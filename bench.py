@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: ViT-B/16 + README RAJNI schedule, batch 256 per GPU, images/sec.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one RAJNIViTWrapper.forward over one synthetic batch (BASELINE.json configs[1]).
@@ -24,6 +24,9 @@ Prints ONE JSON line (rank 0).  Data-parallel: every rank runs the same per-GPU 
               sets against the oracle's own scores with the tie band (tokens within 3 % of the cut score) counted
 
 --impl reference times the reference's CPU implementation alone (rank 0 only).
+--dump-outputs DIR writes what rank 0's last timed step returned as DIR/<name>.npy (see dump_outputs), so that two builds
+can be compared output for output: with the same arguments the weights and input batches are the same on every run.
+It is refused with --impl reference, whose timed path (the reference's evaluate_model) returns no logits to its caller.
 """
 from __future__ import annotations
 
@@ -37,6 +40,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -51,6 +55,7 @@ METRIC = "ViT-B/16 RAJNI images/sec @bs256"
 WORKLOAD = f"C2: {MODEL} random-init + README schedule {{3:.88,4:.88,7:.8,8:.72}}, 224px, bf16 batch 256 per GPU"
 TOKENS = [197, 197, 197, 197, 173, 152, 152, 152, 121, 87, 87, 87]
 TIE_BAND = 0.03          # kept-set disagreements are legitimate only within this relative distance of the cut score
+DUMP_BYTES = 64 << 20    # --dump-outputs writes at most this much in all
 
 # BASELINE.json configs 3-5: (model, schedule, global batch, image size); SURVEY.md 8(d)
 CONFIGS = {
@@ -144,6 +149,21 @@ def host_threads() -> int:
         n = os.cpu_count() or 1
     torch.set_num_threads(n)
     return torch.get_num_threads()
+
+
+def dump_outputs(out_dir, logits, token_counts):
+    """Write one step's results as a caller receives them: the logits [B, classes] (float32) and get_last_stats()'s
+    per-block token counts (float64).  Logits larger than half of DUMP_BYTES are cut to a fixed, seeded sample of images;
+    logits_rows.npy (float64) holds the batch index of every row written."""
+    os.makedirs(out_dir, exist_ok=True)
+    logits = logits.float().cpu().numpy()
+    rows = np.arange(logits.shape[0])
+    if logits.nbytes > DUMP_BYTES // 2:
+        n = DUMP_BYTES // 2 // logits[0].nbytes
+        rows = np.sort(np.random.default_rng(0).choice(logits.shape[0], n, replace=False))
+    np.save(os.path.join(out_dir, "logits.npy"), logits[rows])
+    np.save(os.path.join(out_dir, "logits_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "token_counts.npy"), np.asarray(token_counts, dtype=np.float64))
 
 
 # --------------------------------------------------------------------------- the reference, unmodified (oracle/_ref)
@@ -322,7 +342,12 @@ def main():
     ap.add_argument("--strong", action="store_true",
                     help="strong scaling as the headline: --batch is the GLOBAL batch, sharded over the ranks (the default line "
                          "is weak scaling and carries the sharded reading under the key `strong`)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what rank 0's last timed step returned as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the b200 path; --impl reference has no outputs to write")
 
     if args.impl == "reference":
         args.warmup = max(args.warmup, 1)
@@ -395,6 +420,8 @@ def main():
     clocks = sampler.stop() if rank == 0 else None
     value = world * B * args.steps / (ms_total * 1e-3)
     assert model.get_last_stats()["token_counts"] == TOKENS and torch.isfinite(logits).all()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, logits, model.get_last_stats()["token_counts"])
 
     # ---------------- the same loop for >= 1 s: the power-capped regime ----------------
     sus_steps = max(args.steps, int(math.ceil(1200.0 / (ms_total / args.steps))))

@@ -441,7 +441,7 @@ def test_attention(ops, B, N, Np, H):
             assert torch.equal(outs["pipe"], outs["tc"])
 
 
-def test_attention_packed_tiles_match_one_image_per_tile(ops):
+def test_attention_packed_tiles_match_one_image_per_tile(ops, tmp_path):
     """Short images share a 128-row tile (block-diagonal softmax mask).  Against the same call with one image per tile the
     outputs differ only by the order of the fp32 accumulation of P V (the masked P entries are exactly 0)."""
     import subprocess
@@ -458,7 +458,7 @@ def test_attention_packed_tiles_match_one_image_per_tile(ops):
         "torch.save(out.cpu(), sys.argv[1])\n" % ROOT)
     outs = []
     for nopack in ("", "1"):
-        path = f"/tmp/rajni_pack_{nopack or 0}.pt"
+        path = str(tmp_path / f"pack_{nopack or 0}.pt")
         env = dict(os.environ)
         env.pop("RAJNI_ATTN_NOPACK", None)
         if nopack:
