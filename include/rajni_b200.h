@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define RAJNI_ABI_VERSION 9
+#define RAJNI_ABI_VERSION 10     /* 10: rajni_patch_im2col takes any patch that is a multiple of 8; long-sequence scores */
 
 enum {
     RAJNI_OK = 0,
@@ -74,15 +74,24 @@ int rajni_select(const float* scores, int B, int N, int keep,
                  int32_t* keep_idx, float* next_scores, int32_t* row_map, void* stream);
 
 /* ---- a1+a2 fused: one pass over the K and V planes, then in-CTA select.
- * scores may be NULL when the caller does not need the full score vector. */
+ * scores may be NULL when the caller does not need the full score vector.
+ * rajni_importance and rajni_score_select keep one image's CLS logits and value rows in shared memory; shapes for which
+ * rajni_score_select_needs_workspace(N, H) is 1 (N > ~720 at 12 heads) return RAJNI_EINVAL there: use the split entry. */
 int rajni_score_select(const void* qkv, int B, int N, int C, int H, int keep, float eps,
                        float* scores, int32_t* keep_idx, float* next_scores,
                        int32_t* row_map, void* stream);
 
 /* Same result, bit for bit, in two launches for batches with far fewer images than the GPU has SMs (one CTA per image
  * would leave most SMs idle): the K/V pass is spread over (image, 16-row block) CTAs into `workspace`
- * (rajni_score_select_workspace_bytes(B,N,C,H) bytes, 16-byte aligned, caller-owned), then the per-image kernel finishes. */
+ * (rajni_score_select_workspace_bytes(B,N,C,H) bytes, 16-byte aligned, caller-owned), then the per-image kernel finishes.
+ * Every N <= 4096 works here at any batch: when rajni_score_select_needs_workspace(N, H) is 1 the per-image kernel reads
+ * the logits and value rows from the workspace in place (same arithmetic, same bits).  keep_idx == NULL computes the
+ * scores only (a scores-only call of rajni_importance's meaning): then `scores` is required, keep, next_scores and
+ * row_map are ignored. */
 size_t rajni_score_select_workspace_bytes(int B, int N, int C, int H);
+/* Host-side query, no launch: 1 when one image of N tokens and H heads needs the workspace path of
+ * rajni_score_select_split (its CLS logits and value rows exceed the per-image kernel's shared memory), else 0. */
+int rajni_score_select_needs_workspace(int N, int H);
 int rajni_score_select_split(const void* qkv, int B, int N, int C, int H, int keep, float eps,
                              float* scores, int32_t* keep_idx, float* next_scores, int32_t* row_map,
                              void* workspace, size_t workspace_bytes, void* stream);
@@ -159,8 +168,9 @@ int rajni_attention_fwd_ex(const void* qkv, const int32_t* row_map, void* out,
                            int B, int N_src, int Np, int C, int H, float scale, int reverse, int impl, void* stream);
 
 /* ---- a8: patch-embed front end (model.py:31-37)
- * im2col: images [B,3,S,S] (image_dtype: RAJNI_IMG_BF16 / _F32 / _U8) -> cols [B*P, 3*p*p] bf16
- * in Conv2d weight order (c, ky, kx).  RAJNI_IMG_U8: raw pixels, normalised here as the reference's
+ * im2col: images [B,3,S,S] (image_dtype: RAJNI_IMG_BF16 / _F32 / _U8) -> cols [B*P, 3*p*p] bf16, P = (S/p)^2,
+ * in Conv2d weight order (c, ky, kx).  patch: any multiple of 8 that divides S <= 16384 (8, 16, 24, 32, ...; ABI >= 10,
+ * 16 only before), so 3*p*p is a multiple of 64.  RAJNI_IMG_U8: raw pixels, normalised here as the reference's
  * loader does in fp32 (run.py:62-70: ToTensor + Normalize): (u/255 - norm[c]) / norm[3+c] with
  * norm = HOST array {mean[3], std[3]} (read at call time); other dtypes ignore norm (may be NULL).
  * Also writes the CLS rows

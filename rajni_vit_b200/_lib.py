@@ -15,7 +15,7 @@ LIB_PATH = os.path.join(_HERE, "csrc", "librajni_b200.so")
 RAJNI_OK, RAJNI_EINVAL, RAJNI_ECUDA, RAJNI_EARCH, RAJNI_ERANGE = 0, -1, -2, -3, -4
 ATTN_AUTO, ATTN_PIPE, ATTN_TC, ATTN_LONG = 0, 1, 2, 3
 EPI_BIAS, EPI_GELU, EPI_RESIDUAL, EPI_OUT_F32, EPI_LN_FOLD, EPI_ROW_STATS, HINT_REVERSE_M, HINT_STREAM_K = 1, 2, 4, 8, 16, 32, 64, 128
-ABI_VERSION = 9
+ABI_VERSION = 10
 
 
 class GemmArgs(Structure):
@@ -42,6 +42,7 @@ SIGNATURES = {
     "rajni_score_select": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_float,
                                    c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "rajni_score_select_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int]),
+    "rajni_score_select_needs_workspace": (c_int, [c_int, c_int]),
     "rajni_score_select_split": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_float,
                                          c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "rajni_gather_rows": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p]),

@@ -172,6 +172,118 @@ __global__ void __launch_bounds__(256) im2col16_kernel(const void* __restrict__ 
     }
 }
 
+// ------------------------------------------------------------------ patch im2col (+ CLS rows)
+// Any patch size p that is a multiple of 8.  One thread moves one 8-pixel run of one (patch, channel, patch row): 8 pixels
+// in, 16 bytes of bf16 out.  The run's index inside its (patch, channel) plane (p*p/8 runs) is the fastest thread index, so
+// a warp stores 512 consecutive bytes of one cols row at p >= 16 and four 128-byte planes at p = 8: whole sectors at every
+// p.  Reads are whole image-row segments of p pixels (at p = 8 the warp's four patches are neighbours, so uint8 pixels
+// arrive as whole 32-byte sectors too).  Column order (c, ky, kx) matches Conv2d weight.view(C, -1).
+// DT: 0 = bf16, 1 = fp32, 2 = uint8 pixels normalised here exactly as torchvision's ToTensor + Normalize do in fp32
+// ((u / 255 - mean[c]) / std[c], IEEE divisions; run.py:62-70), so the bf16 result equals that of the fp32 pipeline.
+constexpr int kIm2colUnroll = 4;            // independent runs in flight per thread
+
+template <int DT>
+__device__ __forceinline__ void im2col_load(const void* images, long long pix, uint4 (&r)[2]) {
+    if (DT == 1) {
+        const uint4* s = reinterpret_cast<const uint4*>(static_cast<const float*>(images) + pix);
+        r[0] = __ldg(s);
+        r[1] = __ldg(s + 1);
+    } else if (DT == 2) {
+        const uint2 u = __ldg(reinterpret_cast<const uint2*>(static_cast<const uint8_t*>(images) + pix));
+        r[0] = make_uint4(u.x, u.y, 0u, 0u);
+    } else {
+        r[0] = __ldg(reinterpret_cast<const uint4*>(static_cast<const __nv_bfloat16*>(images) + pix));
+    }
+}
+
+template <int DT>
+__device__ __forceinline__ uint4 im2col_convert(const uint4 (&r)[2], const ImageNorm& norm, int c) {
+    if (DT == 1) {
+        const float4 a = make_float4(__uint_as_float(r[0].x), __uint_as_float(r[0].y), __uint_as_float(r[0].z), __uint_as_float(r[0].w));
+        const float4 b = make_float4(__uint_as_float(r[1].x), __uint_as_float(r[1].y), __uint_as_float(r[1].z), __uint_as_float(r[1].w));
+        return make_uint4(float2_to_bf16x2(a.x, a.y), float2_to_bf16x2(a.z, a.w),
+                          float2_to_bf16x2(b.x, b.y), float2_to_bf16x2(b.z, b.w));
+    } else if (DT == 2) {
+        const float mean = norm.mean[c], sd = norm.std[c];
+        const uint32_t w[2] = {r[0].x, r[0].y};
+        uint32_t o[4];
+#pragma unroll
+        for (int k = 0; k < 2; ++k) {
+            float f[4];
+#pragma unroll
+            for (int j = 0; j < 4; ++j)
+                f[j] = __fdiv_rn(__fsub_rn(__fdiv_rn((float)((w[k] >> (8 * j)) & 0xffu), 255.0f), mean), sd);
+            o[2 * k] = float2_to_bf16x2(f[0], f[1]);
+            o[2 * k + 1] = float2_to_bf16x2(f[2], f[3]);
+        }
+        return make_uint4(o[0], o[1], o[2], o[3]);
+    } else {
+        return r[0];
+    }
+}
+
+template <int DT>
+__global__ void __launch_bounds__(256) im2col_kernel(const void* __restrict__ images, const ImageNorm norm, int B, int S, int p,
+                                                     __nv_bfloat16* __restrict__ cols,
+                                                     const uint4* __restrict__ cls_pos0,
+                                                     uint4* __restrict__ x, int C,
+                                                     float2* __restrict__ row_stats, long long stats_ld, int stats_slots,
+                                                     float cls_sum, float cls_sumsq) {
+    griddep_launch();
+    griddep_wait();
+    const int G = S / p;                        // patches per side
+    const int rpr = p >> 3;                     // runs per patch row
+    const int rpp = p * rpr;                    // runs per (patch, channel) plane
+    const long long plane = (long long)p * p;
+    const int img_runs = G * G * 3 * rpp;       // = 3 S^2 / 8 < 2^31 (checked by the host)
+    const long long runs = (long long)B * img_runs;
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    // run i -> (q = run in plane, px, c, py, b), q fastest; returns the source pixel offset, sets the cols element offset.
+    // One 64-bit division per run; the rest in 32 bits.
+    auto locate = [&](long long i, long long& dst, int& c) {
+        const int b = (int)(i / img_runs);
+        unsigned t = (unsigned)(i - (long long)b * img_runs);
+        const int q = (int)(t % (unsigned)rpp); t /= (unsigned)rpp;
+        const int px = (int)(t % (unsigned)G); t /= (unsigned)G;
+        c = (int)(t % 3u);
+        const int py = (int)(t / 3u);
+        const int ky = q / rpr, kx = (q - ky * rpr) * 8;
+        dst = (((long long)b * G + py) * G + px) * 3 * plane + c * plane + (long long)q * 8;
+        return (((long long)b * 3 + c) * S + (py * p + ky)) * S + px * p + kx;
+    };
+    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    for (; i + (kIm2colUnroll - 1) * stride < runs; i += kIm2colUnroll * stride) {
+        uint4 r[kIm2colUnroll][2];
+        long long dst[kIm2colUnroll];
+        int c[kIm2colUnroll];
+#pragma unroll
+        for (int u = 0; u < kIm2colUnroll; ++u) im2col_load<DT>(images, locate(i + u * stride, dst[u], c[u]), r[u]);
+#pragma unroll
+        for (int u = 0; u < kIm2colUnroll; ++u) *reinterpret_cast<uint4*>(cols + dst[u]) = im2col_convert<DT>(r[u], norm, c[u]);
+    }
+    for (; i < runs; i += stride) {
+        uint4 r[2];
+        long long dst;
+        int c;
+        im2col_load<DT>(images, locate(i, dst, c), r);
+        *reinterpret_cast<uint4*>(cols + dst) = im2col_convert<DT>(r, norm, c);
+    }
+    // CLS rows: x[b,0,:] = cls_token + pos_embed[0]   (model.py:35-37)
+    const int cchunks = C >> 3;
+    const long long P1 = (long long)G * G + 1;
+    for (long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x; k < (long long)B * cchunks; k += stride) {
+        int b = (int)(k / cchunks), j = (int)(k % cchunks);
+        x[(long long)b * P1 * cchunks + j] = __ldg(cls_pos0 + j);
+    }
+    // LayerNorm partials of the CLS rows (the patch rows' partials come from the embed GEMM's epilogue)
+    if (row_stats != nullptr) {
+        for (long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x; k < (long long)B * stats_slots; k += stride) {
+            int b = (int)(k / stats_slots), s = (int)(k % stats_slots);
+            row_stats[(long long)s * stats_ld + (long long)b * P1] = s == 0 ? make_float2(cls_sum, cls_sumsq) : make_float2(0.f, 0.f);
+        }
+    }
+}
+
 }  // namespace rajni
 
 using namespace rajni;
@@ -230,20 +342,34 @@ extern "C" int rajni_patch_im2col(const void* images, int image_dtype, int B, in
             nm.std[i] = norm[3 + i];
             RAJNI_REQUIRE(nm.std[i] > 0.f, RAJNI_EINVAL, "rajni_patch_im2col: std[%d] must be positive", i);
         }
-    RAJNI_REQUIRE(patch == 16 && S > 0 && S % 16 == 0 && B > 0 && C % 8 == 0, RAJNI_EINVAL,
-                  "rajni_patch_im2col: patch=%d S=%d B=%d C=%d unsupported (patch must be 16)", patch, S, B, C);
-    RAJNI_REQUIRE(row_stats == nullptr || (stats_slots > 0 && row_stats_ld >= (long long)B * ((S / 16) * (S / 16) + 1)), RAJNI_EINVAL,
+    RAJNI_REQUIRE(patch >= 8 && patch % 8 == 0 && S > 0 && S <= 16384 && S % patch == 0 && B > 0 && C % 8 == 0, RAJNI_EINVAL,
+                  "rajni_patch_im2col: patch=%d S=%d B=%d C=%d unsupported (patch must be a multiple of 8 dividing S <= 16384)", patch, S, B, C);
+    const int G = S / patch;
+    RAJNI_REQUIRE(row_stats == nullptr || (stats_slots > 0 && row_stats_ld >= (long long)B * (G * G + 1)), RAJNI_EINVAL,
                   "rajni_patch_im2col: row_stats needs stats_slots > 0 and row_stats_ld >= B*(P+1)");
-    const int G = S / 16;
-    const long long strips = (long long)B * G * 3 * 16 * G;
-    long long blocks = (strips + 255) / 256;
-    if (blocks > 148 * 32) blocks = 148 * 32;
     auto s = static_cast<cudaStream_t>(stream);
-    auto kern = image_dtype == RAJNI_IMG_U8 ? im2col16_kernel<2> : image_dtype == RAJNI_IMG_F32 ? im2col16_kernel<1> : im2col16_kernel<0>;
-    cudaError_t le = launch_kernel(kern, dim3((int)blocks), dim3(256), 0, s, 1,
-                                   images, nm, B, S, static_cast<__nv_bfloat16*>(cols), static_cast<const uint4*>(cls_pos0),
-                                   static_cast<uint4*>(x), C, reinterpret_cast<float2*>(row_stats), row_stats_ld, stats_slots,
-                                   cls_sum, cls_sumsq);
+    cudaError_t le;
+    // p = 16 keeps its own kernel: 16-pixel strips, px fastest.  On a B200 at 256 images of 224 px it moves fp32 images in
+    // 41.7 us against the any-patch kernel's 44.3 us, uint8 pixels in 54.5 against 78.6 us (profiles/r3_kbench.txt).
+    if (patch == 16) {
+        const long long strips = (long long)B * G * 3 * 16 * G;
+        long long blocks = (strips + 255) / 256;
+        if (blocks > 148 * 32) blocks = 148 * 32;
+        auto kern = image_dtype == RAJNI_IMG_U8 ? im2col16_kernel<2> : image_dtype == RAJNI_IMG_F32 ? im2col16_kernel<1> : im2col16_kernel<0>;
+        le = launch_kernel(kern, dim3((int)blocks), dim3(256), 0, s, 1,
+                           images, nm, B, S, static_cast<__nv_bfloat16*>(cols), static_cast<const uint4*>(cls_pos0),
+                           static_cast<uint4*>(x), C, reinterpret_cast<float2*>(row_stats), row_stats_ld, stats_slots,
+                           cls_sum, cls_sumsq);
+    } else {
+        const long long runs = (long long)B * G * G * 3 * patch * (patch / 8);
+        long long blocks = (runs + 256 * kIm2colUnroll - 1) / (256 * kIm2colUnroll);
+        if (blocks > 148 * 32) blocks = 148 * 32;
+        auto kern = image_dtype == RAJNI_IMG_U8 ? im2col_kernel<2> : image_dtype == RAJNI_IMG_F32 ? im2col_kernel<1> : im2col_kernel<0>;
+        le = launch_kernel(kern, dim3((int)blocks), dim3(256), 0, s, 1,
+                           images, nm, B, S, patch, static_cast<__nv_bfloat16*>(cols), static_cast<const uint4*>(cls_pos0),
+                           static_cast<uint4*>(x), C, reinterpret_cast<float2*>(row_stats), row_stats_ld, stats_slots,
+                           cls_sum, cls_sumsq);
+    }
     count_launch();
     RAJNI_REQUIRE(le == cudaSuccess, RAJNI_ECUDA, "patch_im2col: launch failed: %s", cudaGetErrorString(le));
     return check_launch("patch_im2col");

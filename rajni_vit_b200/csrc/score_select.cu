@@ -10,8 +10,12 @@
 // per-head CLS logits [H][N], the head-averaged value rows [N][64] (fp32, so the
 // centred norm is computed exactly like the reference without a second HBM pass),
 // and the selection state (radix-select histogram, flags, prefix sums).
+// Sequences whose logits and value rows do not fit there (score_smem_bytes over 227 KB: N > ~720 at 12 heads, e.g. the
+// 785 tokens of a ViT-B/8) take the two-launch path of rajni_score_select_split: score_stream_kernel leaves them in the
+// caller's workspace and score_tail_ws_kernel reads them in place (from L2), keeping only O(N) arrays in shared memory.
 // bf16 tiles in, fp32 arithmetic throughout (SURVEY.md section 4.5).
 #include <algorithm>
+#include <cstdlib>
 
 #include "common.cuh"
 
@@ -364,11 +368,13 @@ __device__ __forceinline__ float row_dist2(const float* row, const float* mu) {
 // barrier that made sm.logit and vm (rows of kVmSmemStride floats, both in shared memory) complete.  Thread-per-token wherever
 // the reference's reductions allow: ~9 block barriers in all.  (NT and the 512 "virtual threads" of block_sum: the overlapped
 // kernel of tools/probes/score_overlap_persistent_experiment.patch runs the same tail on 448 threads with the same bits.)
-template <int NT>
+// VS: float stride of the value rows (kVmSmemStride in shared memory, kHeadDim in the workspace).  sm.logit may point into the
+// workspace too (score_tail_ws_kernel): same reads, same arithmetic, same bits.
+template <int NT, int VS = kVmSmemStride>
 __device__ void score_tail(const SelSmem& sm, const float* vm, const ScoreSelectParams& p, int b, int trace_row = 0) {
     const int N = p.N, H = p.H;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int vs = kVmSmemStride;
+    const int vs = VS;
     const float inv_h = 1.0f / (float)H;
     SC_TRACE(32 + trace_row, 4);
     // ---- mean over tokens of the head-averaged value (importance.py:25): 8 interleaved partial sums per dim, then their sum
@@ -508,6 +514,21 @@ __global__ void __launch_bounds__(kStreamThreads) score_stream_kernel(const __nv
         score_row<CPL>(img + (size_t)n * 3 * C, q, lane, chunks, C, H, N, n, logit_dst, vm_dst, kHeadDim, inv_h);
 }
 
+// Split path, kernel 2 for long sequences: the per-image tail reading the CLS logits and value rows where score_stream_kernel
+// left them (L2-resident: 61 MB at 256 images x 785 tokens x 12 heads) instead of staging them in shared memory, which then
+// holds only the O(N) selection arrays.  The softmax exponentials overwrite the image's logits in the workspace.
+__global__ void __launch_bounds__(kSelThreads) score_tail_ws_kernel(const ScoreSelectParams p, float* logit_g) {
+    extern __shared__ __align__(16) float smem[];
+    griddep_launch();
+    griddep_wait();
+    const int b = blockIdx.x;
+    SelSmem sm = carve_sel_smem(smem, p.N, 0);
+    sm.logit = logit_g + (size_t)b * (((size_t)p.H * p.N + 3) & ~(size_t)3);
+    score_tail<kSelThreads, kHeadDim>(sm, p.pre_vm + (size_t)b * p.N * kHeadDim, p, b);
+}
+
+constexpr size_t kSmemLimit = 227 * 1024;
+
 static size_t score_smem_bytes(int N, int H, bool with_logit, bool with_vm) {
     size_t floats = (size_t)((N + 3) & ~3) + N + 512 + 256 + 4 + 32 + 64 + 64;
     if (with_logit) floats += (size_t)H * N;
@@ -518,7 +539,8 @@ static size_t score_smem_bytes(int N, int H, bool with_logit, bool with_vm) {
 static int launch_score_select(const ScoreSelectParams& p, int B, cudaStream_t stream) {
     const bool with_score = p.qkv != nullptr;
     size_t smem = score_smem_bytes(p.N, p.H, with_score, with_score);
-    RAJNI_REQUIRE(smem <= 227 * 1024, RAJNI_EINVAL, "score_select: N=%d H=%d needs %zu B of shared memory", p.N, p.H, smem);
+    RAJNI_REQUIRE(smem <= kSmemLimit, RAJNI_EINVAL,
+                  "score_select: N=%d H=%d needs %zu B of shared memory (rajni_score_select_split takes such shapes)", p.N, p.H, smem);
     int cpl = with_score ? (p.C + 255) / 256 : 1;
     void (*kern)(const ScoreSelectParams) = nullptr;
     switch (cpl) {
@@ -534,6 +556,19 @@ static int launch_score_select(const ScoreSelectParams& p, int B, cudaStream_t s
     count_launch();
     RAJNI_REQUIRE(e == cudaSuccess, RAJNI_ECUDA, "score_select: launch failed: %s", cudaGetErrorString(e));
     return check_launch("score_select");
+}
+
+// true when one image's CLS logits and value rows do not fit the per-image kernel's shared memory
+static bool needs_workspace_tail(int N, int H) { return score_smem_bytes(N, H, true, true) > kSmemLimit; }
+
+static int launch_score_tail_ws(const ScoreSelectParams& p, float* logit_g, int B, cudaStream_t stream) {
+    const size_t smem = score_smem_bytes(p.N, 0, false, false);
+    cudaError_t e = cudaFuncSetAttribute(score_tail_ws_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    RAJNI_REQUIRE(e == cudaSuccess, RAJNI_ECUDA, "score_tail_ws: smem attribute: %s", cudaGetErrorString(e));
+    e = launch_kernel(score_tail_ws_kernel, dim3(B), dim3(kSelThreads), smem, stream, 1, p, logit_g);
+    count_launch();
+    RAJNI_REQUIRE(e == cudaSuccess, RAJNI_ECUDA, "score_tail_ws: launch failed: %s", cudaGetErrorString(e));
+    return check_launch("score_tail_ws");
 }
 
 static size_t split_workspace_floats(int B, int N, int H) {
@@ -617,10 +652,13 @@ extern "C" size_t rajni_score_select_workspace_bytes(int B, int N, int C, int H)
 extern "C" int rajni_score_select_split(const void* qkv, int B, int N, int C, int H, int keep, float eps,
                                         float* scores, int32_t* keep_idx, float* next_scores, int32_t* row_map,
                                         void* workspace, size_t workspace_bytes, void* stream) {
-    RAJNI_REQUIRE(qkv && keep_idx && next_scores && workspace, RAJNI_EINVAL, "rajni_score_select_split: null pointer");
+    RAJNI_REQUIRE(qkv && workspace && (keep_idx ? next_scores != nullptr : scores != nullptr), RAJNI_EINVAL,
+                  "rajni_score_select_split: null pointer");
     if (int rc = check_score_shape(B, N, C, H)) return rc;
-    RAJNI_REQUIRE(keep >= 1, RAJNI_EINVAL, "rajni_score_select_split: keep=%d < 1", keep);
-    RAJNI_REQUIRE(keep <= N - 1, RAJNI_ERANGE, "selected index k out of range (keep=%d, patches=%d)", keep, N - 1);
+    if (keep_idx != nullptr) {
+        RAJNI_REQUIRE(keep >= 1, RAJNI_EINVAL, "rajni_score_select_split: keep=%d < 1", keep);
+        RAJNI_REQUIRE(keep <= N - 1, RAJNI_ERANGE, "selected index k out of range (keep=%d, patches=%d)", keep, N - 1);
+    }
     RAJNI_REQUIRE(B <= 65535, RAJNI_EINVAL, "rajni_score_select_split: B=%d exceeds the grid limit", B);
     RAJNI_REQUIRE(workspace_bytes >= rajni_score_select_workspace_bytes(B, N, C, H) && (reinterpret_cast<uintptr_t>(workspace) & 15) == 0,
                   RAJNI_EINVAL, "rajni_score_select_split: workspace too small (%zu B) or not 16-byte aligned", workspace_bytes);
@@ -633,6 +671,12 @@ extern "C" int rajni_score_select_split(const void* qkv, int B, int N, int C, in
     p.keep_idx = keep_idx; p.next_scores = next_scores; p.row_map = row_map;
     p.pre_logit = ws;
     p.pre_vm = ws + (size_t)B * (((size_t)H * N + 3) & ~(size_t)3);
-    p.N = N; p.C = C; p.H = H; p.keep = keep; p.eps = eps;
+    p.N = N; p.C = C; p.H = H; p.keep = keep_idx ? keep : 0; p.eps = eps;
+    // RAJNI_SCORE_WS_TAIL=1 (read per call; tests): the long-sequence tail at any N, to compare it with the shared-memory one
+    if (needs_workspace_tail(N, H) || getenv("RAJNI_SCORE_WS_TAIL") != nullptr) return launch_score_tail_ws(p, ws, B, s);
     return launch_score_select(p, B, s);
+}
+
+extern "C" int rajni_score_select_needs_workspace(int N, int H) {
+    return N > 0 && H > 0 && needs_workspace_tail(N, H) ? 1 : 0;
 }

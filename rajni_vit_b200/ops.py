@@ -73,13 +73,22 @@ def _bf16c(t: torch.Tensor) -> torch.Tensor:
     return t
 
 
-def importance(qkv: torch.Tensor, num_heads: int, eps: float = 1e-6) -> torch.Tensor:
-    """qkv [B,N,3C] bf16 -> scores [B,N] fp32.   importance.py:5-34"""
+def importance(qkv: torch.Tensor, num_heads: int, eps: float = 1e-6, workspace: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """qkv [B,N,3C] bf16 -> scores [B,N] fp32.   importance.py:5-34
+    Sequences too long for the one-launch kernel (``needs_score_workspace``) go through the split entry with scratch
+    (``workspace`` as in ``score_select``)."""
     _bf16c(qkv)
     B, N, C3 = qkv.shape
+    C = C3 // 3
     scores = torch.empty((B, N), device=qkv.device, dtype=torch.float32)
-    _call("score_select", B * (2 * N * (C3 // 3) * 2 + (C3 // 3) * 2 + 4 * N), _lib.load().rajni_importance,
-          qkv.data_ptr(), B, N, C3 // 3, num_heads, eps, scores.data_ptr(), _stream(qkv))
+    work = B * (2 * N * C * 2 + C * 2 + 4 * N)
+    lib = _lib.load()
+    if needs_score_workspace(N, num_heads):
+        ws = _checked_score_workspace(qkv.device, B, N, C, num_heads, workspace)
+        _call("score_select", work, lib.rajni_score_select_split, qkv.data_ptr(), B, N, C, num_heads, 0, eps, scores.data_ptr(),
+              None, None, None, ws.data_ptr(), ws.numel(), _stream(qkv))
+    else:
+        _call("score_select", work, lib.rajni_importance, qkv.data_ptr(), B, N, C, num_heads, eps, scores.data_ptr(), _stream(qkv))
     return scores
 
 
@@ -109,6 +118,12 @@ def score_workspace_bytes(B: int, N: int, C: int, num_heads: int) -> int:
     return int(_lib.load().rajni_score_select_workspace_bytes(B, N, C, num_heads))
 
 
+def needs_score_workspace(N: int, num_heads: int) -> bool:
+    """True when scoring N tokens with this many heads needs the split path's workspace at every batch size (the one-launch
+    kernel's shared memory cannot hold the image's logits and value rows).  Host-side query, no launch."""
+    return bool(_lib.load().rajni_score_select_needs_workspace(N, num_heads))
+
+
 def _score_workspace(dev: torch.device, nbytes: int) -> torch.Tensor:
     """Process-wide scratch for callers that do not bring their own (stand-alone ops.score_select calls).  Grow-only and
     NEVER freed: a CUDA graph captured by some other caller may have baked an older buffer's address in, so superseded
@@ -119,13 +134,23 @@ def _score_workspace(dev: torch.device, nbytes: int) -> torch.Tensor:
     return bufs[-1]
 
 
+def _checked_score_workspace(dev: torch.device, B: int, N: int, C: int, num_heads: int,
+                             workspace: Optional[torch.Tensor]) -> torch.Tensor:
+    nbytes = score_workspace_bytes(B, N, C, num_heads)
+    ws = workspace if workspace is not None else _score_workspace(dev, nbytes)
+    if ws.numel() * ws.element_size() < nbytes or ws.device != dev:
+        raise ValueError(f"score_select: workspace of {ws.numel() * ws.element_size()} B on {ws.device}, need {nbytes} B on {dev}")
+    return ws
+
+
 def score_select(qkv: torch.Tensor, num_heads: int, keep: int, eps: float = 1e-6, want_scores: bool = False,
                  keep_idx=None, next_scores=None, row_map=None, scores=None, split: Optional[bool] = None,
                  workspace: Optional[torch.Tensor] = None):
     """Fused importance + selection on qkv [B,N,3C] bf16.
     Returns (scores or None, keep_idx, next_scores, row_map).
-    ``workspace``: uint8 scratch of at least ``score_workspace_bytes(B, N, C, H)`` for the split path (small batches); a
-    caller that replays CUDA graphs must pass one it owns, so that the captured address lives as long as the graph."""
+    ``workspace``: uint8 scratch of at least ``score_workspace_bytes(B, N, C, H)`` for the split path (small batches, and
+    every batch of a sequence for which ``needs_score_workspace``); a caller that replays CUDA graphs must pass one it owns,
+    so that the captured address lives as long as the graph."""
     _bf16c(qkv)
     B, N, C3 = qkv.shape
     dev = qkv.device
@@ -137,14 +162,11 @@ def score_select(qkv: torch.Tensor, num_heads: int, keep: int, eps: float = 1e-6
     C = C3 // 3
     lib = _lib.load()
     if split is None:
-        split = B <= SPLIT_SCORE_MAX_BATCH
+        split = B <= SPLIT_SCORE_MAX_BATCH or needs_score_workspace(N, num_heads)
     # algorithmic bytes (SURVEY 8d): K and V planes + CLS query in, index + carried score out
     work = B * (2 * N * C * 2 + C * 2 + 8 * (keep + 1))
     if split:
-        nbytes = int(lib.rajni_score_select_workspace_bytes(B, N, C, num_heads))
-        ws = workspace if workspace is not None else _score_workspace(dev, nbytes)
-        if ws.numel() * ws.element_size() < nbytes or ws.device != dev:
-            raise ValueError(f"score_select: workspace of {ws.numel() * ws.element_size()} B on {ws.device}, need {nbytes} B on {dev}")
+        ws = _checked_score_workspace(dev, B, N, C, num_heads, workspace)
         _call("score_select", work, lib.rajni_score_select_split, qkv.data_ptr(), B, N, C, num_heads, keep, eps, _ptr(scores),
               keep_idx.data_ptr(), next_scores.data_ptr(), row_map.data_ptr(), ws.data_ptr(), ws.numel(), _stream(qkv))
     else:

@@ -25,7 +25,8 @@ Schedule = Dict[int, Dict]
 
 
 def flops_per_image(token_counts: Sequence[int], C: int, hidden: int, patches: int, classes: int = 1000, patch_dim: int = 768) -> float:
-    """Tensor work of one image under a schedule (SURVEY 8d): token_counts[i] = tokens ENTERING block i."""
+    """Tensor work of one image under a schedule (SURVEY 8d): token_counts[i] = tokens ENTERING block i.
+    ``patch_dim`` = 3 p^2, the patch-embed GEMM's K (768 at p = 16)."""
     total = 2.0 * patches * C * patch_dim + 2.0 * C * classes
     for i, n in enumerate(token_counts):
         kept = token_counts[i + 1] if i + 1 < len(token_counts) else n    # tokens after this block's pruning
@@ -149,11 +150,12 @@ def measure(make_model: Callable[[], torch.nn.Module], schedule: Schedule, batch
     blk = base.blocks[0]
     C = base.patch_embed.proj.out_channels
     size = x0.shape[-1]
+    p = base.patch_embed.proj.kernel_size[0]
     out = {
         "schedule": copy.deepcopy(schedule), "img_s": x0.shape[0] * timing_steps / (e0.elapsed_time(e1) * 1e-3),
         "token_counts": counts,
-        "gflop_per_image": flops_per_image(counts, C, blk.mlp.fc1.out_features, (size // 16) ** 2,
-                                           classes=base.head.out_features) / 1e9,
+        "gflop_per_image": flops_per_image(counts, C, blk.mlp.fc1.out_features, (size // p) ** 2,
+                                           classes=base.head.out_features, patch_dim=3 * p * p) / 1e9,
         "top1": (100.0 * correct / labelled) if labelled else None,
         "agreement": (100.0 * agree / seen) if dense_predictions is not None else 100.0,
         "predictions": preds,

@@ -7,7 +7,7 @@ but only ever touches a small duck-typed surface of it
 this image and there is no network, so this module provides a model with exactly
 those attribute names and timm's ViT semantics:
 
-    patch_embed.proj : Conv2d(3, C, k=16, s=16)  -> flatten(2).transpose(1, 2)
+    patch_embed.proj : Conv2d(3, C, k=p, s=p)  -> flatten(2).transpose(1, 2)   (p = 16, or 8 / 32, see VIT_PATCH)
     cls_token [1,1,C], pos_embed [1,1+P,C], pos_drop
     blocks[i] : norm1, attn{num_heads, scale, qkv, proj, proj_drop}, norm2,
                 mlp{fc1, act=GELU(erf), fc2}, ls1/ls2/drop_path1/drop_path2 = Identity
@@ -22,16 +22,27 @@ import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
-# name -> (embed_dim, depth, heads, img_size)
+# name -> (embed_dim, depth, heads, img_size); the patch size is in VIT_PATCH (callers unpack these four fields)
 VIT_CONFIGS = {
     "vit_tiny_patch16_224": (192, 12, 3, 224),
     "vit_small_patch16_224": (384, 12, 6, 224),
     "vit_base_patch16_224": (768, 12, 12, 224),
     "vit_large_patch16_224": (1024, 24, 16, 224),
     "deit_base_patch16_384": (768, 12, 12, 384),
-    # a 4-block, 17-token model small enough for golden fixtures
+    "vit_small_patch32_224": (384, 12, 6, 224),
+    "vit_base_patch32_224": (768, 12, 12, 224),
+    "vit_small_patch8_224": (384, 12, 6, 224),
+    "vit_base_patch8_224": (768, 12, 12, 224),
+    # 4-block models small enough for golden fixtures and oracle runs: 17 tokens, 82 tokens (72 px is not a multiple of 16)
+    # and 17 tokens again at patch 32
     "vit_micro_patch16_64": (128, 4, 2, 64),
+    "vit_micro_patch8_72": (128, 4, 2, 72),
+    "vit_micro_patch32_128": (128, 4, 2, 128),
 }
+# name -> patch size (pixels per side of a patch; 50 tokens at 224 px for 32, 785 for 8)
+VIT_PATCH = {name: 16 for name in VIT_CONFIGS}
+VIT_PATCH.update({"vit_small_patch32_224": 32, "vit_base_patch32_224": 32, "vit_micro_patch32_128": 32,
+                  "vit_small_patch8_224": 8, "vit_base_patch8_224": 8, "vit_micro_patch8_72": 8})
 
 
 class PatchEmbed(nn.Module):
@@ -151,7 +162,7 @@ def create_model(name: str, seed: int | None = 0, bf16_round: bool = True,
     if seed is not None:
         gen_state = torch.random.get_rng_state()
         torch.manual_seed(seed)
-    model = VisionTransformer(img_size=img, embed_dim=dim, depth=depth, num_heads=heads,
+    model = VisionTransformer(img_size=img, patch_size=VIT_PATCH[name], embed_dim=dim, depth=depth, num_heads=heads,
                               num_classes=num_classes)
     if seed is not None:
         torch.random.set_rng_state(gen_state)

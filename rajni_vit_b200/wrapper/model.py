@@ -92,8 +92,15 @@ class RAJNIViTWrapper(nn.Module):
     def _validate(self):
         m = self.m
         proj = getattr(m.patch_embed, "proj", None)
-        if not isinstance(proj, nn.Conv2d) or proj.kernel_size != (16, 16) or proj.stride != (16, 16) or proj.in_channels != 3:
-            raise NotImplementedError("patch_embed.proj must be Conv2d(3, C, kernel=16, stride=16)")
+        if not isinstance(proj, nn.Conv2d):
+            raise NotImplementedError("patch_embed.proj must be Conv2d(3, C, kernel=p, stride=p)")
+        p = proj.kernel_size[0]
+        if (proj.kernel_size != (p, p) or proj.stride != (p, p) or p % 8 or proj.in_channels != 3
+                or proj.padding != (0, 0) or proj.dilation != (1, 1) or proj.groups != 1):
+            raise NotImplementedError(f"patch_embed.proj is Conv2d(in={proj.in_channels}, kernel={proj.kernel_size}, "
+                                      f"stride={proj.stride}); supported: Conv2d(3, C, kernel=p, stride=p) with p a multiple of 8 "
+                                      f"(8, 16, 24, 32, ...)")
+        self.patch = p
         if not _is_identity(getattr(m.patch_embed, "norm", None)):
             raise NotImplementedError("patch_embed.norm is not supported")
         for name in ("norm_pre", "fc_norm", "patch_drop"):
@@ -147,7 +154,8 @@ class RAJNIViTWrapper(nn.Module):
             return ws
         m = self.m
         C = m.patch_embed.proj.out_channels
-        G = S // 16
+        p = self.patch
+        G = S // p
         P = G * G
         N0 = P + 1
         if m.pos_embed.shape[1] < N0:
@@ -157,7 +165,7 @@ class RAJNIViTWrapper(nn.Module):
         idx = torch.arange(B * P, device=dev, dtype=torch.int32)
         ws = dict(
             P=P, N0=N0, C=C,
-            cols=torch.empty((B * P, 768), **bf),
+            cols=torch.empty((B * P, 3 * p * p), **bf),
             xa=torch.empty((B * N0, C), **bf), xb=torch.empty((B * N0, C), **bf),
             qkv=torch.empty((B * N0, 3 * C), **bf),
             att=torch.empty((B * N0, C), **bf), hid=torch.empty((B * N0, hidden), **bf),
@@ -172,9 +180,12 @@ class RAJNIViTWrapper(nn.Module):
             # stream-K scratch of the long-K GEMMs (fc2), only when asked for: owned here like every other pointer a captured
             # graph bakes in
             gemm_ws=ops.gemm_workspace(dev) if self.stream_k else None,
-            # scratch of the split score path (small batches): owned here, so a captured graph's pointer lives with the graph
+            # scratch of the split score path (small batches, and sequences too long for the one-launch kernel at any batch):
+            # owned here, so a captured graph's pointer lives with the graph.  Sized for N0, the longest sequence of the step.
             score_ws=(torch.empty(max(ops.score_workspace_bytes(B, N0, C, blk.attn.num_heads) for blk in self.blocks),
-                                  device=dev, dtype=torch.uint8) if B <= ops.SPLIT_SCORE_MAX_BATCH else None),
+                                  device=dev, dtype=torch.uint8)
+                      if B <= ops.SPLIT_SCORE_MAX_BATCH or any(ops.needs_score_workspace(N0, blk.attn.num_heads) for blk in self.blocks)
+                      else None),
         )
         self._ws = {key: ws}        # keep one shape resident
         self._graphs = {}           # a captured graph points into the workspace it was captured with
@@ -194,7 +205,7 @@ class RAJNIViTWrapper(nn.Module):
                 return self.forward(x)
         use = self.use_cuda_graph
         if use is None and x.dim() == 4:
-            use = x.shape[0] * ((x.shape[2] // 16) * (x.shape[3] // 16) + 1) <= AUTO_GRAPH_MAX_ROWS
+            use = x.shape[0] * ((x.shape[2] // self.patch) * (x.shape[3] // self.patch) + 1) <= AUTO_GRAPH_MAX_ROWS
         if not use or x.device.type != "cuda" or x.dim() != 4 or ops._prof is not None:      # (the per-kernel profiler times eager launches)
             return self._forward_eager(x)
         # what _forward_eager reads besides the input: the schedule of the pruned blocks (attention.py:25-32) ...
@@ -224,8 +235,8 @@ class RAJNIViTWrapper(nn.Module):
 
     @torch.no_grad()
     def _forward_eager(self, x: torch.Tensor) -> torch.Tensor:
-        if x.dim() != 4 or x.shape[1] != 3 or x.shape[2] != x.shape[3] or x.shape[2] % 16:
-            raise ValueError(f"expected images [B,3,S,S] with S a multiple of 16, got {tuple(x.shape)}")
+        if x.dim() != 4 or x.shape[1] != 3 or x.shape[2] != x.shape[3] or x.shape[2] % self.patch:
+            raise ValueError(f"expected images [B,3,S,S] with S a multiple of the patch size {self.patch}, got {tuple(x.shape)}")
         if x.device.type != "cuda":
             raise RuntimeError("RAJNIViTWrapper (B200) runs on CUDA tensors only; there is no CPU path")
         if self.m.pos_embed.device != x.device or self.m.head.weight.device != x.device:
@@ -261,9 +272,10 @@ class RAJNIViTWrapper(nn.Module):
         pos, cls_pos0, cls_sum, cls_sumsq = pk.tensors(("pos", P), (m.pos_embed, m.cls_token), _pos_pack)
         cur, nxt = ws["xa"], ws["xb"]
         stats, slots = ws["stats"], ws["stat_slots"]
-        ops.patch_im2col(x, 16, ws["cols"], cls_pos0, cur, C, row_stats=stats, stats_slots=slots,
+        kpe = ws["cols"].shape[1]                                                   # 3 p^2
+        ops.patch_im2col(x, self.patch, ws["cols"], cls_pos0, cur, C, row_stats=stats, stats_slots=slots,
                          cls_sum=cls_sum, cls_sumsq=cls_sumsq, norm=self.input_norm if x.dtype == torch.uint8 else None)
-        ops.gemm(ws["cols"], pe_w, pe_b, B * P, C, 768, residual=pos, ldres=C, res_row_map=ws["embed_pos_map"],
+        ops.gemm(ws["cols"], pe_w, pe_b, B * P, C, kpe, residual=pos, ldres=C, res_row_map=ws["embed_pos_map"],
                  out=cur, ldd=C, out_row_map=ws["embed_out_map"], row_stats=stats, tag="embed")
 
         # Zig-zag traversal: every persistent kernel walks its row tiles in the direction opposite to the kernel that

@@ -15,7 +15,13 @@ CASES = [("C1 vit_tiny  bs8", "vit_tiny_patch16_224", C1, 8, 224),
          ("C3 vit_small bs256 (512 over 2 GPUs)", "vit_small_patch16_224", {i: {"keep_ratio": 0.7} for i in range(3, 12)}, 256, 224),
          ("C3 vit_small bs64  (512 over 8 GPUs)", "vit_small_patch16_224", {i: {"keep_ratio": 0.7} for i in range(3, 12)}, 64, 224),
          ("C4 vit_large bs32  (256 over 8 GPUs)", "vit_large_patch16_224", {i: {"keep_ratio": 0.9} for i in range(24)}, 32, 224),
-         ("C5 deit_384  bs16  (128 over 8 GPUs)", "deit_base_patch16_384", README, 16, 384)]
+         ("C5 deit_384  bs16  (128 over 8 GPUs)", "deit_base_patch16_384", README, 16, 384),
+         ("B/32 vit_base_patch32 bs256 dense", "vit_base_patch32_224", {}, 256, 224),
+         ("B/32 vit_base_patch32 bs256 README", "vit_base_patch32_224", README, 256, 224),
+         ("B/8  vit_base_patch8  bs64  dense", "vit_base_patch8_224", {}, 64, 224),
+         ("B/8  vit_base_patch8  bs64  README", "vit_base_patch8_224", README, 64, 224),
+         ("B/8  vit_base_patch8  bs256 dense", "vit_base_patch8_224", {}, 256, 224),
+         ("B/8  vit_base_patch8  bs256 README", "vit_base_patch8_224", README, 256, 224)]
 only = sys.argv[1:]
 for name, model_name, sched, B, S in CASES:
     if only and not any(o in name for o in only):

@@ -72,6 +72,14 @@ def main():
         t = timeit(lambda: ops.score_select(qkv, 12, keep), inner=8)
         nbytes = B * (2 * N * 768 * 2 + 768 * 2 + 8 * (keep + 1))
         print(f"score_select N={N:3d}            {t*1e6:8.1f} us  {nbytes/t/1e9:7.1f} GB/s ({nbytes/t/1e9/PEAKS['hbm_gbs']*100:5.1f}% of measured HBM)")
+    # the long-sequence score path (ViT-B/8, 785 tokens: logits and value rows through the workspace); K/V-plane bytes
+    if want("score_long"):
+        N, keep = 785, 690
+        qkv = torch.randn(B, N, 2304, device="cuda").bfloat16()
+        t = timeit(lambda: ops.score_select(qkv, 12, keep), inner=4)
+        kv = B * 2 * N * 768 * 2
+        print(f"score_select N={N} (workspace)  {t*1e6:8.1f} us  {kv/t/1e9:7.1f} GB/s of K/V planes ({kv/t/1e9/PEAKS['hbm_gbs']*100:5.1f}% of measured HBM)")
+        del qkv
     # attention
     for N, Np in ((197, 197), (197, 173), (173, 152), (152, 121), (121, 87), (87, 87)) if want("attn") else ():
         qkv = torch.randn(B * N, 2304, device="cuda").bfloat16()
@@ -99,6 +107,18 @@ def main():
     c0 = torch.zeros(768, device="cuda", dtype=torch.bfloat16)
     t = timeit(lambda: ops.patch_im2col(img, 16, cols, c0, xx, 768))
     print(f"im2col                       {t*1e6:8.1f} us  {(img.numel()*4+cols.numel()*2)/t/1e9:7.1f} GB/s")
+    # im2col at 8/16/32-pixel patches, fp32 and uint8 pixels: the same bytes at every patch size (3*224*224 pixels in, as
+    # many bf16 out per image)
+    img8 = torch.randint(0, 256, (B, 3, 224, 224), device="cuda", dtype=torch.uint8)
+    norm = ((0.485, 0.456, 0.406), (0.229, 0.224, 0.225))
+    for p in (8, 16, 32):
+        P = (224 // p) ** 2
+        cp = torch.empty(B * P, 3 * p * p, device="cuda", dtype=torch.bfloat16)
+        xp = torch.empty(B * (P + 1), 768, device="cuda", dtype=torch.bfloat16)
+        for im in (img, img8):
+            t = timeit(lambda: ops.patch_im2col(im, p, cp, c0, xp, 768, norm=norm if im.dtype == torch.uint8 else None), inner=4)
+            nb = im.numel() * im.element_size() + cp.numel() * 2
+            print(f"im2col p={p:2d} {str(im.dtype)[6:]:7s}          {t*1e6:8.1f} us  {nb/t/1e9:7.1f} GB/s")
 
 
 if __name__ == "__main__":
