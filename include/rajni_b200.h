@@ -72,6 +72,12 @@ int rajni_importance(const void* qkv, int B, int N, int C, int H, float eps,
  * (global row of each kept token; nullable). keep > N-1 -> RAJNI_ERANGE. */
 int rajni_select(const float* scores, int B, int N, int keep,
                  int32_t* keep_idx, float* next_scores, int32_t* row_map, void* stream);
+/* The same with `prefix` (1 or 2) leading tokens that are always kept: CLS, or CLS and a distillation token.
+ * Top-`keep` of scores[:,prefix:] -> keep_idx [B,keep+prefix] int32, strictly ascending, keep_idx[:,r]==r for
+ * r < prefix; next_scores and row_map [B*(keep+prefix)] as above.  keep > N-prefix -> RAJNI_ERANGE.
+ * rajni_select is this call with prefix 1. */
+int rajni_select_prefix(const float* scores, int B, int N, int prefix, int keep,
+                        int32_t* keep_idx, float* next_scores, int32_t* row_map, void* stream);
 
 /* ---- a1+a2 fused: one pass over the K and V planes, then in-CTA select.
  * scores may be NULL when the caller does not need the full score vector.
@@ -95,6 +101,14 @@ int rajni_score_select_needs_workspace(int N, int H);
 int rajni_score_select_split(const void* qkv, int B, int N, int C, int H, int keep, float eps,
                              float* scores, int32_t* keep_idx, float* next_scores, int32_t* row_map,
                              void* workspace, size_t workspace_bytes, void* stream);
+/* Both of the above with `prefix` (1 or 2) always-kept leading tokens, selection as in rajni_select_prefix.  The scores do
+ * not depend on it: the query is row 0 (CLS), every token (a distillation token too) is a key and value and enters the
+ * value-norm statistics.  workspace == NULL: rajni_score_select's one-launch kernel; else rajni_score_select_split's two
+ * launches (same bits).  keep_idx == NULL computes the scores only.  rajni_score_select and rajni_score_select_split are
+ * this call with prefix 1. */
+int rajni_score_select_prefix(const void* qkv, int B, int N, int C, int H, int prefix, int keep, float eps,
+                              float* scores, int32_t* keep_idx, float* next_scores, int32_t* row_map,
+                              void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- a3 / a9: row gather-compaction (attention.py:42-43, model.py:55-56)
  * dst[r, :] = src[row_map[r], :], rows of `row_elems` bf16 (multiple of 8). */
@@ -106,6 +120,10 @@ int rajni_gather_rows(const void* src, const int32_t* row_map, void* dst,
  * rows only) and written densely at y + r*C. C multiple of 8, C <= 4096. */
 int rajni_layernorm(const void* x, long long in_row_stride, const float* gamma,
                     const float* beta, float eps, void* y, int rows, int C, void* stream);
+/* The same with row r written at y + r*out_row_stride (>= C, multiple of 8): two calls with out_row_stride 2C put the
+ * normalised CLS and distillation rows of each image side by side, the A operand of a distilled model's head. */
+int rajni_layernorm_strided(const void* x, long long in_row_stride, const float* gamma, const float* beta, float eps,
+                            void* y, long long out_row_stride, int rows, int C, void* stream);
 
 /* ---- dense contractions (attention.py:22,55; timm Mlp fc1/fc2; patch_embed; head)
  * D[orow(m), n] = epi( sum_k A[m,k] * W[n,k] ), A [M,K] bf16, W [N,K] bf16
@@ -182,6 +200,15 @@ int rajni_patch_im2col(const void* images, int image_dtype, int B, int S, int pa
                        void* cols, const void* cls_pos0, void* x, int C,
                        float* row_stats, long long row_stats_ld, int stats_slots,
                        float cls_sum, float cls_sumsq, const float* norm, void* stream);
+/* The same with `prefix` (1 or 2) rows in front of each image's patches: x is [B,P+prefix,C], and x[b,r,:] =
+ * prefix_rows[r,:] for r < prefix (prefix_rows [prefix,C] bf16: cls_token + pos_embed[0], dist_token + pos_embed[1]; the
+ * tokens alone for a model that adds positions to the patches only).  With row_stats, prefix_stats_host = HOST array
+ * [prefix][2] of each row's (sum, sum of squares), written to slot 0 (read at call time).  The embed GEMM stores patch q
+ * of image b at row b*(P+prefix) + prefix + q.  rajni_patch_im2col is this call with prefix 1. */
+int rajni_patch_im2col_prefix(const void* images, int image_dtype, int B, int S, int patch,
+                              void* cols, const void* prefix_rows, int prefix, void* x, int C,
+                              float* row_stats, long long row_stats_ld, int stats_slots,
+                              const float* prefix_stats_host, const float* norm, void* stream);
 
 /* ---- f3: the loader's Resize(size, bicubic) + CenterCrop(224) on decoded uint8 RGB frames (run.py:62-66), bit-identical
  * to torchvision on PIL images (Pillow's antialiased two-pass resampler; oracle/resize_oracle.py restates it).

@@ -39,14 +39,19 @@ SIGNATURES = {
     "rajni_launch_count": (c_uint64, []),
     "rajni_importance": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_float, c_void_p, c_void_p]),
     "rajni_select": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "rajni_select_prefix": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     "rajni_score_select": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_float,
                                    c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "rajni_score_select_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int]),
     "rajni_score_select_needs_workspace": (c_int, [c_int, c_int]),
     "rajni_score_select_split": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_float,
                                          c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "rajni_score_select_prefix": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_float,
+                                          c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "rajni_gather_rows": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p]),
     "rajni_layernorm": (c_int, [c_void_p, c_longlong, c_void_p, c_void_p, c_float, c_void_p, c_int, c_int, c_void_p]),
+    "rajni_layernorm_strided": (c_int, [c_void_p, c_longlong, c_void_p, c_void_p, c_float, c_void_p, c_longlong, c_int, c_int,
+                                        c_void_p]),
     "rajni_gemm_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int,
                                 c_void_p, c_longlong, c_void_p, c_longlong, c_void_p, c_void_p]),
     "rajni_gemm_bf16_ex": (c_int, [POINTER(GemmArgs), c_void_p]),
@@ -60,6 +65,8 @@ SIGNATURES = {
     "rajni_resize_status": (c_int, [c_void_p, c_int, c_int, c_void_p]),
     "rajni_patch_im2col": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int,
                                    c_void_p, c_longlong, c_int, c_float, c_float, c_void_p, c_void_p]),
+    "rajni_patch_im2col_prefix": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p, c_int,
+                                          c_void_p, c_longlong, c_int, c_void_p, c_void_p, c_void_p]),
 }
 
 _lib = None

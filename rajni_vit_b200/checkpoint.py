@@ -18,10 +18,13 @@ Accepted key families (SURVEY.md section 5):
 
 The architecture is inferred from the tensors' shapes (width from ``cls_token``, depth from
 the block indices, image size from ``pos_embed``, classes from ``head.weight``); heads =
-width / 64, the only head dimension the kernels (and every BASELINE config) use.
-Checkpoints outside the wrapper's contract — LayerScale (``ls1.gamma``), ``norm_pre``,
-``fc_norm``, distillation / register tokens, qk-norm — raise ``NotImplementedError`` naming
-the offending keys: never a silent partial load.
+width / 64, the only head dimension the kernels (and every BASELINE config) use.  The two DeiT families load too:
+  * DeiT-III: ``blocks.{i}.ls1.gamma`` / ``ls2.gamma`` (LayerScale, accepted only when every block has both), and a
+    ``pos_embed`` with one row per patch (a square length: no position for the class token, timm's ``no_embed_class``);
+  * distilled DeiT: ``dist_token`` together with ``head_dist.*``, ``pos_embed`` of patches + 2.
+Checkpoints outside the wrapper's contract — partial LayerScale, ``norm_pre``, ``fc_norm``, register
+tokens, a distillation token without its head, qk-norm — raise ``NotImplementedError`` naming the offending keys: never a
+silent partial load.
 """
 from __future__ import annotations
 
@@ -38,7 +41,7 @@ from .vit import VisionTransformer
 _SAFETENSORS_DTYPES = {"F32": torch.float32, "F16": torch.float16, "BF16": torch.bfloat16, "F64": torch.float64,
                        "I64": torch.int64, "I32": torch.int32, "U8": torch.uint8, "BOOL": torch.bool}
 
-_UNSUPPORTED = (r"\.ls[12]\.", r"^norm_pre\.", r"^fc_norm\.", r"^dist_token$", r"^reg_token$", r"^head_dist\.",
+_UNSUPPORTED = (r"\.ls[12]\.(?!gamma$)", r"^norm_pre\.", r"^fc_norm\.", r"^reg_token$",
                 r"\.attn\.[qk]_norm\.", r"^patch_embed\.norm\.", r"\.mlp\.norm\.", r"rel_pos", r"^pre_logits\.")
 
 
@@ -130,15 +133,36 @@ def infer_config(sd: Mapping[str, torch.Tensor]) -> Dict[str, int]:
     blocks = {int(m.group(1)) for k in sd for m in [re.match(r"blocks\.(\d+)\.", k)] if m}
     if not blocks or blocks != set(range(len(blocks))):
         raise KeyError(f"block indices {sorted(blocks)} are not 0..depth-1")
+    # LayerScale (DeiT-III): both gammas in every block, or none at all
+    ls = sorted(k for k in sd if re.match(r"blocks\.\d+\.ls[12]\.gamma$", k))
+    if ls and len(ls) != 2 * len(blocks):
+        have = set(ls)
+        odd = sorted(k for i in blocks for k in (f"blocks.{i}.ls1.gamma", f"blocks.{i}.ls2.gamma") if k not in have) or ls
+        raise NotImplementedError(f"LayerScale must be in every block (ls1 and ls2): the checkpoint has {ls[:4]}"
+                                  f"{' ...' if len(ls) > 4 else ''} but not {odd[:4]}")
+    # distillation token (distilled DeiT): only together with its head
+    dist = "dist_token" in sd
+    head_dist = sorted(k for k in sd if k.startswith("head_dist."))
+    if dist != bool(head_dist) or (dist and "head_dist.weight" not in sd):
+        raise NotImplementedError("a distillation token needs its head and the head needs the token: checkpoint has "
+                                  f"{['dist_token'] if dist else []} {head_dist}")
+    # pos_embed layout from its length: patches (square, no position for the class token), + 1 (class token), + 2 (distilled)
     n_tok = sd["pos_embed"].shape[1]
-    grid = int(round((n_tok - 1) ** 0.5))
-    if grid * grid != n_tok - 1:
-        raise NotImplementedError(f"pos_embed has {n_tok} positions: not 1 + a square grid (class token + patches)")
+    prefix = 2 if dist else 1
+    grid = int(round(max(n_tok - prefix, 0) ** 0.5))
+    no_embed_class = False
+    if grid * grid != n_tok - prefix:
+        grid = int(round(n_tok ** 0.5))
+        no_embed_class = True
+        if grid * grid != n_tok:
+            raise NotImplementedError(f"pos_embed has {n_tok} positions: not a square grid of patches, plus {prefix} "
+                                      f"({'class and distillation tokens' if dist else 'class token'}) or plus none")
     if C % 64:
         raise NotImplementedError(f"width {C} is not a multiple of the head dimension 64")
     hidden = sd["blocks.0.mlp.fc1.weight"].shape[0]
     return dict(embed_dim=C, depth=len(blocks), num_heads=C // 64, img_size=grid * patch, patch_size=patch,
-                num_classes=sd["head.weight"].shape[0], mlp_ratio=hidden / C)
+                num_classes=sd["head.weight"].shape[0], mlp_ratio=hidden / C, init_values=1.0 if ls else None,
+                no_embed_class=no_embed_class, distilled=dist)
 
 
 def load_checkpoint(source: Union[str, os.PathLike, Mapping[str, torch.Tensor]], model: Optional[torch.nn.Module] = None,

@@ -41,7 +41,7 @@ __global__ void __launch_bounds__(256) gather_rows_kernel(const uint4* __restric
 template <int CPL>
 __global__ void __launch_bounds__(256) layernorm_kernel(const __nv_bfloat16* __restrict__ x, long long in_stride,
                                                         const float* __restrict__ gamma, const float* __restrict__ beta,
-                                                        float eps, __nv_bfloat16* __restrict__ y, int rows, int C) {
+                                                        float eps, __nv_bfloat16* __restrict__ y, long long out_stride, int rows, int C) {
     griddep_launch();
     griddep_wait();
     const int lane = threadIdx.x & 31;
@@ -76,7 +76,7 @@ __global__ void __launch_bounds__(256) layernorm_kernel(const __nv_bfloat16* __r
         }
     }
     const float rstd = rsqrtf(warp_sum(sq) / (float)C + eps);
-    __nv_bfloat16* yr = y + (long long)row * C;
+    __nv_bfloat16* yr = y + (long long)row * out_stride;
 #pragma unroll
     for (int i = 0; i < CPL; ++i) {
         int j = lane + 32 * i;
@@ -95,7 +95,38 @@ __global__ void __launch_bounds__(256) layernorm_kernel(const __nv_bfloat16* __r
     }
 }
 
-// ------------------------------------------------------------------ patch im2col (+ CLS rows)
+// ------------------------------------------------------------------ patch im2col (+ prefix rows)
+// Prefix rows: the P0 rows in front of each image's patches (CLS, or CLS + distillation token), copied from a [P0, C] block
+// the host prepared (token + its position embedding, or the token alone when the model adds no position to it), and
+// their LayerNorm partial sums (slot 0 = the host's (sum, sum of squares) of the row, the other slots zero).
+constexpr int kMaxPrefix = 2;
+struct PrefixStats { float sum[kMaxPrefix], sumsq[kMaxPrefix]; };
+
+__device__ __forceinline__ void write_prefix_rows(const uint4* __restrict__ prefix_rows, int P0, const PrefixStats& ps,
+                                                  uint4* __restrict__ x, int C, int B, long long P,
+                                                  float2* __restrict__ row_stats, long long stats_ld, int stats_slots) {
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    const long long t0 = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const int cchunks = C >> 3;
+    const long long N0 = P + P0;                 // rows per image
+    const long long pre = (long long)P0 * cchunks;
+    for (long long i = t0; i < (long long)B * pre; i += stride) {
+        const int b = (int)(i / pre);
+        const int k = (int)(i - (long long)b * pre);          // r * cchunks + j: row-major in prefix_rows and in x alike
+        x[(long long)b * N0 * cchunks + k] = __ldg(prefix_rows + k);
+    }
+    // LayerNorm partials of the prefix rows (the patch rows' partials come from the embed GEMM's epilogue)
+    if (row_stats != nullptr) {
+        const long long per = (long long)stats_slots * P0;
+        for (long long i = t0; i < (long long)B * per; i += stride) {
+            const int b = (int)(i / per);
+            const int k = (int)(i - (long long)b * per);
+            const int s = k / P0, r = k - s * P0;
+            row_stats[(long long)s * stats_ld + (long long)b * N0 + r] = s == 0 ? make_float2(ps.sum[r], ps.sumsq[r]) : make_float2(0.f, 0.f);
+        }
+    }
+}
+
 // One thread moves one (patch, channel, ky) strip: 16 pixels in, 16 bf16 out (two 16-byte
 // stores = one full 32-byte sector).  px is the fastest thread index, so a warp reads
 // contiguous image rows.  Column order (c, ky, kx) matches Conv2d weight.view(C, -1).
@@ -105,10 +136,9 @@ struct ImageNorm { float mean[3], std[3]; };
 template <int DT>
 __global__ void __launch_bounds__(256) im2col16_kernel(const void* __restrict__ images, const ImageNorm norm, int B, int S,
                                                        __nv_bfloat16* __restrict__ cols,
-                                                       const uint4* __restrict__ cls_pos0,
+                                                       const uint4* __restrict__ prefix_rows, int P0, const PrefixStats ps,
                                                        uint4* __restrict__ x, int C,
-                                                       float2* __restrict__ row_stats, long long stats_ld, int stats_slots,
-                                                       float cls_sum, float cls_sumsq) {
+                                                       float2* __restrict__ row_stats, long long stats_ld, int stats_slots) {
     griddep_launch();
     griddep_wait();
     const int G = S >> 4;                       // patches per side
@@ -156,23 +186,11 @@ __global__ void __launch_bounds__(256) im2col16_kernel(const void* __restrict__ 
         dst[0] = o0;
         dst[1] = o1;
     }
-    // CLS rows: x[b,0,:] = cls_token + pos_embed[0]   (model.py:35-37)
-    const int cchunks = C >> 3;
-    const long long P1 = (long long)G * G + 1;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < (long long)B * cchunks; i += stride) {
-        int b = (int)(i / cchunks), j = (int)(i % cchunks);
-        x[(long long)b * P1 * cchunks + j] = __ldg(cls_pos0 + j);
-    }
-    // LayerNorm partials of the CLS rows (the patch rows' partials come from the embed GEMM's epilogue)
-    if (row_stats != nullptr) {
-        for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < (long long)B * stats_slots; i += stride) {
-            int b = (int)(i / stats_slots), s = (int)(i % stats_slots);
-            row_stats[(long long)s * stats_ld + (long long)b * P1] = s == 0 ? make_float2(cls_sum, cls_sumsq) : make_float2(0.f, 0.f);
-        }
-    }
+    // prefix rows: x[b,0,:] = cls_token + pos_embed[0]   (model.py:35-37), and the distillation token's row after it
+    write_prefix_rows(prefix_rows, P0, ps, x, C, B, (long long)G * G, row_stats, stats_ld, stats_slots);
 }
 
-// ------------------------------------------------------------------ patch im2col (+ CLS rows)
+// ------------------------------------------------------------------ patch im2col (+ prefix rows)
 // Any patch size p that is a multiple of 8.  One thread moves one 8-pixel run of one (patch, channel, patch row): 8 pixels
 // in, 16 bytes of bf16 out.  The run's index inside its (patch, channel) plane (p*p/8 runs) is the fastest thread index, so
 // a warp stores 512 consecutive bytes of one cols row at p >= 16 and four 128-byte planes at p = 8: whole sectors at every
@@ -225,10 +243,9 @@ __device__ __forceinline__ uint4 im2col_convert(const uint4 (&r)[2], const Image
 template <int DT>
 __global__ void __launch_bounds__(256) im2col_kernel(const void* __restrict__ images, const ImageNorm norm, int B, int S, int p,
                                                      __nv_bfloat16* __restrict__ cols,
-                                                     const uint4* __restrict__ cls_pos0,
+                                                     const uint4* __restrict__ prefix_rows, int P0, const PrefixStats ps,
                                                      uint4* __restrict__ x, int C,
-                                                     float2* __restrict__ row_stats, long long stats_ld, int stats_slots,
-                                                     float cls_sum, float cls_sumsq) {
+                                                     float2* __restrict__ row_stats, long long stats_ld, int stats_slots) {
     griddep_launch();
     griddep_wait();
     const int G = S / p;                        // patches per side
@@ -268,20 +285,8 @@ __global__ void __launch_bounds__(256) im2col_kernel(const void* __restrict__ im
         im2col_load<DT>(images, locate(i, dst, c), r);
         *reinterpret_cast<uint4*>(cols + dst) = im2col_convert<DT>(r, norm, c);
     }
-    // CLS rows: x[b,0,:] = cls_token + pos_embed[0]   (model.py:35-37)
-    const int cchunks = C >> 3;
-    const long long P1 = (long long)G * G + 1;
-    for (long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x; k < (long long)B * cchunks; k += stride) {
-        int b = (int)(k / cchunks), j = (int)(k % cchunks);
-        x[(long long)b * P1 * cchunks + j] = __ldg(cls_pos0 + j);
-    }
-    // LayerNorm partials of the CLS rows (the patch rows' partials come from the embed GEMM's epilogue)
-    if (row_stats != nullptr) {
-        for (long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x; k < (long long)B * stats_slots; k += stride) {
-            int b = (int)(k / stats_slots), s = (int)(k % stats_slots);
-            row_stats[(long long)s * stats_ld + (long long)b * P1] = s == 0 ? make_float2(cls_sum, cls_sumsq) : make_float2(0.f, 0.f);
-        }
-    }
+    // prefix rows: x[b,0,:] = cls_token + pos_embed[0]   (model.py:35-37), and the distillation token's row after it
+    write_prefix_rows(prefix_rows, P0, ps, x, C, B, (long long)G * G, row_stats, stats_ld, stats_slots);
 }
 
 }  // namespace rajni
@@ -304,35 +309,49 @@ extern "C" int rajni_gather_rows(const void* src, const int32_t* row_map, void* 
     return check_launch("gather_rows");
 }
 
-extern "C" int rajni_layernorm(const void* x, long long in_row_stride, const float* gamma,
-                               const float* beta, float eps, void* y, int rows, int C, void* stream) {
+extern "C" int rajni_layernorm_strided(const void* x, long long in_row_stride, const float* gamma, const float* beta, float eps,
+                                       void* y, long long out_row_stride, int rows, int C, void* stream) {
     RAJNI_REQUIRE(x && gamma && beta && y, RAJNI_EINVAL, "rajni_layernorm: null pointer");
-    RAJNI_REQUIRE(rows > 0 && C > 0 && C % 8 == 0 && C <= 2048 && in_row_stride % 8 == 0, RAJNI_EINVAL,
-                  "rajni_layernorm: rows=%d C=%d stride=%lld unsupported", rows, C, in_row_stride);
+    RAJNI_REQUIRE(rows > 0 && C > 0 && C % 8 == 0 && C <= 2048 && in_row_stride % 8 == 0 && out_row_stride % 8 == 0 && out_row_stride >= C,
+                  RAJNI_EINVAL, "rajni_layernorm: rows=%d C=%d stride=%lld out stride=%lld unsupported", rows, C, in_row_stride, out_row_stride);
     const int cpl = (C / 8 + 31) / 32;
     const int wpb = 8;
     dim3 grid((rows + wpb - 1) / wpb), block(wpb * 32);
     auto s = static_cast<cudaStream_t>(stream);
     auto xb = static_cast<const __nv_bfloat16*>(x);
     auto yb = static_cast<__nv_bfloat16*>(y);
+    const long long os = out_row_stride;
     cudaError_t le = cudaSuccess;
     switch (cpl) {
-        case 1: le = launch_kernel(layernorm_kernel<1>, grid, block, 0, s, 1, xb, in_row_stride, gamma, beta, eps, yb, rows, C); break;
-        case 2: le = launch_kernel(layernorm_kernel<2>, grid, block, 0, s, 1, xb, in_row_stride, gamma, beta, eps, yb, rows, C); break;
-        case 3: le = launch_kernel(layernorm_kernel<3>, grid, block, 0, s, 1, xb, in_row_stride, gamma, beta, eps, yb, rows, C); break;
-        case 4: le = launch_kernel(layernorm_kernel<4>, grid, block, 0, s, 1, xb, in_row_stride, gamma, beta, eps, yb, rows, C); break;
-        default: le = launch_kernel(layernorm_kernel<8>, grid, block, 0, s, 1, xb, in_row_stride, gamma, beta, eps, yb, rows, C); break;
+        case 1: le = launch_kernel(layernorm_kernel<1>, grid, block, 0, s, 1, xb, in_row_stride, gamma, beta, eps, yb, os, rows, C); break;
+        case 2: le = launch_kernel(layernorm_kernel<2>, grid, block, 0, s, 1, xb, in_row_stride, gamma, beta, eps, yb, os, rows, C); break;
+        case 3: le = launch_kernel(layernorm_kernel<3>, grid, block, 0, s, 1, xb, in_row_stride, gamma, beta, eps, yb, os, rows, C); break;
+        case 4: le = launch_kernel(layernorm_kernel<4>, grid, block, 0, s, 1, xb, in_row_stride, gamma, beta, eps, yb, os, rows, C); break;
+        default: le = launch_kernel(layernorm_kernel<8>, grid, block, 0, s, 1, xb, in_row_stride, gamma, beta, eps, yb, os, rows, C); break;
     }
     count_launch();
     RAJNI_REQUIRE(le == cudaSuccess, RAJNI_ECUDA, "layernorm: launch failed: %s", cudaGetErrorString(le));
     return check_launch("layernorm");
 }
 
-extern "C" int rajni_patch_im2col(const void* images, int image_dtype, int B, int S, int patch,
-                                  void* cols, const void* cls_pos0, void* x, int C,
-                                  float* row_stats, long long row_stats_ld, int stats_slots,
-                                  float cls_sum, float cls_sumsq, const float* norm, void* stream) {
-    RAJNI_REQUIRE(images && cols && cls_pos0 && x, RAJNI_EINVAL, "rajni_patch_im2col: null pointer");
+extern "C" int rajni_layernorm(const void* x, long long in_row_stride, const float* gamma,
+                               const float* beta, float eps, void* y, int rows, int C, void* stream) {
+    return rajni_layernorm_strided(x, in_row_stride, gamma, beta, eps, y, C, rows, C, stream);
+}
+
+extern "C" int rajni_patch_im2col_prefix(const void* images, int image_dtype, int B, int S, int patch,
+                                         void* cols, const void* prefix_rows, int prefix, void* x, int C,
+                                         float* row_stats, long long row_stats_ld, int stats_slots,
+                                         const float* prefix_stats_host, const float* norm, void* stream) {
+    RAJNI_REQUIRE(images && cols && prefix_rows && x, RAJNI_EINVAL, "rajni_patch_im2col: null pointer");
+    RAJNI_REQUIRE(prefix >= 1 && prefix <= kMaxPrefix, RAJNI_EINVAL, "rajni_patch_im2col: prefix=%d (1: CLS, 2: CLS + distillation token)", prefix);
+    RAJNI_REQUIRE(row_stats == nullptr || prefix_stats_host != nullptr, RAJNI_EINVAL, "rajni_patch_im2col: row_stats needs prefix_stats_host");
+    PrefixStats ps{};
+    if (row_stats != nullptr)
+        for (int r = 0; r < prefix; ++r) {
+            ps.sum[r] = prefix_stats_host[2 * r];
+            ps.sumsq[r] = prefix_stats_host[2 * r + 1];
+        }
     RAJNI_REQUIRE(image_dtype >= RAJNI_IMG_BF16 && image_dtype <= RAJNI_IMG_U8, RAJNI_EINVAL, "rajni_patch_im2col: image_dtype %d", image_dtype);
     RAJNI_REQUIRE(image_dtype != RAJNI_IMG_U8 || norm != nullptr, RAJNI_EINVAL, "rajni_patch_im2col: uint8 images need norm (mean[3], std[3])");
     ImageNorm nm{{0.f, 0.f, 0.f}, {1.f, 1.f, 1.f}};
@@ -345,8 +364,8 @@ extern "C" int rajni_patch_im2col(const void* images, int image_dtype, int B, in
     RAJNI_REQUIRE(patch >= 8 && patch % 8 == 0 && S > 0 && S <= 16384 && S % patch == 0 && B > 0 && C % 8 == 0, RAJNI_EINVAL,
                   "rajni_patch_im2col: patch=%d S=%d B=%d C=%d unsupported (patch must be a multiple of 8 dividing S <= 16384)", patch, S, B, C);
     const int G = S / patch;
-    RAJNI_REQUIRE(row_stats == nullptr || (stats_slots > 0 && row_stats_ld >= (long long)B * (G * G + 1)), RAJNI_EINVAL,
-                  "rajni_patch_im2col: row_stats needs stats_slots > 0 and row_stats_ld >= B*(P+1)");
+    RAJNI_REQUIRE(row_stats == nullptr || (stats_slots > 0 && row_stats_ld >= (long long)B * (G * G + prefix)), RAJNI_EINVAL,
+                  "rajni_patch_im2col: row_stats needs stats_slots > 0 and row_stats_ld >= B*(P+prefix)");
     auto s = static_cast<cudaStream_t>(stream);
     cudaError_t le;
     // p = 16 keeps its own kernel: 16-pixel strips, px fastest.  On a B200 at 256 images of 224 px it moves fp32 images in
@@ -357,20 +376,27 @@ extern "C" int rajni_patch_im2col(const void* images, int image_dtype, int B, in
         if (blocks > 148 * 32) blocks = 148 * 32;
         auto kern = image_dtype == RAJNI_IMG_U8 ? im2col16_kernel<2> : image_dtype == RAJNI_IMG_F32 ? im2col16_kernel<1> : im2col16_kernel<0>;
         le = launch_kernel(kern, dim3((int)blocks), dim3(256), 0, s, 1,
-                           images, nm, B, S, static_cast<__nv_bfloat16*>(cols), static_cast<const uint4*>(cls_pos0),
-                           static_cast<uint4*>(x), C, reinterpret_cast<float2*>(row_stats), row_stats_ld, stats_slots,
-                           cls_sum, cls_sumsq);
+                           images, nm, B, S, static_cast<__nv_bfloat16*>(cols), static_cast<const uint4*>(prefix_rows), prefix, ps,
+                           static_cast<uint4*>(x), C, reinterpret_cast<float2*>(row_stats), row_stats_ld, stats_slots);
     } else {
         const long long runs = (long long)B * G * G * 3 * patch * (patch / 8);
         long long blocks = (runs + 256 * kIm2colUnroll - 1) / (256 * kIm2colUnroll);
         if (blocks > 148 * 32) blocks = 148 * 32;
         auto kern = image_dtype == RAJNI_IMG_U8 ? im2col_kernel<2> : image_dtype == RAJNI_IMG_F32 ? im2col_kernel<1> : im2col_kernel<0>;
         le = launch_kernel(kern, dim3((int)blocks), dim3(256), 0, s, 1,
-                           images, nm, B, S, patch, static_cast<__nv_bfloat16*>(cols), static_cast<const uint4*>(cls_pos0),
-                           static_cast<uint4*>(x), C, reinterpret_cast<float2*>(row_stats), row_stats_ld, stats_slots,
-                           cls_sum, cls_sumsq);
+                           images, nm, B, S, patch, static_cast<__nv_bfloat16*>(cols), static_cast<const uint4*>(prefix_rows), prefix, ps,
+                           static_cast<uint4*>(x), C, reinterpret_cast<float2*>(row_stats), row_stats_ld, stats_slots);
     }
     count_launch();
     RAJNI_REQUIRE(le == cudaSuccess, RAJNI_ECUDA, "patch_im2col: launch failed: %s", cudaGetErrorString(le));
     return check_launch("patch_im2col");
+}
+
+extern "C" int rajni_patch_im2col(const void* images, int image_dtype, int B, int S, int patch,
+                                  void* cols, const void* cls_pos0, void* x, int C,
+                                  float* row_stats, long long row_stats_ld, int stats_slots,
+                                  float cls_sum, float cls_sumsq, const float* norm, void* stream) {
+    const float cls_stats[2] = {cls_sum, cls_sumsq};
+    return rajni_patch_im2col_prefix(images, image_dtype, B, S, patch, cols, cls_pos0, 1, x, C, row_stats, row_stats_ld,
+                                     stats_slots, cls_stats, norm, stream);
 }

@@ -1,7 +1,8 @@
 // Fused token scoring + selection for one image per CTA.
 //
 //   score  : rajni/wrapper/importance.py:5-34   (CLS attention x sigmoid(z-scored value norm))
-//   select : rajni/wrapper/attention.py:31-39   (top-k of scores[:,1:], ascending, CLS prepended)
+//   select : rajni/wrapper/attention.py:31-39   (top-k of scores[:,1:], ascending, CLS prepended); generalised to P0
+//            prefix tokens (CLS, or CLS + distillation token): top-k of scores[:,P0:], tokens 0..P0-1 prepended
 //   carry  : rajni/wrapper/attention.py:58      (next_scores = scores[keep_idx])
 //
 // HBM-bound: the only large traffic is ONE pass over the K and V planes of the
@@ -41,12 +42,13 @@ struct ScoreSelectParams {
     const __nv_bfloat16* qkv;   // [B,N,3C] or null (select-only)
     const float* scores_in;     // [B,N] when qkv == null
     float* scores_out;          // [B,N] or null
-    int32_t* keep_idx;          // [B,keep+1] or null (score-only)
-    float* next_scores;         // [B,keep+1]
-    int32_t* row_map;           // [B*(keep+1)] or null
+    int32_t* keep_idx;          // [B,keep+P0] or null (score-only)
+    float* next_scores;         // [B,keep+P0]
+    int32_t* row_map;           // [B*(keep+P0)] or null
     const float* pre_logit;     // [B][pad4(H*N)] CLS logits already computed by score_stream_kernel, or null
     const float* pre_vm;        // [B][N*64] head-averaged value rows already computed, or null
     int N, C, H, keep;
+    int P0;                     // prefix tokens, always kept (1: CLS; 2: CLS + distillation token)
     float eps;
 };
 
@@ -109,19 +111,19 @@ __device__ __forceinline__ uint32_t float_key(float f) {
     return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
 }
 
-// Select the `keep` largest of score[1..N-1] (ties: lower index first), always keep token 0,
+// Select the `keep` largest of score[P0..N-1] (ties: lower index first), always keep tokens 0..P0-1,
 // and emit ascending indices.  All threads of the CTA call this; score[] is in smem.
 template <int NT>
 __device__ void select_and_emit(const float* score, uint32_t* s_hist, int* s_misc, int* s_warp_off,
                                 const ScoreSelectParams& p, int b) {
-    const int N = p.N, keep = p.keep, tid = threadIdx.x;
+    const int N = p.N, keep = p.keep, P0 = p.P0, tid = threadIdx.x;
     // ---- radix select: key of the keep-th largest patch score, 8 bits per pass
     uint32_t prefix = 0, mask = 0;
     int remaining = keep;
     for (int shift = 24; shift >= 0; shift -= 8) {
         for (int i = tid; i < 256; i += NT) s_hist[i] = 0;
         tail_sync<NT>();
-        for (int n = 1 + tid; n < N; n += NT) {
+        for (int n = P0 + tid; n < N; n += NT) {
             uint32_t k = float_key(score[n]);
             if ((k & mask) == prefix) atomicAdd(&s_hist[(k >> shift) & 0xff], 1u);
         }
@@ -166,13 +168,14 @@ __device__ void select_and_emit(const float* score, uint32_t* s_hist, int* s_mis
     int n_gt = 0, n_eq = 0;
     for (int i = 0; i < ipt; ++i) {
         int n = n0 + i;
-        if (n >= 1 && n < N) {
+        if (n < P0) {
+            n_gt += 1;                      // prefix tokens are always kept (counted as "greater")
+        } else if (n < N) {
             uint32_t k = float_key(score[n]);
             n_gt += (k > thresh);
             n_eq += (k == thresh);
         }
     }
-    if (n0 == 0 && N > 0) n_gt += 1;        // CLS is always kept (counted as "greater")
     // block exclusive scan of (n_gt, n_eq) packed: both < 2^15
     int packed = (n_gt << 16) | n_eq;
     int incl = packed;
@@ -197,15 +200,15 @@ __device__ void select_and_emit(const float* score, uint32_t* s_hist, int* s_mis
     tail_sync<NT>();
     int excl = incl - packed + s_warp_off[warp];
     int gt_before = excl >> 16, eq_before = excl & 0xffff;
-    const int stride = keep + 1;
+    const int stride = keep + P0;
     for (int i = 0; i < ipt; ++i) {
         int n = n0 + i;
         if (n < N) {
             bool take;
             int pos;
-            if (n == 0) {
+            if (n < P0) {
                 take = true;
-                pos = 0;
+                pos = gt_before;            // = n: only prefix tokens precede it
             } else {
                 uint32_t k = float_key(score[n]);
                 bool gt = k > thresh, eq = k == thresh;
@@ -218,7 +221,7 @@ __device__ void select_and_emit(const float* score, uint32_t* s_hist, int* s_mis
                 p.next_scores[(size_t)b * stride + pos] = score[n];
                 if (p.row_map) p.row_map[(size_t)b * stride + pos] = b * N + n;
             }
-            gt_before += take && (n == 0 || float_key(score[n]) > thresh);
+            gt_before += take && (n < P0 || float_key(score[n]) > thresh);
         }
     }
 }
@@ -298,18 +301,18 @@ __device__ __forceinline__ void load_cls_query(const __nv_bfloat16* img, int lan
 }
 
 // Selection for N <= 256 (every 224-px configuration): rank by counting instead of four radix passes with their twelve
-// block barriers.  Thread n counts the patches with a larger key (keys in shared memory, read four at a time; slot 0 and the
-// padding hold key 0, which no score maps to); equal keys - rare - are found through a counter per rank and ordered by index
+// block barriers.  Thread n counts the patches with a larger key (keys in shared memory, read four at a time; the prefix
+// slots and the padding hold key 0, which no score maps to); equal keys - rare - are found through a counter per rank and ordered by index
 // in a second loop only their threads run.  Positions come from one ballot per warp.  Same output as select_and_emit.
 template <int NT>
 __device__ void select_rank_emit(const float* score, uint32_t* key, uint32_t* s_cnt, int* s_warp_cnt, const ScoreSelectParams& p, int b) {
-    const int N = p.N, keep = p.keep, tid = threadIdx.x, lane = tid & 31;
+    const int N = p.N, keep = p.keep, P0 = p.P0, tid = threadIdx.x, lane = tid & 31;
     const int N4 = (N + 3) & ~3;
-    for (int n = tid; n < N4; n += NT) key[n] = (n >= 1 && n < N) ? float_key(score[n]) : 0u;
+    for (int n = tid; n < N4; n += NT) key[n] = (n >= P0 && n < N) ? float_key(score[n]) : 0u;
     for (int i = tid; i < 256; i += NT) s_cnt[i] = 0;
     tail_sync<NT>();
     const int n = tid;                                   // N <= 256 <= NT
-    const bool live = n >= 1 && n < N;
+    const bool live = n >= P0 && n < N;
     const uint32_t kn = live ? key[n] : 0xffffffffu;
     int gt = 0;
     if ((n & ~31) < N) {                                 // warps past the last token have nothing to count
@@ -320,15 +323,15 @@ __device__ void select_rank_emit(const float* score, uint32_t* key, uint32_t* s_
             gt += (k.x > kn) + (k.y > kn) + (k.z > kn) + (k.w > kn);
         }
     }
-    if (live) atomicAdd(&s_cnt[gt], 1u);                 // gt <= N - 2 <= 254
+    if (live) atomicAdd(&s_cnt[gt], 1u);                 // gt <= N - P0 - 1 <= 254
     tail_sync<NT>();
     bool take = false;
-    if (n == 0) {
-        take = true;                                     // CLS is always kept
+    if (n < P0) {
+        take = true;                                     // prefix tokens are always kept
     } else if (n < N) {
         int rank = gt;
         if (s_cnt[gt] > 1u && gt < keep) {               // tied with other patches: lower index first
-            for (int m = 1; m < n; ++m) rank += (key[m] == kn);
+            for (int m = P0; m < n; ++m) rank += (key[m] == kn);
         }
         take = rank < keep;
     }
@@ -338,7 +341,7 @@ __device__ void select_rank_emit(const float* score, uint32_t* key, uint32_t* s_
     if (take) {
         int pos = __popc(bal & ((1u << lane) - 1u));
         for (int w = 0; w < (tid >> 5); ++w) pos += s_warp_cnt[w];
-        const size_t o = (size_t)b * (keep + 1) + pos;
+        const size_t o = (size_t)b * (keep + P0) + pos;
         p.keep_idx[o] = n;
         p.next_scores[o] = score[n];
         if (p.row_map) p.row_map[o] = b * N + n;
@@ -600,6 +603,53 @@ static int check_score_shape(int B, int N, int C, int H) {
     return 0;
 }
 
+static int check_keep(const char* fn, int N, int P0, int keep) {
+    RAJNI_REQUIRE(P0 >= 1 && P0 <= 2, RAJNI_EINVAL, "%s: prefix=%d (1: CLS, 2: CLS + distillation token)", fn, P0);
+    RAJNI_REQUIRE(keep >= 1, RAJNI_EINVAL, "%s: keep=%d < 1", fn, keep);
+    RAJNI_REQUIRE(keep <= N - P0, RAJNI_ERANGE, "selected index k out of range (keep=%d, patches=%d)", keep, N - P0);
+    return 0;
+}
+
+static int select_prefix(const char* fn, const float* scores, int B, int N, int P0, int keep, int32_t* keep_idx,
+                         float* next_scores, int32_t* row_map, cudaStream_t stream) {
+    RAJNI_REQUIRE(scores && keep_idx && next_scores, RAJNI_EINVAL, "%s: null pointer", fn);
+    RAJNI_REQUIRE(B > 0 && N >= 2 && N <= 16384, RAJNI_EINVAL, "%s: bad B=%d N=%d", fn, B, N);
+    if (int rc = check_keep(fn, N, P0, keep)) return rc;
+    ScoreSelectParams p{};
+    p.scores_in = scores;
+    p.keep_idx = keep_idx; p.next_scores = next_scores; p.row_map = row_map;
+    p.N = N; p.C = 0; p.H = 0; p.keep = keep; p.P0 = P0; p.eps = 0.f;
+    return launch_score_select(p, B, stream);
+}
+
+// workspace == null: the one-launch kernel; else the split path (K/V pass over (image, row-block) CTAs, then the tail).
+// keep_idx == null: scores only.
+static int score_select_prefix(const char* fn, const void* qkv, int B, int N, int C, int H, int P0, int keep, float eps,
+                               float* scores, int32_t* keep_idx, float* next_scores, int32_t* row_map,
+                               void* workspace, size_t workspace_bytes, cudaStream_t s) {
+    RAJNI_REQUIRE(qkv && (keep_idx ? next_scores != nullptr : scores != nullptr), RAJNI_EINVAL, "%s: null pointer", fn);
+    if (int rc = check_score_shape(B, N, C, H)) return rc;
+    if (keep_idx != nullptr) {
+        if (int rc = check_keep(fn, N, P0, keep)) return rc;
+    }
+    ScoreSelectParams p{};
+    p.qkv = static_cast<const __nv_bfloat16*>(qkv);
+    p.scores_out = scores;
+    p.keep_idx = keep_idx; p.next_scores = next_scores; p.row_map = row_map;
+    p.N = N; p.C = C; p.H = H; p.keep = keep_idx ? keep : 0; p.P0 = P0; p.eps = eps;
+    if (workspace == nullptr) return launch_score_select(p, B, s);
+    RAJNI_REQUIRE(B <= 65535, RAJNI_EINVAL, "%s: B=%d exceeds the grid limit", fn, B);
+    RAJNI_REQUIRE(workspace_bytes >= split_workspace_floats(B, N, H) * sizeof(float) && (reinterpret_cast<uintptr_t>(workspace) & 15) == 0,
+                  RAJNI_EINVAL, "%s: workspace too small (%zu B) or not 16-byte aligned", fn, workspace_bytes);
+    float* ws = static_cast<float*>(workspace);
+    if (int rc = launch_score_stream(p.qkv, B, N, C, H, ws, s)) return rc;
+    p.pre_logit = ws;
+    p.pre_vm = ws + (size_t)B * (((size_t)H * N + 3) & ~(size_t)3);
+    // RAJNI_SCORE_WS_TAIL=1 (read per call; tests): the long-sequence tail at any N, to compare it with the shared-memory one
+    if (needs_workspace_tail(N, H) || getenv("RAJNI_SCORE_WS_TAIL") != nullptr) return launch_score_tail_ws(p, ws, B, s);
+    return launch_score_select(p, B, s);
+}
+
 }  // namespace rajni
 
 using namespace rajni;
@@ -615,32 +665,30 @@ extern "C" int rajni_importance(const void* qkv, int B, int N, int C, int H, flo
     return launch_score_select(p, B, static_cast<cudaStream_t>(stream));
 }
 
+extern "C" int rajni_select_prefix(const float* scores, int B, int N, int prefix, int keep, int32_t* keep_idx,
+                                   float* next_scores, int32_t* row_map, void* stream) {
+    return select_prefix("rajni_select_prefix", scores, B, N, prefix, keep, keep_idx, next_scores, row_map,
+                         static_cast<cudaStream_t>(stream));
+}
+
 extern "C" int rajni_select(const float* scores, int B, int N, int keep, int32_t* keep_idx,
                             float* next_scores, int32_t* row_map, void* stream) {
-    RAJNI_REQUIRE(scores && keep_idx && next_scores, RAJNI_EINVAL, "rajni_select: null pointer");
-    RAJNI_REQUIRE(B > 0 && N >= 2 && N <= 16384, RAJNI_EINVAL, "rajni_select: bad B=%d N=%d", B, N);
-    RAJNI_REQUIRE(keep >= 1, RAJNI_EINVAL, "rajni_select: keep=%d < 1", keep);
-    RAJNI_REQUIRE(keep <= N - 1, RAJNI_ERANGE, "selected index k out of range (keep=%d, patches=%d)", keep, N - 1);
-    ScoreSelectParams p{};
-    p.scores_in = scores;
-    p.keep_idx = keep_idx; p.next_scores = next_scores; p.row_map = row_map;
-    p.N = N; p.C = 0; p.H = 0; p.keep = keep; p.eps = 0.f;
-    return launch_score_select(p, B, static_cast<cudaStream_t>(stream));
+    return select_prefix("rajni_select", scores, B, N, 1, keep, keep_idx, next_scores, row_map, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int rajni_score_select_prefix(const void* qkv, int B, int N, int C, int H, int prefix, int keep, float eps,
+                                         float* scores, int32_t* keep_idx, float* next_scores, int32_t* row_map,
+                                         void* workspace, size_t workspace_bytes, void* stream) {
+    return score_select_prefix("rajni_score_select_prefix", qkv, B, N, C, H, prefix, keep, eps, scores, keep_idx, next_scores,
+                               row_map, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
 }
 
 extern "C" int rajni_score_select(const void* qkv, int B, int N, int C, int H, int keep, float eps,
                                   float* scores, int32_t* keep_idx, float* next_scores,
                                   int32_t* row_map, void* stream) {
-    RAJNI_REQUIRE(qkv && keep_idx && next_scores, RAJNI_EINVAL, "rajni_score_select: null pointer");
-    if (int rc = check_score_shape(B, N, C, H)) return rc;
-    RAJNI_REQUIRE(keep >= 1, RAJNI_EINVAL, "rajni_score_select: keep=%d < 1", keep);
-    RAJNI_REQUIRE(keep <= N - 1, RAJNI_ERANGE, "selected index k out of range (keep=%d, patches=%d)", keep, N - 1);
-    ScoreSelectParams p{};
-    p.qkv = static_cast<const __nv_bfloat16*>(qkv);
-    p.scores_out = scores;
-    p.keep_idx = keep_idx; p.next_scores = next_scores; p.row_map = row_map;
-    p.N = N; p.C = C; p.H = H; p.keep = keep; p.eps = eps;
-    return launch_score_select(p, B, static_cast<cudaStream_t>(stream));
+    RAJNI_REQUIRE(keep_idx, RAJNI_EINVAL, "rajni_score_select: null pointer");
+    return score_select_prefix("rajni_score_select", qkv, B, N, C, H, 1, keep, eps, scores, keep_idx, next_scores, row_map,
+                               nullptr, 0, static_cast<cudaStream_t>(stream));
 }
 
 extern "C" size_t rajni_score_select_workspace_bytes(int B, int N, int C, int H) {
@@ -652,29 +700,9 @@ extern "C" size_t rajni_score_select_workspace_bytes(int B, int N, int C, int H)
 extern "C" int rajni_score_select_split(const void* qkv, int B, int N, int C, int H, int keep, float eps,
                                         float* scores, int32_t* keep_idx, float* next_scores, int32_t* row_map,
                                         void* workspace, size_t workspace_bytes, void* stream) {
-    RAJNI_REQUIRE(qkv && workspace && (keep_idx ? next_scores != nullptr : scores != nullptr), RAJNI_EINVAL,
-                  "rajni_score_select_split: null pointer");
-    if (int rc = check_score_shape(B, N, C, H)) return rc;
-    if (keep_idx != nullptr) {
-        RAJNI_REQUIRE(keep >= 1, RAJNI_EINVAL, "rajni_score_select_split: keep=%d < 1", keep);
-        RAJNI_REQUIRE(keep <= N - 1, RAJNI_ERANGE, "selected index k out of range (keep=%d, patches=%d)", keep, N - 1);
-    }
-    RAJNI_REQUIRE(B <= 65535, RAJNI_EINVAL, "rajni_score_select_split: B=%d exceeds the grid limit", B);
-    RAJNI_REQUIRE(workspace_bytes >= rajni_score_select_workspace_bytes(B, N, C, H) && (reinterpret_cast<uintptr_t>(workspace) & 15) == 0,
-                  RAJNI_EINVAL, "rajni_score_select_split: workspace too small (%zu B) or not 16-byte aligned", workspace_bytes);
-    float* ws = static_cast<float*>(workspace);
-    auto s = static_cast<cudaStream_t>(stream);
-    if (int rc = launch_score_stream(static_cast<const __nv_bfloat16*>(qkv), B, N, C, H, ws, s)) return rc;
-    ScoreSelectParams p{};
-    p.qkv = static_cast<const __nv_bfloat16*>(qkv);
-    p.scores_out = scores;
-    p.keep_idx = keep_idx; p.next_scores = next_scores; p.row_map = row_map;
-    p.pre_logit = ws;
-    p.pre_vm = ws + (size_t)B * (((size_t)H * N + 3) & ~(size_t)3);
-    p.N = N; p.C = C; p.H = H; p.keep = keep_idx ? keep : 0; p.eps = eps;
-    // RAJNI_SCORE_WS_TAIL=1 (read per call; tests): the long-sequence tail at any N, to compare it with the shared-memory one
-    if (needs_workspace_tail(N, H) || getenv("RAJNI_SCORE_WS_TAIL") != nullptr) return launch_score_tail_ws(p, ws, B, s);
-    return launch_score_select(p, B, s);
+    RAJNI_REQUIRE(workspace, RAJNI_EINVAL, "rajni_score_select_split: null pointer");
+    return score_select_prefix("rajni_score_select_split", qkv, B, N, C, H, 1, keep, eps, scores, keep_idx, next_scores, row_map,
+                               workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
 }
 
 extern "C" int rajni_score_select_needs_workspace(int N, int H) {

@@ -73,10 +73,19 @@ def _bf16c(t: torch.Tensor) -> torch.Tensor:
     return t
 
 
-def importance(qkv: torch.Tensor, num_heads: int, eps: float = 1e-6, workspace: Optional[torch.Tensor] = None) -> torch.Tensor:
+def _check_prefix(prefix: int) -> int:
+    if prefix not in (1, 2):
+        raise ValueError(f"prefix={prefix}: 1 (CLS) or 2 (CLS + distillation token) leading tokens are supported")
+    return prefix
+
+
+def importance(qkv: torch.Tensor, num_heads: int, eps: float = 1e-6, workspace: Optional[torch.Tensor] = None,
+               prefix: int = 1) -> torch.Tensor:
     """qkv [B,N,3C] bf16 -> scores [B,N] fp32.   importance.py:5-34
     Sequences too long for the one-launch kernel (``needs_score_workspace``) go through the split entry with scratch
-    (``workspace`` as in ``score_select``)."""
+    (``workspace`` as in ``score_select``).  ``prefix`` (1 or 2 leading tokens) does not change the scores: the query is
+    row 0 and every token, a distillation token too, is a key and value."""
+    _check_prefix(prefix)
     _bf16c(qkv)
     B, N, C3 = qkv.shape
     C = C3 // 3
@@ -92,17 +101,20 @@ def importance(qkv: torch.Tensor, num_heads: int, eps: float = 1e-6, workspace: 
     return scores
 
 
-def select(scores: torch.Tensor, keep: int, keep_idx=None, next_scores=None, row_map=None
+def select(scores: torch.Tensor, keep: int, keep_idx=None, next_scores=None, row_map=None, prefix: int = 1
            ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
-    """scores [B,N] fp32 -> (keep_idx int32 [B,keep+1], next_scores fp32, row_map int32 [B*(keep+1)])."""
+    """scores [B,N] fp32 -> (keep_idx int32 [B,keep+prefix], next_scores fp32, row_map int32 [B*(keep+prefix)]).
+    The first ``prefix`` tokens (CLS, or CLS + distillation token) are always kept; the top ``keep`` of the rest follow."""
     if scores.dtype != torch.float32 or not scores.is_contiguous():
         raise ValueError("scores must be contiguous fp32")
+    _check_prefix(prefix)
     B, N = scores.shape
     dev = scores.device
-    keep_idx = torch.empty((B, keep + 1), device=dev, dtype=torch.int32) if keep_idx is None else keep_idx
-    next_scores = torch.empty((B, keep + 1), device=dev, dtype=torch.float32) if next_scores is None else next_scores
-    row_map = torch.empty((B * (keep + 1),), device=dev, dtype=torch.int32) if row_map is None else row_map
-    _call("select", B * (4 * N + 12 * (keep + 1)), _lib.load().rajni_select, scores.data_ptr(), B, N, keep,
+    Np = keep + prefix
+    keep_idx = torch.empty((B, Np), device=dev, dtype=torch.int32) if keep_idx is None else keep_idx
+    next_scores = torch.empty((B, Np), device=dev, dtype=torch.float32) if next_scores is None else next_scores
+    row_map = torch.empty((B * Np,), device=dev, dtype=torch.int32) if row_map is None else row_map
+    _call("select", B * (4 * N + 12 * Np), _lib.load().rajni_select_prefix, scores.data_ptr(), B, N, prefix, keep,
           keep_idx.data_ptr(), next_scores.data_ptr(), row_map.data_ptr(), _stream(scores))
     return keep_idx, next_scores, row_map
 
@@ -145,33 +157,32 @@ def _checked_score_workspace(dev: torch.device, B: int, N: int, C: int, num_head
 
 def score_select(qkv: torch.Tensor, num_heads: int, keep: int, eps: float = 1e-6, want_scores: bool = False,
                  keep_idx=None, next_scores=None, row_map=None, scores=None, split: Optional[bool] = None,
-                 workspace: Optional[torch.Tensor] = None):
+                 workspace: Optional[torch.Tensor] = None, prefix: int = 1):
     """Fused importance + selection on qkv [B,N,3C] bf16.
-    Returns (scores or None, keep_idx, next_scores, row_map).
+    Returns (scores or None, keep_idx [B,keep+prefix], next_scores, row_map); ``prefix`` as in ``select``.
     ``workspace``: uint8 scratch of at least ``score_workspace_bytes(B, N, C, H)`` for the split path (small batches, and
     every batch of a sequence for which ``needs_score_workspace``); a caller that replays CUDA graphs must pass one it owns,
     so that the captured address lives as long as the graph."""
     _bf16c(qkv)
+    _check_prefix(prefix)
     B, N, C3 = qkv.shape
     dev = qkv.device
+    Np = keep + prefix
     if want_scores and scores is None:
         scores = torch.empty((B, N), device=dev, dtype=torch.float32)
-    keep_idx = torch.empty((B, keep + 1), device=dev, dtype=torch.int32) if keep_idx is None else keep_idx
-    next_scores = torch.empty((B, keep + 1), device=dev, dtype=torch.float32) if next_scores is None else next_scores
-    row_map = torch.empty((B * (keep + 1),), device=dev, dtype=torch.int32) if row_map is None else row_map
+    keep_idx = torch.empty((B, Np), device=dev, dtype=torch.int32) if keep_idx is None else keep_idx
+    next_scores = torch.empty((B, Np), device=dev, dtype=torch.float32) if next_scores is None else next_scores
+    row_map = torch.empty((B * Np,), device=dev, dtype=torch.int32) if row_map is None else row_map
     C = C3 // 3
     lib = _lib.load()
     if split is None:
         split = B <= SPLIT_SCORE_MAX_BATCH or needs_score_workspace(N, num_heads)
     # algorithmic bytes (SURVEY 8d): K and V planes + CLS query in, index + carried score out
-    work = B * (2 * N * C * 2 + C * 2 + 8 * (keep + 1))
-    if split:
-        ws = _checked_score_workspace(dev, B, N, C, num_heads, workspace)
-        _call("score_select", work, lib.rajni_score_select_split, qkv.data_ptr(), B, N, C, num_heads, keep, eps, _ptr(scores),
-              keep_idx.data_ptr(), next_scores.data_ptr(), row_map.data_ptr(), ws.data_ptr(), ws.numel(), _stream(qkv))
-    else:
-        _call("score_select", work, lib.rajni_score_select, qkv.data_ptr(), B, N, C, num_heads, keep, eps, _ptr(scores),
-              keep_idx.data_ptr(), next_scores.data_ptr(), row_map.data_ptr(), _stream(qkv))
+    work = B * (2 * N * C * 2 + C * 2 + 8 * Np)
+    ws = _checked_score_workspace(dev, B, N, C, num_heads, workspace) if split else None
+    _call("score_select", work, lib.rajni_score_select_prefix, qkv.data_ptr(), B, N, C, num_heads, prefix, keep, eps,
+          _ptr(scores), keep_idx.data_ptr(), next_scores.data_ptr(), row_map.data_ptr(), _ptr(ws),
+          0 if ws is None else ws.numel(), _stream(qkv))
     return scores, keep_idx, next_scores, row_map
 
 
@@ -186,12 +197,18 @@ def gather_rows(src: torch.Tensor, row_map: torch.Tensor, out: Optional[torch.Te
 
 
 def layernorm(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps: float, rows: int, C: int,
-              in_row_stride: Optional[int] = None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """Row LayerNorm, bf16 -> bf16; row r read at x.data_ptr + r*in_row_stride elements."""
+              in_row_stride: Optional[int] = None, out: Optional[torch.Tensor] = None, in_offset: int = 0,
+              out_row_stride: Optional[int] = None, out_offset: int = 0) -> torch.Tensor:
+    """Row LayerNorm, bf16 -> bf16; row r read at x.data_ptr + in_offset + r*in_row_stride elements and written at
+    out.data_ptr + out_offset + r*out_row_stride (default C: dense rows)."""
     out = torch.empty((rows, C), device=x.device, dtype=torch.bfloat16) if out is None else out
-    _call("layernorm", rows * C * 4, _lib.load().rajni_layernorm, x.data_ptr(),
-          C if in_row_stride is None else in_row_stride, gamma.data_ptr(), beta.data_ptr(), eps, out.data_ptr(),
-          rows, C, _stream(x))
+    stride = C if in_row_stride is None else in_row_stride
+    ostride = C if out_row_stride is None else out_row_stride
+    if in_offset + (rows - 1) * stride + C > x.numel() or out_offset + (rows - 1) * ostride + C > out.numel():
+        raise ValueError(f"layernorm: {rows} rows (strides {stride} / {ostride}, offsets {in_offset} / {out_offset}) exceed "
+                         f"the input ({x.numel()}) or output ({out.numel()} elements)")
+    _call("layernorm", rows * C * 4, _lib.load().rajni_layernorm_strided, x.data_ptr() + 2 * in_offset, stride,
+          gamma.data_ptr(), beta.data_ptr(), eps, out.data_ptr() + 2 * out_offset, ostride, rows, C, _stream(x))
     return out
 
 
@@ -283,10 +300,12 @@ _IMG_DTYPES = {torch.bfloat16: 0, torch.float32: 1, torch.uint8: 2}      # RAJNI
 
 def patch_im2col(images: torch.Tensor, patch: int, cols: torch.Tensor, cls_pos0: torch.Tensor,
                  x: torch.Tensor, C: int, row_stats: Optional[torch.Tensor] = None, stats_slots: int = 0,
-                 cls_sum: float = 0.0, cls_sumsq: float = 0.0, norm: Optional[tuple] = None) -> None:
+                 cls_sum=0.0, cls_sumsq=0.0, norm: Optional[tuple] = None, prefix: int = 1) -> None:
     """images [B,3,S,S] fp32|bf16|uint8 -> cols [B*P, 3*p*p] bf16; also writes the CLS rows of x (and their
     LayerNorm partial sums into row_stats fp32 [slots, rows, 2]).  uint8 pixels are normalised in the kernel with
-    ``norm = (mean[3], std[3])`` exactly as ToTensor + Normalize do in fp32 (run.py:62-70)."""
+    ``norm = (mean[3], std[3])`` exactly as ToTensor + Normalize do in fp32 (run.py:62-70).
+    ``prefix`` = 2 (CLS + distillation token): x is [B, P+2, C], ``cls_pos0`` is the [2, C] block of the two prefix rows
+    and ``cls_sum`` / ``cls_sumsq`` are sequences of two, one per row."""
     if images.dtype not in _IMG_DTYPES or not images.is_contiguous():
         raise ValueError("images must be contiguous fp32, bf16 or uint8")
     norm_arr = None
@@ -297,10 +316,18 @@ def patch_im2col(images: torch.Tensor, patch: int, cols: torch.Tensor, cls_pos0:
     B, ch, S, S2 = images.shape
     if ch != 3 or S != S2:
         raise ValueError(f"images must be [B,3,S,S], got {tuple(images.shape)}")
-    _call("patch_im2col", images.numel() * images.element_size() + images.numel() * 2 + B * C * 2,
-          _lib.load().rajni_patch_im2col, images.data_ptr(), _IMG_DTYPES[images.dtype], B, S, patch,
-          cols.data_ptr(), cls_pos0.data_ptr(), x.data_ptr(), C, _ptr(row_stats),
-          0 if row_stats is None else row_stats.shape[1], stats_slots, cls_sum, cls_sumsq, norm_arr, _stream(images))
+    _check_prefix(prefix)
+    if cls_pos0.dtype != torch.bfloat16 or not cls_pos0.is_contiguous() or cls_pos0.numel() != prefix * C:
+        raise ValueError(f"cls_pos0 must be {prefix} contiguous bf16 row(s) of {C}")
+    sums = [float(v) for v in (cls_sum if prefix > 1 else [cls_sum])]
+    sqs = [float(v) for v in (cls_sumsq if prefix > 1 else [cls_sumsq])]
+    if len(sums) != prefix or len(sqs) != prefix:
+        raise ValueError(f"cls_sum and cls_sumsq need one value per prefix row ({prefix})")
+    stats_arr = (ctypes.c_float * (2 * prefix))(*[v for pair in zip(sums, sqs) for v in pair])
+    _call("patch_im2col", images.numel() * images.element_size() + images.numel() * 2 + B * prefix * C * 2,
+          _lib.load().rajni_patch_im2col_prefix, images.data_ptr(), _IMG_DTYPES[images.dtype], B, S, patch,
+          cols.data_ptr(), cls_pos0.data_ptr(), prefix, x.data_ptr(), C, _ptr(row_stats),
+          0 if row_stats is None else row_stats.shape[1], stats_slots, stats_arr, norm_arr, _stream(images))
 
 
 def resize_center_crop(frames: torch.Tensor, meta: torch.Tensor, max_h: int, size: int = 256, crop: int = 224,

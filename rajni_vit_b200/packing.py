@@ -59,6 +59,24 @@ class PackCache:
         self._store[key] = (sig, packed)
         return packed
 
+    def linear_ls(self, lin: nn.Module, ls: nn.Module) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
+        """LayerScale folded into the Linear that feeds the residual (DeiT-III's ls1 after proj, ls2 after fc2):
+        x + gamma*(W a + b) = x + (gamma[:,None]*W) a + gamma*b  ->  (bf16(gamma[:,None]*W) [N,K], fp32 gamma*b [N] or None).
+        The product is rounded to bf16 once; bf16 keeps its relative precision down to ~1e-38, so a gamma of 1e-6 costs no
+        more than the weights' own rounding."""
+        sig = _sig(lin.weight, getattr(lin, "bias", None), ls.gamma)
+        key = (id(lin), "ls")
+        hit = self._store.get(key)
+        if hit is not None and hit[0] == sig:
+            return hit[1]
+        gamma = ls.gamma.detach().to(torch.float32)
+        w = lin.weight.detach().to(torch.float32)
+        b = getattr(lin, "bias", None)
+        packed = ((w * gamma[:, None]).to(torch.bfloat16).contiguous(),
+                  None if b is None else (b.detach().to(torch.float32) * gamma).contiguous())
+        self._store[key] = (sig, packed)
+        return packed
+
     def norm(self, m: nn.LayerNorm) -> Tuple[torch.Tensor, torch.Tensor, float]:
         sig = _sig(m.weight, m.bias)
         hit = self._store.get(id(m))

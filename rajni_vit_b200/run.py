@@ -37,7 +37,9 @@ def get_args(argv=None):
     ap.add_argument("--batch_size", type=int, default=256)
     ap.add_argument("--num_workers", type=int, default=8)
     ap.add_argument("--pin_mem", action="store_true", default=True)
-    ap.add_argument("--model", type=str, default="vit_base_patch16_224", help="timm model name")
+    ap.add_argument("--model", type=str, default="vit_base_patch16_224",
+                    help="timm model name; without timm, a stand-in of vit.VIT_CONFIGS (e.g. vit_base_patch16_224, "
+                         "deit3_base_patch16_224, deit_base_distilled_patch16_224)")
     ap.add_argument("--device", type=str, default="cuda")
     ap.add_argument("--schedule", type=str, default=None, help="JSON file with the RAJNI pruning schedule")
     ap.add_argument("--warmup", type=int, default=5)

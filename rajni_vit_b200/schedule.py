@@ -34,14 +34,15 @@ def flops_per_image(token_counts: Sequence[int], C: int, hidden: int, patches: i
     return total
 
 
-def token_counts(schedule: Schedule, depth: int, tokens: int) -> List[int]:
-    """Tokens entering each block: block i listed in the schedule keeps max(1, int(r * (N - 1))) patches + CLS
-    (attention.py:31-32), and the kept tokens are what the block's own attention and MLP run on."""
+def token_counts(schedule: Schedule, depth: int, tokens: int, prefix: int = 1) -> List[int]:
+    """Tokens entering each block: block i listed in the schedule keeps max(1, int(r * (N - prefix))) patches + the
+    ``prefix`` leading tokens (attention.py:31-32; prefix 2 for a distilled DeiT's CLS + distillation token), and the kept
+    tokens are what the block's own attention and MLP run on."""
     out, n = [], tokens
     for i in range(depth):
         out.append(n)
         if i in schedule:
-            n = max(1, int(float(schedule[i].get("keep_ratio", 1.0)) * (n - 1))) + 1
+            n = max(1, int(float(schedule[i].get("keep_ratio", 1.0)) * (n - prefix))) + prefix
     return out
 
 

@@ -13,6 +13,14 @@ those attribute names and timm's ViT semantics:
                 mlp{fc1, act=GELU(erf), fc2}, ls1/ls2/drop_path1/drop_path2 = Identity
     norm, head
 
+and the two DeiT families (extra fields in VIT_VARIANT):
+
+    DeiT-III (``deit3_*``): ls1/ls2 = LayerScale (``gamma`` [C]), and no position for the class token
+        (timm's ``no_embed_class``: pos_embed [1,P,C] is added to the patches before the class token is prepended);
+    distilled DeiT (``deit_*_distilled_*``): a distillation token after the class token (``dist_token``,
+        ``num_prefix_tokens = 2``, pos_embed [1,2+P,C]) and a second head ``head_dist`` on it; in eval mode the output is
+        ``(head(x[:,0]) + head_dist(x[:,1])) / 2``.
+
 It is a plain eager PyTorch module.  It is NOT on the accelerated path: the
 B200 wrapper reads its leaf parameters and runs its own kernels.
 """
@@ -38,11 +46,29 @@ VIT_CONFIGS = {
     "vit_micro_patch16_64": (128, 4, 2, 64),
     "vit_micro_patch8_72": (128, 4, 2, 72),
     "vit_micro_patch32_128": (128, 4, 2, 128),
+    # DeiT-III (LayerScale, class token without a position) and distilled DeiT (class + distillation token, two heads)
+    "deit3_small_patch16_224": (384, 12, 6, 224),
+    "deit3_medium_patch16_224": (512, 12, 8, 224),
+    "deit3_base_patch16_224": (768, 12, 12, 224),
+    "deit3_large_patch16_224": (1024, 24, 16, 224),
+    "deit3_base_patch16_384": (768, 12, 12, 384),
+    "deit_tiny_distilled_patch16_224": (192, 12, 3, 224),
+    "deit_small_distilled_patch16_224": (384, 12, 6, 224),
+    "deit_base_distilled_patch16_224": (768, 12, 12, 224),
+    "deit_base_distilled_patch16_384": (768, 12, 12, 384),
+    # 4-block test models of the two families: 16 + 1 and 16 + 2 tokens
+    "deit3_micro_patch16_64": (128, 4, 2, 64),
+    "deit_micro_distilled_patch16_64": (128, 4, 2, 64),
 }
 # name -> patch size (pixels per side of a patch; 50 tokens at 224 px for 32, 785 for 8)
 VIT_PATCH = {name: 16 for name in VIT_CONFIGS}
 VIT_PATCH.update({"vit_small_patch32_224": 32, "vit_base_patch32_224": 32, "vit_micro_patch32_128": 32,
                   "vit_small_patch8_224": 8, "vit_base_patch8_224": 8, "vit_micro_patch8_72": 8})
+# name -> extra VisionTransformer arguments of the DeiT families (timm's deit3_* use init_values=1e-6 and no_embed_class;
+# create_model spreads the LayerScale gammas, see spread_layer_scale)
+_DEIT3 = dict(init_values=1e-6, no_embed_class=True)
+VIT_VARIANT = {name: dict(_DEIT3) for name in VIT_CONFIGS if name.startswith("deit3_")}
+VIT_VARIANT.update({name: dict(distilled=True) for name in VIT_CONFIGS if "_distilled_" in name})
 
 
 class PatchEmbed(nn.Module):
@@ -97,16 +123,27 @@ class Mlp(nn.Module):
         return self.drop2(self.fc2(self.norm(self.drop1(self.act(self.fc1(x))))))
 
 
+class LayerScale(nn.Module):
+    """timm's LayerScale: x * gamma, gamma [C] learnt per channel (DeiT-III, CaiT)."""
+
+    def __init__(self, dim, init_values=1e-5):
+        super().__init__()
+        self.gamma = nn.Parameter(init_values * torch.ones(dim))
+
+    def forward(self, x):
+        return x * self.gamma
+
+
 class Block(nn.Module):
-    def __init__(self, dim, num_heads, mlp_ratio=4.0):
+    def __init__(self, dim, num_heads, mlp_ratio=4.0, init_values=None):
         super().__init__()
         self.norm1 = nn.LayerNorm(dim, eps=1e-6)
         self.attn = Attention(dim, num_heads)
-        self.ls1 = nn.Identity()
+        self.ls1 = LayerScale(dim, init_values) if init_values else nn.Identity()
         self.drop_path1 = nn.Identity()
         self.norm2 = nn.LayerNorm(dim, eps=1e-6)
         self.mlp = Mlp(dim, int(dim * mlp_ratio))
-        self.ls2 = nn.Identity()
+        self.ls2 = LayerScale(dim, init_values) if init_values else nn.Identity()
         self.drop_path2 = nn.Identity()
 
     def forward(self, x):
@@ -116,37 +153,54 @@ class Block(nn.Module):
 
 
 class VisionTransformer(nn.Module):
+    """``init_values``: LayerScale after attention and MLP (None: Identity).  ``no_embed_class``: pos_embed covers the patches
+    only.  ``distilled``: a distillation token and ``head_dist`` (timm's VisionTransformerDistilled, eval-mode output)."""
+
     def __init__(self, img_size=224, patch_size=16, in_chans=3, num_classes=1000,
-                 embed_dim=768, depth=12, num_heads=12, mlp_ratio=4.0):
+                 embed_dim=768, depth=12, num_heads=12, mlp_ratio=4.0, init_values=None, no_embed_class=False,
+                 distilled=False):
         super().__init__()
         self.num_classes = num_classes
         self.embed_dim = self.num_features = embed_dim
         self.global_pool = "token"
-        self.num_prefix_tokens = 1
+        self.num_prefix_tokens = 2 if distilled else 1
+        self.no_embed_class = no_embed_class
         self.patch_embed = PatchEmbed(img_size, patch_size, in_chans, embed_dim)
-        n_tok = self.patch_embed.num_patches + 1
+        n_tok = self.patch_embed.num_patches + (0 if no_embed_class else self.num_prefix_tokens)
         self.cls_token = nn.Parameter(torch.zeros(1, 1, embed_dim))
+        self.dist_token = nn.Parameter(torch.zeros(1, 1, embed_dim)) if distilled else None
         self.pos_embed = nn.Parameter(torch.zeros(1, n_tok, embed_dim))
         self.pos_drop = nn.Dropout(0.0)
         self.patch_drop = nn.Identity()
         self.norm_pre = nn.Identity()
-        self.blocks = nn.Sequential(*[Block(embed_dim, num_heads, mlp_ratio) for _ in range(depth)])
+        self.blocks = nn.Sequential(*[Block(embed_dim, num_heads, mlp_ratio, init_values) for _ in range(depth)])
         self.norm = nn.LayerNorm(embed_dim, eps=1e-6)
         self.fc_norm = nn.Identity()
         self.head_drop = nn.Dropout(0.0)
         self.head = nn.Linear(embed_dim, num_classes)
+        self.head_dist = nn.Linear(embed_dim, num_classes) if distilled else None
         nn.init.normal_(self.cls_token, std=0.02)
         nn.init.normal_(self.pos_embed, std=0.02)
+        if distilled:
+            nn.init.normal_(self.dist_token, std=0.02)
+
+    def _pos_embed(self, x):
+        prefix = [self.cls_token.expand(x.shape[0], -1, -1)]
+        if self.dist_token is not None:
+            prefix.append(self.dist_token.expand(x.shape[0], -1, -1))
+        if self.no_embed_class:                                 # timm: positions for the patches only, tokens prepended after
+            return self.pos_drop(torch.cat(prefix + [x + self.pos_embed], dim=1))
+        return self.pos_drop(torch.cat(prefix + [x], dim=1) + self.pos_embed)
 
     def forward_features(self, x):
-        x = self.patch_embed(x)
-        x = torch.cat([self.cls_token.expand(x.shape[0], -1, -1), x], dim=1)
-        x = self.pos_drop(x + self.pos_embed)
+        x = self._pos_embed(self.patch_embed(x))
         x = self.blocks(self.norm_pre(self.patch_drop(x)))
         return self.norm(x)
 
     def forward(self, x):
         x = self.forward_features(x)
+        if self.head_dist is not None:                          # timm VisionTransformerDistilled, eval mode
+            return (self.head(self.head_drop(x[:, 0])) + self.head_dist(self.head_drop(x[:, 1]))) / 2
         return self.head(self.head_drop(self.fc_norm(x[:, 0])))
 
 
@@ -162,15 +216,34 @@ def create_model(name: str, seed: int | None = 0, bf16_round: bool = True,
     if seed is not None:
         gen_state = torch.random.get_rng_state()
         torch.manual_seed(seed)
+    variant = VIT_VARIANT.get(name, {})
     model = VisionTransformer(img_size=img, patch_size=VIT_PATCH[name], embed_dim=dim, depth=depth, num_heads=heads,
-                              num_classes=num_classes)
+                              num_classes=num_classes, **variant)
     if seed is not None:
         torch.random.set_rng_state(gen_state)
+    if variant.get("init_values"):
+        spread_layer_scale(model, seed=0 if seed is None else seed, bf16_round=False)
     if bf16_round:
         with torch.no_grad():
             for p in model.parameters():
                 p.copy_(p.to(torch.bfloat16).to(torch.float32))
     return model.eval()
+
+
+def spread_layer_scale(model: VisionTransformer, seed: int = 0, lo: float = 1e-6, hi: float = 1.0,
+                       bf16_round: bool = True) -> VisionTransformer:
+    """Give every LayerScale gamma values spread log-uniformly over [lo, hi] (DeiT-III's trained gammas range from its
+    1e-6 init to O(1)); a constant gamma would leave the per-channel fold untested.  Own generator: the other parameters
+    are not touched."""
+    g = torch.Generator().manual_seed(1000 + seed)
+    lo_, hi_ = torch.log(torch.tensor(lo)), torch.log(torch.tensor(hi))
+    with torch.no_grad():
+        for name, p in model.named_parameters():
+            if name.endswith(".gamma"):
+                p.copy_(torch.exp(lo_ + (hi_ - lo_) * torch.rand(p.shape, generator=g)))
+                if bf16_round:
+                    p.copy_(p.to(torch.bfloat16).to(torch.float32))
+    return model
 
 
 def randomize_trained_like(model: VisionTransformer, seed: int = 0, outlier_channels: int = 4, outlier_scale: float = 20.0,

@@ -10,10 +10,11 @@ from .. import ops
 from ..packing import PackCache
 
 
-def keep_count(num_tokens: int, keep_ratio: float) -> int:
-    """Patches kept out of ``num_tokens - 1``: Python double multiply, truncation, floor of 1
-    (rajni/wrapper/attention.py:31-32)."""
-    return max(1, int(keep_ratio * (num_tokens - 1)))
+def keep_count(num_tokens: int, keep_ratio: float, prefix: int = 1) -> int:
+    """Patches kept out of ``num_tokens - prefix``: Python double multiply, truncation, floor of 1
+    (rajni/wrapper/attention.py:31-32).  ``prefix``: the leading tokens that are always kept (1: CLS; 2: CLS and the
+    distillation token of a distilled DeiT)."""
+    return max(1, int(keep_ratio * (num_tokens - prefix)))
 
 
 class RAJNIAttention(nn.Module):
@@ -22,7 +23,8 @@ class RAJNIAttention(nn.Module):
     Same constructor, attributes and return contract as the reference:
     ``forward(x[B,N,C], prev_scores=None) -> (out[B,Np,C], keep_idx[B,Np] int64, next_scores[B,Np])``.
     Shares (does not copy) the wrapped attention's ``qkv`` / ``proj`` modules
-    (attention.py:10-11).
+    (attention.py:10-11).  ``num_prefix_tokens`` (set by RAJNIViTWrapper from its base model) leading tokens are always
+    kept: Np = keep + num_prefix_tokens.
     """
 
     def __init__(self, attn: nn.Module, keep_ratio: float, update: bool):
@@ -34,6 +36,7 @@ class RAJNIAttention(nn.Module):
         self.proj_drop = attn.proj_drop
         self.keep_ratio = keep_ratio
         self.update = update
+        self.num_prefix_tokens = 1
         for name in ("q_norm", "k_norm"):
             sub = getattr(attn, name, None)
             if sub is not None and not isinstance(sub, nn.Identity):
@@ -59,18 +62,19 @@ class RAJNIAttention(nn.Module):
         qw, qb = self._packs.linear(self.qkv)
         pw, pb = self._packs.linear(self.proj)
         qkv = ops.gemm(xn, qw, qb, B * N, 3 * C, C)                                   # attention.py:22
-        keep = keep_count(N, self.keep_ratio)
-        if keep > N - 1:
+        P0 = self.num_prefix_tokens
+        keep = keep_count(N, self.keep_ratio, P0)
+        if keep > N - P0:
             raise RuntimeError("selected index k out of range")                       # torch.topk's error, attention.py:35
         scores = None
         if self.update or prev_scores is None:                                        # attention.py:25-28
             scores, keep_idx, next_scores, row_map = ops.score_select(
-                qkv.view(B, N, 3 * C), H, keep, want_scores=want_scores)
+                qkv.view(B, N, 3 * C), H, keep, want_scores=want_scores, prefix=P0)
         else:
             scores = prev_scores.detach().to(torch.float32).contiguous()
-            keep_idx, next_scores, row_map = ops.select(scores, keep)
-        att = ops.attention(qkv, row_map, B, N, keep + 1, C, H, float(self.scale))    # attention.py:42-54
-        out = ops.gemm(att, pw, pb, B * (keep + 1), C, C)                             # attention.py:55
+            keep_idx, next_scores, row_map = ops.select(scores, keep, prefix=P0)
+        att = ops.attention(qkv, row_map, B, N, keep + P0, C, H, float(self.scale))   # attention.py:42-54
+        out = ops.gemm(att, pw, pb, B * (keep + P0), C, C)                            # attention.py:55
         return out, keep_idx, next_scores, row_map, scores
 
     @torch.no_grad()

@@ -12,6 +12,10 @@ Deliberate deviations from the reference (SURVEY.md section 5):
   * activations are bf16 with fp32 accumulation, scores are fp32;
   * ties in the top-k are broken by lower index (torch.topk leaves it undefined);
   * unsupported base models raise instead of silently diverging.
+
+Beyond the reference's models it runs the two DeiT families: LayerScale (DeiT-III's ``ls1`` / ``ls2``, folded into the
+proj / fc2 weights), a class token without a position (``no_embed_class``), and a distillation token (distilled DeiT:
+two prefix tokens, always kept, and the eval-mode average of ``head`` and ``head_dist``).
 """
 from __future__ import annotations
 
@@ -43,6 +47,14 @@ def _is_identity(m) -> bool:
     return m is None or isinstance(m, nn.Identity) or (isinstance(m, nn.Dropout) and m.p == 0.0)
 
 
+def _is_layer_scale(m, C: int) -> bool:
+    """timm's LayerScale (x * gamma): a module of that name whose only parameter is ``gamma`` [C] and that holds nothing else."""
+    if type(m).__name__ != "LayerScale" or list(m.children()) or list(m.buffers()):
+        return False
+    params = dict(m.named_parameters())
+    return list(params) == ["gamma"] and tuple(params["gamma"].shape) == (C,)
+
+
 AUTO_GRAPH_MAX_ROWS = 16384       # batch x tokens up to which forward() replays a CUDA graph by default
 
 
@@ -71,6 +83,8 @@ class RAJNIViTWrapper(nn.Module):
         # None = automatic: replay a captured CUDA graph when the batch is small enough to be launch-bound
         env = os.environ.get("RAJNI_CUDA_GRAPH", "")
         self.use_cuda_graph: Optional[bool] = None if env == "" else env != "0"
+        self.prefix = 1                  # leading tokens that are always kept (set by _validate: 2 for a distilled DeiT)
+        self.no_embed_class = False      # pos_embed covers the patches only (DeiT-III)
         self.input_norm: Optional[tuple] = None       # (mean[3], std[3]) for uint8 images, see set_input_normalization
         # Stream-K tail of the fc2 GEMMs (gemm_tcgen05.cu): +1.4 % at 32 images per GPU, nothing at 64 and above.  OFF by default
         # because the fp32 summation order of a split tile depends on the tile count, i.e. on the batch size: without it an
@@ -111,8 +125,33 @@ class RAJNIViTWrapper(nn.Module):
         if not isinstance(m.norm, nn.LayerNorm) or not isinstance(m.head, nn.Linear):
             raise NotImplementedError("norm must be LayerNorm and head must be Linear")
         C = proj.out_channels
+        # prefix tokens: CLS, or CLS + distillation token (distilled DeiT); register tokens are not supported
+        if getattr(m, "cls_token", None) is None:
+            raise NotImplementedError("a class token (cls_token) is required")
+        if getattr(m, "reg_token", None) is not None or getattr(m, "num_reg_tokens", 0):
+            raise NotImplementedError("register tokens (reg_token) are not supported")
+        dist, head_dist = getattr(m, "dist_token", None), getattr(m, "head_dist", None)
+        prefix = int(getattr(m, "num_prefix_tokens", 1))
+        if dist is not None:
+            if not isinstance(head_dist, nn.Linear) or head_dist.weight.shape != m.head.weight.shape:
+                raise NotImplementedError("a dist_token needs head_dist, a Linear of the head's shape")
+            if prefix != 2:
+                raise NotImplementedError(f"num_prefix_tokens = {prefix} with a dist_token: expected 2 (CLS + distillation)")
+            if getattr(m, "distilled_training", False):
+                raise NotImplementedError("distilled_training (the (x, x_dist) training output) is not supported")
+        elif head_dist is not None and not _is_identity(head_dist):
+            raise NotImplementedError("head_dist without a dist_token is not supported")
+        elif prefix != 1:
+            raise NotImplementedError(f"num_prefix_tokens = {prefix}: only CLS (1) or CLS + dist_token (2) are supported")
+        self.prefix = prefix
+        self.no_embed_class = bool(getattr(m, "no_embed_class", False))
         for i, blk in enumerate(self.blocks):
-            for name in ("ls1", "ls2", "drop_path1", "drop_path2"):
+            for name in ("ls1", "ls2"):
+                ls = getattr(blk, name, None)
+                if not _is_identity(ls) and not _is_layer_scale(ls, C):
+                    raise NotImplementedError(f"blocks[{i}].{name} = {type(ls).__name__} is not supported "
+                                              "(Identity or LayerScale with gamma [C])")
+            for name in ("drop_path1", "drop_path2"):
                 if not _is_identity(getattr(blk, name, None)):
                     raise NotImplementedError(f"blocks[{i}].{name} = {type(getattr(blk, name)).__name__} is not supported")
             attn = blk.attn
@@ -130,6 +169,8 @@ class RAJNIViTWrapper(nn.Module):
                 raise NotImplementedError(f"blocks[{i}].mlp.norm is not supported")
             if not isinstance(blk.norm1, nn.LayerNorm) or not isinstance(blk.norm2, nn.LayerNorm):
                 raise NotImplementedError(f"blocks[{i}]: norm1/norm2 must be LayerNorm")
+            if blk.has_pruner:
+                blk.attn.num_prefix_tokens = prefix
 
     def _apply(self, fn, *a, **kw):
         self._packs.clear()
@@ -146,6 +187,9 @@ class RAJNIViTWrapper(nn.Module):
     def get_last_stats(self):
         return self._last_stats
 
+    def _distilled(self) -> bool:
+        return getattr(self.m, "dist_token", None) is not None
+
     # ------------------------------------------------------------------ workspace
     def _workspace(self, B: int, S: int, dev: torch.device):
         key = (B, S, dev, self.stream_k)
@@ -157,9 +201,11 @@ class RAJNIViTWrapper(nn.Module):
         p = self.patch
         G = S // p
         P = G * G
-        N0 = P + 1
-        if m.pos_embed.shape[1] < N0:
-            raise ValueError(f"pos_embed has {m.pos_embed.shape[1]} positions, input needs {N0}")
+        P0 = self.prefix
+        N0 = P + P0
+        pos_off = 0 if self.no_embed_class else P0          # pos_embed row of patch 0
+        if m.pos_embed.shape[1] < P + pos_off:
+            raise ValueError(f"pos_embed has {m.pos_embed.shape[1]} positions, input needs {P + pos_off}")
         hidden = max(blk.mlp.fc1.out_features for blk in self.blocks)
         bf = dict(device=dev, dtype=torch.bfloat16)
         idx = torch.arange(B * P, device=dev, dtype=torch.int32)
@@ -169,9 +215,10 @@ class RAJNIViTWrapper(nn.Module):
             xa=torch.empty((B * N0, C), **bf), xb=torch.empty((B * N0, C), **bf),
             qkv=torch.empty((B * N0, 3 * C), **bf),
             att=torch.empty((B * N0, C), **bf), hid=torch.empty((B * N0, hidden), **bf),
-            cls=torch.empty((B, C), **bf),
-            embed_out_map=((idx // P) * N0 + 1 + idx % P).to(torch.int32),
-            embed_pos_map=(1 + idx % P).to(torch.int32),
+            # final-norm rows feeding the head: CLS, or [CLS | distillation token] side by side (K = 2C)
+            cls=torch.empty((B, (2 if self._distilled() else 1) * C), **bf),
+            embed_out_map=((idx // P) * N0 + P0 + idx % P).to(torch.int32),
+            embed_pos_map=(pos_off + idx % P).to(torch.int32),
             # LayerNorm partial sums (sum, sum of squares) of the rows of x, one slot per (n-tile, column half)
             # of the GEMM that produced them; consumed by the LN-folded qkv / fc1 GEMMs
             stat_slots=ops.row_stats_slots(C),
@@ -205,7 +252,7 @@ class RAJNIViTWrapper(nn.Module):
                 return self.forward(x)
         use = self.use_cuda_graph
         if use is None and x.dim() == 4:
-            use = x.shape[0] * ((x.shape[2] // self.patch) * (x.shape[3] // self.patch) + 1) <= AUTO_GRAPH_MAX_ROWS
+            use = x.shape[0] * ((x.shape[2] // self.patch) * (x.shape[3] // self.patch) + self.prefix) <= AUTO_GRAPH_MAX_ROWS
         if not use or x.device.type != "cuda" or x.dim() != 4 or ops._prof is not None:      # (the per-kernel profiler times eager launches)
             return self._forward_eager(x)
         # what _forward_eager reads besides the input: the schedule of the pruned blocks (attention.py:25-32) ...
@@ -261,20 +308,29 @@ class RAJNIViTWrapper(nn.Module):
         pk = self._packs
 
         # ---- patch + CLS + pos (model.py:31-37): im2col, then one GEMM whose epilogue adds
-        #      bias and pos_embed and scatters into rows 1..P of each image
+        #      bias and pos_embed and scatters into rows P0..P0+P-1 of each image (P0 = 1, or 2 with a distillation token)
         pe_w, pe_b = pk.linear(m.patch_embed.proj)
-        def _pos_pack():
-            pos_ = m.pos_embed.detach()[0, : P + 1].to(torch.bfloat16).contiguous()
-            cls_ = (m.cls_token.detach()[0, 0] + m.pos_embed.detach()[0, 0]).to(torch.bfloat16).contiguous()
-            c32 = cls_.to(torch.float32)
-            return pos_, cls_, float(c32.sum()), float((c32 * c32).sum())
+        P0 = self.prefix
+        dist = getattr(m, "dist_token", None)
 
-        pos, cls_pos0, cls_sum, cls_sumsq = pk.tensors(("pos", P), (m.pos_embed, m.cls_token), _pos_pack)
+        def _pos_pack():
+            pos_ = m.pos_embed.detach()[0, : P + (0 if self.no_embed_class else P0)].to(torch.bfloat16).contiguous()
+            tok = [m.cls_token.detach()[0, 0]] + ([dist.detach()[0, 0]] if dist is not None else [])
+            if not self.no_embed_class:                     # the tokens' own positions; DeiT-III adds none to its class token
+                tok = [t + m.pos_embed.detach()[0, r] for r, t in enumerate(tok)]
+            rows = torch.stack(tok).to(torch.bfloat16).contiguous()
+            r32 = rows.to(torch.float32)
+            sums = [float(r32[r].sum()) for r in range(P0)]               # one full reduction per row
+            sqs = [float((r32[r] * r32[r]).sum()) for r in range(P0)]
+            return pos_, rows, sums if P0 > 1 else sums[0], sqs if P0 > 1 else sqs[0]
+
+        pos, prefix_rows, pre_sum, pre_sumsq = pk.tensors(("pos", P), (m.pos_embed, m.cls_token, dist), _pos_pack)
         cur, nxt = ws["xa"], ws["xb"]
         stats, slots = ws["stats"], ws["stat_slots"]
         kpe = ws["cols"].shape[1]                                                   # 3 p^2
-        ops.patch_im2col(x, self.patch, ws["cols"], cls_pos0, cur, C, row_stats=stats, stats_slots=slots,
-                         cls_sum=cls_sum, cls_sumsq=cls_sumsq, norm=self.input_norm if x.dtype == torch.uint8 else None)
+        ops.patch_im2col(x, self.patch, ws["cols"], prefix_rows, cur, C, row_stats=stats, stats_slots=slots,
+                         cls_sum=pre_sum, cls_sumsq=pre_sumsq, norm=self.input_norm if x.dtype == torch.uint8 else None,
+                         prefix=P0)
         ops.gemm(ws["cols"], pe_w, pe_b, B * P, C, kpe, residual=pos, ldres=C, res_row_map=ws["embed_pos_map"],
                  out=cur, ldd=C, out_row_map=ws["embed_out_map"], row_stats=stats, tag="embed")
 
@@ -290,19 +346,21 @@ class RAJNIViTWrapper(nn.Module):
             H = blk.attn.num_heads
             # norm1 / norm2 are folded into the qkv / fc1 GEMMs: x itself is the A operand, the row statistics
             # come from the epilogue of whichever GEMM stored x (embed, proj or fc2)
+            # LayerScale (DeiT-III) is folded into the GEMMs that feed the residual: proj (ls1) and fc2 (ls2)
             qw, qb, qsum, e1 = pk.linear_ln(blk.attn.qkv, blk.norm1)
-            pw, pb = pk.linear(blk.attn.proj)
+            ls1, ls2 = getattr(blk, "ls1", None), getattr(blk, "ls2", None)
+            pw, pb = pk.linear(blk.attn.proj) if _is_identity(ls1) else pk.linear_ls(blk.attn.proj, ls1)
             f1w, f1b, f1sum, e2 = pk.linear_ln(blk.mlp.fc1, blk.norm2)
-            f2w, f2b = pk.linear(blk.mlp.fc2)
+            f2w, f2b = pk.linear(blk.mlp.fc2) if _is_identity(ls2) else pk.linear_ls(blk.mlp.fc2, ls2)
             hidden = f1w.shape[0]
             M = B * N
             ops.gemm(cur, qw, qb, M, 3 * C, C, out=ws["qkv"], ln=(stats, slots, qsum, e1), tag="qkv", reverse=rev)   # model.py:51 + attention.py:22
             if blk.has_pruner:
                 attn: RAJNIAttention = blk.attn
-                keep = keep_count(N, attn.keep_ratio)                                 # attention.py:31-32
-                if keep > N - 1:
+                keep = keep_count(N, attn.keep_ratio, P0)                             # attention.py:31-32
+                if keep > N - P0:
                     raise RuntimeError("selected index k out of range")               # attention.py:35
-                Np = keep + 1
+                Np = keep + P0
                 sel = ws["sel"].get(i)
                 if sel is None or sel[0].shape[1] != Np:
                     sel = (torch.empty((B, Np), device=x.device, dtype=torch.int32),
@@ -311,10 +369,10 @@ class RAJNIViTWrapper(nn.Module):
                     ws["sel"][i] = sel
                 keep_idx, next_scores, row_map = sel
                 if attn.update or scores is None:                                     # attention.py:25-28
-                    ops.score_select(ws["qkv"][: B * N].view(B, N, 3 * C), H, keep,
-                                     keep_idx=keep_idx, next_scores=next_scores, row_map=row_map, workspace=ws["score_ws"])
+                    ops.score_select(ws["qkv"][: B * N].view(B, N, 3 * C), H, keep, keep_idx=keep_idx, next_scores=next_scores,
+                                     row_map=row_map, workspace=ws["score_ws"], prefix=P0)
                 else:
-                    ops.select(scores, keep, keep_idx=keep_idx, next_scores=next_scores, row_map=row_map)
+                    ops.select(scores, keep, keep_idx=keep_idx, next_scores=next_scores, row_map=row_map, prefix=P0)
                 if Np > ops.LONG_SEQ and "qkvc" not in ws:                             # compaction buffer, long sequences only
                     ws["qkvc"] = torch.empty((B * ws["N0"], 3 * C), device=x.device, dtype=torch.bfloat16)
                 ops.attention(ws["qkv"], row_map, B, N, Np, C, H, float(attn.scale), out=ws["att"], reverse=zig and not rev,
@@ -340,10 +398,26 @@ class RAJNIViTWrapper(nn.Module):
 
         # ---- final norm on the CLS rows only (LayerNorm is row-wise) + head   model.py:65-66
         gn, bn, en = pk.norm(m.norm)
-        hw, hb = pk.linear(m.head)
-        ops.layernorm(cur, gn, bn, en, B, C, in_row_stride=N * C, out=ws["cls"])
-        logits = ops.gemm(ws["cls"], hw, hb, B, hw.shape[0], C, out_f32=True, tag="head")
+        if dist is None:
+            hw, hb = pk.linear(m.head)
+            ops.layernorm(cur, gn, bn, en, B, C, in_row_stride=N * C, out=ws["cls"])
+            logits = ops.gemm(ws["cls"], hw, hb, B, hw.shape[0], C, out_f32=True, tag="head")
+        else:
+            # distilled: (head(LN(x0)) + head_dist(LN(x1))) / 2 as ONE GEMM over [LN(x0) | LN(x1)] (K = 2C) with the weights
+            # [W_head | W_dist] / 2 (halving is exact in bf16) and the bias (b + b_dist) / 2
+            hw, hb = pk.tensors(("head2",), (m.head.weight, m.head.bias, m.head_dist.weight, m.head_dist.bias), self._head_pack)
+            for r in range(2):
+                ops.layernorm(cur, gn, bn, en, B, C, in_row_stride=N * C, in_offset=r * C, out=ws["cls"],
+                              out_row_stride=2 * C, out_offset=r * C)
+            logits = ops.gemm(ws["cls"], hw, hb, B, hw.shape[0], 2 * C, out_f32=True, tag="head")
 
         self._last_stats = {"token_counts": token_counts}                            # model.py:68
         self._last_keep_idx = keep_log
         return logits if out_dtype == torch.float32 else logits.to(out_dtype)
+
+    def _head_pack(self):
+        m = self.m
+        w = torch.cat([m.head.weight.detach(), m.head_dist.weight.detach()], dim=1).to(torch.bfloat16) / 2
+        b = [t.detach().to(torch.float32) if t is not None else torch.zeros(m.head.out_features, device=m.head.weight.device)
+             for t in (m.head.bias, m.head_dist.bias)]
+        return w.contiguous(), ((b[0] + b[1]) / 2).contiguous()
