@@ -40,8 +40,7 @@ static int attention_dispatch(const void* qkv, const int32_t* row_map, void* out
     if (impl == RAJNI_ATTN_AUTO) {
         static const bool force_tc = getenv("RAJNI_ATTN_TC") != nullptr, force_pipe = getenv("RAJNI_ATTN_PIPE") != nullptr;
         const int np_pad = (Np + 15) & ~15;
-        int sms = 148;
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, current_device());
+        const int sms = num_sms();
         const long long items = (long long)B * H;
         const bool big = Np > 128;
         const bool one_tile = Np > 64 && Np <= 128 && (row_map == nullptr ? items >= sms : items <= 4LL * sms);

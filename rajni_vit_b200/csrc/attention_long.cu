@@ -53,23 +53,6 @@ struct AttnLongParams {
     float scale_log2;
 };
 
-__device__ __forceinline__ void al_cp_async16(uint32_t smem_dst, const void* gsrc, int src_bytes) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" :: "r"(smem_dst), "l"(gsrc), "r"(src_bytes) : "memory");
-}
-__device__ __forceinline__ void al_cp_async_arrive(uint64_t* bar) {
-    asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" :: "r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ float al_ex2(float x) {
-    float y;
-    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-    return y;
-}
-__device__ __forceinline__ float al_fmax3(float a, float b, float c) {
-    float d;
-    asm("max.f32 %0, %1, %2, %3;" : "=f"(d) : "f"(a), "f"(b), "f"(c));
-    return d;
-}
-
 __global__ void __launch_bounds__(kAlThreads, 1)
 attention_long_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_kv, const AttnLongParams p) {
     extern __shared__ uint8_t smem_raw[];
@@ -180,9 +163,9 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_c
                 for (int i = 0; i < 32; ++i) {
                     const int r = grp + 4 * i;
                     const bool ok = grow[i] >= 0;
-                    al_cp_async16(s_q + qb * kAlQBytes + r * 128 + ((chunk ^ (r & 7)) << 4), head + (ok ? grow[i] : 0) * C3, ok ? 16 : 0);
+                    cp_async16(s_q + qb * kAlQBytes + r * 128 + ((chunk ^ (r & 7)) << 4), head + (ok ? grow[i] : 0) * C3, ok ? 16 : 0);
                 }
-                al_cp_async_arrive(&q_full[qb]);
+                cp_async_arrive_noinc(&q_full[qb]);
             }
             // ---- key blocks: pass 1 needs K only, pass 2 K and V
             for (int pass = 0; pass < 2; ++pass) {
@@ -206,12 +189,12 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_c
                                 const bool ok = grow[i] >= 0;
                                 const __nv_bfloat16* src = head + (ok ? grow[i] : 0) * C3;
                                 const uint32_t off = r * 128 + ((chunk ^ (r & 7)) << 4);
-                                al_cp_async16(sk + off, src + p.C, ok ? 16 : 0);
-                                if (pass == 1) al_cp_async16(sv + off, src + 2 * p.C, ok ? 16 : 0);   // 0 * V must stay 0 past Np
+                                cp_async16(sk + off, src + p.C, ok ? 16 : 0);
+                                if (pass == 1) cp_async16(sv + off, src + 2 * p.C, ok ? 16 : 0);   // 0 * V must stay 0 past Np
                             }
                         }
                     }
-                    al_cp_async_arrive(&full_bar[stage]);
+                    cp_async_arrive_noinc(&full_bar[stage]);
                     if (lane == 0) AL_TRACE(n, 1 + pass * 3 + (j < 3 ? j : 2));
                 }
             }
@@ -313,8 +296,8 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_c
                         if (c0 + 64 <= ncol) {
 #pragma unroll
                             for (int g = 0; g < 8; ++g) {
-                                mx0 = al_fmax3(mx0, __uint_as_float(cur[4 * g]), __uint_as_float(cur[4 * g + 1]));
-                                mx1 = al_fmax3(mx1, __uint_as_float(cur[4 * g + 2]), __uint_as_float(cur[4 * g + 3]));
+                                mx0 = fmax3(mx0, __uint_as_float(cur[4 * g]), __uint_as_float(cur[4 * g + 1]));
+                                mx1 = fmax3(mx1, __uint_as_float(cur[4 * g + 2]), __uint_as_float(cur[4 * g + 3]));
                             }
                         } else {
 #pragma unroll
@@ -360,8 +343,8 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_c
                     const uint32_t ts = twin + buf * kAlKB;
                     // one 8-column group: this thread's 2 rows x 2 columns -> one packed P word per row
                     auto exp_group = [&](uint32_t s00, uint32_t s01, uint32_t s10, uint32_t s11, int c, bool masked, uint32_t& p0, uint32_t& p1) {
-                        float e00 = al_ex2(fmaf(__uint_as_float(s00), sl2, -mb0)), e01 = al_ex2(fmaf(__uint_as_float(s01), sl2, -mb0));
-                        float e10 = al_ex2(fmaf(__uint_as_float(s10), sl2, -mb1)), e11 = al_ex2(fmaf(__uint_as_float(s11), sl2, -mb1));
+                        float e00 = ex2_approx(fmaf(__uint_as_float(s00), sl2, -mb0)), e01 = ex2_approx(fmaf(__uint_as_float(s01), sl2, -mb0));
+                        float e10 = ex2_approx(fmaf(__uint_as_float(s10), sl2, -mb1)), e11 = ex2_approx(fmaf(__uint_as_float(s11), sl2, -mb1));
                         if (masked) {                                             // key columns past Np contribute nothing
                             if (c + 1 >= ncol) { e01 = 0.f; e11 = 0.f; }
                             if (c >= ncol) { e00 = 0.f; e10 = 0.f; }
@@ -467,18 +450,6 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_c
     }
 }
 
-int make_tmap_bf16_3d_ld(CUtensorMap* map, const void* base, long long batch, long long rows, long long cols, int box_rows);   // gemm_tcgen05.cu
-
-static int al_num_sms() {
-    static int n_dev[kMaxDevices] = {};          // per device: one process may drive several GPUs
-    int& n = n_dev[current_device()];
-    if (!n) {
-        cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, current_device());
-        if (n <= 0) n = 148;
-    }
-    return n;
-}
-
 // returns 1 if handled, <0 on error
 int launch_attention_long(const void* qkv, const int32_t* row_map, void* out, int B, int N_src, int Np,
                           int C, int H, float scale, int reverse, cudaStream_t stream) {
@@ -495,21 +466,14 @@ int launch_attention_long(const void* qkv, const int32_t* row_map, void* out, in
     const long long items = (long long)p.BH * p.QT;
     RAJNI_REQUIRE(items < (1LL << 31), RAJNI_EINVAL, "attention_long: too many work items");
     p.n_items = (int)items;
-    static bool attr_done_dev[kMaxDevices] = {};
-    bool& attr_done = attr_done_dev[current_device()];
-    if (!attr_done) {
-        cudaError_t e = cudaFuncSetAttribute(attention_long_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kAlSmem);
-        RAJNI_REQUIRE(e == cudaSuccess, RAJNI_ECUDA, "attention_long: smem attribute (%d B): %s", kAlSmem, cudaGetErrorString(e));
-        attr_done = true;
-    }
+    static int smem_granted[kMaxDevices] = {};
+    if (int rc = raise_smem_limit("attention_long", attention_long_kernel, kAlSmem, smem_granted)) return rc;
     CUtensorMap tq, tkv;
     if (int rc = make_tmap_bf16_3d_ld(&tq, qkv, B, N_src, 3LL * C, 128)) return rc;           // per image: a box never reads the next image
     if (int rc = make_tmap_bf16_3d_ld(&tkv, qkv, B, N_src, 3LL * C, kAlKB)) return rc;
-    const int grid = p.n_items < al_num_sms() ? p.n_items : al_num_sms();
-    cudaError_t le = launch_kernel(attention_long_kernel, dim3(grid), dim3(kAlThreads), (size_t)kAlSmem, stream, 1, tq, tkv, p);
-    count_launch();
-    RAJNI_REQUIRE(le == cudaSuccess, RAJNI_ECUDA, "attention_long: launch failed: %s", cudaGetErrorString(le));
-    int rc = check_launch("attention_long");
+    const int grid = p.n_items < num_sms() ? p.n_items : num_sms();
+    const int rc = launch_checked("attention_long", attention_long_kernel, dim3(grid), dim3(kAlThreads), (size_t)kAlSmem, stream, 1,
+                                  tq, tkv, p);
     return rc ? rc : 1;
 }
 

@@ -79,27 +79,8 @@ struct AttnPipeParams {
     float scale_log2;
 };
 
-__device__ __forceinline__ void ap_cp_async16(uint32_t smem_dst, const void* gsrc, int src_bytes) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" :: "r"(smem_dst), "l"(gsrc), "r"(src_bytes) : "memory");
-}
-__device__ __forceinline__ void ap_cp_async_arrive(uint64_t* bar) {
-    asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" :: "r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void ap_sts128(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
-    asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" :: "r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
-}
-__device__ __forceinline__ float ap_ex2(float x) {
-    float y;
-    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-    return y;
-}
 __device__ __forceinline__ void ap_bar_sync(int id, int threads) {
     asm volatile("bar.sync %0, %1;" :: "r"(id), "r"(threads) : "memory");
-}
-__device__ __forceinline__ float ap_fmax3(float a, float b, float c) {
-    float d;
-    asm("max.f32 %0, %1, %2, %3;" : "=f"(d) : "f"(a), "f"(b), "f"(c));
-    return d;
 }
 // Register re-partitioning between warpgroups (4 consecutive warps): the load/MMA and the epilogue warpgroups give registers
 // back, the exp warpgroups (a half row of S = 112 registers) take them.  8*160 + 4*112 + 4*80 = 2048 = 64 K / 32.
@@ -177,10 +158,10 @@ __device__ __forceinline__ float ap_exp_half(uint32_t sb, int cb, uint32_t pcol,
     // ---- row maximum of this half (four independent chains), then of the row (the other half's through shared memory)
     float m4[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
 #pragma unroll
-    for (int i = 0; i < 32 * N32; i += 2) m4[(i >> 1) & 3] = ap_fmax3(m4[(i >> 1) & 3], __uint_as_float(s[i]), __uint_as_float(s[i + 1]));
+    for (int i = 0; i < 32 * N32; i += 2) m4[(i >> 1) & 3] = fmax3(m4[(i >> 1) & 3], __uint_as_float(s[i]), __uint_as_float(s[i + 1]));
     if (HAS16) {
 #pragma unroll
-        for (int i = 0; i < 16; i += 2) m4[(i >> 1) & 3] = ap_fmax3(m4[(i >> 1) & 3], __uint_as_float(s[96 + i]), __uint_as_float(s[97 + i]));
+        for (int i = 0; i < 16; i += 2) m4[(i >> 1) & 3] = fmax3(m4[(i >> 1) & 3], __uint_as_float(s[96 + i]), __uint_as_float(s[97 + i]));
     }
     const float mx = fmaxf(fmaxf(m4[0], m4[1]), fmaxf(m4[2], m4[3]));
     *pm_mine = mx;
@@ -198,8 +179,8 @@ __device__ __forceinline__ float ap_exp_half(uint32_t sb, int cb, uint32_t pcol,
 #pragma unroll
         for (int j = 0; j < N; j += 2) {
             const float x0 = fmaf(__uint_as_float(s[R0 + j]), sl2, -mb), x1 = fmaf(__uint_as_float(s[R0 + j + 1]), sl2, -mb);
-            const float e0 = ap_ex2(x0);
-            const float e1 = (kApPolyEvery > 0 && (j + 1) % (kApPolyEvery > 0 ? kApPolyEvery : 1) == kApPolyEvery - 1) ? ap_ex2_poly(x1) : ap_ex2(x1);
+            const float e0 = ex2_approx(x0);
+            const float e1 = (kApPolyEvery > 0 && (j + 1) % (kApPolyEvery > 0 ? kApPolyEvery : 1) == kApPolyEvery - 1) ? ap_ex2_poly(x1) : ex2_approx(x1);
             sum0 += e0;
             sum1 += e1;
             s[W0 + (j >> 1)] = float2_to_bf16x2(e0, e1);
@@ -247,13 +228,13 @@ __device__ __forceinline__ void ap_exp_full(uint32_t sb, uint32_t pcol, int Np, 
     }
     float m4[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
 #pragma unroll
-    for (int i = 0; i < NCOL; i += 2) m4[(i >> 1) & 3] = ap_fmax3(m4[(i >> 1) & 3], __uint_as_float(s[i]), __uint_as_float(s[i + 1]));
+    for (int i = 0; i < NCOL; i += 2) m4[(i >> 1) & 3] = fmax3(m4[(i >> 1) & 3], __uint_as_float(s[i]), __uint_as_float(s[i + 1]));
     const float mb = fmaxf(fmaxf(m4[0], m4[1]), fmaxf(m4[2], m4[3])) * sl2;
     float sum0 = 0.f, sum1 = 0.f;
 #pragma unroll
     for (int j = 0; j < NCOL; j += 2) {
         if (j == SPLIT) { sum_a = sum0 + sum1; sum0 = 0.f; sum1 = 0.f; }
-        const float e0 = ap_ex2(fmaf(__uint_as_float(s[j]), sl2, -mb)), e1 = ap_ex2(fmaf(__uint_as_float(s[j + 1]), sl2, -mb));
+        const float e0 = ex2_approx(fmaf(__uint_as_float(s[j]), sl2, -mb)), e1 = ex2_approx(fmaf(__uint_as_float(s[j + 1]), sl2, -mb));
         sum0 += e0;
         sum1 += e1;
         s[j >> 1] = float2_to_bf16x2(e0, e1);
@@ -380,14 +361,14 @@ attention_pipe_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid
                     const uint32_t off = j * 128 + ((chunk ^ (j & 7)) << 4);
                     if (pass == 0) {
                         if (ok) {                                     // rows past Np: dead query rows / masked key columns
-                            ap_cp_async16(sq + off, src, 16);
-                            ap_cp_async16(sk + off, src + p.C, 16);
+                            cp_async16(sq + off, src, 16);
+                            cp_async16(sk + off, src + p.C, 16);
                         }
                     } else {
-                        ap_cp_async16(sv + off, src + 2 * p.C, ok ? 16 : 0);      // zero-filled: 0 * V must stay 0
+                        cp_async16(sv + off, src + 2 * p.C, ok ? 16 : 0);      // zero-filled: 0 * V must stay 0
                     }
                 }
-                ap_cp_async_arrive(pass == 0 ? &qk_full[stage] : &v_full[stage]);
+                cp_async_arrive_noinc(pass == 0 ? &qk_full[stage] : &v_full[stage]);
             }
             if (++stage == p.stages) { stage = 0; phase ^= 1; }
         }
@@ -496,7 +477,7 @@ attention_pipe_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid
                 for (int c = 0; c < 8; ++c) {
                     const uint32_t (&src)[32] = c < 4 ? o0 : o1;
                     const int j = (c & 3) * 8;
-                    ap_sts128(srow + ((c ^ (lane & 7)) << 4),
+                    sts128(srow + ((c ^ (lane & 7)) << 4),
                               float2_to_bf16x2(__uint_as_float(src[j]) * inv, __uint_as_float(src[j + 1]) * inv),
                               float2_to_bf16x2(__uint_as_float(src[j + 2]) * inv, __uint_as_float(src[j + 3]) * inv),
                               float2_to_bf16x2(__uint_as_float(src[j + 4]) * inv, __uint_as_float(src[j + 5]) * inv),
@@ -615,19 +596,6 @@ attention_pipe_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid
     }
 }
 
-int make_tmap_bf16_3d_box(CUtensorMap* map, const void* base, long long batch, long long rows, long long cols, int box_rows);   // gemm_tcgen05.cu
-int make_tmap_bf16_3d_ld(CUtensorMap* map, const void* base, long long batch, long long rows, long long cols, int box_rows);
-
-static int ap_num_sms() {
-    static int n_dev[kMaxDevices] = {};
-    int& n = n_dev[current_device()];
-    if (!n) {
-        cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, current_device());
-        if (n <= 0) n = 148;
-    }
-    return n;
-}
-
 // returns 1 if this kernel handled the call, 0 if the shape is outside its range, <0 on error
 int launch_attention_pipe(const void* qkv, const int32_t* row_map, void* out, int B, int N_src, int Np,
                           int C, int H, float scale, int reverse, cudaStream_t stream) {
@@ -672,20 +640,13 @@ int launch_attention_pipe(const void* qkv, const int32_t* row_map, void* out, in
     CUtensorMap tmap_out;
     RAJNI_REQUIRE((reinterpret_cast<uintptr_t>(out) & 15u) == 0, RAJNI_EINVAL, "attention_pipe: out must be 16-byte aligned (TMA store)");
     if (int rc = make_tmap_bf16_3d_box(&tmap_out, out, B, Np, C, 32)) return rc;
-    static int attr_smem_dev[kMaxDevices] = {};
-    int& attr_smem = attr_smem_dev[current_device()];
-    if (smem > attr_smem) {
-        cudaError_t e = cudaFuncSetAttribute(attention_pipe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        RAJNI_REQUIRE(e == cudaSuccess, RAJNI_ECUDA, "attention_pipe: smem attribute (%d B): %s", smem, cudaGetErrorString(e));
-        attr_smem = smem;
-    }
-    int grid = p.BH < ap_num_sms() ? p.BH : ap_num_sms();
+    static int smem_granted[kMaxDevices] = {};
+    if (int rc = raise_smem_limit("attention_pipe", attention_pipe_kernel, smem, smem_granted)) return rc;
+    int grid = p.BH < num_sms() ? p.BH : num_sms();
     static const int cta_cap = getenv("RAJNI_ATTN_MAX_CTAS") ? atoi(getenv("RAJNI_ATTN_MAX_CTAS")) : 0;      // experiments: share the GPU
     if (cta_cap > 0 && grid > cta_cap) grid = cta_cap;
-    cudaError_t le = launch_kernel(attention_pipe_kernel, dim3(grid), dim3(kApThreads), (size_t)smem, stream, 1, tmap, tmap_out, p);
-    count_launch();
-    RAJNI_REQUIRE(le == cudaSuccess, RAJNI_ECUDA, "attention_pipe: launch failed: %s", cudaGetErrorString(le));
-    int rc = check_launch("attention_pipe");
+    const int rc = launch_checked("attention_pipe", attention_pipe_kernel, dim3(grid), dim3(kApThreads), (size_t)smem, stream, 1,
+                                  tmap, tmap_out, p);
     return rc ? rc : 1;
 }
 

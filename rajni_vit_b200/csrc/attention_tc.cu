@@ -66,31 +66,6 @@ struct AttnTcParams {
     float scale_log2;
 };
 
-__device__ __forceinline__ void cp_async16(uint32_t smem_dst, const void* gsrc, int src_bytes) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" :: "r"(smem_dst), "l"(gsrc), "r"(src_bytes) : "memory");
-}
-// arrive on `bar` once every cp.async issued so far by this thread has landed
-__device__ __forceinline__ void cp_async_arrive_noinc(uint64_t* bar) {
-    asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" :: "r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void sts128(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
-    asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" :: "r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
-}
-__device__ __forceinline__ float ex2_approx(float x) {
-    float y;
-    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-    return y;
-}
-__device__ __forceinline__ float fmax3(float a, float b, float c) {
-    float d;
-    asm("max.f32 %0, %1, %2, %3;" : "=f"(d) : "f"(a), "f"(b), "f"(c));
-    return d;
-}
-__device__ __forceinline__ void st_global_256(void* p, const uint32_t (&v)[8]) {
-    asm volatile("st.global.v8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};"
-                 :: "l"(p), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]) : "memory");
-}
-
 // (image*H + head) handled by tile `t` of unit `u`, or -1
 __device__ __forceinline__ int unit_item(const AttnTcParams& p, int u, int t) {
     const int item = p.two_tiles ? u : 2 * u + t;
@@ -514,21 +489,6 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_c
     }
 }
 
-int make_tmap_bf16_2d_box(CUtensorMap* map, const void* base, long long rows, long long cols, long long ld_elems,
-                          int box_cols, int box_rows);      // gemm_tcgen05.cu
-int make_tmap_bf16_3d_box(CUtensorMap* map, const void* base, long long batch, long long rows, long long cols, int box_rows);
-int make_tmap_bf16_3d_ld(CUtensorMap* map, const void* base, long long batch, long long rows, long long cols, int box_rows);
-
-static int at_num_sms() {
-    static int n_dev[kMaxDevices] = {};          // per device: one process may drive several GPUs
-    int& n = n_dev[current_device()];
-    if (!n) {
-        cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, current_device());
-        if (n <= 0) n = 148;
-    }
-    return n;
-}
-
 // returns 1 if the tcgen05 kernel handled the call, 0 if the shape is outside its range, <0 on error
 int launch_attention_tc(const void* qkv, const int32_t* row_map, void* out, int B, int N_src, int Np,
                         int C, int H, float scale, int reverse, cudaStream_t stream) {
@@ -578,20 +538,12 @@ int launch_attention_tc(const void* qkv, const int32_t* row_map, void* out, int 
     if (int rc = make_tmap_bf16_3d_box(&tmap_out, out, B, Np, C, 32)) return rc;
     const bool packed = seg < Np;
     auto kern = packed ? attention_tc_kernel<true> : attention_tc_kernel<false>;
-    static int attr_smem_dev[2][kMaxDevices] = {};
-    int& attr_smem = attr_smem_dev[packed][current_device()];
-    if (smem > attr_smem) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        RAJNI_REQUIRE(e == cudaSuccess, RAJNI_ECUDA, "attention_tc: smem attribute (%d B): %s", smem, cudaGetErrorString(e));
-        attr_smem = smem;
-    }
-    int grid = p.n_units < at_num_sms() ? p.n_units : at_num_sms();
+    static int smem_granted[2][kMaxDevices] = {};
+    if (int rc = raise_smem_limit("attention_tc", kern, smem, smem_granted[packed])) return rc;
+    int grid = p.n_units < num_sms() ? p.n_units : num_sms();
     static const int cta_cap = getenv("RAJNI_ATTN_MAX_CTAS") ? atoi(getenv("RAJNI_ATTN_MAX_CTAS")) : 0;      // experiments: share the GPU
     if (cta_cap > 0 && grid > cta_cap) grid = cta_cap;
-    cudaError_t le = launch_kernel(kern, dim3(grid), dim3(kAtThreads), (size_t)smem, stream, 1, tmap, tmap_out, p);
-    count_launch();
-    RAJNI_REQUIRE(le == cudaSuccess, RAJNI_ECUDA, "attention_tc: launch failed: %s", cudaGetErrorString(le));
-    int rc = check_launch("attention_tc");
+    const int rc = launch_checked("attention_tc", kern, dim3(grid), dim3(kAtThreads), (size_t)smem, stream, 1, tmap, tmap_out, p);
     return rc ? rc : 1;
 }
 

@@ -1,7 +1,9 @@
-// Shared device helpers for the sm_100a kernels: mbarrier, TMA, tcgen05/TMEM wrappers,
-// warp reductions, vector loads.  Inline PTX only — no CUTLASS.
+// Shared helpers for the sm_100a kernels.  Host side: errors, the launch path (launch_kernel, launch_checked,
+// raise_smem_limit), the SM count and the TMA tensor-map builders.  Device side: mbarrier, TMA, cp.async, tcgen05/TMEM
+// wrappers, warp reductions, vector loads and stores.  Inline PTX only — no CUTLASS.
 #pragma once
 
+#include <cuda.h>
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -63,6 +65,51 @@ inline cudaError_t launch_kernel(void (*kern)(KArgs...), dim3 grid, dim3 block, 
     cfg.numAttrs = n;
     return cudaLaunchKernelEx(&cfg, kern, std::forward<Args>(args)...);
 }
+
+// launch_kernel, counted in rajni_launch_count() whether or not the launch call succeeds.  Returns RAJNI_OK, or
+// RAJNI_ECUDA with `name` in the error text when the launch call or cudaGetLastError reports an error.
+template <typename... KArgs, typename... Args>
+inline int launch_checked(const char* name, void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
+                          int cluster_x, Args&&... args) {
+    const cudaError_t e = launch_kernel(kern, grid, block, smem, stream, cluster_x, std::forward<Args>(args)...);
+    count_launch();
+    RAJNI_REQUIRE(e == cudaSuccess, RAJNI_ECUDA, "%s: launch failed: %s", name, cudaGetErrorString(e));
+    return check_launch(name);
+}
+
+// Raises `kern`'s dynamic shared-memory limit on the current device to `bytes`, calling the runtime only when `bytes`
+// exceeds what `granted` (the caller's static record for this kernel, per device) says was already set there.
+template <typename... KArgs>
+inline int raise_smem_limit(const char* name, void (*kern)(KArgs...), int bytes, int (&granted)[kMaxDevices]) {
+    int& g = granted[current_device()];
+    if (bytes > g) {
+        const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+        RAJNI_REQUIRE(e == cudaSuccess, RAJNI_ECUDA, "%s: smem attribute (%d B): %s", name, bytes, cudaGetErrorString(e));
+        g = bytes;
+    }
+    return RAJNI_OK;
+}
+
+// SM count of the current device, queried once per device (one process may drive several GPUs); 148 if the query fails.
+inline int num_sms() {
+    static int n_dev[kMaxDevices] = {};
+    const int dev = current_device();
+    int& n = n_dev[dev];
+    if (!n) {
+        cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
+        if (n <= 0) n = 148;
+    }
+    return n;
+}
+
+// ------------------------------------------------------------------ TMA tensor maps (gemm_tcgen05.cu)
+// bf16, 128-byte swizzle, out-of-bounds elements read as zero.  Return 0 or RAJNI_ECUDA.
+// 2-D row-major [rows, cols] with a leading dimension of ld_elems, box = box_rows x 64 columns (L2 promotion 256 B).
+int make_tmap_bf16_2d(CUtensorMap* map, const void* base, long long rows, long long cols, long long ld_elems, int box_rows);
+// 3-D densely packed [batch][rows][cols], box = box_rows x 64 columns of one batch entry: a box never crosses into the next
+// entry's rows (stores are clipped there, loads zero-filled).  _box: no L2 promotion (stores); _ld: 256 B (loads).
+int make_tmap_bf16_3d_box(CUtensorMap* map, const void* base, long long batch, long long rows, long long cols, int box_rows);
+int make_tmap_bf16_3d_ld(CUtensorMap* map, const void* base, long long batch, long long rows, long long cols, int box_rows);
 
 // ------------------------------------------------------------------ small device utils
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
@@ -142,6 +189,21 @@ __device__ __forceinline__ void stg256(void* p, const uint32_t (&v)[8]) {
     asm volatile("st.global.v8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};"
                  :: "l"(p), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]) : "memory");
 }
+// explicit shared-state-space store (a generic pointer into dynamic smem compiles to ST.E)
+__device__ __forceinline__ void sts128(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
+    asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" :: "r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
+}
+
+__device__ __forceinline__ float ex2_approx(float x) {
+    float y;
+    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
+    return y;
+}
+__device__ __forceinline__ float fmax3(float a, float b, float c) {
+    float d;
+    asm("max.f32 %0, %1, %2, %3;" : "=f"(d) : "f"(a), "f"(b), "f"(c));
+    return d;
+}
 
 __device__ __forceinline__ bool elect_one() {
     uint32_t pred;
@@ -187,6 +249,16 @@ __device__ __forceinline__ bool mbar_test(uint64_t* bar, uint32_t parity) {
         "selp.u32 %0, 1, 0, p;\n\t}"
         : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
     return ok != 0;
+}
+
+// ------------------------------------------------------------------ cp.async
+// 16-byte global -> shared copy; the bytes past src_bytes (0 or 16) are zero-filled
+__device__ __forceinline__ void cp_async16(uint32_t smem_dst, const void* gsrc, int src_bytes) {
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" :: "r"(smem_dst), "l"(gsrc), "r"(src_bytes) : "memory");
+}
+// arrive on `bar` once every cp.async issued so far by this thread has landed
+__device__ __forceinline__ void cp_async_arrive_noinc(uint64_t* bar) {
+    asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" :: "r"(smem_u32(bar)) : "memory");
 }
 
 // ------------------------------------------------------------------ TMA

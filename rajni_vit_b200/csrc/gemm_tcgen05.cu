@@ -142,9 +142,7 @@ __device__ __forceinline__ float gelu_erf(float x) {
     p = fmaf(p, a, 5.0176125e-02f);
     p = fmaf(p, a, 0.4615304f);
     p = fmaf(p, a, 1.1504223f);
-    float e;
-    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e) : "f"(-a * p));
-    const float s = x * (0.5f * e);
+    const float s = x * (0.5f * ex2_approx(-a * p));
     return x >= 0.f ? x - s : s;
 }
 
@@ -160,17 +158,12 @@ __device__ __forceinline__ uint64_t gelu_erf2(uint64_t x2) {
     q = fma2(q, na, f2pack(-0.4615304f, -0.4615304f));
     q = fma2(q, na, f2pack(1.1504223f, 1.1504223f));
     const uint64_t arg = fma2(na, q, f2pack(-1.0f, -1.0f));
-    float a0, a1, t0, t1;
+    float a0, a1;
     f2unpack(arg, a0, a1);
-    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(t0) : "f"(a0));
-    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(t1) : "f"(a1));
-    return fma2(na, f2pack(t0, t1), f2pack(fmaxf(x0, 0.0f), fmaxf(x1, 0.0f)));
+    return fma2(na, f2pack(ex2_approx(a0), ex2_approx(a1)), f2pack(fmaxf(x0, 0.0f), fmaxf(x1, 0.0f)));
 }
 
-// explicit shared-state-space accesses (a generic pointer into dynamic smem compiles to LD.E/ST.E)
-__device__ __forceinline__ void sts128(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
-    asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" :: "r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
-}
+// explicit shared-state-space load (a generic pointer into dynamic smem compiles to LD.E)
 __device__ __forceinline__ float4 lds128(uint32_t addr) {
     float4 v;
     asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(addr) : "memory");
@@ -706,68 +699,49 @@ static EncodeTiledFn get_encode_fn() {
     return fn;
 }
 
-// 2-D bf16 row-major [rows, cols] tensor, box = [box_rows, box_cols], 128-byte swizzle, zero OOB fill.
-int make_tmap_bf16_2d_box(CUtensorMap* map, const void* base, long long rows, long long cols,
-                          long long ld_elems, int box_cols, int box_rows) {
+// One cuTensorMapEncodeTiled call on a bf16 tensor of `rank` <= 3 dimensions (dims and box innermost first, strides in
+// bytes for dims 1..rank-1): unit element strides, 128-byte swizzle, zero OOB fill.  Sets `r` to the driver's result and
+// returns 0, or RAJNI_ECUDA when the driver lacks the entry point.
+static int encode_tmap_bf16(CUtensorMap* map, const void* base, cuuint32_t rank, const cuuint64_t* dims, const cuuint64_t* strides,
+                            const cuuint32_t* box, CUtensorMapL2promotion l2, CUresult& r) {
     EncodeTiledFn fn = get_encode_fn();
     RAJNI_REQUIRE(fn != nullptr, RAJNI_ECUDA, "cuTensorMapEncodeTiled is not available from the driver");
-    cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-    cuuint64_t strides[1] = {(cuuint64_t)ld_elems * 2};
-    cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
-    cuuint32_t estr[2] = {1u, 1u};
-    CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    RAJNI_REQUIRE(r == CUDA_SUCCESS, RAJNI_ECUDA, "cuTensorMapEncodeTiled failed (%d) rows=%lld cols=%lld ld=%lld box=%dx%d",
-                  (int)r, rows, cols, ld_elems, box_rows, box_cols);
+    const cuuint32_t estr[3] = {1u, 1u, 1u};
+    r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, rank, const_cast<void*>(base), dims, strides, box, estr,
+           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, l2, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     return 0;
 }
-// [batch][rows][cols] bf16 tensor, densely packed, box = box_rows x 64 columns of one batch entry, 128-byte swizzle.
-// (Used for stores that must be clipped at the end of each batch entry's rows.)
+
+int make_tmap_bf16_2d(CUtensorMap* map, const void* base, long long rows, long long cols, long long ld_elems, int box_rows) {
+    const cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
+    const cuuint64_t strides[1] = {(cuuint64_t)ld_elems * 2};
+    const cuuint32_t box[2] = {64u, (cuuint32_t)box_rows};
+    CUresult r;
+    if (int rc = encode_tmap_bf16(map, base, 2, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, r)) return rc;
+    RAJNI_REQUIRE(r == CUDA_SUCCESS, RAJNI_ECUDA, "cuTensorMapEncodeTiled failed (%d) rows=%lld cols=%lld ld=%lld box=%dx%d",
+                  (int)r, rows, cols, ld_elems, box_rows, 64);
+    return 0;
+}
+// [batch][rows][cols], densely packed: the two 3-D views differ only in L2 promotion
 int make_tmap_bf16_3d_box(CUtensorMap* map, const void* base, long long batch, long long rows, long long cols, int box_rows) {
-    EncodeTiledFn fn = get_encode_fn();
-    RAJNI_REQUIRE(fn != nullptr, RAJNI_ECUDA, "cuTensorMapEncodeTiled is not available from the driver");
-    cuuint64_t dims[3] = {(cuuint64_t)cols, (cuuint64_t)rows, (cuuint64_t)batch};
-    cuuint64_t strides[2] = {(cuuint64_t)cols * 2, (cuuint64_t)rows * (cuuint64_t)cols * 2};
-    cuuint32_t box[3] = {64u, (cuuint32_t)box_rows, 1u};
-    cuuint32_t estr[3] = {1u, 1u, 1u};
-    CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), dims, strides, box, estr,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    const cuuint64_t dims[3] = {(cuuint64_t)cols, (cuuint64_t)rows, (cuuint64_t)batch};
+    const cuuint64_t strides[2] = {(cuuint64_t)cols * 2, (cuuint64_t)rows * (cuuint64_t)cols * 2};
+    const cuuint32_t box[3] = {64u, (cuuint32_t)box_rows, 1u};
+    CUresult r;
+    if (int rc = encode_tmap_bf16(map, base, 3, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_NONE, r)) return rc;
     RAJNI_REQUIRE(r == CUDA_SUCCESS, RAJNI_ECUDA, "cuTensorMapEncodeTiled (3d) failed (%d) batch=%lld rows=%lld cols=%lld",
                   (int)r, batch, rows, cols);
     return 0;
 }
-// The same 3-d view for LOADS: box = box_rows x 64 columns of one batch entry; rows past the entry's `rows` are zero-filled,
-// so a box that starts in one image can never pull in the next image's values.
 int make_tmap_bf16_3d_ld(CUtensorMap* map, const void* base, long long batch, long long rows, long long cols, int box_rows) {
-    EncodeTiledFn fn = get_encode_fn();
-    RAJNI_REQUIRE(fn != nullptr, RAJNI_ECUDA, "cuTensorMapEncodeTiled is not available from the driver");
-    cuuint64_t dims[3] = {(cuuint64_t)cols, (cuuint64_t)rows, (cuuint64_t)batch};
-    cuuint64_t strides[2] = {(cuuint64_t)cols * 2, (cuuint64_t)rows * (cuuint64_t)cols * 2};
-    cuuint32_t box[3] = {64u, (cuuint32_t)box_rows, 1u};
-    cuuint32_t estr[3] = {1u, 1u, 1u};
-    CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), dims, strides, box, estr,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    const cuuint64_t dims[3] = {(cuuint64_t)cols, (cuuint64_t)rows, (cuuint64_t)batch};
+    const cuuint64_t strides[2] = {(cuuint64_t)cols * 2, (cuuint64_t)rows * (cuuint64_t)cols * 2};
+    const cuuint32_t box[3] = {64u, (cuuint32_t)box_rows, 1u};
+    CUresult r;
+    if (int rc = encode_tmap_bf16(map, base, 3, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, r)) return rc;
     RAJNI_REQUIRE(r == CUDA_SUCCESS, RAJNI_ECUDA, "cuTensorMapEncodeTiled (3d load) failed (%d) batch=%lld rows=%lld cols=%lld box_rows=%d",
                   (int)r, batch, rows, cols, box_rows);
     return 0;
-}
-int make_tmap_bf16_2d(CUtensorMap* map, const void* base, long long rows, long long cols,
-                      long long ld_elems, int box_rows) {
-    return make_tmap_bf16_2d_box(map, base, rows, cols, ld_elems, 64, box_rows);
-}
-
-static int num_sms() {
-    static int n_dev[kMaxDevices] = {};
-    const int dev = current_device();
-    int& n = n_dev[dev];
-    if (!n) {
-        cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
-        if (n <= 0) n = 148;
-    }
-    return n;
 }
 
 // Stream-K scratch: a 4 KB header of counters, then one fp32 slot per (pair, piece, CTA rank) of 128 x 256 accumulators.
@@ -830,17 +804,9 @@ static int launch_gemm_mode(const void* A, const void* W, GemmParams& p, void* w
     }
     auto kern = gemm_bf16_kernel<BN, CG, MODE, LN, false>;
     if constexpr (kSkCapable) { if (sk) kern = gemm_bf16_kernel<BN, CG, MODE, LN, true>; }
-    static bool attr_done_dev[kMaxDevices][2] = {};       // the attribute is per device (one process may drive several GPUs)
-    bool& attr_done = attr_done_dev[current_device()][sk ? 1 : 0];
-    if (!attr_done) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes);
-        RAJNI_REQUIRE(e == cudaSuccess, RAJNI_ECUDA, "gemm: smem attribute (%d B): %s", Cfg::kSmemBytes, cudaGetErrorString(e));
-        attr_done = true;
-    }
-    cudaError_t e = launch_kernel(kern, dim3(grid), dim3(kGemmThreads), Cfg::kSmemBytes, stream, CG, ta, tb, p);
-    count_launch();
-    RAJNI_REQUIRE(e == cudaSuccess, RAJNI_ECUDA, "gemm_bf16: launch failed: %s", cudaGetErrorString(e));
-    return check_launch("gemm_bf16");
+    static int smem_granted[2][kMaxDevices] = {};
+    if (int rc = raise_smem_limit("gemm", kern, Cfg::kSmemBytes, smem_granted[sk ? 1 : 0])) return rc;
+    return launch_checked("gemm_bf16", kern, dim3(grid), dim3(kGemmThreads), Cfg::kSmemBytes, stream, CG, ta, tb, p);
 }
 
 static bool aligned32(const void* ptr) { return (reinterpret_cast<uintptr_t>(ptr) & 31u) == 0; }

@@ -186,14 +186,12 @@ extern "C" int rajni_resize_center_crop_u8(const void* frames, const long long* 
     int* err = reinterpret_cast<int*>(ws + (size_t)B * rs_image_bytes(max_h));
     cudaError_t e = cudaMemsetAsync(err, 0, sizeof(int), st);
     RAJNI_REQUIRE(e == cudaSuccess, RAJNI_ECUDA, "rajni_resize_center_crop_u8: memset: %s", cudaGetErrorString(e));
-    e = launch_kernel(resize_plan_kernel, dim3(B), dim3(2 * kRsCrop), 0, st, 1, meta, size, ws, max_h, err);
-    RAJNI_REQUIRE(e == cudaSuccess, RAJNI_ECUDA, "resize_plan: launch failed: %s", cudaGetErrorString(e));
-    e = launch_kernel(resize_h_kernel, dim3(max_h, B), dim3(kRsCrop), 0, st, 1, static_cast<const uint8_t*>(frames), meta, ws, max_h);
-    RAJNI_REQUIRE(e == cudaSuccess, RAJNI_ECUDA, "resize_h: launch failed: %s", cudaGetErrorString(e));
-    e = launch_kernel(resize_v_kernel, dim3(kRsCrop, B), dim3(kRsCrop), 0, st, 1, ws, max_h, static_cast<uint8_t*>(out));
-    RAJNI_REQUIRE(e == cudaSuccess, RAJNI_ECUDA, "resize_v: launch failed: %s", cudaGetErrorString(e));
-    count_launch(3);
-    return check_launch("resize_center_crop_u8");
+    if (int rc = launch_checked("resize_plan", resize_plan_kernel, dim3(B), dim3(2 * kRsCrop), 0, st, 1, meta, size, ws, max_h, err))
+        return rc;
+    if (int rc = launch_checked("resize_h", resize_h_kernel, dim3(max_h, B), dim3(kRsCrop), 0, st, 1,
+                                static_cast<const uint8_t*>(frames), meta, ws, max_h))
+        return rc;
+    return launch_checked("resize_v", resize_v_kernel, dim3(kRsCrop, B), dim3(kRsCrop), 0, st, 1, ws, max_h, static_cast<uint8_t*>(out));
 }
 
 /* 0 if every frame of the last call on this workspace was resized; 1 + the index of a frame that was rejected (smaller than

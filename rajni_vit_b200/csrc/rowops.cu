@@ -302,11 +302,8 @@ extern "C" int rajni_gather_rows(const void* src, const int32_t* row_map, void* 
     const long long total = (long long)rows_out * cpr;
     long long blocks = (total + 256 * 4 - 1) / (256 * 4);
     if (blocks > 148 * 16) blocks = 148 * 16;
-    cudaError_t e = launch_kernel(gather_rows_kernel, dim3((int)blocks), dim3(256), 0, static_cast<cudaStream_t>(stream), 1,
-                                  static_cast<const uint4*>(src), row_map, static_cast<uint4*>(dst), total, cpr);
-    count_launch();
-    RAJNI_REQUIRE(e == cudaSuccess, RAJNI_ECUDA, "gather_rows: launch failed: %s", cudaGetErrorString(e));
-    return check_launch("gather_rows");
+    return launch_checked("gather_rows", gather_rows_kernel, dim3((int)blocks), dim3(256), 0, static_cast<cudaStream_t>(stream), 1,
+                          static_cast<const uint4*>(src), row_map, static_cast<uint4*>(dst), total, cpr);
 }
 
 extern "C" int rajni_layernorm_strided(const void* x, long long in_row_stride, const float* gamma, const float* beta, float eps,
@@ -317,21 +314,15 @@ extern "C" int rajni_layernorm_strided(const void* x, long long in_row_stride, c
     const int cpl = (C / 8 + 31) / 32;
     const int wpb = 8;
     dim3 grid((rows + wpb - 1) / wpb), block(wpb * 32);
-    auto s = static_cast<cudaStream_t>(stream);
-    auto xb = static_cast<const __nv_bfloat16*>(x);
-    auto yb = static_cast<__nv_bfloat16*>(y);
-    const long long os = out_row_stride;
-    cudaError_t le = cudaSuccess;
+    auto kern = layernorm_kernel<8>;                          // cpl 5..8
     switch (cpl) {
-        case 1: le = launch_kernel(layernorm_kernel<1>, grid, block, 0, s, 1, xb, in_row_stride, gamma, beta, eps, yb, os, rows, C); break;
-        case 2: le = launch_kernel(layernorm_kernel<2>, grid, block, 0, s, 1, xb, in_row_stride, gamma, beta, eps, yb, os, rows, C); break;
-        case 3: le = launch_kernel(layernorm_kernel<3>, grid, block, 0, s, 1, xb, in_row_stride, gamma, beta, eps, yb, os, rows, C); break;
-        case 4: le = launch_kernel(layernorm_kernel<4>, grid, block, 0, s, 1, xb, in_row_stride, gamma, beta, eps, yb, os, rows, C); break;
-        default: le = launch_kernel(layernorm_kernel<8>, grid, block, 0, s, 1, xb, in_row_stride, gamma, beta, eps, yb, os, rows, C); break;
+        case 1: kern = layernorm_kernel<1>; break;
+        case 2: kern = layernorm_kernel<2>; break;
+        case 3: kern = layernorm_kernel<3>; break;
+        case 4: kern = layernorm_kernel<4>; break;
     }
-    count_launch();
-    RAJNI_REQUIRE(le == cudaSuccess, RAJNI_ECUDA, "layernorm: launch failed: %s", cudaGetErrorString(le));
-    return check_launch("layernorm");
+    return launch_checked("layernorm", kern, grid, block, 0, static_cast<cudaStream_t>(stream), 1, static_cast<const __nv_bfloat16*>(x),
+                          in_row_stride, gamma, beta, eps, static_cast<__nv_bfloat16*>(y), out_row_stride, rows, C);
 }
 
 extern "C" int rajni_layernorm(const void* x, long long in_row_stride, const float* gamma,
@@ -367,7 +358,6 @@ extern "C" int rajni_patch_im2col_prefix(const void* images, int image_dtype, in
     RAJNI_REQUIRE(row_stats == nullptr || (stats_slots > 0 && row_stats_ld >= (long long)B * (G * G + prefix)), RAJNI_EINVAL,
                   "rajni_patch_im2col: row_stats needs stats_slots > 0 and row_stats_ld >= B*(P+prefix)");
     auto s = static_cast<cudaStream_t>(stream);
-    cudaError_t le;
     // p = 16 keeps its own kernel: 16-pixel strips, px fastest.  On a B200 at 256 images of 224 px it moves fp32 images in
     // 41.7 us against the any-patch kernel's 44.3 us, uint8 pixels in 54.5 against 78.6 us (profiles/r3_kbench.txt).
     if (patch == 16) {
@@ -375,21 +365,18 @@ extern "C" int rajni_patch_im2col_prefix(const void* images, int image_dtype, in
         long long blocks = (strips + 255) / 256;
         if (blocks > 148 * 32) blocks = 148 * 32;
         auto kern = image_dtype == RAJNI_IMG_U8 ? im2col16_kernel<2> : image_dtype == RAJNI_IMG_F32 ? im2col16_kernel<1> : im2col16_kernel<0>;
-        le = launch_kernel(kern, dim3((int)blocks), dim3(256), 0, s, 1,
-                           images, nm, B, S, static_cast<__nv_bfloat16*>(cols), static_cast<const uint4*>(prefix_rows), prefix, ps,
-                           static_cast<uint4*>(x), C, reinterpret_cast<float2*>(row_stats), row_stats_ld, stats_slots);
+        return launch_checked("patch_im2col", kern, dim3((int)blocks), dim3(256), 0, s, 1,
+                              images, nm, B, S, static_cast<__nv_bfloat16*>(cols), static_cast<const uint4*>(prefix_rows), prefix, ps,
+                              static_cast<uint4*>(x), C, reinterpret_cast<float2*>(row_stats), row_stats_ld, stats_slots);
     } else {
         const long long runs = (long long)B * G * G * 3 * patch * (patch / 8);
         long long blocks = (runs + 256 * kIm2colUnroll - 1) / (256 * kIm2colUnroll);
         if (blocks > 148 * 32) blocks = 148 * 32;
         auto kern = image_dtype == RAJNI_IMG_U8 ? im2col_kernel<2> : image_dtype == RAJNI_IMG_F32 ? im2col_kernel<1> : im2col_kernel<0>;
-        le = launch_kernel(kern, dim3((int)blocks), dim3(256), 0, s, 1,
-                           images, nm, B, S, patch, static_cast<__nv_bfloat16*>(cols), static_cast<const uint4*>(prefix_rows), prefix, ps,
-                           static_cast<uint4*>(x), C, reinterpret_cast<float2*>(row_stats), row_stats_ld, stats_slots);
+        return launch_checked("patch_im2col", kern, dim3((int)blocks), dim3(256), 0, s, 1,
+                              images, nm, B, S, patch, static_cast<__nv_bfloat16*>(cols), static_cast<const uint4*>(prefix_rows), prefix, ps,
+                              static_cast<uint4*>(x), C, reinterpret_cast<float2*>(row_stats), row_stats_ld, stats_slots);
     }
-    count_launch();
-    RAJNI_REQUIRE(le == cudaSuccess, RAJNI_ECUDA, "patch_im2col: launch failed: %s", cudaGetErrorString(le));
-    return check_launch("patch_im2col");
 }
 
 extern "C" int rajni_patch_im2col(const void* images, int image_dtype, int B, int S, int patch,

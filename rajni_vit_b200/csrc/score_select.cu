@@ -553,12 +553,9 @@ static int launch_score_select(const ScoreSelectParams& p, int B, cudaStream_t s
         case 4: kern = score_select_kernel<4>; break;
         default: RAJNI_REQUIRE(false, RAJNI_EINVAL, "score_select: C=%d > 1024 unsupported", p.C);
     }
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    RAJNI_REQUIRE(e == cudaSuccess, RAJNI_ECUDA, "score_select: smem attribute: %s", cudaGetErrorString(e));
-    e = launch_kernel(kern, dim3(B), dim3(kSelThreads), smem, stream, 1, p);
-    count_launch();
-    RAJNI_REQUIRE(e == cudaSuccess, RAJNI_ECUDA, "score_select: launch failed: %s", cudaGetErrorString(e));
-    return check_launch("score_select");
+    static int smem_granted[4][kMaxDevices] = {};
+    if (int rc = raise_smem_limit("score_select", kern, (int)smem, smem_granted[cpl - 1])) return rc;
+    return launch_checked("score_select", kern, dim3(B), dim3(kSelThreads), smem, stream, 1, p);
 }
 
 // true when one image's CLS logits and value rows do not fit the per-image kernel's shared memory
@@ -566,12 +563,9 @@ static bool needs_workspace_tail(int N, int H) { return score_smem_bytes(N, H, t
 
 static int launch_score_tail_ws(const ScoreSelectParams& p, float* logit_g, int B, cudaStream_t stream) {
     const size_t smem = score_smem_bytes(p.N, 0, false, false);
-    cudaError_t e = cudaFuncSetAttribute(score_tail_ws_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    RAJNI_REQUIRE(e == cudaSuccess, RAJNI_ECUDA, "score_tail_ws: smem attribute: %s", cudaGetErrorString(e));
-    e = launch_kernel(score_tail_ws_kernel, dim3(B), dim3(kSelThreads), smem, stream, 1, p, logit_g);
-    count_launch();
-    RAJNI_REQUIRE(e == cudaSuccess, RAJNI_ECUDA, "score_tail_ws: launch failed: %s", cudaGetErrorString(e));
-    return check_launch("score_tail_ws");
+    static int smem_granted[kMaxDevices] = {};
+    if (int rc = raise_smem_limit("score_tail_ws", score_tail_ws_kernel, (int)smem, smem_granted)) return rc;
+    return launch_checked("score_tail_ws", score_tail_ws_kernel, dim3(B), dim3(kSelThreads), smem, stream, 1, p, logit_g);
 }
 
 static size_t split_workspace_floats(int B, int N, int H) {
@@ -590,11 +584,8 @@ static int launch_score_stream(const __nv_bfloat16* qkv, int B, int N, int C, in
         case 4: kern = score_stream_kernel<4>; break;
         default: RAJNI_REQUIRE(false, RAJNI_EINVAL, "score_select: C=%d > 1024 unsupported", C);
     }
-    cudaError_t e = launch_kernel(kern, dim3((N + kStreamRows - 1) / kStreamRows, B), dim3(kStreamThreads), 0, stream, 1,
-                                  qkv, logit_g, vm_g, N, C, H);
-    count_launch();
-    RAJNI_REQUIRE(e == cudaSuccess, RAJNI_ECUDA, "score_stream: launch failed: %s", cudaGetErrorString(e));
-    return check_launch("score_stream");
+    return launch_checked("score_stream", kern, dim3((N + kStreamRows - 1) / kStreamRows, B), dim3(kStreamThreads), 0, stream, 1,
+                          qkv, logit_g, vm_g, N, C, H);
 }
 
 static int check_score_shape(int B, int N, int C, int H) {
