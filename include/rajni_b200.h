@@ -124,6 +124,21 @@ int rajni_layernorm(const void* x, long long in_row_stride, const float* gamma,
  * normalised CLS and distillation rows of each image side by side, the A operand of a distilled model's head. */
 int rajni_layernorm_strided(const void* x, long long in_row_stride, const float* gamma, const float* beta, float eps,
                             void* y, long long out_row_stride, int rows, int C, void* stream);
+/* The same over a whole activation matrix, also emitting the rows' LayerNorm partial sums for an LN-folded GEMM
+ * (RAJNI_EPI_LN_FOLD) that reads y next: row_stats[s*row_stats_ld + r] = (sum, sum of squares) of the bf16 row r as stored
+ * for s = 0, zero for s = 1..stats_slots-1 (the slot layout of RAJNI_EPI_ROW_STATS).  y may be x (in place).  This is the
+ * pre-norm stem of CLIP ViTs (timm's norm_pre), applied to the embedded tokens before block 0.  C <= 2048. */
+int rajni_layernorm_row_stats(const void* x, long long in_row_stride, const float* gamma, const float* beta, float eps,
+                              void* y, long long out_row_stride, int rows, int C,
+                              float* row_stats, long long row_stats_ld, int stats_slots, void* stream);
+
+/* ---- average-pooled head (timm global_pool='avg' with fc_norm: MAE fine-tuned ViTs)
+ * y[b*out_row_stride + c] = LN(mean_{n = prefix..N-1} x[b*N + n, :])[c] in bf16, x [B*N, C] bf16 dense, gamma / beta fp32
+ * [C].  The mean is an fp32 sum of the bf16 rows divided by N - prefix (the patch tokens; prefix 1 or 2), the LayerNorm is
+ * fp32 with a centred variance.  The summation order depends on N, prefix and C only, so an image's row is bit-identical
+ * in any batch.  C a multiple of 64 up to 2048, B <= 65535. */
+int rajni_mean_pool_layernorm(const void* x, int B, int N, int prefix, int C, const float* gamma, const float* beta,
+                              float eps, void* y, long long out_row_stride, void* stream);
 
 /* ---- dense contractions (attention.py:22,55; timm Mlp fc1/fc2; patch_embed; head)
  * D[orow(m), n] = epi( sum_k A[m,k] * W[n,k] ), A [M,K] bf16, W [N,K] bf16

@@ -22,9 +22,16 @@ width / 64, the only head dimension the kernels (and every BASELINE config) use.
   * DeiT-III: ``blocks.{i}.ls1.gamma`` / ``ls2.gamma`` (LayerScale, accepted only when every block has both), and a
     ``pos_embed`` with one row per patch (a square length: no position for the class token, timm's ``no_embed_class``);
   * distilled DeiT: ``dist_token`` together with ``head_dist.*``, ``pos_embed`` of patches + 2.
-Checkpoints outside the wrapper's contract — partial LayerScale, ``norm_pre``, ``fc_norm``, register
-tokens, a distillation token without its head, qk-norm — raise ``NotImplementedError`` naming the offending keys: never a
-silent partial load.
+So do the two head / stem variants:
+  * average pooling (MAE fine-tunes): ``fc_norm.weight`` and ``fc_norm.bias`` and no ``norm.*`` (timm
+    ``global_pool='avg'``: the head reads fc_norm of the patch tokens' mean);
+  * a pre-norm stem (CLIP fine-tunes): ``norm_pre.weight`` and ``norm_pre.bias``.  A checkpoint does not record LayerNorm
+    eps; timm's CLIP ViTs, the models with this stem, use 1e-5 everywhere, so that is what a pre-norm model gets (1e-6
+    otherwise);
+  * a patch embedding without bias (CLIP): no ``patch_embed.proj.bias``.
+Checkpoints outside the wrapper's contract — partial LayerScale, a partial ``norm_pre`` or ``fc_norm``, ``fc_norm`` next
+to ``norm``, register tokens, a distillation token without its head, qk-norm — raise ``NotImplementedError`` naming the
+offending keys: never a silent partial load.
 """
 from __future__ import annotations
 
@@ -41,7 +48,7 @@ from .vit import VisionTransformer
 _SAFETENSORS_DTYPES = {"F32": torch.float32, "F16": torch.float16, "BF16": torch.bfloat16, "F64": torch.float64,
                        "I64": torch.int64, "I32": torch.int32, "U8": torch.uint8, "BOOL": torch.bool}
 
-_UNSUPPORTED = (r"\.ls[12]\.(?!gamma$)", r"^norm_pre\.", r"^fc_norm\.", r"^reg_token$",
+_UNSUPPORTED = (r"\.ls[12]\.(?!gamma$)", r"^norm_pre\.(?!(weight|bias)$)", r"^fc_norm\.(?!(weight|bias)$)", r"^reg_token$",
                 r"\.attn\.[qk]_norm\.", r"^patch_embed\.norm\.", r"\.mlp\.norm\.", r"rel_pos", r"^pre_logits\.")
 
 
@@ -118,13 +125,26 @@ def normalise_keys(sd: Mapping[str, torch.Tensor]) -> Dict[str, torch.Tensor]:
 
 
 def infer_config(sd: Mapping[str, torch.Tensor]) -> Dict[str, int]:
-    for k in ("cls_token", "pos_embed", "patch_embed.proj.weight", "head.weight", "norm.weight"):
+    for k in ("cls_token", "pos_embed", "patch_embed.proj.weight", "head.weight"):
         if k not in sd:
             raise KeyError(f"checkpoint has no {k!r}: not a timm-named ViT state dict (keys start with {sorted(sd)[:4]})")
     bad = sorted(k for k in sd if any(re.search(p, k) for p in _UNSUPPORTED))
     if bad:
         raise NotImplementedError(f"checkpoint uses features outside the RAJNI wrapper's contract: {bad[:6]}"
                                   f"{' ...' if len(bad) > 6 else ''}")
+    # the final LayerNorm: `norm` before class-token pooling, or `fc_norm` after average pooling - never both, never partial
+    fam = {name: sorted(k for k in sd if k.startswith(name + ".")) for name in ("norm", "fc_norm", "norm_pre")}
+    for name, keys in fam.items():
+        if keys and keys != [f"{name}.bias", f"{name}.weight"]:
+            raise NotImplementedError(f"{name} must be a LayerNorm with weight and bias: the checkpoint has {keys}")
+    if fam["fc_norm"] and fam["norm"]:
+        raise NotImplementedError(f"fc_norm next to norm is not supported (average pooling has norm = Identity): {fam['fc_norm']} "
+                                  f"and {fam['norm']}")
+    if not fam["fc_norm"] and not fam["norm"]:
+        raise KeyError("checkpoint has neither 'norm.weight' nor 'fc_norm.weight': not a timm-named ViT state dict")
+    avg_pool, pre_norm = bool(fam["fc_norm"]), bool(fam["norm_pre"])
+    if avg_pool and "dist_token" in sd:
+        raise NotImplementedError("fc_norm (global_pool='avg') with a distillation token is not supported")
     C = sd["cls_token"].shape[-1]
     pw = sd["patch_embed.proj.weight"]
     if pw.dim() != 4 or pw.shape[1] != 3 or pw.shape[2] != pw.shape[3]:
@@ -162,7 +182,8 @@ def infer_config(sd: Mapping[str, torch.Tensor]) -> Dict[str, int]:
     hidden = sd["blocks.0.mlp.fc1.weight"].shape[0]
     return dict(embed_dim=C, depth=len(blocks), num_heads=C // 64, img_size=grid * patch, patch_size=patch,
                 num_classes=sd["head.weight"].shape[0], mlp_ratio=hidden / C, init_values=1.0 if ls else None,
-                no_embed_class=no_embed_class, distilled=dist)
+                no_embed_class=no_embed_class, distilled=dist, global_pool="avg" if avg_pool else "token", fc_norm=avg_pool,
+                pre_norm=pre_norm, patch_bias="patch_embed.proj.bias" in sd, norm_eps=1e-5 if pre_norm else 1e-6)
 
 
 def load_checkpoint(source: Union[str, os.PathLike, Mapping[str, torch.Tensor]], model: Optional[torch.nn.Module] = None,

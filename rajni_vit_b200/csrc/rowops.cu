@@ -38,10 +38,14 @@ __global__ void __launch_bounds__(256) gather_rows_kernel(const uint4* __restric
 // ------------------------------------------------------------------ LayerNorm
 // One warp per row, the row held in registers (CPL 16-byte chunks per lane), fp32 math:
 // mean, then centred variance (biased, like nn.LayerNorm), y = (x-mean)*rstd*gamma+beta.
-template <int CPL>
+// STATS: also write the row's LayerNorm partial sums in the RAJNI_EPI_ROW_STATS layout that the LN-folded GEMMs read
+// (slot 0 = (sum, sum of squares) of the stored bf16 row, the other slots zero, as write_prefix_rows does).  Every load
+// of a row precedes its first store (the stores need the row's mean), so y may be x.
+template <int CPL, bool STATS = false>
 __global__ void __launch_bounds__(256) layernorm_kernel(const __nv_bfloat16* __restrict__ x, long long in_stride,
                                                         const float* __restrict__ gamma, const float* __restrict__ beta,
-                                                        float eps, __nv_bfloat16* __restrict__ y, long long out_stride, int rows, int C) {
+                                                        float eps, __nv_bfloat16* __restrict__ y, long long out_stride, int rows, int C,
+                                                        float2* __restrict__ row_stats, long long stats_ld, int stats_slots) {
     griddep_launch();
     griddep_wait();
     const int lane = threadIdx.x & 31;
@@ -77,6 +81,7 @@ __global__ void __launch_bounds__(256) layernorm_kernel(const __nv_bfloat16* __r
     }
     const float rstd = rsqrtf(warp_sum(sq) / (float)C + eps);
     __nv_bfloat16* yr = y + (long long)row * out_stride;
+    float osum = 0.f, osq = 0.f;
 #pragma unroll
     for (int i = 0; i < CPL; ++i) {
         int j = lane + 32 * i;
@@ -91,8 +96,120 @@ __global__ void __launch_bounds__(256) layernorm_kernel(const __nv_bfloat16* __r
             o.z = float2_to_bf16x2((v[i][4] - mean) * rstd * g1.x + b1.x, (v[i][5] - mean) * rstd * g1.y + b1.y);
             o.w = float2_to_bf16x2((v[i][6] - mean) * rstd * g1.z + b1.z, (v[i][7] - mean) * rstd * g1.w + b1.w);
             st_stream16(yr + j * 8, o);
+            if (STATS) {
+                const uint32_t w[4] = {o.x, o.y, o.z, o.w};
+#pragma unroll
+                for (int k = 0; k < 4; ++k) {
+                    const float2 f = bf16x2_to_float2(w[k]);
+                    osum += f.x + f.y;
+                    osq += f.x * f.x + f.y * f.y;
+                }
+            }
         }
     }
+    if (STATS) {
+        osum = warp_sum(osum);
+        osq = warp_sum(osq);
+        for (int s = lane; s < stats_slots; s += 32)
+            row_stats[(long long)s * stats_ld + row] = s == 0 ? make_float2(osum, osq) : make_float2(0.f, 0.f);
+    }
+}
+
+// ------------------------------------------------------------------ average pooling + fc_norm
+// y[b,:] = LN(mean(x[b*N + P0 .. b*N + N-1, :])): timm's head with global_pool='avg' (fc_norm over the mean of the patch
+// tokens).  One cluster of kPoolCluster CTAs per image, CTA r owning columns [r*C/8, (r+1)*C/8): at 256 images that is
+// 2048 CTAs to stream the rows, and the LayerNorm statistics of the mean row are combined over the cluster through DSMEM.
+// Thread t sums chunk t % K (8 columns, K = C/64 chunks per CTA) over rows P0 + t/K, P0 + t/K + G, ... (G = 256/K row
+// groups) in fp32, then the G partials of a column are added in group order and divided by N - P0.  The order depends on
+// N, P0 and C only: an image's pooled row is bit-identical in any batch.
+constexpr int kPoolCluster = 8;
+constexpr int kPoolThreads = 256;
+constexpr int kPoolUnroll = 4;              // row loads in flight per thread
+
+__device__ __forceinline__ float ld_cluster_f32(uint32_t addr) {
+    float v;
+    asm volatile("ld.shared::cluster.f32 %0, [%1];" : "=f"(v) : "r"(addr) : "memory");
+    return v;
+}
+
+// Sum of v over the CTA (fixed order: lanes, then warps 0..7), then over the cluster's CTAs 0..7 (every CTA adds the same
+// eight values in the same order, so all get the same bits).  slot: this CTA's shared word that its partial goes to.
+__device__ __forceinline__ float pool_cluster_sum(float v, float* warp_part, float* slot) {
+    v = warp_sum(v);
+    if ((threadIdx.x & 31) == 0) warp_part[threadIdx.x >> 5] = v;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        float t = 0.f;
+#pragma unroll
+        for (int w = 0; w < kPoolThreads / 32; ++w) t += warp_part[w];
+        *slot = t;
+    }
+    cluster_sync_all();
+    float t = 0.f;
+#pragma unroll
+    for (int r = 0; r < kPoolCluster; ++r) t += ld_cluster_f32(mapa_u32(smem_u32(slot), r));
+    return t;
+}
+
+__global__ void __launch_bounds__(kPoolThreads, 4) mean_pool_layernorm_kernel(const __nv_bfloat16* __restrict__ x, int N, int P0, int C,
+                                                                           const float* __restrict__ gamma, const float* __restrict__ beta,
+                                                                           float eps, __nv_bfloat16* __restrict__ y, long long out_stride) {
+    __shared__ float part[kPoolThreads * 8];
+    __shared__ float warp_part[kPoolThreads / 32];
+    __shared__ float red[2];
+    griddep_launch();
+    griddep_wait();
+    const int b = blockIdx.y;
+    const int cs = C / kPoolCluster;                            // columns of this CTA (multiple of 8)
+    const int K = cs >> 3, G = kPoolThreads / K;
+    const int c0 = (int)cluster_ctarank() * cs;
+    const int t = threadIdx.x, j = t % K, g = t / K;
+    if (g < G) {
+        float acc[8];
+#pragma unroll
+        for (int e = 0; e < 8; ++e) acc[e] = 0.f;
+        const __nv_bfloat16* base = x + (long long)b * N * C + c0 + j * 8;
+        int n = P0 + g;
+        for (; n + (kPoolUnroll - 1) * G < N; n += kPoolUnroll * G) {
+            uint4 u[kPoolUnroll];
+#pragma unroll
+            for (int k = 0; k < kPoolUnroll; ++k) u[k] = ld_stream16(base + (long long)(n + k * G) * C);
+#pragma unroll
+            for (int k = 0; k < kPoolUnroll; ++k) {
+                const uint32_t w[4] = {u[k].x, u[k].y, u[k].z, u[k].w};
+#pragma unroll
+                for (int q = 0; q < 4; ++q) {
+                    const float2 f = bf16x2_to_float2(w[q]);
+                    acc[2 * q] += f.x;
+                    acc[2 * q + 1] += f.y;
+                }
+            }
+        }
+        for (; n < N; n += G) {
+            const uint4 u = ld_stream16(base + (long long)n * C);
+            const uint32_t w[4] = {u.x, u.y, u.z, u.w};
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                const float2 f = bf16x2_to_float2(w[q]);
+                acc[2 * q] += f.x;
+                acc[2 * q + 1] += f.y;
+            }
+        }
+#pragma unroll
+        for (int e = 0; e < 8; ++e) part[g * cs + j * 8 + e] = acc[e];
+    }
+    __syncthreads();
+    float m = 0.f;                                              // this thread's column of the mean row (t < cs)
+    if (t < cs) {
+        float s = 0.f;
+        for (int q = 0; q < G; ++q) s += part[q * cs + t];
+        m = s / (float)(N - P0);
+    }
+    const float mean = pool_cluster_sum(m, warp_part, &red[0]) / (float)C;
+    const float d = t < cs ? m - mean : 0.f;
+    const float rstd = rsqrtf(pool_cluster_sum(d * d, warp_part, &red[1]) / (float)C + eps);
+    if (t < cs) y[(long long)b * out_stride + c0 + t] = __float2bfloat16_rn(d * rstd * gamma[c0 + t] + beta[c0 + t]);
+    cluster_sync_all();                                         // no CTA leaves while another may still read its red[]
 }
 
 // ------------------------------------------------------------------ patch im2col (+ prefix rows)
@@ -322,7 +439,45 @@ extern "C" int rajni_layernorm_strided(const void* x, long long in_row_stride, c
         case 4: kern = layernorm_kernel<4>; break;
     }
     return launch_checked("layernorm", kern, grid, block, 0, static_cast<cudaStream_t>(stream), 1, static_cast<const __nv_bfloat16*>(x),
-                          in_row_stride, gamma, beta, eps, static_cast<__nv_bfloat16*>(y), out_row_stride, rows, C);
+                          in_row_stride, gamma, beta, eps, static_cast<__nv_bfloat16*>(y), out_row_stride, rows, C,
+                          static_cast<float2*>(nullptr), 0LL, 0);
+}
+
+extern "C" int rajni_layernorm_row_stats(const void* x, long long in_row_stride, const float* gamma, const float* beta, float eps,
+                                         void* y, long long out_row_stride, int rows, int C,
+                                         float* row_stats, long long row_stats_ld, int stats_slots, void* stream) {
+    RAJNI_REQUIRE(x && gamma && beta && y && row_stats, RAJNI_EINVAL, "rajni_layernorm_row_stats: null pointer");
+    RAJNI_REQUIRE(rows > 0 && C > 0 && C % 8 == 0 && C <= 2048 && in_row_stride % 8 == 0 && out_row_stride % 8 == 0 && out_row_stride >= C,
+                  RAJNI_EINVAL, "rajni_layernorm_row_stats: rows=%d C=%d stride=%lld out stride=%lld unsupported", rows, C, in_row_stride,
+                  out_row_stride);
+    RAJNI_REQUIRE(stats_slots > 0 && row_stats_ld >= rows, RAJNI_EINVAL,
+                  "rajni_layernorm_row_stats: stats_slots=%d row_stats_ld=%lld (need slots > 0 and ld >= rows=%d)", stats_slots,
+                  row_stats_ld, rows);
+    const int cpl = (C / 8 + 31) / 32;
+    const int wpb = 8;
+    dim3 grid((rows + wpb - 1) / wpb), block(wpb * 32);
+    auto kern = layernorm_kernel<8, true>;                    // cpl 5..8
+    switch (cpl) {
+        case 1: kern = layernorm_kernel<1, true>; break;
+        case 2: kern = layernorm_kernel<2, true>; break;
+        case 3: kern = layernorm_kernel<3, true>; break;
+        case 4: kern = layernorm_kernel<4, true>; break;
+    }
+    return launch_checked("layernorm_row_stats", kern, grid, block, 0, static_cast<cudaStream_t>(stream), 1,
+                          static_cast<const __nv_bfloat16*>(x), in_row_stride, gamma, beta, eps, static_cast<__nv_bfloat16*>(y),
+                          out_row_stride, rows, C, reinterpret_cast<float2*>(row_stats), row_stats_ld, stats_slots);
+}
+
+extern "C" int rajni_mean_pool_layernorm(const void* x, int B, int N, int prefix, int C, const float* gamma, const float* beta,
+                                         float eps, void* y, long long out_row_stride, void* stream) {
+    RAJNI_REQUIRE(x && gamma && beta && y, RAJNI_EINVAL, "rajni_mean_pool_layernorm: null pointer");
+    RAJNI_REQUIRE(B > 0 && B <= 65535 && prefix >= 1 && prefix <= kMaxPrefix && N > prefix && C > 0 && C % 64 == 0 && C <= 2048 &&
+                  out_row_stride >= C && out_row_stride % 8 == 0, RAJNI_EINVAL,
+                  "rajni_mean_pool_layernorm: B=%d N=%d prefix=%d C=%d out stride=%lld unsupported (C a multiple of 64 up to 2048, "
+                  "N > prefix, prefix 1 or 2)", B, N, prefix, C, out_row_stride);
+    return launch_checked("mean_pool_layernorm", mean_pool_layernorm_kernel, dim3(kPoolCluster, B), dim3(kPoolThreads), 0,
+                          static_cast<cudaStream_t>(stream), kPoolCluster, static_cast<const __nv_bfloat16*>(x), N, prefix, C, gamma,
+                          beta, eps, static_cast<__nv_bfloat16*>(y), out_row_stride);
 }
 
 extern "C" int rajni_layernorm(const void* x, long long in_row_stride, const float* gamma,

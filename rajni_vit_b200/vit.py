@@ -13,13 +13,20 @@ those attribute names and timm's ViT semantics:
                 mlp{fc1, act=GELU(erf), fc2}, ls1/ls2/drop_path1/drop_path2 = Identity
     norm, head
 
-and the two DeiT families (extra fields in VIT_VARIANT):
+(and timm's ``norm_pre``, ``fc_norm`` = Identity), and the two DeiT families (extra fields in VIT_VARIANT):
 
     DeiT-III (``deit3_*``): ls1/ls2 = LayerScale (``gamma`` [C]), and no position for the class token
         (timm's ``no_embed_class``: pos_embed [1,P,C] is added to the patches before the class token is prepended);
     distilled DeiT (``deit_*_distilled_*``): a distillation token after the class token (``dist_token``,
         ``num_prefix_tokens = 2``, pos_embed [1,2+P,C]) and a second head ``head_dist`` on it; in eval mode the output is
-        ``(head(x[:,0]) + head_dist(x[:,1])) / 2``.
+        ``(head(x[:,0]) + head_dist(x[:,1])) / 2``;
+
+and two head / stem variants (extra fields in VIT_POOL_PRENORM):
+
+    average pooling (MAE fine-tunes, ``*_mae``): ``global_pool='avg'``, ``norm`` = Identity and ``fc_norm`` = LayerNorm,
+        the output is ``head(fc_norm(x[:, 1:].mean(1)))`` (timm's ``forward_head``);
+    a pre-norm stem (CLIP, ``*_clip_*``): a patch embedding without bias, ``norm_pre`` = LayerNorm applied to the embedded
+        tokens before block 0, and LayerNorm eps 1e-5 everywhere.
 
 It is a plain eager PyTorch module.  It is NOT on the accelerated path: the
 B200 wrapper reads its leaf parameters and runs its own kernels.
@@ -59,26 +66,38 @@ VIT_CONFIGS = {
     # 4-block test models of the two families: 16 + 1 and 16 + 2 tokens
     "deit3_micro_patch16_64": (128, 4, 2, 64),
     "deit_micro_distilled_patch16_64": (128, 4, 2, 64),
+    # average pooling with fc_norm (MAE fine-tunes) and a pre-norm stem (CLIP fine-tunes), and a 4-block test model of each
+    "vit_base_patch16_224_mae": (768, 12, 12, 224),
+    "vit_large_patch16_224_mae": (1024, 24, 16, 224),
+    "vit_base_patch16_clip_224": (768, 12, 12, 224),
+    "vit_base_patch32_clip_224": (768, 12, 12, 224),
+    "vit_base_patch16_clip_384": (768, 12, 12, 384),
+    "vit_micro_patch16_64_mae": (128, 4, 2, 64),
+    "vit_micro_patch16_64_clip": (128, 4, 2, 64),
 }
 # name -> patch size (pixels per side of a patch; 50 tokens at 224 px for 32, 785 for 8)
 VIT_PATCH = {name: 16 for name in VIT_CONFIGS}
-VIT_PATCH.update({"vit_small_patch32_224": 32, "vit_base_patch32_224": 32, "vit_micro_patch32_128": 32,
+VIT_PATCH.update({"vit_small_patch32_224": 32, "vit_base_patch32_224": 32, "vit_micro_patch32_128": 32, "vit_base_patch32_clip_224": 32,
                   "vit_small_patch8_224": 8, "vit_base_patch8_224": 8, "vit_micro_patch8_72": 8})
 # name -> extra VisionTransformer arguments of the DeiT families (timm's deit3_* use init_values=1e-6 and no_embed_class;
 # create_model spreads the LayerScale gammas, see spread_layer_scale)
 _DEIT3 = dict(init_values=1e-6, no_embed_class=True)
 VIT_VARIANT = {name: dict(_DEIT3) for name in VIT_CONFIGS if name.startswith("deit3_")}
 VIT_VARIANT.update({name: dict(distilled=True) for name in VIT_CONFIGS if "_distilled_" in name})
+# name -> extra VisionTransformer arguments of the pooled and pre-norm families (timm's *_mae fine-tunes: global_pool='avg',
+# fc_norm; *_clip_*: pre_norm, no patch-embed bias, LayerNorm eps 1e-5)
+VIT_POOL_PRENORM = {name: dict(global_pool="avg", fc_norm=True) for name in VIT_CONFIGS if name.endswith("_mae")}
+VIT_POOL_PRENORM.update({name: dict(pre_norm=True, patch_bias=False, norm_eps=1e-5) for name in VIT_CONFIGS if "_clip" in name})
 
 
 class PatchEmbed(nn.Module):
-    def __init__(self, img_size, patch, in_chans, dim):
+    def __init__(self, img_size, patch, in_chans, dim, bias=True):
         super().__init__()
         self.img_size = (img_size, img_size)
         self.patch_size = (patch, patch)
         self.grid_size = (img_size // patch, img_size // patch)
         self.num_patches = self.grid_size[0] * self.grid_size[1]
-        self.proj = nn.Conv2d(in_chans, dim, kernel_size=patch, stride=patch)
+        self.proj = nn.Conv2d(in_chans, dim, kernel_size=patch, stride=patch, bias=bias)
         self.norm = nn.Identity()
 
     def forward(self, x):
@@ -135,13 +154,13 @@ class LayerScale(nn.Module):
 
 
 class Block(nn.Module):
-    def __init__(self, dim, num_heads, mlp_ratio=4.0, init_values=None):
+    def __init__(self, dim, num_heads, mlp_ratio=4.0, init_values=None, norm_eps=1e-6):
         super().__init__()
-        self.norm1 = nn.LayerNorm(dim, eps=1e-6)
+        self.norm1 = nn.LayerNorm(dim, eps=norm_eps)
         self.attn = Attention(dim, num_heads)
         self.ls1 = LayerScale(dim, init_values) if init_values else nn.Identity()
         self.drop_path1 = nn.Identity()
-        self.norm2 = nn.LayerNorm(dim, eps=1e-6)
+        self.norm2 = nn.LayerNorm(dim, eps=norm_eps)
         self.mlp = Mlp(dim, int(dim * mlp_ratio))
         self.ls2 = LayerScale(dim, init_values) if init_values else nn.Identity()
         self.drop_path2 = nn.Identity()
@@ -154,28 +173,32 @@ class Block(nn.Module):
 
 class VisionTransformer(nn.Module):
     """``init_values``: LayerScale after attention and MLP (None: Identity).  ``no_embed_class``: pos_embed covers the patches
-    only.  ``distilled``: a distillation token and ``head_dist`` (timm's VisionTransformerDistilled, eval-mode output)."""
+    only.  ``distilled``: a distillation token and ``head_dist`` (timm's VisionTransformerDistilled, eval-mode output).
+    ``global_pool``: 'token' (class token) or 'avg' (mean of the tokens after the prefix); ``fc_norm``: the final LayerNorm
+    after pooling instead of before it (None: timm's default, on for 'avg').  ``pre_norm``: ``norm_pre`` LayerNorm after the
+    embedding.  ``patch_bias``: the patch projection has a bias.  ``norm_eps``: eps of every LayerNorm."""
 
     def __init__(self, img_size=224, patch_size=16, in_chans=3, num_classes=1000,
                  embed_dim=768, depth=12, num_heads=12, mlp_ratio=4.0, init_values=None, no_embed_class=False,
-                 distilled=False):
+                 distilled=False, global_pool="token", fc_norm=None, pre_norm=False, patch_bias=True, norm_eps=1e-6):
         super().__init__()
+        use_fc_norm = global_pool == "avg" if fc_norm is None else fc_norm
         self.num_classes = num_classes
         self.embed_dim = self.num_features = embed_dim
-        self.global_pool = "token"
+        self.global_pool = global_pool
         self.num_prefix_tokens = 2 if distilled else 1
         self.no_embed_class = no_embed_class
-        self.patch_embed = PatchEmbed(img_size, patch_size, in_chans, embed_dim)
+        self.patch_embed = PatchEmbed(img_size, patch_size, in_chans, embed_dim, bias=patch_bias)
         n_tok = self.patch_embed.num_patches + (0 if no_embed_class else self.num_prefix_tokens)
         self.cls_token = nn.Parameter(torch.zeros(1, 1, embed_dim))
         self.dist_token = nn.Parameter(torch.zeros(1, 1, embed_dim)) if distilled else None
         self.pos_embed = nn.Parameter(torch.zeros(1, n_tok, embed_dim))
         self.pos_drop = nn.Dropout(0.0)
         self.patch_drop = nn.Identity()
-        self.norm_pre = nn.Identity()
-        self.blocks = nn.Sequential(*[Block(embed_dim, num_heads, mlp_ratio, init_values) for _ in range(depth)])
-        self.norm = nn.LayerNorm(embed_dim, eps=1e-6)
-        self.fc_norm = nn.Identity()
+        self.norm_pre = nn.LayerNorm(embed_dim, eps=norm_eps) if pre_norm else nn.Identity()
+        self.blocks = nn.Sequential(*[Block(embed_dim, num_heads, mlp_ratio, init_values, norm_eps) for _ in range(depth)])
+        self.norm = nn.Identity() if use_fc_norm else nn.LayerNorm(embed_dim, eps=norm_eps)
+        self.fc_norm = nn.LayerNorm(embed_dim, eps=norm_eps) if use_fc_norm else nn.Identity()
         self.head_drop = nn.Dropout(0.0)
         self.head = nn.Linear(embed_dim, num_classes)
         self.head_dist = nn.Linear(embed_dim, num_classes) if distilled else None
@@ -201,7 +224,8 @@ class VisionTransformer(nn.Module):
         x = self.forward_features(x)
         if self.head_dist is not None:                          # timm VisionTransformerDistilled, eval mode
             return (self.head(self.head_drop(x[:, 0])) + self.head_dist(self.head_drop(x[:, 1]))) / 2
-        return self.head(self.head_drop(self.fc_norm(x[:, 0])))
+        x = x[:, self.num_prefix_tokens:].mean(dim=1) if self.global_pool == "avg" else x[:, 0]     # timm forward_head
+        return self.head(self.head_drop(self.fc_norm(x)))
 
 
 def create_model(name: str, seed: int | None = 0, bf16_round: bool = True,
@@ -216,7 +240,7 @@ def create_model(name: str, seed: int | None = 0, bf16_round: bool = True,
     if seed is not None:
         gen_state = torch.random.get_rng_state()
         torch.manual_seed(seed)
-    variant = VIT_VARIANT.get(name, {})
+    variant = {**VIT_VARIANT.get(name, {}), **VIT_POOL_PRENORM.get(name, {})}
     model = VisionTransformer(img_size=img, patch_size=VIT_PATCH[name], embed_dim=dim, depth=depth, num_heads=heads,
                               num_classes=num_classes, **variant)
     if seed is not None:
@@ -258,9 +282,10 @@ def randomize_trained_like(model: VisionTransformer, seed: int = 0, outlier_chan
     hot = torch.randperm(C, generator=g)[:outlier_channels]
     with torch.no_grad():
         for name, p in model.named_parameters():
-            if name.endswith("norm1.weight") or name.endswith("norm2.weight") or name == "norm.weight":
+            if name.endswith("norm1.weight") or name.endswith("norm2.weight") or name in ("norm.weight", "fc_norm.weight",
+                                                                                        "norm_pre.weight"):
                 p.copy_(0.3 + 2.2 * torch.rand(p.shape, generator=g))
-            elif name.endswith("norm1.bias") or name.endswith("norm2.bias") or name == "norm.bias":
+            elif name.endswith("norm1.bias") or name.endswith("norm2.bias") or name in ("norm.bias", "fc_norm.bias", "norm_pre.bias"):
                 p.copy_(0.3 * torch.randn(p.shape, generator=g))
             elif name.endswith(".bias"):
                 p.copy_(0.5 * torch.randn(p.shape, generator=g))

@@ -15,7 +15,10 @@ Deliberate deviations from the reference (SURVEY.md section 5):
 
 Beyond the reference's models it runs the two DeiT families: LayerScale (DeiT-III's ``ls1`` / ``ls2``, folded into the
 proj / fc2 weights), a class token without a position (``no_embed_class``), and a distillation token (distilled DeiT:
-two prefix tokens, always kept, and the eval-mode average of ``head`` and ``head_dist``).
+two prefix tokens, always kept, and the eval-mode average of ``head`` and ``head_dist``).  It also runs average-pooled
+heads (``global_pool='avg'`` with ``fc_norm``, MAE fine-tunes: the mean of the patch tokens the last block kept, then
+fc_norm, in one kernel) and a pre-norm stem (``norm_pre``, CLIP fine-tunes: one LayerNorm pass over the embedded tokens
+that also writes block 0's LayerNorm statistics), with or without a patch-embedding bias.
 """
 from __future__ import annotations
 
@@ -45,6 +48,10 @@ def _normalise_schedule(schedule: Dict) -> Dict[int, Dict]:
 
 def _is_identity(m) -> bool:
     return m is None or isinstance(m, nn.Identity) or (isinstance(m, nn.Dropout) and m.p == 0.0)
+
+
+def _is_layer_norm(m, C: int) -> bool:
+    return isinstance(m, nn.LayerNorm) and tuple(m.normalized_shape) == (C,) and m.weight is not None and m.bias is not None
 
 
 def _is_layer_scale(m, C: int) -> bool:
@@ -85,6 +92,8 @@ class RAJNIViTWrapper(nn.Module):
         self.use_cuda_graph: Optional[bool] = None if env == "" else env != "0"
         self.prefix = 1                  # leading tokens that are always kept (set by _validate: 2 for a distilled DeiT)
         self.no_embed_class = False      # pos_embed covers the patches only (DeiT-III)
+        self.pre_norm = False            # norm_pre LayerNorm after the embedding (CLIP)
+        self.avg_pool = False            # head on fc_norm(mean of the patch tokens) (global_pool='avg', MAE)
         self.input_norm: Optional[tuple] = None       # (mean[3], std[3]) for uint8 images, see set_input_normalization
         # Stream-K tail of the fc2 GEMMs (gemm_tcgen05.cu): +1.4 % at 32 images per GPU, nothing at 64 and above.  OFF by default
         # because the fp32 summation order of a split tile depends on the tile count, i.e. on the batch size: without it an
@@ -117,14 +126,36 @@ class RAJNIViTWrapper(nn.Module):
         self.patch = p
         if not _is_identity(getattr(m.patch_embed, "norm", None)):
             raise NotImplementedError("patch_embed.norm is not supported")
-        for name in ("norm_pre", "fc_norm", "patch_drop"):
-            if not _is_identity(getattr(m, name, None)):
-                raise NotImplementedError(f"{name} = {type(getattr(m, name)).__name__} is not supported")
-        if getattr(m, "global_pool", "token") != "token":
-            raise NotImplementedError("only global_pool='token' (CLS) is supported")
-        if not isinstance(m.norm, nn.LayerNorm) or not isinstance(m.head, nn.Linear):
-            raise NotImplementedError("norm must be LayerNorm and head must be Linear")
+        if not _is_identity(getattr(m, "patch_drop", None)):
+            raise NotImplementedError(f"patch_drop = {type(m.patch_drop).__name__} is not supported")
         C = proj.out_channels
+        # pre-norm stem (CLIP): a LayerNorm over the embedded tokens before block 0
+        norm_pre = getattr(m, "norm_pre", None)
+        if not _is_identity(norm_pre) and not _is_layer_norm(norm_pre, C):
+            raise NotImplementedError(f"norm_pre = {type(norm_pre).__name__} is not supported (Identity or an affine LayerNorm [C])")
+        self.pre_norm = not _is_identity(norm_pre)
+        # head: the class token through `norm`, or the mean of the patch tokens through `fc_norm` (MAE fine-tunes)
+        pool, fc_norm = getattr(m, "global_pool", "token"), getattr(m, "fc_norm", None)
+        if pool == "avg":
+            if getattr(m, "dist_token", None) is not None:
+                raise NotImplementedError("global_pool='avg' with a distillation token is not supported")
+            if _is_identity(fc_norm):
+                raise NotImplementedError("global_pool='avg' without fc_norm (timm fc_norm=False) is not supported")
+            if not _is_layer_norm(fc_norm, C):
+                raise NotImplementedError(f"fc_norm = {type(fc_norm).__name__} is not supported (an affine LayerNorm [C])")
+            if not _is_identity(m.norm):
+                raise NotImplementedError(f"fc_norm together with norm = {type(m.norm).__name__} is not supported "
+                                          "(timm's avg-pooled models have norm = Identity)")
+        elif pool == "token":
+            if not _is_identity(fc_norm):
+                raise NotImplementedError(f"fc_norm = {type(fc_norm).__name__} with global_pool='token' is not supported")
+            if not isinstance(m.norm, nn.LayerNorm):
+                raise NotImplementedError("norm must be LayerNorm")
+        else:
+            raise NotImplementedError(f"global_pool={pool!r} is not supported ('token' or 'avg')")
+        self.avg_pool = pool == "avg"
+        if not isinstance(m.head, nn.Linear):
+            raise NotImplementedError("head must be Linear")
         # prefix tokens: CLS, or CLS + distillation token (distilled DeiT); register tokens are not supported
         if getattr(m, "cls_token", None) is None:
             raise NotImplementedError("a class token (cls_token) is required")
@@ -164,7 +195,8 @@ class RAJNIViTWrapper(nn.Module):
                     raise NotImplementedError(f"blocks[{i}].attn.{name} is not supported")
             act = blk.mlp.act
             if not isinstance(act, nn.GELU) or getattr(act, "approximate", "none") != "none":
-                raise NotImplementedError(f"blocks[{i}].mlp.act must be exact (erf) nn.GELU")
+                raise NotImplementedError(f"blocks[{i}].mlp.act = {type(act).__name__} is not supported: "
+                                          f"blocks[{i}].mlp.act must be exact (erf) nn.GELU")
             if not _is_identity(getattr(blk.mlp, "norm", None)):
                 raise NotImplementedError(f"blocks[{i}].mlp.norm is not supported")
             if not isinstance(blk.norm1, nn.LayerNorm) or not isinstance(blk.norm2, nn.LayerNorm):
@@ -310,6 +342,9 @@ class RAJNIViTWrapper(nn.Module):
         # ---- patch + CLS + pos (model.py:31-37): im2col, then one GEMM whose epilogue adds
         #      bias and pos_embed and scatters into rows P0..P0+P-1 of each image (P0 = 1, or 2 with a distillation token)
         pe_w, pe_b = pk.linear(m.patch_embed.proj)
+        if pe_b is None:                # CLIP: no patch bias.  A zero bias keeps the GEMM's bias + residual epilogue, the one
+            pe_b = pk.tensors(("pe_zero_bias",), (m.patch_embed.proj.weight,),          # that also writes row statistics
+                              lambda: torch.zeros(C, device=x.device, dtype=torch.float32))
         P0 = self.prefix
         dist = getattr(m, "dist_token", None)
 
@@ -333,6 +368,9 @@ class RAJNIViTWrapper(nn.Module):
                          prefix=P0)
         ops.gemm(ws["cols"], pe_w, pe_b, B * P, C, kpe, residual=pos, ldres=C, res_row_map=ws["embed_pos_map"],
                  out=cur, ldd=C, out_row_map=ws["embed_out_map"], row_stats=stats, tag="embed")
+        if self.pre_norm:               # x = norm_pre(x) in place, with the row statistics block 0's LN-folded qkv GEMM reads
+            gp, bp, ep = pk.norm(m.norm_pre)
+            ops.layernorm(cur, gp, bp, ep, B * N, C, out=cur, row_stats=stats, stats_slots=slots)
 
         # Zig-zag traversal: every persistent kernel walks its row tiles in the direction opposite to the kernel that
         # produced its main operand, so it starts on the rows that kernel wrote last and that still sit in L2.
@@ -397,14 +435,20 @@ class RAJNIViTWrapper(nn.Module):
             rev = zig and not rev
 
         # ---- final norm on the CLS rows only (LayerNorm is row-wise) + head   model.py:65-66
-        gn, bn, en = pk.norm(m.norm)
-        if dist is None:
+        if self.avg_pool:               # timm forward_head, global_pool='avg': head(fc_norm(mean of the kept patch tokens))
+            gf, bf_, ef = pk.norm(m.fc_norm)
+            hw, hb = pk.linear(m.head)
+            ops.mean_pool_layernorm(cur, B, N, C, gf, bf_, ef, prefix=P0, out=ws["cls"])
+            logits = ops.gemm(ws["cls"], hw, hb, B, hw.shape[0], C, out_f32=True, tag="head")
+        elif dist is None:
+            gn, bn, en = pk.norm(m.norm)
             hw, hb = pk.linear(m.head)
             ops.layernorm(cur, gn, bn, en, B, C, in_row_stride=N * C, out=ws["cls"])
             logits = ops.gemm(ws["cls"], hw, hb, B, hw.shape[0], C, out_f32=True, tag="head")
         else:
             # distilled: (head(LN(x0)) + head_dist(LN(x1))) / 2 as ONE GEMM over [LN(x0) | LN(x1)] (K = 2C) with the weights
             # [W_head | W_dist] / 2 (halving is exact in bf16) and the bias (b + b_dist) / 2
+            gn, bn, en = pk.norm(m.norm)
             hw, hb = pk.tensors(("head2",), (m.head.weight, m.head.bias, m.head_dist.weight, m.head_dist.bias), self._head_pack)
             for r in range(2):
                 ops.layernorm(cur, gn, bn, en, B, C, in_row_stride=N * C, in_offset=r * C, out=ws["cls"],
