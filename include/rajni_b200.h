@@ -124,6 +124,10 @@ int rajni_layernorm(const void* x, long long in_row_stride, const float* gamma,
  * normalised CLS and distillation rows of each image side by side, the A operand of a distilled model's head. */
 int rajni_layernorm_strided(const void* x, long long in_row_stride, const float* gamma, const float* beta, float eps,
                             void* y, long long out_row_stride, int rows, int C, void* stream);
+/* The same values stored as fp32 (the features of a headless model, num_classes = 0): y + r*out_row_stride floats,
+ * out_row_stride >= C and a multiple of 4.  bf16_rn of each value is what rajni_layernorm_strided stores. */
+int rajni_layernorm_strided_f32(const void* x, long long in_row_stride, const float* gamma, const float* beta, float eps,
+                                float* y, long long out_row_stride, int rows, int C, void* stream);
 /* The same over a whole activation matrix, also emitting the rows' LayerNorm partial sums for an LN-folded GEMM
  * (RAJNI_EPI_LN_FOLD) that reads y next: row_stats[s*row_stats_ld + r] = (sum, sum of squares) of the bf16 row r as stored
  * for s = 0, zero for s = 1..stats_slots-1 (the slot layout of RAJNI_EPI_ROW_STATS).  y may be x (in place).  This is the
@@ -139,6 +143,10 @@ int rajni_layernorm_row_stats(const void* x, long long in_row_stride, const floa
  * in any batch.  C a multiple of 64 up to 2048, B <= 65535. */
 int rajni_mean_pool_layernorm(const void* x, int B, int N, int prefix, int C, const float* gamma, const float* beta,
                               float eps, void* y, long long out_row_stride, void* stream);
+/* The same values stored as fp32 (the pooled features of a headless model): y + b*out_row_stride floats, out_row_stride
+ * >= C and a multiple of 4.  Same summation order; bf16_rn of each value is what rajni_mean_pool_layernorm stores. */
+int rajni_mean_pool_layernorm_f32(const void* x, int B, int N, int prefix, int C, const float* gamma, const float* beta,
+                                  float eps, float* y, long long out_row_stride, void* stream);
 
 /* ---- dense contractions (attention.py:22,55; timm Mlp fc1/fc2; patch_embed; head)
  * D[orow(m), n] = epi( sum_k A[m,k] * W[n,k] ), A [M,K] bf16, W [N,K] bf16

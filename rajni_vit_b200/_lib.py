@@ -52,10 +52,14 @@ SIGNATURES = {
     "rajni_layernorm": (c_int, [c_void_p, c_longlong, c_void_p, c_void_p, c_float, c_void_p, c_int, c_int, c_void_p]),
     "rajni_layernorm_strided": (c_int, [c_void_p, c_longlong, c_void_p, c_void_p, c_float, c_void_p, c_longlong, c_int, c_int,
                                         c_void_p]),
+    "rajni_layernorm_strided_f32": (c_int, [c_void_p, c_longlong, c_void_p, c_void_p, c_float, c_void_p, c_longlong, c_int, c_int,
+                                            c_void_p]),
     "rajni_layernorm_row_stats": (c_int, [c_void_p, c_longlong, c_void_p, c_void_p, c_float, c_void_p, c_longlong, c_int, c_int,
                                           c_void_p, c_longlong, c_int, c_void_p]),
     "rajni_mean_pool_layernorm": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_float, c_void_p, c_longlong,
                                           c_void_p]),
+    "rajni_mean_pool_layernorm_f32": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_float, c_void_p,
+                                              c_longlong, c_void_p]),
     "rajni_gemm_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int,
                                 c_void_p, c_longlong, c_void_p, c_longlong, c_void_p, c_void_p]),
     "rajni_gemm_bf16_ex": (c_int, [POINTER(GemmArgs), c_void_p]),

@@ -17,7 +17,8 @@ Accepted key families (SURVEY.md section 5):
   * wrappers around either: ``module.`` (DataParallel), ``model.``, and ``{"state_dict": ...}`` / ``{"model": ...}`` nesting
 
 The architecture is inferred from the tensors' shapes (width from ``cls_token``, depth from
-the block indices, image size from ``pos_embed``, classes from ``head.weight``); heads =
+the block indices, image size from ``pos_embed``, classes from ``head.weight``, none without ``head.*``: timm's
+``num_classes=0``, whose output is the pooled features); heads =
 width / 64, the only head dimension the kernels (and every BASELINE config) use.  The two DeiT families load too:
   * DeiT-III: ``blocks.{i}.ls1.gamma`` / ``ls2.gamma`` (LayerScale, accepted only when every block has both), and a
     ``pos_embed`` with one row per patch (a square length: no position for the class token, timm's ``no_embed_class``);
@@ -125,9 +126,16 @@ def normalise_keys(sd: Mapping[str, torch.Tensor]) -> Dict[str, torch.Tensor]:
 
 
 def infer_config(sd: Mapping[str, torch.Tensor]) -> Dict[str, int]:
-    for k in ("cls_token", "pos_embed", "patch_embed.proj.weight", "head.weight"):
+    for k in ("cls_token", "pos_embed", "patch_embed.proj.weight"):
         if k not in sd:
             raise KeyError(f"checkpoint has no {k!r}: not a timm-named ViT state dict (keys start with {sorted(sd)[:4]})")
+    # no head.* at all: a headless backbone (num_classes=0: DINO, MAE pretraining, in21k backbones)
+    headless = "head.weight" not in sd
+    if headless and "head.bias" in sd:
+        raise KeyError("checkpoint has 'head.bias' but no 'head.weight'")
+    if headless and ("dist_token" in sd or any(k.startswith("head_dist.") for k in sd)):
+        raise NotImplementedError("a distillation token ('dist_token' / 'head_dist.*') without 'head.weight' is not supported: "
+                                  "distilled models need their classifier heads")
     bad = sorted(k for k in sd if any(re.search(p, k) for p in _UNSUPPORTED))
     if bad:
         raise NotImplementedError(f"checkpoint uses features outside the RAJNI wrapper's contract: {bad[:6]}"
@@ -181,7 +189,7 @@ def infer_config(sd: Mapping[str, torch.Tensor]) -> Dict[str, int]:
         raise NotImplementedError(f"width {C} is not a multiple of the head dimension 64")
     hidden = sd["blocks.0.mlp.fc1.weight"].shape[0]
     return dict(embed_dim=C, depth=len(blocks), num_heads=C // 64, img_size=grid * patch, patch_size=patch,
-                num_classes=sd["head.weight"].shape[0], mlp_ratio=hidden / C, init_values=1.0 if ls else None,
+                num_classes=0 if headless else sd["head.weight"].shape[0], mlp_ratio=hidden / C, init_values=1.0 if ls else None,
                 no_embed_class=no_embed_class, distilled=dist, global_pool="avg" if avg_pool else "token", fc_norm=avg_pool,
                 pre_norm=pre_norm, patch_bias="patch_embed.proj.bias" in sd, norm_eps=1e-5 if pre_norm else 1e-6)
 

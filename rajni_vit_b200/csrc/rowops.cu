@@ -1,5 +1,7 @@
 // HBM-bound row kernels: gather-compaction, LayerNorm, patch im2col.
 // All use 16-byte vector accesses, contiguous along the fastest dimension per warp.
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace rajni {
@@ -41,11 +43,13 @@ __global__ void __launch_bounds__(256) gather_rows_kernel(const uint4* __restric
 // STATS: also write the row's LayerNorm partial sums in the RAJNI_EPI_ROW_STATS layout that the LN-folded GEMMs read
 // (slot 0 = (sum, sum of squares) of the stored bf16 row, the other slots zero, as write_prefix_rows does).  Every load
 // of a row precedes its first store (the stores need the row's mean), so y may be x.
-template <int CPL, bool STATS = false>
+// OutT = float: the same values stored unrounded (a headless model's features), 8 columns as two 16-byte stores.
+template <int CPL, bool STATS = false, typename OutT = __nv_bfloat16>
 __global__ void __launch_bounds__(256) layernorm_kernel(const __nv_bfloat16* __restrict__ x, long long in_stride,
                                                         const float* __restrict__ gamma, const float* __restrict__ beta,
-                                                        float eps, __nv_bfloat16* __restrict__ y, long long out_stride, int rows, int C,
+                                                        float eps, OutT* __restrict__ y, long long out_stride, int rows, int C,
                                                         float2* __restrict__ row_stats, long long stats_ld, int stats_slots) {
+    static_assert(!STATS || std::is_same<OutT, __nv_bfloat16>::value, "row statistics are those of a stored bf16 row");
     griddep_launch();
     griddep_wait();
     const int lane = threadIdx.x & 31;
@@ -80,7 +84,7 @@ __global__ void __launch_bounds__(256) layernorm_kernel(const __nv_bfloat16* __r
         }
     }
     const float rstd = rsqrtf(warp_sum(sq) / (float)C + eps);
-    __nv_bfloat16* yr = y + (long long)row * out_stride;
+    OutT* yr = y + (long long)row * out_stride;
     float osum = 0.f, osq = 0.f;
 #pragma unroll
     for (int i = 0; i < CPL; ++i) {
@@ -90,19 +94,28 @@ __global__ void __launch_bounds__(256) layernorm_kernel(const __nv_bfloat16* __r
             const float4 g1 = __ldg(reinterpret_cast<const float4*>(gamma + j * 8 + 4));
             const float4 b0 = __ldg(reinterpret_cast<const float4*>(beta + j * 8));
             const float4 b1 = __ldg(reinterpret_cast<const float4*>(beta + j * 8 + 4));
-            uint4 o;
-            o.x = float2_to_bf16x2((v[i][0] - mean) * rstd * g0.x + b0.x, (v[i][1] - mean) * rstd * g0.y + b0.y);
-            o.y = float2_to_bf16x2((v[i][2] - mean) * rstd * g0.z + b0.z, (v[i][3] - mean) * rstd * g0.w + b0.w);
-            o.z = float2_to_bf16x2((v[i][4] - mean) * rstd * g1.x + b1.x, (v[i][5] - mean) * rstd * g1.y + b1.y);
-            o.w = float2_to_bf16x2((v[i][6] - mean) * rstd * g1.z + b1.z, (v[i][7] - mean) * rstd * g1.w + b1.w);
-            st_stream16(yr + j * 8, o);
-            if (STATS) {
-                const uint32_t w[4] = {o.x, o.y, o.z, o.w};
+            if constexpr (std::is_same<OutT, float>::value) {
+                const float4 o0 = make_float4((v[i][0] - mean) * rstd * g0.x + b0.x, (v[i][1] - mean) * rstd * g0.y + b0.y,
+                                              (v[i][2] - mean) * rstd * g0.z + b0.z, (v[i][3] - mean) * rstd * g0.w + b0.w);
+                const float4 o1 = make_float4((v[i][4] - mean) * rstd * g1.x + b1.x, (v[i][5] - mean) * rstd * g1.y + b1.y,
+                                              (v[i][6] - mean) * rstd * g1.z + b1.z, (v[i][7] - mean) * rstd * g1.w + b1.w);
+                st_stream16(yr + j * 8, *reinterpret_cast<const uint4*>(&o0));
+                st_stream16(yr + j * 8 + 4, *reinterpret_cast<const uint4*>(&o1));
+            } else {
+                uint4 o;
+                o.x = float2_to_bf16x2((v[i][0] - mean) * rstd * g0.x + b0.x, (v[i][1] - mean) * rstd * g0.y + b0.y);
+                o.y = float2_to_bf16x2((v[i][2] - mean) * rstd * g0.z + b0.z, (v[i][3] - mean) * rstd * g0.w + b0.w);
+                o.z = float2_to_bf16x2((v[i][4] - mean) * rstd * g1.x + b1.x, (v[i][5] - mean) * rstd * g1.y + b1.y);
+                o.w = float2_to_bf16x2((v[i][6] - mean) * rstd * g1.z + b1.z, (v[i][7] - mean) * rstd * g1.w + b1.w);
+                st_stream16(yr + j * 8, o);
+                if (STATS) {
+                    const uint32_t w[4] = {o.x, o.y, o.z, o.w};
 #pragma unroll
-                for (int k = 0; k < 4; ++k) {
-                    const float2 f = bf16x2_to_float2(w[k]);
-                    osum += f.x + f.y;
-                    osq += f.x * f.x + f.y * f.y;
+                    for (int k = 0; k < 4; ++k) {
+                        const float2 f = bf16x2_to_float2(w[k]);
+                        osum += f.x + f.y;
+                        osq += f.x * f.x + f.y * f.y;
+                    }
                 }
             }
         }
@@ -151,9 +164,11 @@ __device__ __forceinline__ float pool_cluster_sum(float v, float* warp_part, flo
     return t;
 }
 
+// OutT = float: the same values stored unrounded (a headless model's features).
+template <typename OutT = __nv_bfloat16>
 __global__ void __launch_bounds__(kPoolThreads, 4) mean_pool_layernorm_kernel(const __nv_bfloat16* __restrict__ x, int N, int P0, int C,
                                                                            const float* __restrict__ gamma, const float* __restrict__ beta,
-                                                                           float eps, __nv_bfloat16* __restrict__ y, long long out_stride) {
+                                                                           float eps, OutT* __restrict__ y, long long out_stride) {
     __shared__ float part[kPoolThreads * 8];
     __shared__ float warp_part[kPoolThreads / 32];
     __shared__ float red[2];
@@ -208,7 +223,10 @@ __global__ void __launch_bounds__(kPoolThreads, 4) mean_pool_layernorm_kernel(co
     const float mean = pool_cluster_sum(m, warp_part, &red[0]) / (float)C;
     const float d = t < cs ? m - mean : 0.f;
     const float rstd = rsqrtf(pool_cluster_sum(d * d, warp_part, &red[1]) / (float)C + eps);
-    if (t < cs) y[(long long)b * out_stride + c0 + t] = __float2bfloat16_rn(d * rstd * gamma[c0 + t] + beta[c0 + t]);
+    if (t < cs) {
+        if constexpr (std::is_same<OutT, float>::value) y[(long long)b * out_stride + c0 + t] = d * rstd * gamma[c0 + t] + beta[c0 + t];
+        else y[(long long)b * out_stride + c0 + t] = __float2bfloat16_rn(d * rstd * gamma[c0 + t] + beta[c0 + t]);
+    }
     cluster_sync_all();                                         // no CTA leaves while another may still read its red[]
 }
 
@@ -423,24 +441,38 @@ extern "C" int rajni_gather_rows(const void* src, const int32_t* row_map, void* 
                           static_cast<const uint4*>(src), row_map, static_cast<uint4*>(dst), total, cpr);
 }
 
-extern "C" int rajni_layernorm_strided(const void* x, long long in_row_stride, const float* gamma, const float* beta, float eps,
-                                       void* y, long long out_row_stride, int rows, int C, void* stream) {
-    RAJNI_REQUIRE(x && gamma && beta && y, RAJNI_EINVAL, "rajni_layernorm: null pointer");
-    RAJNI_REQUIRE(rows > 0 && C > 0 && C % 8 == 0 && C <= 2048 && in_row_stride % 8 == 0 && out_row_stride % 8 == 0 && out_row_stride >= C,
-                  RAJNI_EINVAL, "rajni_layernorm: rows=%d C=%d stride=%lld out stride=%lld unsupported", rows, C, in_row_stride, out_row_stride);
+// y: bf16 or fp32 rows at out_row_stride elements (a multiple of 16 bytes, as the kernel stores 16-byte chunks)
+template <typename OutT>
+static int layernorm_strided(const char* name, const char* kname, const void* x, long long in_row_stride, const float* gamma, const float* beta,
+                             float eps, OutT* y, long long out_row_stride, int rows, int C, void* stream) {
+    constexpr int kOutAlign = 16 / sizeof(OutT);
+    RAJNI_REQUIRE(x && gamma && beta && y, RAJNI_EINVAL, "%s: null pointer", name);
+    RAJNI_REQUIRE(rows > 0 && C > 0 && C % 8 == 0 && C <= 2048 && in_row_stride % 8 == 0 && out_row_stride % kOutAlign == 0 &&
+                  out_row_stride >= C, RAJNI_EINVAL, "%s: rows=%d C=%d stride=%lld out stride=%lld unsupported", name, rows, C,
+                  in_row_stride, out_row_stride);
     const int cpl = (C / 8 + 31) / 32;
     const int wpb = 8;
     dim3 grid((rows + wpb - 1) / wpb), block(wpb * 32);
-    auto kern = layernorm_kernel<8>;                          // cpl 5..8
+    auto kern = layernorm_kernel<8, false, OutT>;             // cpl 5..8
     switch (cpl) {
-        case 1: kern = layernorm_kernel<1>; break;
-        case 2: kern = layernorm_kernel<2>; break;
-        case 3: kern = layernorm_kernel<3>; break;
-        case 4: kern = layernorm_kernel<4>; break;
+        case 1: kern = layernorm_kernel<1, false, OutT>; break;
+        case 2: kern = layernorm_kernel<2, false, OutT>; break;
+        case 3: kern = layernorm_kernel<3, false, OutT>; break;
+        case 4: kern = layernorm_kernel<4, false, OutT>; break;
     }
-    return launch_checked("layernorm", kern, grid, block, 0, static_cast<cudaStream_t>(stream), 1, static_cast<const __nv_bfloat16*>(x),
-                          in_row_stride, gamma, beta, eps, static_cast<__nv_bfloat16*>(y), out_row_stride, rows, C,
-                          static_cast<float2*>(nullptr), 0LL, 0);
+    return launch_checked(kname, kern, grid, block, 0, static_cast<cudaStream_t>(stream), 1, static_cast<const __nv_bfloat16*>(x),
+                          in_row_stride, gamma, beta, eps, y, out_row_stride, rows, C, static_cast<float2*>(nullptr), 0LL, 0);
+}
+
+extern "C" int rajni_layernorm_strided(const void* x, long long in_row_stride, const float* gamma, const float* beta, float eps,
+                                       void* y, long long out_row_stride, int rows, int C, void* stream) {
+    return layernorm_strided("rajni_layernorm", "layernorm", x, in_row_stride, gamma, beta, eps, static_cast<__nv_bfloat16*>(y), out_row_stride,
+                             rows, C, stream);
+}
+
+extern "C" int rajni_layernorm_strided_f32(const void* x, long long in_row_stride, const float* gamma, const float* beta, float eps,
+                                           float* y, long long out_row_stride, int rows, int C, void* stream) {
+    return layernorm_strided("rajni_layernorm_f32", "layernorm_f32", x, in_row_stride, gamma, beta, eps, y, out_row_stride, rows, C, stream);
 }
 
 extern "C" int rajni_layernorm_row_stats(const void* x, long long in_row_stride, const float* gamma, const float* beta, float eps,
@@ -468,16 +500,29 @@ extern "C" int rajni_layernorm_row_stats(const void* x, long long in_row_stride,
                           out_row_stride, rows, C, reinterpret_cast<float2*>(row_stats), row_stats_ld, stats_slots);
 }
 
+template <typename OutT>
+static int mean_pool_layernorm(const char* name, const char* kname, const void* x, int B, int N, int prefix, int C, const float* gamma, const float* beta,
+                               float eps, OutT* y, long long out_row_stride, void* stream) {
+    constexpr int kOutAlign = 16 / sizeof(OutT);
+    RAJNI_REQUIRE(x && gamma && beta && y, RAJNI_EINVAL, "%s: null pointer", name);
+    RAJNI_REQUIRE(B > 0 && B <= 65535 && prefix >= 1 && prefix <= kMaxPrefix && N > prefix && C > 0 && C % 64 == 0 && C <= 2048 &&
+                  out_row_stride >= C && out_row_stride % kOutAlign == 0, RAJNI_EINVAL,
+                  "%s: B=%d N=%d prefix=%d C=%d out stride=%lld unsupported (C a multiple of 64 up to 2048, "
+                  "N > prefix, prefix 1 or 2)", name, B, N, prefix, C, out_row_stride);
+    return launch_checked(kname, mean_pool_layernorm_kernel<OutT>, dim3(kPoolCluster, B), dim3(kPoolThreads), 0,
+                          static_cast<cudaStream_t>(stream), kPoolCluster, static_cast<const __nv_bfloat16*>(x), N, prefix, C, gamma,
+                          beta, eps, y, out_row_stride);
+}
+
 extern "C" int rajni_mean_pool_layernorm(const void* x, int B, int N, int prefix, int C, const float* gamma, const float* beta,
                                          float eps, void* y, long long out_row_stride, void* stream) {
-    RAJNI_REQUIRE(x && gamma && beta && y, RAJNI_EINVAL, "rajni_mean_pool_layernorm: null pointer");
-    RAJNI_REQUIRE(B > 0 && B <= 65535 && prefix >= 1 && prefix <= kMaxPrefix && N > prefix && C > 0 && C % 64 == 0 && C <= 2048 &&
-                  out_row_stride >= C && out_row_stride % 8 == 0, RAJNI_EINVAL,
-                  "rajni_mean_pool_layernorm: B=%d N=%d prefix=%d C=%d out stride=%lld unsupported (C a multiple of 64 up to 2048, "
-                  "N > prefix, prefix 1 or 2)", B, N, prefix, C, out_row_stride);
-    return launch_checked("mean_pool_layernorm", mean_pool_layernorm_kernel, dim3(kPoolCluster, B), dim3(kPoolThreads), 0,
-                          static_cast<cudaStream_t>(stream), kPoolCluster, static_cast<const __nv_bfloat16*>(x), N, prefix, C, gamma,
-                          beta, eps, static_cast<__nv_bfloat16*>(y), out_row_stride);
+    return mean_pool_layernorm("rajni_mean_pool_layernorm", "mean_pool_layernorm", x, B, N, prefix, C, gamma, beta, eps, static_cast<__nv_bfloat16*>(y),
+                               out_row_stride, stream);
+}
+
+extern "C" int rajni_mean_pool_layernorm_f32(const void* x, int B, int N, int prefix, int C, const float* gamma, const float* beta,
+                                             float eps, float* y, long long out_row_stride, void* stream) {
+    return mean_pool_layernorm("rajni_mean_pool_layernorm_f32", "mean_pool_layernorm_f32", x, B, N, prefix, C, gamma, beta, eps, y, out_row_stride, stream);
 }
 
 extern "C" int rajni_layernorm(const void* x, long long in_row_stride, const float* gamma,

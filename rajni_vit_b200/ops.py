@@ -200,20 +200,28 @@ def layernorm(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps: flo
               in_row_stride: Optional[int] = None, out: Optional[torch.Tensor] = None, in_offset: int = 0,
               out_row_stride: Optional[int] = None, out_offset: int = 0, row_stats: Optional[torch.Tensor] = None,
               stats_slots: int = 0) -> torch.Tensor:
-    """Row LayerNorm, bf16 -> bf16; row r read at x.data_ptr + in_offset + r*in_row_stride elements and written at
-    out.data_ptr + out_offset + r*out_row_stride (default C: dense rows).  ``out`` may be ``x`` (in place).
+    """Row LayerNorm, bf16 -> bf16 or fp32 (the dtype of ``out``; bf16 when ``out`` is None); row r read at
+    x.data_ptr + in_offset + r*in_row_stride elements and written at out.data_ptr + out_offset + r*out_row_stride elements
+    (default C: dense rows).  ``out`` may be ``x`` (in place).  An fp32 ``out`` holds the values that the bf16 output rounds.
     ``row_stats`` fp32 [>= stats_slots, >= rows, 2]: also write the LayerNorm partial sums of the stored rows for an LN-folded
-    ``gemm`` (slot 0 = (sum, sum of squares) of row r as stored in bf16, slots 1..stats_slots-1 zero)."""
+    ``gemm`` (slot 0 = (sum, sum of squares) of row r as stored in bf16, slots 1..stats_slots-1 zero); bf16 ``out`` only."""
     out = torch.empty((rows, C), device=x.device, dtype=torch.bfloat16) if out is None else out
+    if out.dtype not in (torch.bfloat16, torch.float32):
+        raise ValueError(f"layernorm: out must be bf16 or fp32, got {out.dtype}")
+    f32 = out.dtype == torch.float32
     stride = C if in_row_stride is None else in_row_stride
     ostride = C if out_row_stride is None else out_row_stride
     if in_offset + (rows - 1) * stride + C > x.numel() or out_offset + (rows - 1) * ostride + C > out.numel():
         raise ValueError(f"layernorm: {rows} rows (strides {stride} / {ostride}, offsets {in_offset} / {out_offset}) exceed "
                          f"the input ({x.numel()}) or output ({out.numel()} elements)")
     if row_stats is None:
-        _call("layernorm", rows * C * 4, _lib.load().rajni_layernorm_strided, x.data_ptr() + 2 * in_offset, stride,
-              gamma.data_ptr(), beta.data_ptr(), eps, out.data_ptr() + 2 * out_offset, ostride, rows, C, _stream(x))
+        _call("layernorm_f32" if f32 else "layernorm", rows * C * (6 if f32 else 4),
+              _lib.load().rajni_layernorm_strided_f32 if f32 else _lib.load().rajni_layernorm_strided, x.data_ptr() + 2 * in_offset,
+              stride, gamma.data_ptr(), beta.data_ptr(), eps, out.data_ptr() + out.element_size() * out_offset, ostride, rows, C,
+              _stream(x))
         return out
+    if f32:
+        raise ValueError("layernorm: row_stats are the sums of the stored bf16 rows; out must be bf16")
     if (row_stats.dtype != torch.float32 or not row_stats.is_contiguous() or row_stats.dim() != 3 or row_stats.shape[2] != 2
             or row_stats.shape[0] < stats_slots or row_stats.shape[1] < rows):
         raise ValueError(f"layernorm: row_stats must be contiguous fp32 [>= {stats_slots}, >= {rows}, 2], got "
@@ -227,17 +235,21 @@ def layernorm(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps: flo
 def mean_pool_layernorm(x: torch.Tensor, B: int, N: int, C: int, gamma: torch.Tensor, beta: torch.Tensor, eps: float,
                         prefix: int = 1, out: Optional[torch.Tensor] = None, out_row_stride: Optional[int] = None) -> torch.Tensor:
     """timm's average-pooled head input: out[b] = LayerNorm(mean of x[b*N + prefix .. b*N + N-1]) (fc_norm over the patch
-    tokens' mean), x [>= B*N, C] bf16 dense; -> bf16 rows at out.data_ptr + b*out_row_stride (default C).  fp32 sums in an
-    order that does not depend on B."""
+    tokens' mean), x [>= B*N, C] bf16 dense; -> bf16 or fp32 rows (the dtype of ``out``; bf16 when ``out`` is None) at
+    out.data_ptr + b*out_row_stride elements (default C).  fp32 sums in an order that does not depend on B; an fp32 ``out``
+    holds the values that the bf16 output rounds."""
     _check_prefix(prefix)
     if x.dtype != torch.bfloat16 or not x.is_contiguous() or x.numel() < B * N * C:
         raise ValueError(f"mean_pool_layernorm: x must be contiguous bf16 with at least {B}*{N} rows of {C}")
     ostride = C if out_row_stride is None else out_row_stride
     out = torch.empty((B, C), device=x.device, dtype=torch.bfloat16) if out is None else out
-    if out.dtype != torch.bfloat16 or out.numel() < (B - 1) * ostride + C:
-        raise ValueError(f"mean_pool_layernorm: out must be bf16 with room for {B} rows at stride {ostride}")
-    _call("mean_pool_layernorm", B * ((N - prefix) * C * 2 + C * 2), _lib.load().rajni_mean_pool_layernorm, x.data_ptr(), B, N,
-          prefix, C, gamma.data_ptr(), beta.data_ptr(), eps, out.data_ptr(), ostride, _stream(x))
+    if out.dtype not in (torch.bfloat16, torch.float32) or out.numel() < (B - 1) * ostride + C:
+        raise ValueError(f"mean_pool_layernorm: out must be bf16 or fp32 with room for {B} rows at stride {ostride}")
+    f32 = out.dtype == torch.float32
+    lib = _lib.load()
+    _call("mean_pool_layernorm_f32" if f32 else "mean_pool_layernorm", B * ((N - prefix) * C * 2 + C * out.element_size()),
+          lib.rajni_mean_pool_layernorm_f32 if f32 else lib.rajni_mean_pool_layernorm, x.data_ptr(), B, N, prefix, C,
+          gamma.data_ptr(), beta.data_ptr(), eps, out.data_ptr(), ostride, _stream(x))
     return out
 
 

@@ -16,7 +16,8 @@ Differences from the reference CLI, all deliberate (SURVEY.md section 5):
     ``csrc/resize.cu`` (bit-identical to torchvision on PIL images), ToTensor + Normalize in the patch kernel;
   * ``--ckpt file`` loads timm-named weights from a .safetensors / .pt file (no hub access needed);
   * under torchrun every rank decodes only its shard of each batch (``data.sharded_loader``);
-  * without ``timm`` (not installable here) the stand-in ViT with random weights is used and the fact is printed.
+  * without ``timm`` (not installable here) the stand-in ViT with random weights is used and the fact is printed;
+  * a headless model (num_classes=0) is refused: it has no class scores to take a top-1 accuracy of.
 """
 from __future__ import annotations
 
@@ -28,6 +29,7 @@ import torch
 
 from .eval import evaluate_model
 from .wrapper import RAJNIViTWrapper
+from .wrapper.model import _is_identity
 
 
 def get_args(argv=None):
@@ -122,6 +124,10 @@ def main(argv=None):
 
     base, origin = build_model(args.model, args.ckpt)
     say(f"model {args.model}: {origin}")
+    if hasattr(base, "head") and _is_identity(base.head):
+        raise ValueError(f"{args.model} is headless (head = Identity, num_classes=0): it outputs features, not class scores, "
+                         "so it has no top-1 accuracy to measure; rajni_vit_b200.schedule.measure reports the features' cosine "
+                         "agreement with the un-pruned model instead")
     size = getattr(getattr(base, "patch_embed", None), "img_size", (224, 224))
     size = size[0] if isinstance(size, (tuple, list)) else int(size)
     loader = build_loader(args, size, rank, world)

@@ -6,7 +6,9 @@ This module measures candidates on the device the model will run on and picks on
 * ``measure(make_model, schedule, batches)`` - images/s of the wrapped model, tensor work per image, and the accuracy axis:
   top-1 accuracy when the batches carry labels (real weights: ``load_checkpoint`` + an ImageNet loader), and always the
   agreement with the UN-PRUNED model's predictions on the same inputs (with random-init stand-ins this only says how much
-  the pruning perturbs the logits - it is the axis the tests use).
+  the pruning perturbs the logits - it is the axis the tests use).  A headless model (``head`` = Identity, num_classes=0)
+  has no predictions: its accuracy axis is the mean cosine similarity, in %, between each image's pruned and dense features
+  (``cosine_agreement``).
 * ``pareto_front(results)`` - the candidates no other candidate beats on both axes.
 * ``search(make_model, batches, ...)`` - greedy descent from the dense model: repeatedly lower the keep ratio of the one
   block whose step buys the most images/s per point of accuracy lost, while the accuracy stays above the floor.
@@ -112,6 +114,16 @@ def greedy_search(measure_fn: Callable[[Schedule], Dict], depth: int, floor: flo
 
 
 # ------------------------------------------------------------------ measurement (GPU)
+def cosine_agreement(features: Sequence[torch.Tensor], dense_features: Sequence[torch.Tensor]) -> float:
+    """Mean over images of the cosine similarity between an image's features and its dense features, in % (batches of
+    [B, C] in the same order on both sides; fp64 arithmetic)."""
+    total, seen = 0.0, 0
+    for f, d in zip(features, dense_features, strict=True):
+        total += float(torch.nn.functional.cosine_similarity(f.double(), d.to(f.device).double(), dim=1).sum())
+        seen += f.shape[0]
+    return 100.0 * total / seen
+
+
 def _split(batch):
     if isinstance(batch, (tuple, list)):
         return batch[0], (batch[1] if len(batch) > 1 else None)
@@ -123,13 +135,18 @@ def measure(make_model: Callable[[], torch.nn.Module], schedule: Schedule, batch
             dense_predictions: Optional[List[torch.Tensor]] = None, timing_steps: int = 10) -> Dict:
     """One candidate: wrap a FRESH base model (the wrapper replaces its attention modules: `model.py:7-25`), run every batch
     once for the accuracy axis, then time `timing_steps` forwards of the first batch with CUDA events.
-    ``accuracy`` is top-1 against the labels when the batches have them, else the agreement with `dense_predictions`."""
+    ``accuracy`` is top-1 against the labels when the batches have them, else the agreement with `dense_predictions`.
+    A headless model's ``predictions`` are its features, and ``accuracy`` is their ``cosine_agreement`` with
+    `dense_predictions`, labels or not."""
     from .wrapper import RAJNIViTWrapper
     base = make_model()
     model = RAJNIViTWrapper(base, copy.deepcopy(schedule)).to(device).eval()
     preds, correct, labelled, agree, seen = [], 0, 0, 0, 0
     for i, batch in enumerate(batches):
         x, y = _split(batch)
+        if model.headless:
+            preds.append(model(x.to(device, non_blocking=True)))
+            continue
         p = model(x.to(device, non_blocking=True)).argmax(dim=1)
         preds.append(p)
         seen += p.numel()
@@ -156,9 +173,10 @@ def measure(make_model: Callable[[], torch.nn.Module], schedule: Schedule, batch
         "schedule": copy.deepcopy(schedule), "img_s": x0.shape[0] * timing_steps / (e0.elapsed_time(e1) * 1e-3),
         "token_counts": counts,
         "gflop_per_image": flops_per_image(counts, C, blk.mlp.fc1.out_features, (size // p) ** 2,
-                                           classes=base.head.out_features, patch_dim=3 * p * p) / 1e9,
+                                           classes=0 if model.headless else base.head.out_features, patch_dim=3 * p * p) / 1e9,
         "top1": (100.0 * correct / labelled) if labelled else None,
-        "agreement": (100.0 * agree / seen) if dense_predictions is not None else 100.0,
+        "agreement": (100.0 if dense_predictions is None else cosine_agreement(preds, dense_predictions) if model.headless
+                      else 100.0 * agree / seen),
         "predictions": preds,
     }
     out["accuracy"] = out["top1"] if out["top1"] is not None else out["agreement"]
@@ -180,7 +198,8 @@ def sweep(make_model, batches, candidates: Optional[Sequence[Tuple[str, Schedule
 def search(make_model, batches, floor: float, device="cuda", blocks: Optional[Sequence[int]] = None,
            ratios: Sequence[float] = (1.0, 0.9, 0.8, 0.7, 0.6, 0.5), timing_steps: int = 5) -> Tuple[Schedule, List[Dict]]:
     """`greedy_search` with `measure` as the evaluator: the fastest schedule found whose accuracy (top-1 with labels, else
-    agreement with the dense model, both in %) stays at or above `floor`."""
+    agreement with the dense model; for a headless model the features' cosine agreement; all in %) stays at or above
+    `floor`."""
     dense = measure(make_model, {}, batches, device, None, timing_steps)
     depth = len(make_model().blocks)
     cache: Dict[str, Dict] = {}

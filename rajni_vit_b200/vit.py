@@ -28,6 +28,9 @@ and two head / stem variants (extra fields in VIT_POOL_PRENORM):
     a pre-norm stem (CLIP, ``*_clip_*``): a patch embedding without bias, ``norm_pre`` = LayerNorm applied to the embedded
         tokens before block 0, and LayerNorm eps 1e-5 everywhere.
 
+Any of them built with ``num_classes=0`` is headless, as in timm: ``head`` = Identity and the output is the pooled,
+normalised features [B, C].  The DINO backbones (``*_dino``, extra fields in VIT_HEADLESS) are built that way.
+
 It is a plain eager PyTorch module.  It is NOT on the accelerated path: the
 B200 wrapper reads its leaf parameters and runs its own kernels.
 """
@@ -74,11 +77,19 @@ VIT_CONFIGS = {
     "vit_base_patch16_clip_384": (768, 12, 12, 384),
     "vit_micro_patch16_64_mae": (128, 4, 2, 64),
     "vit_micro_patch16_64_clip": (128, 4, 2, 64),
+    # headless self-supervised backbones (DINO: num_classes=0, the output is the normalised class token), and a 4-block test
+    # model
+    "vit_small_patch16_224_dino": (384, 12, 6, 224),
+    "vit_base_patch16_224_dino": (768, 12, 12, 224),
+    "vit_small_patch8_224_dino": (384, 12, 6, 224),
+    "vit_base_patch8_224_dino": (768, 12, 12, 224),
+    "vit_micro_patch16_64_dino": (128, 4, 2, 64),
 }
 # name -> patch size (pixels per side of a patch; 50 tokens at 224 px for 32, 785 for 8)
 VIT_PATCH = {name: 16 for name in VIT_CONFIGS}
 VIT_PATCH.update({"vit_small_patch32_224": 32, "vit_base_patch32_224": 32, "vit_micro_patch32_128": 32, "vit_base_patch32_clip_224": 32,
-                  "vit_small_patch8_224": 8, "vit_base_patch8_224": 8, "vit_micro_patch8_72": 8})
+                  "vit_small_patch8_224": 8, "vit_base_patch8_224": 8, "vit_micro_patch8_72": 8,
+                  "vit_small_patch8_224_dino": 8, "vit_base_patch8_224_dino": 8})
 # name -> extra VisionTransformer arguments of the DeiT families (timm's deit3_* use init_values=1e-6 and no_embed_class;
 # create_model spreads the LayerScale gammas, see spread_layer_scale)
 _DEIT3 = dict(init_values=1e-6, no_embed_class=True)
@@ -88,6 +99,8 @@ VIT_VARIANT.update({name: dict(distilled=True) for name in VIT_CONFIGS if "_dist
 # fc_norm; *_clip_*: pre_norm, no patch-embed bias, LayerNorm eps 1e-5)
 VIT_POOL_PRENORM = {name: dict(global_pool="avg", fc_norm=True) for name in VIT_CONFIGS if name.endswith("_mae")}
 VIT_POOL_PRENORM.update({name: dict(pre_norm=True, patch_bias=False, norm_eps=1e-5) for name in VIT_CONFIGS if "_clip" in name})
+# name -> extra VisionTransformer arguments of the headless models (timm's *.dino weights: num_classes=0, head = Identity)
+VIT_HEADLESS = {name: dict(num_classes=0) for name in VIT_CONFIGS if name.endswith("_dino")}
 
 
 class PatchEmbed(nn.Module):
@@ -176,7 +189,8 @@ class VisionTransformer(nn.Module):
     only.  ``distilled``: a distillation token and ``head_dist`` (timm's VisionTransformerDistilled, eval-mode output).
     ``global_pool``: 'token' (class token) or 'avg' (mean of the tokens after the prefix); ``fc_norm``: the final LayerNorm
     after pooling instead of before it (None: timm's default, on for 'avg').  ``pre_norm``: ``norm_pre`` LayerNorm after the
-    embedding.  ``patch_bias``: the patch projection has a bias.  ``norm_eps``: eps of every LayerNorm."""
+    embedding.  ``patch_bias``: the patch projection has a bias.  ``norm_eps``: eps of every LayerNorm.  ``num_classes=0``:
+    ``head`` (and ``head_dist``) = Identity, timm's headless model."""
 
     def __init__(self, img_size=224, patch_size=16, in_chans=3, num_classes=1000,
                  embed_dim=768, depth=12, num_heads=12, mlp_ratio=4.0, init_values=None, no_embed_class=False,
@@ -200,8 +214,8 @@ class VisionTransformer(nn.Module):
         self.norm = nn.Identity() if use_fc_norm else nn.LayerNorm(embed_dim, eps=norm_eps)
         self.fc_norm = nn.LayerNorm(embed_dim, eps=norm_eps) if use_fc_norm else nn.Identity()
         self.head_drop = nn.Dropout(0.0)
-        self.head = nn.Linear(embed_dim, num_classes)
-        self.head_dist = nn.Linear(embed_dim, num_classes) if distilled else None
+        self.head = nn.Linear(embed_dim, num_classes) if num_classes > 0 else nn.Identity()
+        self.head_dist = (nn.Linear(embed_dim, num_classes) if num_classes > 0 else nn.Identity()) if distilled else None
         nn.init.normal_(self.cls_token, std=0.02)
         nn.init.normal_(self.pos_embed, std=0.02)
         if distilled:
@@ -229,20 +243,22 @@ class VisionTransformer(nn.Module):
 
 
 def create_model(name: str, seed: int | None = 0, bf16_round: bool = True,
-                 num_classes: int = 1000) -> VisionTransformer:
+                 num_classes: int | None = None) -> VisionTransformer:
     """Random-init stand-in for ``timm.create_model(name)`` (no pretrained weights exist here).
 
     seed: torch CPU RNG seed for the init (SURVEY.md section 8d: manual_seed(0)).
     bf16_round: round every parameter to a bf16-representable fp32 value so that the
         fp32 oracle and the bf16 kernel path share bit-identical weights.
+    num_classes: None = the model's own (1000, or 0 for the headless models of VIT_HEADLESS); 0 = headless.
     """
     dim, depth, heads, img = VIT_CONFIGS[name]
     if seed is not None:
         gen_state = torch.random.get_rng_state()
         torch.manual_seed(seed)
-    variant = {**VIT_VARIANT.get(name, {}), **VIT_POOL_PRENORM.get(name, {})}
-    model = VisionTransformer(img_size=img, patch_size=VIT_PATCH[name], embed_dim=dim, depth=depth, num_heads=heads,
-                              num_classes=num_classes, **variant)
+    variant = {"num_classes": 1000, **VIT_VARIANT.get(name, {}), **VIT_POOL_PRENORM.get(name, {}), **VIT_HEADLESS.get(name, {})}
+    if num_classes is not None:
+        variant["num_classes"] = num_classes
+    model = VisionTransformer(img_size=img, patch_size=VIT_PATCH[name], embed_dim=dim, depth=depth, num_heads=heads, **variant)
     if seed is not None:
         torch.random.set_rng_state(gen_state)
     if variant.get("init_values"):

@@ -18,7 +18,9 @@ proj / fc2 weights), a class token without a position (``no_embed_class``), and 
 two prefix tokens, always kept, and the eval-mode average of ``head`` and ``head_dist``).  It also runs average-pooled
 heads (``global_pool='avg'`` with ``fc_norm``, MAE fine-tunes: the mean of the patch tokens the last block kept, then
 fc_norm, in one kernel) and a pre-norm stem (``norm_pre``, CLIP fine-tunes: one LayerNorm pass over the embedded tokens
-that also writes block 0's LayerNorm statistics), with or without a patch-embedding bias.
+that also writes block 0's LayerNorm statistics), with or without a patch-embedding bias.  A headless model (``head`` =
+Identity, timm's ``num_classes=0``: DINO and other backbones) returns its pooled, normalised features [B, C], stored in fp32
+by the final LayerNorm or pooling kernel itself.
 """
 from __future__ import annotations
 
@@ -94,6 +96,7 @@ class RAJNIViTWrapper(nn.Module):
         self.no_embed_class = False      # pos_embed covers the patches only (DeiT-III)
         self.pre_norm = False            # norm_pre LayerNorm after the embedding (CLIP)
         self.avg_pool = False            # head on fc_norm(mean of the patch tokens) (global_pool='avg', MAE)
+        self.headless = False            # head = Identity: forward returns the features the head would read (num_classes=0)
         self.input_norm: Optional[tuple] = None       # (mean[3], std[3]) for uint8 images, see set_input_normalization
         # Stream-K tail of the fc2 GEMMs (gemm_tcgen05.cu): +1.4 % at 32 images per GPU, nothing at 64 and above.  OFF by default
         # because the fp32 summation order of a split tile depends on the tile count, i.e. on the batch size: without it an
@@ -154,8 +157,9 @@ class RAJNIViTWrapper(nn.Module):
         else:
             raise NotImplementedError(f"global_pool={pool!r} is not supported ('token' or 'avg')")
         self.avg_pool = pool == "avg"
-        if not isinstance(m.head, nn.Linear):
-            raise NotImplementedError("head must be Linear")
+        if not isinstance(m.head, nn.Linear) and not _is_identity(m.head):
+            raise NotImplementedError(f"head = {type(m.head).__name__} is not supported (Linear, or Identity for a headless model)")
+        self.headless = _is_identity(m.head)
         # prefix tokens: CLS, or CLS + distillation token (distilled DeiT); register tokens are not supported
         if getattr(m, "cls_token", None) is None:
             raise NotImplementedError("a class token (cls_token) is required")
@@ -164,6 +168,9 @@ class RAJNIViTWrapper(nn.Module):
         dist, head_dist = getattr(m, "dist_token", None), getattr(m, "head_dist", None)
         prefix = int(getattr(m, "num_prefix_tokens", 1))
         if dist is not None:
+            if self.headless:
+                raise NotImplementedError("a dist_token with head = Identity (headless) is not supported: timm would return the "
+                                          "mean of the normalised class and distillation tokens")
             if not isinstance(head_dist, nn.Linear) or head_dist.weight.shape != m.head.weight.shape:
                 raise NotImplementedError("a dist_token needs head_dist, a Linear of the head's shape")
             if prefix != 2:
@@ -318,7 +325,8 @@ class RAJNIViTWrapper(nn.Module):
             raise ValueError(f"expected images [B,3,S,S] with S a multiple of the patch size {self.patch}, got {tuple(x.shape)}")
         if x.device.type != "cuda":
             raise RuntimeError("RAJNIViTWrapper (B200) runs on CUDA tensors only; there is no CPU path")
-        if self.m.pos_embed.device != x.device or self.m.head.weight.device != x.device:
+        last = self.m.head if not self.headless else self.m.fc_norm if self.avg_pool else self.m.norm      # the last module with weights
+        if self.m.pos_embed.device != x.device or last.weight.device != x.device:
             raise RuntimeError(f"Expected all tensors to be on the same device: input on {x.device}, model on "
                                f"{self.m.pos_embed.device} (call .to(device) on the wrapper first)")
         if self.training:
@@ -435,7 +443,13 @@ class RAJNIViTWrapper(nn.Module):
             rev = zig and not rev
 
         # ---- final norm on the CLS rows only (LayerNorm is row-wise) + head   model.py:65-66
-        if self.avg_pool:               # timm forward_head, global_pool='avg': head(fc_norm(mean of the kept patch tokens))
+        if self.headless:               # the head's input is the output, stored in fp32 by the kernel that computes it
+            logits = torch.empty((B, C), device=x.device, dtype=torch.float32)
+            if self.avg_pool:
+                ops.mean_pool_layernorm(cur, B, N, C, *pk.norm(m.fc_norm), prefix=P0, out=logits)
+            else:
+                ops.layernorm(cur, *pk.norm(m.norm), B, C, in_row_stride=N * C, out=logits)
+        elif self.avg_pool:             # timm forward_head, global_pool='avg': head(fc_norm(mean of the kept patch tokens))
             gf, bf_, ef = pk.norm(m.fc_norm)
             hw, hb = pk.linear(m.head)
             ops.mean_pool_layernorm(cur, B, N, C, gf, bf_, ef, prefix=P0, out=ws["cls"])

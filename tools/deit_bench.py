@@ -15,7 +15,8 @@
 e.g. ``vit_base_patch16_224,vit_base_patch16_224_mae,vit_base_patch16_clip_224`` for the average-pooled and pre-norm models.
 3. ``--kernels``: the two kernels of those models in isolation - the pooled head (mean of the patch rows + fc_norm) and the
    LayerNorm pass that also writes row statistics (norm_pre) - at ViT-B/16 shapes (197 tokens, C = 768) for 256 and 8
-   images.  Each launch timed alone with CUDA events after a 256 MB write has flushed L2; median over the launches.
+   images, and the final LayerNorm on the class-token rows and the pooled head with bf16 and with fp32 rows out (fp32: a
+   headless model's features).  Each launch timed alone with CUDA events after a 256 MB write has flushed L2; median over the launches.
    Achieved bytes/s are the bytes each kernel must move (rows read, rows and statistics written) over that time, and
    are also given as a share of the 6.45 TB/s a device-to-device copy reaches on a B200.
 The card name and power limit are read in the same run and printed first."""
@@ -100,7 +101,7 @@ def kernel_report(say):
     g = torch.Generator(device="cuda").manual_seed(0)
     gamma = 0.5 + torch.rand(C, device="cuda", generator=g)
     beta = 0.1 * torch.randn(C, device="cuda", generator=g)
-    say("## pooled head and norm_pre kernels, C = %d, %d tokens per image, L2 flushed before each launch" % (C, N))
+    say("## pooled head, final LayerNorm and norm_pre kernels, C = %d, %d tokens per image, L2 flushed before each launch" % (C, N))
     for B in (256, 8):
         x = torch.randn(B * N, C, device="cuda", generator=g).to(torch.bfloat16)
         out = torch.empty(B, C, device="cuda", dtype=torch.bfloat16)
@@ -108,6 +109,15 @@ def kernel_report(say):
         nbytes = B * (N - 1) * C * 2 + B * C * 2
         say(f"mean_pool_layernorm   B={B:3d}: {t:8.2f} us  {nbytes / 1e6:8.2f} MB  {nbytes / t / 1e6:7.3f} TB/s  "
             f"{nbytes / t / 1e-6 / COPY_BYTES_PER_S * 100:5.1f} % of copy")
+        outf = torch.empty(B, C, device="cuda", dtype=torch.float32)
+        t = time_kernel_cold(lambda: ops.mean_pool_layernorm(x, B, N, C, gamma, beta, 1e-6, prefix=1, out=outf))
+        nbytes = B * (N - 1) * C * 2 + B * C * 4
+        say(f"mean_pool_layernorm_f32 B={B:3d}: {t:8.2f} us  {nbytes / 1e6:8.2f} MB  {nbytes / t / 1e6:7.3f} TB/s  "
+            f"{nbytes / t / 1e-6 / COPY_BYTES_PER_S * 100:5.1f} % of copy")
+        for kname, o in (("layernorm (CLS rows)", out), ("layernorm_f32 (CLS rows)", outf)):
+            t = time_kernel_cold(lambda: ops.layernorm(x, gamma, beta, 1e-6, B, C, in_row_stride=N * C, out=o))
+            nbytes = B * C * 2 + B * C * o.element_size()
+            say(f"{kname:24s} B={B:3d}: {t:8.2f} us  {nbytes / 1e6:8.2f} MB  {nbytes / t / 1e6:7.3f} TB/s")
         st = torch.empty(slots, B * N, 2, device="cuda")
         y = torch.empty_like(x)
         t = time_kernel_cold(lambda: ops.layernorm(x, gamma, beta, 1e-5, B * N, C, out=y, row_stats=st, stats_slots=slots))
@@ -124,7 +134,7 @@ def main():
     ap.add_argument("--rounds", type=int, default=3)
     ap.add_argument("--out", help="also write the report to this file")
     ap.add_argument("--models", default=",".join(MODELS), help="comma-separated stand-ins; the first is the baseline")
-    ap.add_argument("--kernels", action="store_true", help="also time the pooled-head and norm_pre kernels")
+    ap.add_argument("--kernels", action="store_true", help="also time the pooled-head, final LayerNorm and norm_pre kernels")
     args = ap.parse_args()
     models = args.models.split(",")
     lines = []
