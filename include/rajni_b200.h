@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define RAJNI_ABI_VERSION 10     /* 10: rajni_patch_im2col takes any patch that is a multiple of 8; long-sequence scores */
+#define RAJNI_ABI_VERSION 11     /* 11: one entry point per operation; the superseded calls are gone */
 
 enum {
     RAJNI_OK = 0,
@@ -38,7 +38,7 @@ enum {
     RAJNI_ERANGE = -4    /* keep > N-1: the reference's topk raises here         */
 };
 
-/* epilogue flags for rajni_gemm_bf16 */
+/* epilogue flags for rajni_gemm_bf16_ex (rajni_gemm_args.flags) */
 enum {
     RAJNI_EPI_BIAS = 1,       /* + bias[n]                                       */
     RAJNI_EPI_GELU = 2,       /* exact erf GELU (timm nn.GELU) after bias        */
@@ -59,56 +59,35 @@ int rajni_device_check(void);
 /* number of kernels this library has launched in this process (bench.py's gpu_launches). */
 uint64_t rajni_launch_count(void);
 
-/* ---- a1: compute_importance (rajni/wrapper/importance.py:5-34) ------------------
- * qkv [B,N,3C] bf16 with the last dim laid out (3,H,D); scores [B,N] fp32.
- * bf16 tiles in, fp32 arithmetic (SURVEY.md section 4.5). D must be 64. */
-int rajni_importance(const void* qkv, int B, int N, int C, int H, float eps,
-                     float* scores, void* stream);
-
-/* ---- a2: token selection (rajni/wrapper/attention.py:31-39) and score carry (:58)
- * Top-`keep` of scores[:,1:] -> keep_idx [B,keep+1] int32, strictly ascending,
- * keep_idx[:,0]==0. Tie rule: greater score first, then lower index.
- * next_scores [B,keep+1] = scores[keep_idx]. row_map [B*(keep+1)] = b*N+keep_idx
- * (global row of each kept token; nullable). keep > N-1 -> RAJNI_ERANGE. */
-int rajni_select(const float* scores, int B, int N, int keep,
-                 int32_t* keep_idx, float* next_scores, int32_t* row_map, void* stream);
-/* The same with `prefix` (1 or 2) leading tokens that are always kept: CLS, or CLS and a distillation token.
- * Top-`keep` of scores[:,prefix:] -> keep_idx [B,keep+prefix] int32, strictly ascending, keep_idx[:,r]==r for
- * r < prefix; next_scores and row_map [B*(keep+prefix)] as above.  keep > N-prefix -> RAJNI_ERANGE.
- * rajni_select is this call with prefix 1. */
+/* ---- a2: token selection on carried scores (rajni/wrapper/attention.py:31-39) and score carry (:58)
+ * `prefix` (1 or 2) leading tokens are always kept: CLS, or CLS and a distillation token.  Top-`keep` of
+ * scores[:,prefix:] -> keep_idx [B,keep+prefix] int32, strictly ascending, keep_idx[:,r]==r for r < prefix.  Tie rule:
+ * greater score first, then lower index.  next_scores [B,keep+prefix] = scores[keep_idx].  row_map [B*(keep+prefix)] =
+ * b*N+keep_idx (global row of each kept token; nullable).  keep > N-prefix -> RAJNI_ERANGE. */
 int rajni_select_prefix(const float* scores, int B, int N, int prefix, int keep,
                         int32_t* keep_idx, float* next_scores, int32_t* row_map, void* stream);
 
-/* ---- a1+a2 fused: one pass over the K and V planes, then in-CTA select.
- * scores may be NULL when the caller does not need the full score vector.
- * rajni_importance and rajni_score_select keep one image's CLS logits and value rows in shared memory; shapes for which
- * rajni_score_select_needs_workspace(N, H) is 1 (N > ~720 at 12 heads) return RAJNI_EINVAL there: use the split entry. */
-int rajni_score_select(const void* qkv, int B, int N, int C, int H, int keep, float eps,
-                       float* scores, int32_t* keep_idx, float* next_scores,
-                       int32_t* row_map, void* stream);
-
-/* Same result, bit for bit, in two launches for batches with far fewer images than the GPU has SMs (one CTA per image
- * would leave most SMs idle): the K/V pass is spread over (image, 16-row block) CTAs into `workspace`
+/* ---- a1: compute_importance (rajni/wrapper/importance.py:5-34) fused with a2: one pass over the K and V planes, then
+ * the selection of rajni_select_prefix in the same CTA.
+ * qkv [B,N,3C] bf16 with the last dim laid out (3,H,D), D must be 64; scores [B,N] fp32, may be NULL when the caller does
+ * not need the full score vector.  bf16 tiles in, fp32 arithmetic (SURVEY.md section 4.5).  The scores do not depend on
+ * `prefix`: the query is row 0 (CLS), every token (a distillation token too) is a key and value and enters the value-norm
+ * statistics.  keep_idx == NULL computes the scores only: then `scores` is required, and prefix, keep, next_scores and
+ * row_map are ignored.
+ * workspace == NULL: one launch, one CTA per image, which keeps the image's CLS logits and value rows in shared memory;
+ * shapes for which rajni_score_select_needs_workspace(N, H) is 1 (N > ~720 at 12 heads) return RAJNI_EINVAL.
+ * workspace != NULL: the same result, bit for bit, in two launches, for batches with far fewer images than the GPU has SMs
+ * (one CTA per image would leave most SMs idle): the K/V pass is spread over (image, 16-row block) CTAs into `workspace`
  * (rajni_score_select_workspace_bytes(B,N,C,H) bytes, 16-byte aligned, caller-owned), then the per-image kernel finishes.
- * Every N <= 4096 works here at any batch: when rajni_score_select_needs_workspace(N, H) is 1 the per-image kernel reads
- * the logits and value rows from the workspace in place (same arithmetic, same bits).  keep_idx == NULL computes the
- * scores only (a scores-only call of rajni_importance's meaning): then `scores` is required, keep, next_scores and
- * row_map are ignored. */
-size_t rajni_score_select_workspace_bytes(int B, int N, int C, int H);
-/* Host-side query, no launch: 1 when one image of N tokens and H heads needs the workspace path of
- * rajni_score_select_split (its CLS logits and value rows exceed the per-image kernel's shared memory), else 0. */
-int rajni_score_select_needs_workspace(int N, int H);
-int rajni_score_select_split(const void* qkv, int B, int N, int C, int H, int keep, float eps,
-                             float* scores, int32_t* keep_idx, float* next_scores, int32_t* row_map,
-                             void* workspace, size_t workspace_bytes, void* stream);
-/* Both of the above with `prefix` (1 or 2) always-kept leading tokens, selection as in rajni_select_prefix.  The scores do
- * not depend on it: the query is row 0 (CLS), every token (a distillation token too) is a key and value and enters the
- * value-norm statistics.  workspace == NULL: rajni_score_select's one-launch kernel; else rajni_score_select_split's two
- * launches (same bits).  keep_idx == NULL computes the scores only.  rajni_score_select and rajni_score_select_split are
- * this call with prefix 1. */
+ * Every N <= 4096 works this way at any batch: when rajni_score_select_needs_workspace(N, H) is 1 the per-image kernel
+ * reads the logits and value rows from the workspace in place (same arithmetic, same bits). */
 int rajni_score_select_prefix(const void* qkv, int B, int N, int C, int H, int prefix, int keep, float eps,
                               float* scores, int32_t* keep_idx, float* next_scores, int32_t* row_map,
                               void* workspace, size_t workspace_bytes, void* stream);
+size_t rajni_score_select_workspace_bytes(int B, int N, int C, int H);
+/* Host-side query, no launch: 1 when one image of N tokens and H heads needs the workspace of rajni_score_select_prefix
+ * (its CLS logits and value rows exceed the per-image kernel's shared memory), else 0. */
+int rajni_score_select_needs_workspace(int N, int H);
 
 /* ---- a3 / a9: row gather-compaction (attention.py:42-43, model.py:55-56)
  * dst[r, :] = src[row_map[r], :], rows of `row_elems` bf16 (multiple of 8). */
@@ -116,22 +95,21 @@ int rajni_gather_rows(const void* src, const int32_t* row_map, void* dst,
                       int rows_out, int row_elems, void* stream);
 
 /* ---- LayerNorm over the last dim (model.py:51,59,65), bf16 -> bf16, fp32 math.
- * Row r is read at x + r*in_row_stride elements (lets the final norm touch CLS
- * rows only) and written densely at y + r*C. C multiple of 8, C <= 4096. */
-int rajni_layernorm(const void* x, long long in_row_stride, const float* gamma,
-                    const float* beta, float eps, void* y, int rows, int C, void* stream);
-/* The same with row r written at y + r*out_row_stride (>= C, multiple of 8): two calls with out_row_stride 2C put the
- * normalised CLS and distillation rows of each image side by side, the A operand of a distilled model's head. */
+ * Row r is read at x + r*in_row_stride elements (multiple of 8; lets the final norm touch CLS rows only) and written at
+ * y + r*out_row_stride (>= C, multiple of 8; C for dense rows).  Two calls with out_row_stride 2C put the normalised CLS
+ * and distillation rows of each image side by side, the A operand of a distilled model's head.  C multiple of 8,
+ * C <= 2048. */
 int rajni_layernorm_strided(const void* x, long long in_row_stride, const float* gamma, const float* beta, float eps,
                             void* y, long long out_row_stride, int rows, int C, void* stream);
-/* The same values stored as fp32 (the features of a headless model, num_classes = 0): y + r*out_row_stride floats,
- * out_row_stride >= C and a multiple of 4.  bf16_rn of each value is what rajni_layernorm_strided stores. */
+/* rajni_layernorm_strided's values stored as fp32 (the features of a headless model, num_classes = 0):
+ * y + r*out_row_stride floats, out_row_stride >= C and a multiple of 4.  bf16_rn of each value is what
+ * rajni_layernorm_strided stores. */
 int rajni_layernorm_strided_f32(const void* x, long long in_row_stride, const float* gamma, const float* beta, float eps,
                                 float* y, long long out_row_stride, int rows, int C, void* stream);
-/* The same over a whole activation matrix, also emitting the rows' LayerNorm partial sums for an LN-folded GEMM
- * (RAJNI_EPI_LN_FOLD) that reads y next: row_stats[s*row_stats_ld + r] = (sum, sum of squares) of the bf16 row r as stored
- * for s = 0, zero for s = 1..stats_slots-1 (the slot layout of RAJNI_EPI_ROW_STATS).  y may be x (in place).  This is the
- * pre-norm stem of CLIP ViTs (timm's norm_pre), applied to the embedded tokens before block 0.  C <= 2048. */
+/* rajni_layernorm_strided over a whole activation matrix, also emitting the rows' LayerNorm partial sums for an
+ * LN-folded GEMM (RAJNI_EPI_LN_FOLD) that reads y next: row_stats[s*row_stats_ld + r] = (sum, sum of squares) of the bf16
+ * row r as stored for s = 0, zero for s = 1..stats_slots-1 (the slot layout of RAJNI_EPI_ROW_STATS).  y may be x (in
+ * place).  This is the pre-norm stem of CLIP ViTs (timm's norm_pre), applied to the embedded tokens before block 0. */
 int rajni_layernorm_row_stats(const void* x, long long in_row_stride, const float* gamma, const float* beta, float eps,
                               void* y, long long out_row_stride, int rows, int C,
                               float* row_stats, long long row_stats_ld, int stats_slots, void* stream);
@@ -150,16 +128,13 @@ int rajni_mean_pool_layernorm_f32(const void* x, int B, int N, int prefix, int C
 
 /* ---- dense contractions (attention.py:22,55; timm Mlp fc1/fc2; patch_embed; head)
  * D[orow(m), n] = epi( sum_k A[m,k] * W[n,k] ), A [M,K] bf16, W [N,K] bf16
- * (nn.Linear layout), fp32 accumulation in TMEM (tcgen05.mma, TMA-fed).
+ * (nn.Linear layout), fp32 accumulation in TMEM (tcgen05.mma, TMA-fed); epi as set by the RAJNI_EPI_* flags.
  *   orow(m) = out_row_map ? out_row_map[m] : m
  *   res row = res_row_map ? res_row_map[m] : m      (gathered residual, model.py:55-58)
- * K multiple of 8; ldd/ldres are row strides in elements (multiples of 8). */
-int rajni_gemm_bf16(const void* A, const void* W, const float* bias, void* D,
-                    int M, int N, int K, int flags,
-                    const void* residual, long long ldres, const int32_t* res_row_map,
-                    long long ldd, const int32_t* out_row_map, void* stream);
-
-/* ---- the same contraction with LayerNorm folded in (model.py:51 norm1 -> qkv, model.py:59 norm2 -> fc1)
+ * K multiple of 8; ldd/ldres are row strides in elements (multiples of 8).  The arguments travel in a struct; the fields a
+ * call does not use are zero.
+ *
+ * LayerNorm folded in (model.py:51 norm1 -> qkv, model.py:59 norm2 -> fc1):
  *
  *   LN(x) W^T + b  =  rstd[m] * ( x (W.gamma)^T )[m,n]  -  rstd[m]*mean[m] * wsum[n]  +  ( b + W beta )[n]
  *
@@ -198,12 +173,10 @@ int rajni_gemm_row_stats_slots(int N);
  * reverse != 0: process the images last-to-first (L2 reuse hint, see RAJNI_HINT_REVERSE_M).
  * Images are independent for finite inputs.  Np > 64: also for non-finite ones (a NaN/Inf in one image never reaches
  * another's output).  Np <= 64: consecutive images may share a tile and one P V product (masked softmax): a NaN/Inf VALUE row
- * then reaches the images packed with it (0 * NaN); the environment variable RAJNI_ATTN_NOPACK=1 keeps one image per tile. */
-int rajni_attention_fwd(const void* qkv, const int32_t* row_map, void* out,
-                        int B, int N_src, int Np, int C, int H, float scale, int reverse, void* stream);
-/* The same call with the kernel chosen by the caller (tests and A/B timing; results agree within bf16 rounding):
- * AUTO = what rajni_attention_fwd picks; PIPE = role-pipelined kernel (Np_pad <= 224); TC = two-tile kernel (Np <= 256);
- * LONG = key-block kernel (built for Np > 256).  A kernel asked for a shape it does not cover returns RAJNI_EINVAL. */
+ * then reaches the images packed with it (0 * NaN); the environment variable RAJNI_ATTN_NOPACK=1 keeps one image per tile.
+ * impl picks the kernel: AUTO = the library's choice by shape (every caller but tests and A/B timing); PIPE =
+ * role-pipelined kernel (Np_pad <= 224); TC = two-tile kernel (Np <= 256); LONG = key-block kernel (built for Np > 256).
+ * Their results agree within bf16 rounding.  A kernel asked for a shape it does not cover returns RAJNI_EINVAL. */
 enum { RAJNI_ATTN_AUTO = 0, RAJNI_ATTN_PIPE = 1, RAJNI_ATTN_TC = 2, RAJNI_ATTN_LONG = 3 };
 int rajni_attention_fwd_ex(const void* qkv, const int32_t* row_map, void* out,
                            int B, int N_src, int Np, int C, int H, float scale, int reverse, int impl, void* stream);
@@ -214,20 +187,13 @@ int rajni_attention_fwd_ex(const void* qkv, const int32_t* row_map, void* out,
  * 16 only before), so 3*p*p is a multiple of 64.  RAJNI_IMG_U8: raw pixels, normalised here as the reference's
  * loader does in fp32 (run.py:62-70: ToTensor + Normalize): (u/255 - norm[c]) / norm[3+c] with
  * norm = HOST array {mean[3], std[3]} (read at call time); other dtypes ignore norm (may be NULL).
- * Also writes the CLS rows
- * x[b,0,:] = cls_pos0[:] (= cls_token + pos_embed[0], precomputed) into x [B,1+P,C] and, when
- * row_stats != NULL, the LayerNorm partials of those rows (slot 0 = (cls_sum, cls_sumsq), the
- * other `stats_slots-1` slots zero) in the layout RAJNI_EPI_ROW_STATS uses. */
+ * Also writes the `prefix` (1 or 2) rows in front of each image's patches: x is [B,P+prefix,C], and x[b,r,:] =
+ * prefix_rows[r,:] for r < prefix (prefix_rows [prefix,C] bf16: cls_token + pos_embed[0], then dist_token + pos_embed[1]
+ * for a distilled DeiT; the tokens alone for a model that adds positions to the patches only).  The embed GEMM stores
+ * patch q of image b at row b*(P+prefix) + prefix + q.  When row_stats != NULL, also the LayerNorm partials of the prefix
+ * rows in the layout RAJNI_EPI_ROW_STATS uses: slot 0 of row r = prefix_stats_host[r] (a HOST array [prefix][2] of each
+ * row's sum and sum of squares, read at call time), the other `stats_slots-1` slots zero. */
 enum { RAJNI_IMG_BF16 = 0, RAJNI_IMG_F32 = 1, RAJNI_IMG_U8 = 2 };
-int rajni_patch_im2col(const void* images, int image_dtype, int B, int S, int patch,
-                       void* cols, const void* cls_pos0, void* x, int C,
-                       float* row_stats, long long row_stats_ld, int stats_slots,
-                       float cls_sum, float cls_sumsq, const float* norm, void* stream);
-/* The same with `prefix` (1 or 2) rows in front of each image's patches: x is [B,P+prefix,C], and x[b,r,:] =
- * prefix_rows[r,:] for r < prefix (prefix_rows [prefix,C] bf16: cls_token + pos_embed[0], dist_token + pos_embed[1]; the
- * tokens alone for a model that adds positions to the patches only).  With row_stats, prefix_stats_host = HOST array
- * [prefix][2] of each row's (sum, sum of squares), written to slot 0 (read at call time).  The embed GEMM stores patch q
- * of image b at row b*(P+prefix) + prefix + q.  rajni_patch_im2col is this call with prefix 1. */
 int rajni_patch_im2col_prefix(const void* images, int image_dtype, int B, int S, int patch,
                               void* cols, const void* prefix_rows, int prefix, void* x, int C,
                               float* row_stats, long long row_stats_ld, int stats_slots,
@@ -237,7 +203,7 @@ int rajni_patch_im2col_prefix(const void* images, int image_dtype, int B, int S,
  * to torchvision on PIL images (Pillow's antialiased two-pass resampler; oracle/resize_oracle.py restates it).
  * frames: device buffer, the B decoded frames (HWC, uint8) back to back; meta: DEVICE int64 [B][3] = (byte offset of the
  * frame in `frames`, height, width); max_h >= every height.  out: uint8 [B,3,224,224] planar - what PILToTensor gives after
- * the two transforms; feed it to rajni_patch_im2col (RAJNI_IMG_U8) for ToTensor + Normalize.
+ * the two transforms; feed it to rajni_patch_im2col_prefix (RAJNI_IMG_U8) for ToTensor + Normalize.
  * workspace: rajni_resize_workspace_bytes(B, max_h) bytes.  A frame that cannot be handled (shorter edge would end up
  * below the crop, height above max_h, downscale beyond ~23x) is skipped and reported by rajni_resize_status (which
  * synchronises the stream): 0 = all frames done, else 1 + index of a rejected frame. */

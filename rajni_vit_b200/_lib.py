@@ -15,7 +15,7 @@ LIB_PATH = os.path.join(_HERE, "csrc", "librajni_b200.so")
 RAJNI_OK, RAJNI_EINVAL, RAJNI_ECUDA, RAJNI_EARCH, RAJNI_ERANGE = 0, -1, -2, -3, -4
 ATTN_AUTO, ATTN_PIPE, ATTN_TC, ATTN_LONG = 0, 1, 2, 3
 EPI_BIAS, EPI_GELU, EPI_RESIDUAL, EPI_OUT_F32, EPI_LN_FOLD, EPI_ROW_STATS, HINT_REVERSE_M, HINT_STREAM_K = 1, 2, 4, 8, 16, 32, 64, 128
-ABI_VERSION = 10
+ABI_VERSION = 11
 
 
 class GemmArgs(Structure):
@@ -37,19 +37,12 @@ SIGNATURES = {
     "rajni_last_error": (c_char_p, []),
     "rajni_device_check": (c_int, []),
     "rajni_launch_count": (c_uint64, []),
-    "rajni_importance": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_float, c_void_p, c_void_p]),
-    "rajni_select": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     "rajni_select_prefix": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
-    "rajni_score_select": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_float,
-                                   c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "rajni_score_select_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int]),
     "rajni_score_select_needs_workspace": (c_int, [c_int, c_int]),
-    "rajni_score_select_split": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_float,
-                                         c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "rajni_score_select_prefix": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_float,
                                           c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "rajni_gather_rows": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p]),
-    "rajni_layernorm": (c_int, [c_void_p, c_longlong, c_void_p, c_void_p, c_float, c_void_p, c_int, c_int, c_void_p]),
     "rajni_layernorm_strided": (c_int, [c_void_p, c_longlong, c_void_p, c_void_p, c_float, c_void_p, c_longlong, c_int, c_int,
                                         c_void_p]),
     "rajni_layernorm_strided_f32": (c_int, [c_void_p, c_longlong, c_void_p, c_void_p, c_float, c_void_p, c_longlong, c_int, c_int,
@@ -60,19 +53,14 @@ SIGNATURES = {
                                           c_void_p]),
     "rajni_mean_pool_layernorm_f32": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_float, c_void_p,
                                               c_longlong, c_void_p]),
-    "rajni_gemm_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int,
-                                c_void_p, c_longlong, c_void_p, c_longlong, c_void_p, c_void_p]),
     "rajni_gemm_bf16_ex": (c_int, [POINTER(GemmArgs), c_void_p]),
     "rajni_gemm_row_stats_slots": (c_int, [c_int]),
     "rajni_gemm_workspace_bytes": (c_size_t, []),
     "rajni_gemm_stream_k_plan": (c_int, [c_int, c_int, c_int, c_int, c_void_p]),
-    "rajni_attention_fwd": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_float, c_int, c_void_p]),
     "rajni_attention_fwd_ex": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_float, c_int, c_int, c_void_p]),
     "rajni_resize_workspace_bytes": (c_size_t, [c_int, c_int]),
     "rajni_resize_center_crop_u8": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
     "rajni_resize_status": (c_int, [c_void_p, c_int, c_int, c_void_p]),
-    "rajni_patch_im2col": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int,
-                                   c_void_p, c_longlong, c_int, c_float, c_float, c_void_p, c_void_p]),
     "rajni_patch_im2col_prefix": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p, c_int,
                                           c_void_p, c_longlong, c_int, c_void_p, c_void_p, c_void_p]),
 }

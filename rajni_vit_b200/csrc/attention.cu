@@ -30,12 +30,13 @@ int launch_attention_long(const void* qkv, const int32_t* row_map, void* out, in
 
 using namespace rajni;
 
-static int attention_dispatch(const void* qkv, const int32_t* row_map, void* out, int B, int N_src, int Np, int C, int H,
-                              float scale, int reverse, int impl, cudaStream_t st) {
-    RAJNI_REQUIRE(qkv && out, RAJNI_EINVAL, "rajni_attention_fwd: null pointer");
+extern "C" int rajni_attention_fwd_ex(const void* qkv, const int32_t* row_map, void* out,
+                                      int B, int N_src, int Np, int C, int H, float scale, int reverse, int impl, void* stream) {
+    auto st = static_cast<cudaStream_t>(stream);
+    RAJNI_REQUIRE(qkv && out, RAJNI_EINVAL, "rajni_attention_fwd_ex: null pointer");
     RAJNI_REQUIRE(B > 0 && Np > 0 && N_src >= Np && H > 0 && C == H * 64, RAJNI_EINVAL,
-                  "rajni_attention_fwd: B=%d N_src=%d Np=%d C=%d H=%d (head dim must be 64)", B, N_src, Np, C, H);
-    RAJNI_REQUIRE(row_map || N_src == Np, RAJNI_EINVAL, "rajni_attention_fwd: N_src != Np needs a row_map");
+                  "rajni_attention_fwd_ex: B=%d N_src=%d Np=%d C=%d H=%d (head dim must be 64)", B, N_src, Np, C, H);
+    RAJNI_REQUIRE(row_map || N_src == Np, RAJNI_EINVAL, "rajni_attention_fwd_ex: N_src != Np needs a row_map");
     RAJNI_REQUIRE(impl >= RAJNI_ATTN_AUTO && impl <= RAJNI_ATTN_LONG, RAJNI_EINVAL, "rajni_attention_fwd_ex: impl %d", impl);
     if (impl == RAJNI_ATTN_AUTO) {
         static const bool force_tc = getenv("RAJNI_ATTN_TC") != nullptr, force_pipe = getenv("RAJNI_ATTN_PIPE") != nullptr;
@@ -52,18 +53,8 @@ static int attention_dispatch(const void* qkv, const int32_t* row_map, void* out
     else if (impl == RAJNI_ATTN_TC) rc = launch_attention_tc(qkv, row_map, out, B, N_src, Np, C, H, scale, reverse, st);
     else rc = launch_attention_long(qkv, row_map, out, B, N_src, Np, C, H, scale, reverse, st);
     if (rc == 0) {
-        set_error("rajni_attention_fwd: kernel %d does not cover Np=%d", impl, Np);
+        set_error("rajni_attention_fwd_ex: kernel %d does not cover Np=%d", impl, Np);
         return RAJNI_EINVAL;
     }
     return rc < 0 ? rc : RAJNI_OK;
-}
-
-extern "C" int rajni_attention_fwd(const void* qkv, const int32_t* row_map, void* out,
-                                   int B, int N_src, int Np, int C, int H, float scale, int reverse, void* stream) {
-    return attention_dispatch(qkv, row_map, out, B, N_src, Np, C, H, scale, reverse, RAJNI_ATTN_AUTO, static_cast<cudaStream_t>(stream));
-}
-
-extern "C" int rajni_attention_fwd_ex(const void* qkv, const int32_t* row_map, void* out,
-                                      int B, int N_src, int Np, int C, int H, float scale, int reverse, int impl, void* stream) {
-    return attention_dispatch(qkv, row_map, out, B, N_src, Np, C, H, scale, reverse, impl, static_cast<cudaStream_t>(stream));
 }

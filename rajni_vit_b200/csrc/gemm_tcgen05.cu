@@ -828,7 +828,7 @@ static int launch_gemm(const void* A, const void* W, GemmParams& p, void* ws, si
             return launch_gemm_mode<BN, CG, MODE_BIAS_RES, false>(A, W, p, ws, ws_bytes, stream);
     }
     RAJNI_REQUIRE(!ln && !stats, RAJNI_EINVAL,
-                  "rajni_gemm_bf16: LN_FOLD / ROW_STATS need N %% %d == 0, ldd/ldres multiples of 16 and 32-byte aligned rows "
+                  "rajni_gemm_bf16_ex: LN_FOLD / ROW_STATS need N %% %d == 0, ldd/ldres multiples of 16 and 32-byte aligned rows "
                   "(N=%d ldd=%lld ldres=%lld flags=%d)", BN, p.N, p.ldd, p.ldres, p.flags);
     return launch_gemm_mode<BN, CG, MODE_GENERIC, false>(A, W, p, ws, ws_bytes, stream);
 }
@@ -906,18 +906,18 @@ extern "C" int rajni_gemm_stream_k_plan(int M, int N, int K, int flags, int* sk_
 extern "C" int rajni_gemm_bf16_ex(const rajni_gemm_args* a, void* stream) {
     RAJNI_REQUIRE(a != nullptr, RAJNI_EINVAL, "rajni_gemm_bf16_ex: null argument block");
     const int M = a->M, N = a->N, K = a->K, flags = a->flags;
-    RAJNI_REQUIRE(a->A && a->W && a->D, RAJNI_EINVAL, "rajni_gemm_bf16: null pointer");
-    RAJNI_REQUIRE(M > 0 && N > 0 && K > 0 && K % 8 == 0, RAJNI_EINVAL, "rajni_gemm_bf16: M=%d N=%d K=%d (K must be a multiple of 8)", M, N, K);
-    RAJNI_REQUIRE(!(flags & RAJNI_EPI_BIAS) || a->bias, RAJNI_EINVAL, "rajni_gemm_bf16: bias flag without bias");
-    RAJNI_REQUIRE(!(flags & RAJNI_EPI_RESIDUAL) || a->residual, RAJNI_EINVAL, "rajni_gemm_bf16: residual flag without residual");
+    RAJNI_REQUIRE(a->A && a->W && a->D, RAJNI_EINVAL, "rajni_gemm_bf16_ex: null pointer");
+    RAJNI_REQUIRE(M > 0 && N > 0 && K > 0 && K % 8 == 0, RAJNI_EINVAL, "rajni_gemm_bf16_ex: M=%d N=%d K=%d (K must be a multiple of 8)", M, N, K);
+    RAJNI_REQUIRE(!(flags & RAJNI_EPI_BIAS) || a->bias, RAJNI_EINVAL, "rajni_gemm_bf16_ex: bias flag without bias");
+    RAJNI_REQUIRE(!(flags & RAJNI_EPI_RESIDUAL) || a->residual, RAJNI_EINVAL, "rajni_gemm_bf16_ex: residual flag without residual");
     RAJNI_REQUIRE(a->ldd >= N && a->ldd % 4 == 0 && (!(flags & RAJNI_EPI_RESIDUAL) || a->ldres % 4 == 0), RAJNI_EINVAL,
-                  "rajni_gemm_bf16: ldd=%lld ldres=%lld must be multiples of 4 and ldd >= N", a->ldd, a->ldres);
+                  "rajni_gemm_bf16_ex: ldd=%lld ldres=%lld must be multiples of 4 and ldd >= N", a->ldd, a->ldres);
     if (flags & RAJNI_EPI_LN_FOLD)
         RAJNI_REQUIRE(a->ln_stats && a->ln_wsum && a->ln_slots > 0 && a->ln_stats_ld >= M && (flags & RAJNI_EPI_BIAS) && !(flags & RAJNI_EPI_OUT_F32),
-                      RAJNI_EINVAL, "rajni_gemm_bf16: LN_FOLD needs ln_stats, ln_wsum, ln_slots > 0, ln_stats_ld >= M, a bias and bf16 output");
+                      RAJNI_EINVAL, "rajni_gemm_bf16_ex: LN_FOLD needs ln_stats, ln_wsum, ln_slots > 0, ln_stats_ld >= M, a bias and bf16 output");
     if (flags & RAJNI_EPI_ROW_STATS)
         RAJNI_REQUIRE(a->row_stats && a->row_stats_ld > 0 && (flags & RAJNI_EPI_RESIDUAL) && !(flags & RAJNI_EPI_OUT_F32), RAJNI_EINVAL,
-                      "rajni_gemm_bf16: ROW_STATS needs row_stats, row_stats_ld and the bias+residual bf16 epilogue");
+                      "rajni_gemm_bf16_ex: ROW_STATS needs row_stats, row_stats_ld and the bias+residual bf16 epilogue");
     GemmParams p{};
     p.bias = a->bias; p.D = a->D;
     p.residual = static_cast<const __nv_bfloat16*>(a->residual);
@@ -935,7 +935,7 @@ extern "C" int rajni_gemm_bf16_ex(const rajni_gemm_args* a, void* stream) {
     p.row_stats_ld = a->row_stats_ld;
     p.stat_shift = stat_shift_for(N);
     const bool exact = (flags & (RAJNI_EPI_LN_FOLD | RAJNI_EPI_ROW_STATS)) != 0;
-    RAJNI_REQUIRE(!exact || N % 64 == 0, RAJNI_EINVAL, "rajni_gemm_bf16: LN_FOLD / ROW_STATS need N %% 64 == 0 (N=%d)", N);
+    RAJNI_REQUIRE(!exact || N % 64 == 0, RAJNI_EINVAL, "rajni_gemm_bf16_ex: LN_FOLD / ROW_STATS need N %% 64 == 0 (N=%d)", N);
     // (a producer of 64-column statistics slots cannot use the 192-wide tile)
     int bn = pick_bn(N, M, K, exact, (flags & RAJNI_EPI_ROW_STATS) && stat_shift_for(N) == 6,
                      a->workspace != nullptr && (size_t)a->workspace_bytes >= sk_workspace_bytes(), (flags & RAJNI_HINT_STREAM_K) != 0);   // < 0: exact CTA-pair tile of width -bn
@@ -951,18 +951,4 @@ extern "C" int rajni_gemm_bf16_ex(const rajni_gemm_args* a, void* stream) {
         case 128: return launch_gemm<128, 1>(a->A, a->W, p, a->workspace, (size_t)a->workspace_bytes, s);
         default: return launch_gemm<64, 1>(a->A, a->W, p, a->workspace, (size_t)a->workspace_bytes, s);
     }
-}
-
-extern "C" int rajni_gemm_bf16(const void* A, const void* W, const float* bias, void* D,
-                               int M, int N, int K, int flags,
-                               const void* residual, long long ldres, const int32_t* res_row_map,
-                               long long ldd, const int32_t* out_row_map, void* stream) {
-    RAJNI_REQUIRE(!(flags & (RAJNI_EPI_LN_FOLD | RAJNI_EPI_ROW_STATS)), RAJNI_EINVAL,
-                  "rajni_gemm_bf16: LN_FOLD / ROW_STATS need rajni_gemm_bf16_ex");
-    rajni_gemm_args a{};
-    a.A = A; a.W = W; a.bias = bias; a.D = D;
-    a.M = M; a.N = N; a.K = K; a.flags = flags;
-    a.residual = residual; a.ldres = ldres; a.res_row_map = res_row_map;
-    a.ldd = ldd; a.out_row_map = out_row_map;
-    return rajni_gemm_bf16_ex(&a, stream);
 }

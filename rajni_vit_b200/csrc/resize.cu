@@ -13,7 +13,7 @@
 //                        explicitly unfused multiplies/adds (the weights must match the CPU's to the last bit)
 //   resize_h_kernel      temp[b][r][xx][c] for the source rows the crop needs            (HBM-bound: reads the frames once)
 //   resize_v_kernel      out[b][c][yy][xx] uint8 planar - the tensor PILToTensor would give; the patch kernel then applies
-//                        ToTensor + Normalize in fp32 (rajni_patch_im2col, RAJNI_IMG_U8)
+//                        ToTensor + Normalize in fp32 (rajni_patch_im2col_prefix, RAJNI_IMG_U8)
 #include "common.cuh"
 
 namespace rajni {

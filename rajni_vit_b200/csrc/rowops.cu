@@ -441,63 +441,54 @@ extern "C" int rajni_gather_rows(const void* src, const int32_t* row_map, void* 
                           static_cast<const uint4*>(src), row_map, static_cast<uint4*>(dst), total, cpr);
 }
 
-// y: bf16 or fp32 rows at out_row_stride elements (a multiple of 16 bytes, as the kernel stores 16-byte chunks)
-template <typename OutT>
-static int layernorm_strided(const char* name, const char* kname, const void* x, long long in_row_stride, const float* gamma, const float* beta,
-                             float eps, OutT* y, long long out_row_stride, int rows, int C, void* stream) {
+// The host side of the three LayerNorm entry points.  y: bf16 or fp32 rows at out_row_stride elements (a multiple of 16
+// bytes, as the kernel stores 16-byte chunks).  STATS: also the rows' partial sums (bf16 rows only, see layernorm_kernel).
+template <bool STATS, typename OutT>
+static int launch_layernorm(const char* name, const char* kname, const void* x, long long in_row_stride, const float* gamma,
+                            const float* beta, float eps, OutT* y, long long out_row_stride, int rows, int C,
+                            float* row_stats, long long row_stats_ld, int stats_slots, void* stream) {
     constexpr int kOutAlign = 16 / sizeof(OutT);
-    RAJNI_REQUIRE(x && gamma && beta && y, RAJNI_EINVAL, "%s: null pointer", name);
+    RAJNI_REQUIRE(x && gamma && beta && y && (!STATS || row_stats), RAJNI_EINVAL, "%s: null pointer", name);
     RAJNI_REQUIRE(rows > 0 && C > 0 && C % 8 == 0 && C <= 2048 && in_row_stride % 8 == 0 && out_row_stride % kOutAlign == 0 &&
                   out_row_stride >= C, RAJNI_EINVAL, "%s: rows=%d C=%d stride=%lld out stride=%lld unsupported", name, rows, C,
                   in_row_stride, out_row_stride);
+    if (STATS)
+        RAJNI_REQUIRE(stats_slots > 0 && row_stats_ld >= rows, RAJNI_EINVAL,
+                      "%s: stats_slots=%d row_stats_ld=%lld (need slots > 0 and ld >= rows=%d)", name, stats_slots,
+                      row_stats_ld, rows);
     const int cpl = (C / 8 + 31) / 32;
     const int wpb = 8;
     dim3 grid((rows + wpb - 1) / wpb), block(wpb * 32);
-    auto kern = layernorm_kernel<8, false, OutT>;             // cpl 5..8
+    auto kern = layernorm_kernel<8, STATS, OutT>;             // cpl 5..8
     switch (cpl) {
-        case 1: kern = layernorm_kernel<1, false, OutT>; break;
-        case 2: kern = layernorm_kernel<2, false, OutT>; break;
-        case 3: kern = layernorm_kernel<3, false, OutT>; break;
-        case 4: kern = layernorm_kernel<4, false, OutT>; break;
+        case 1: kern = layernorm_kernel<1, STATS, OutT>; break;
+        case 2: kern = layernorm_kernel<2, STATS, OutT>; break;
+        case 3: kern = layernorm_kernel<3, STATS, OutT>; break;
+        case 4: kern = layernorm_kernel<4, STATS, OutT>; break;
     }
     return launch_checked(kname, kern, grid, block, 0, static_cast<cudaStream_t>(stream), 1, static_cast<const __nv_bfloat16*>(x),
-                          in_row_stride, gamma, beta, eps, y, out_row_stride, rows, C, static_cast<float2*>(nullptr), 0LL, 0);
+                          in_row_stride, gamma, beta, eps, y, out_row_stride, rows, C, reinterpret_cast<float2*>(row_stats),
+                          row_stats_ld, stats_slots);
 }
 
 extern "C" int rajni_layernorm_strided(const void* x, long long in_row_stride, const float* gamma, const float* beta, float eps,
                                        void* y, long long out_row_stride, int rows, int C, void* stream) {
-    return layernorm_strided("rajni_layernorm", "layernorm", x, in_row_stride, gamma, beta, eps, static_cast<__nv_bfloat16*>(y), out_row_stride,
-                             rows, C, stream);
+    return launch_layernorm<false>("rajni_layernorm_strided", "layernorm", x, in_row_stride, gamma, beta, eps,
+                                   static_cast<__nv_bfloat16*>(y), out_row_stride, rows, C, nullptr, 0, 0, stream);
 }
 
 extern "C" int rajni_layernorm_strided_f32(const void* x, long long in_row_stride, const float* gamma, const float* beta, float eps,
                                            float* y, long long out_row_stride, int rows, int C, void* stream) {
-    return layernorm_strided("rajni_layernorm_f32", "layernorm_f32", x, in_row_stride, gamma, beta, eps, y, out_row_stride, rows, C, stream);
+    return launch_layernorm<false>("rajni_layernorm_f32", "layernorm_f32", x, in_row_stride, gamma, beta, eps, y,
+                                   out_row_stride, rows, C, nullptr, 0, 0, stream);
 }
 
 extern "C" int rajni_layernorm_row_stats(const void* x, long long in_row_stride, const float* gamma, const float* beta, float eps,
                                          void* y, long long out_row_stride, int rows, int C,
                                          float* row_stats, long long row_stats_ld, int stats_slots, void* stream) {
-    RAJNI_REQUIRE(x && gamma && beta && y && row_stats, RAJNI_EINVAL, "rajni_layernorm_row_stats: null pointer");
-    RAJNI_REQUIRE(rows > 0 && C > 0 && C % 8 == 0 && C <= 2048 && in_row_stride % 8 == 0 && out_row_stride % 8 == 0 && out_row_stride >= C,
-                  RAJNI_EINVAL, "rajni_layernorm_row_stats: rows=%d C=%d stride=%lld out stride=%lld unsupported", rows, C, in_row_stride,
-                  out_row_stride);
-    RAJNI_REQUIRE(stats_slots > 0 && row_stats_ld >= rows, RAJNI_EINVAL,
-                  "rajni_layernorm_row_stats: stats_slots=%d row_stats_ld=%lld (need slots > 0 and ld >= rows=%d)", stats_slots,
-                  row_stats_ld, rows);
-    const int cpl = (C / 8 + 31) / 32;
-    const int wpb = 8;
-    dim3 grid((rows + wpb - 1) / wpb), block(wpb * 32);
-    auto kern = layernorm_kernel<8, true>;                    // cpl 5..8
-    switch (cpl) {
-        case 1: kern = layernorm_kernel<1, true>; break;
-        case 2: kern = layernorm_kernel<2, true>; break;
-        case 3: kern = layernorm_kernel<3, true>; break;
-        case 4: kern = layernorm_kernel<4, true>; break;
-    }
-    return launch_checked("layernorm_row_stats", kern, grid, block, 0, static_cast<cudaStream_t>(stream), 1,
-                          static_cast<const __nv_bfloat16*>(x), in_row_stride, gamma, beta, eps, static_cast<__nv_bfloat16*>(y),
-                          out_row_stride, rows, C, reinterpret_cast<float2*>(row_stats), row_stats_ld, stats_slots);
+    return launch_layernorm<true>("rajni_layernorm_row_stats", "layernorm_row_stats", x, in_row_stride, gamma, beta, eps,
+                                  static_cast<__nv_bfloat16*>(y), out_row_stride, rows, C, row_stats, row_stats_ld, stats_slots,
+                                  stream);
 }
 
 template <typename OutT>
@@ -525,38 +516,33 @@ extern "C" int rajni_mean_pool_layernorm_f32(const void* x, int B, int N, int pr
     return mean_pool_layernorm("rajni_mean_pool_layernorm_f32", "mean_pool_layernorm_f32", x, B, N, prefix, C, gamma, beta, eps, y, out_row_stride, stream);
 }
 
-extern "C" int rajni_layernorm(const void* x, long long in_row_stride, const float* gamma,
-                               const float* beta, float eps, void* y, int rows, int C, void* stream) {
-    return rajni_layernorm_strided(x, in_row_stride, gamma, beta, eps, y, C, rows, C, stream);
-}
-
 extern "C" int rajni_patch_im2col_prefix(const void* images, int image_dtype, int B, int S, int patch,
                                          void* cols, const void* prefix_rows, int prefix, void* x, int C,
                                          float* row_stats, long long row_stats_ld, int stats_slots,
                                          const float* prefix_stats_host, const float* norm, void* stream) {
-    RAJNI_REQUIRE(images && cols && prefix_rows && x, RAJNI_EINVAL, "rajni_patch_im2col: null pointer");
-    RAJNI_REQUIRE(prefix >= 1 && prefix <= kMaxPrefix, RAJNI_EINVAL, "rajni_patch_im2col: prefix=%d (1: CLS, 2: CLS + distillation token)", prefix);
-    RAJNI_REQUIRE(row_stats == nullptr || prefix_stats_host != nullptr, RAJNI_EINVAL, "rajni_patch_im2col: row_stats needs prefix_stats_host");
+    RAJNI_REQUIRE(images && cols && prefix_rows && x, RAJNI_EINVAL, "rajni_patch_im2col_prefix: null pointer");
+    RAJNI_REQUIRE(prefix >= 1 && prefix <= kMaxPrefix, RAJNI_EINVAL, "rajni_patch_im2col_prefix: prefix=%d (1: CLS, 2: CLS + distillation token)", prefix);
+    RAJNI_REQUIRE(row_stats == nullptr || prefix_stats_host != nullptr, RAJNI_EINVAL, "rajni_patch_im2col_prefix: row_stats needs prefix_stats_host");
     PrefixStats ps{};
     if (row_stats != nullptr)
         for (int r = 0; r < prefix; ++r) {
             ps.sum[r] = prefix_stats_host[2 * r];
             ps.sumsq[r] = prefix_stats_host[2 * r + 1];
         }
-    RAJNI_REQUIRE(image_dtype >= RAJNI_IMG_BF16 && image_dtype <= RAJNI_IMG_U8, RAJNI_EINVAL, "rajni_patch_im2col: image_dtype %d", image_dtype);
-    RAJNI_REQUIRE(image_dtype != RAJNI_IMG_U8 || norm != nullptr, RAJNI_EINVAL, "rajni_patch_im2col: uint8 images need norm (mean[3], std[3])");
+    RAJNI_REQUIRE(image_dtype >= RAJNI_IMG_BF16 && image_dtype <= RAJNI_IMG_U8, RAJNI_EINVAL, "rajni_patch_im2col_prefix: image_dtype %d", image_dtype);
+    RAJNI_REQUIRE(image_dtype != RAJNI_IMG_U8 || norm != nullptr, RAJNI_EINVAL, "rajni_patch_im2col_prefix: uint8 images need norm (mean[3], std[3])");
     ImageNorm nm{{0.f, 0.f, 0.f}, {1.f, 1.f, 1.f}};
     if (image_dtype == RAJNI_IMG_U8)
         for (int i = 0; i < 3; ++i) {
             nm.mean[i] = norm[i];
             nm.std[i] = norm[3 + i];
-            RAJNI_REQUIRE(nm.std[i] > 0.f, RAJNI_EINVAL, "rajni_patch_im2col: std[%d] must be positive", i);
+            RAJNI_REQUIRE(nm.std[i] > 0.f, RAJNI_EINVAL, "rajni_patch_im2col_prefix: std[%d] must be positive", i);
         }
     RAJNI_REQUIRE(patch >= 8 && patch % 8 == 0 && S > 0 && S <= 16384 && S % patch == 0 && B > 0 && C % 8 == 0, RAJNI_EINVAL,
-                  "rajni_patch_im2col: patch=%d S=%d B=%d C=%d unsupported (patch must be a multiple of 8 dividing S <= 16384)", patch, S, B, C);
+                  "rajni_patch_im2col_prefix: patch=%d S=%d B=%d C=%d unsupported (patch must be a multiple of 8 dividing S <= 16384)", patch, S, B, C);
     const int G = S / patch;
     RAJNI_REQUIRE(row_stats == nullptr || (stats_slots > 0 && row_stats_ld >= (long long)B * (G * G + prefix)), RAJNI_EINVAL,
-                  "rajni_patch_im2col: row_stats needs stats_slots > 0 and row_stats_ld >= B*(P+prefix)");
+                  "rajni_patch_im2col_prefix: row_stats needs stats_slots > 0 and row_stats_ld >= B*(P+prefix)");
     auto s = static_cast<cudaStream_t>(stream);
     // p = 16 keeps its own kernel: 16-pixel strips, px fastest.  On a B200 at 256 images of 224 px it moves fp32 images in
     // 41.7 us against the any-patch kernel's 44.3 us, uint8 pixels in 54.5 against 78.6 us (profiles/r3_kbench.txt).
@@ -577,13 +563,4 @@ extern "C" int rajni_patch_im2col_prefix(const void* images, int image_dtype, in
                               images, nm, B, S, patch, static_cast<__nv_bfloat16*>(cols), static_cast<const uint4*>(prefix_rows), prefix, ps,
                               static_cast<uint4*>(x), C, reinterpret_cast<float2*>(row_stats), row_stats_ld, stats_slots);
     }
-}
-
-extern "C" int rajni_patch_im2col(const void* images, int image_dtype, int B, int S, int patch,
-                                  void* cols, const void* cls_pos0, void* x, int C,
-                                  float* row_stats, long long row_stats_ld, int stats_slots,
-                                  float cls_sum, float cls_sumsq, const float* norm, void* stream) {
-    const float cls_stats[2] = {cls_sum, cls_sumsq};
-    return rajni_patch_im2col_prefix(images, image_dtype, B, S, patch, cols, cls_pos0, 1, x, C, row_stats, row_stats_ld,
-                                     stats_slots, cls_stats, norm, stream);
 }

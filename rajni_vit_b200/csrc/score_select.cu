@@ -12,8 +12,9 @@
 // centred norm is computed exactly like the reference without a second HBM pass),
 // and the selection state (radix-select histogram, flags, prefix sums).
 // Sequences whose logits and value rows do not fit there (score_smem_bytes over 227 KB: N > ~720 at 12 heads, e.g. the
-// 785 tokens of a ViT-B/8) take the two-launch path of rajni_score_select_split: score_stream_kernel leaves them in the
-// caller's workspace and score_tail_ws_kernel reads them in place (from L2), keeping only O(N) arrays in shared memory.
+// 785 tokens of a ViT-B/8) take the two-launch path of rajni_score_select_prefix with a workspace: score_stream_kernel
+// leaves them in the caller's workspace and score_tail_ws_kernel reads them in place (from L2), keeping only O(N) arrays in
+// shared memory.
 // bf16 tiles in, fp32 arithmetic throughout (SURVEY.md section 4.5).
 #include <algorithm>
 #include <cstdlib>
@@ -442,8 +443,8 @@ __device__ void score_tail(const SelSmem& sm, const float* vm, const ScoreSelect
 }
 
 // CPL = 16-byte chunks per lane per plane = ceil(C / 256).
-// One CTA per image, everything in shared memory, no scratch: the stand-alone entry points (rajni_importance, rajni_select,
-// rajni_score_select).  64 registers per thread so that two CTAs (two images) share an SM.  All images of a batch are
+// One CTA per image, everything in shared memory, no scratch: rajni_select_prefix, and rajni_score_select_prefix without a
+// workspace.  64 registers per thread so that two CTAs (two images) share an SM.  All images of a batch are
 // resident at once and march in lock-step - pass, then tail - so the tail (~25 % of the time) is never hidden.  A persistent
 // kernel that overlaps the two across images was built and measured (tools/probes/score_overlap_persistent_experiment.patch,
 // profiles/r2_score_select.md): the tail's ~8 us latency is still exposed after the last image, so it did not win.
@@ -543,7 +544,7 @@ static int launch_score_select(const ScoreSelectParams& p, int B, cudaStream_t s
     const bool with_score = p.qkv != nullptr;
     size_t smem = score_smem_bytes(p.N, p.H, with_score, with_score);
     RAJNI_REQUIRE(smem <= kSmemLimit, RAJNI_EINVAL,
-                  "score_select: N=%d H=%d needs %zu B of shared memory (rajni_score_select_split takes such shapes)", p.N, p.H, smem);
+                  "score_select: N=%d H=%d needs %zu B of shared memory (rajni_score_select_prefix with a workspace takes such shapes)", p.N, p.H, smem);
     int cpl = with_score ? (p.C + 255) / 256 : 1;
     void (*kern)(const ScoreSelectParams) = nullptr;
     switch (cpl) {
@@ -601,33 +602,40 @@ static int check_keep(const char* fn, int N, int P0, int keep) {
     return 0;
 }
 
-static int select_prefix(const char* fn, const float* scores, int B, int N, int P0, int keep, int32_t* keep_idx,
-                         float* next_scores, int32_t* row_map, cudaStream_t stream) {
+}  // namespace rajni
+
+using namespace rajni;
+
+extern "C" int rajni_select_prefix(const float* scores, int B, int N, int prefix, int keep, int32_t* keep_idx,
+                                   float* next_scores, int32_t* row_map, void* stream) {
+    const char* fn = "rajni_select_prefix";
     RAJNI_REQUIRE(scores && keep_idx && next_scores, RAJNI_EINVAL, "%s: null pointer", fn);
     RAJNI_REQUIRE(B > 0 && N >= 2 && N <= 16384, RAJNI_EINVAL, "%s: bad B=%d N=%d", fn, B, N);
-    if (int rc = check_keep(fn, N, P0, keep)) return rc;
+    if (int rc = check_keep(fn, N, prefix, keep)) return rc;
     ScoreSelectParams p{};
     p.scores_in = scores;
     p.keep_idx = keep_idx; p.next_scores = next_scores; p.row_map = row_map;
-    p.N = N; p.C = 0; p.H = 0; p.keep = keep; p.P0 = P0; p.eps = 0.f;
-    return launch_score_select(p, B, stream);
+    p.N = N; p.C = 0; p.H = 0; p.keep = keep; p.P0 = prefix; p.eps = 0.f;
+    return launch_score_select(p, B, static_cast<cudaStream_t>(stream));
 }
 
 // workspace == null: the one-launch kernel; else the split path (K/V pass over (image, row-block) CTAs, then the tail).
 // keep_idx == null: scores only.
-static int score_select_prefix(const char* fn, const void* qkv, int B, int N, int C, int H, int P0, int keep, float eps,
-                               float* scores, int32_t* keep_idx, float* next_scores, int32_t* row_map,
-                               void* workspace, size_t workspace_bytes, cudaStream_t s) {
+extern "C" int rajni_score_select_prefix(const void* qkv, int B, int N, int C, int H, int prefix, int keep, float eps,
+                                         float* scores, int32_t* keep_idx, float* next_scores, int32_t* row_map,
+                                         void* workspace, size_t workspace_bytes, void* stream) {
+    const char* fn = "rajni_score_select_prefix";
+    auto s = static_cast<cudaStream_t>(stream);
     RAJNI_REQUIRE(qkv && (keep_idx ? next_scores != nullptr : scores != nullptr), RAJNI_EINVAL, "%s: null pointer", fn);
     if (int rc = check_score_shape(B, N, C, H)) return rc;
     if (keep_idx != nullptr) {
-        if (int rc = check_keep(fn, N, P0, keep)) return rc;
+        if (int rc = check_keep(fn, N, prefix, keep)) return rc;
     }
     ScoreSelectParams p{};
     p.qkv = static_cast<const __nv_bfloat16*>(qkv);
     p.scores_out = scores;
     p.keep_idx = keep_idx; p.next_scores = next_scores; p.row_map = row_map;
-    p.N = N; p.C = C; p.H = H; p.keep = keep_idx ? keep : 0; p.P0 = P0; p.eps = eps;
+    p.N = N; p.C = C; p.H = H; p.keep = keep_idx ? keep : 0; p.P0 = prefix; p.eps = eps;
     if (workspace == nullptr) return launch_score_select(p, B, s);
     RAJNI_REQUIRE(B <= 65535, RAJNI_EINVAL, "%s: B=%d exceeds the grid limit", fn, B);
     RAJNI_REQUIRE(workspace_bytes >= split_workspace_floats(B, N, H) * sizeof(float) && (reinterpret_cast<uintptr_t>(workspace) & 15) == 0,
@@ -641,59 +649,10 @@ static int score_select_prefix(const char* fn, const void* qkv, int B, int N, in
     return launch_score_select(p, B, s);
 }
 
-}  // namespace rajni
-
-using namespace rajni;
-
-extern "C" int rajni_importance(const void* qkv, int B, int N, int C, int H, float eps,
-                                float* scores, void* stream) {
-    RAJNI_REQUIRE(qkv && scores, RAJNI_EINVAL, "rajni_importance: null pointer");
-    if (int rc = check_score_shape(B, N, C, H)) return rc;
-    ScoreSelectParams p{};
-    p.qkv = static_cast<const __nv_bfloat16*>(qkv);
-    p.scores_out = scores;
-    p.N = N; p.C = C; p.H = H; p.keep = 0; p.eps = eps;
-    return launch_score_select(p, B, static_cast<cudaStream_t>(stream));
-}
-
-extern "C" int rajni_select_prefix(const float* scores, int B, int N, int prefix, int keep, int32_t* keep_idx,
-                                   float* next_scores, int32_t* row_map, void* stream) {
-    return select_prefix("rajni_select_prefix", scores, B, N, prefix, keep, keep_idx, next_scores, row_map,
-                         static_cast<cudaStream_t>(stream));
-}
-
-extern "C" int rajni_select(const float* scores, int B, int N, int keep, int32_t* keep_idx,
-                            float* next_scores, int32_t* row_map, void* stream) {
-    return select_prefix("rajni_select", scores, B, N, 1, keep, keep_idx, next_scores, row_map, static_cast<cudaStream_t>(stream));
-}
-
-extern "C" int rajni_score_select_prefix(const void* qkv, int B, int N, int C, int H, int prefix, int keep, float eps,
-                                         float* scores, int32_t* keep_idx, float* next_scores, int32_t* row_map,
-                                         void* workspace, size_t workspace_bytes, void* stream) {
-    return score_select_prefix("rajni_score_select_prefix", qkv, B, N, C, H, prefix, keep, eps, scores, keep_idx, next_scores,
-                               row_map, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
-}
-
-extern "C" int rajni_score_select(const void* qkv, int B, int N, int C, int H, int keep, float eps,
-                                  float* scores, int32_t* keep_idx, float* next_scores,
-                                  int32_t* row_map, void* stream) {
-    RAJNI_REQUIRE(keep_idx, RAJNI_EINVAL, "rajni_score_select: null pointer");
-    return score_select_prefix("rajni_score_select", qkv, B, N, C, H, 1, keep, eps, scores, keep_idx, next_scores, row_map,
-                               nullptr, 0, static_cast<cudaStream_t>(stream));
-}
-
 extern "C" size_t rajni_score_select_workspace_bytes(int B, int N, int C, int H) {
     (void)C;
     if (B <= 0 || N <= 0 || H <= 0) return 0;
     return split_workspace_floats(B, N, H) * sizeof(float);
-}
-
-extern "C" int rajni_score_select_split(const void* qkv, int B, int N, int C, int H, int keep, float eps,
-                                        float* scores, int32_t* keep_idx, float* next_scores, int32_t* row_map,
-                                        void* workspace, size_t workspace_bytes, void* stream) {
-    RAJNI_REQUIRE(workspace, RAJNI_EINVAL, "rajni_score_select_split: null pointer");
-    return score_select_prefix("rajni_score_select_split", qkv, B, N, C, H, 1, keep, eps, scores, keep_idx, next_scores, row_map,
-                               workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
 }
 
 extern "C" int rajni_score_select_needs_workspace(int N, int H) {

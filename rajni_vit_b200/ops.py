@@ -82,7 +82,7 @@ def _check_prefix(prefix: int) -> int:
 def importance(qkv: torch.Tensor, num_heads: int, eps: float = 1e-6, workspace: Optional[torch.Tensor] = None,
                prefix: int = 1) -> torch.Tensor:
     """qkv [B,N,3C] bf16 -> scores [B,N] fp32.   importance.py:5-34
-    Sequences too long for the one-launch kernel (``needs_score_workspace``) go through the split entry with scratch
+    Sequences too long for the one-launch kernel (``needs_score_workspace``) take the two-launch path with scratch
     (``workspace`` as in ``score_select``).  ``prefix`` (1 or 2 leading tokens) does not change the scores: the query is
     row 0 and every token, a distillation token too, is a key and value."""
     _check_prefix(prefix)
@@ -91,13 +91,9 @@ def importance(qkv: torch.Tensor, num_heads: int, eps: float = 1e-6, workspace: 
     C = C3 // 3
     scores = torch.empty((B, N), device=qkv.device, dtype=torch.float32)
     work = B * (2 * N * C * 2 + C * 2 + 4 * N)
-    lib = _lib.load()
-    if needs_score_workspace(N, num_heads):
-        ws = _checked_score_workspace(qkv.device, B, N, C, num_heads, workspace)
-        _call("score_select", work, lib.rajni_score_select_split, qkv.data_ptr(), B, N, C, num_heads, 0, eps, scores.data_ptr(),
-              None, None, None, ws.data_ptr(), ws.numel(), _stream(qkv))
-    else:
-        _call("score_select", work, lib.rajni_importance, qkv.data_ptr(), B, N, C, num_heads, eps, scores.data_ptr(), _stream(qkv))
+    ws = _checked_score_workspace(qkv.device, B, N, C, num_heads, workspace) if needs_score_workspace(N, num_heads) else None
+    _call("score_select", work, _lib.load().rajni_score_select_prefix, qkv.data_ptr(), B, N, C, num_heads, prefix, 0, eps,
+          scores.data_ptr(), None, None, None, _ptr(ws), 0 if ws is None else ws.numel(), _stream(qkv))
     return scores
 
 

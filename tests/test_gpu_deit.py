@@ -1,7 +1,7 @@
-"""The two DeiT families on the B200: selection with two always-kept prefix tokens on every score/select path, the
-prefix-aware entry points against the old ones at one prefix token, the im2col prefix rows, and the wrapper end to end
-(LayerScale folded into proj / fc2, no position for DeiT-III's class token, the distilled model's two-head average)
-against the DeiT reference (tests/deit_oracle.py, the oracle extended to the two families)."""
+"""The two DeiT families on the B200: selection with two always-kept prefix tokens on every score/select path, the im2col
+prefix rows, and the wrapper end to end (LayerScale folded into proj / fc2, no position for DeiT-III's class token, the
+distilled model's two-head average) against the DeiT reference (tests/deit_oracle.py, the oracle extended to the two
+families)."""
 import copy
 
 import pytest
@@ -106,56 +106,6 @@ def test_select_on_carried_scores_two_prefix_tokens(ops, B, N):
     from rajni_vit_b200._lib import RajniError
     with pytest.raises(RajniError, match="selected index k out of range"):
         ops.select(s.cuda(), N - 1, prefix=2)
-
-
-def test_one_prefix_token_through_the_new_entry_points_is_bit_identical(ops):
-    """ops calls the *_prefix entry points; at prefix 1 they reproduce the old entry points bit for bit on every path."""
-    from rajni_vit_b200 import _lib
-    lib = _lib.load()
-    stream = torch.cuda.current_stream().cuda_stream
-    for B, N, H in ((3, 197, 12), (200, 197, 6), (3, 577, 12), (2, 785, 12)):
-        qkv = _qkv(B, N, H, B + N)
-        keep = dorc.keep_count(N, 0.8)
-        C = 64 * H
-        for split in (False, True):
-            if not split and ops.needs_score_workspace(N, H):
-                continue
-            new = ops.score_select(qkv, H, keep, want_scores=True, split=split)
-            old = [torch.empty_like(new[0]), torch.empty_like(new[1]), torch.empty_like(new[2]), torch.empty_like(new[3])]
-            if split:
-                ws = torch.empty(ops.score_workspace_bytes(B, N, C, H), device="cuda", dtype=torch.uint8)
-                rc = lib.rajni_score_select_split(qkv.data_ptr(), B, N, C, H, keep, 1e-6, old[0].data_ptr(), old[1].data_ptr(),
-                                                  old[2].data_ptr(), old[3].data_ptr(), ws.data_ptr(), ws.numel(), stream)
-            else:
-                rc = lib.rajni_score_select(qkv.data_ptr(), B, N, C, H, keep, 1e-6, old[0].data_ptr(), old[1].data_ptr(),
-                                            old[2].data_ptr(), old[3].data_ptr(), stream)
-            _lib.check(rc)
-            for a, b in zip(new, old):
-                assert torch.equal(a, b), (B, N, split)
-        sel_new = ops.select(new[0], keep)
-        sel_old = [torch.empty_like(t) for t in sel_new]
-        _lib.check(lib.rajni_select(new[0].data_ptr(), B, N, keep, sel_old[0].data_ptr(), sel_old[1].data_ptr(),
-                                    sel_old[2].data_ptr(), stream))
-        for a, b in zip(sel_new, sel_old):
-            assert torch.equal(a, b)
-    # im2col at prefix 1: same cols, CLS rows and LayerNorm partials as rajni_patch_im2col
-    for p, S in ((16, 224), (8, 72)):
-        img = torch.randn(3, 3, S, S, device="cuda")
-        P, C = (S // p) ** 2, 192
-        cls_pos0 = torch.randn(C, device="cuda").to(torch.bfloat16)
-        outs = []
-        for use_new in (True, False):
-            cols = torch.zeros(3 * P, 3 * p * p, device="cuda", dtype=torch.bfloat16)
-            x = torch.zeros(3 * (P + 1), C, device="cuda", dtype=torch.bfloat16)
-            st = torch.full((3, 3 * (P + 1), 2), 7.0, device="cuda")
-            if use_new:
-                ops.patch_im2col(img, p, cols, cls_pos0, x, C, row_stats=st, stats_slots=3, cls_sum=1.25, cls_sumsq=3.5)
-            else:
-                _lib.check(lib.rajni_patch_im2col(img.data_ptr(), 1, 3, S, p, cols.data_ptr(), cls_pos0.data_ptr(), x.data_ptr(), C,
-                                                  st.data_ptr(), st.shape[1], 3, 1.25, 3.5, None, stream))
-            outs.append((cols, x, st))
-        for a, b in zip(*outs):
-            assert torch.equal(a, b)
 
 
 # ------------------------------------------------------------------ im2col prefix rows

@@ -516,7 +516,7 @@ def test_patch_embed(ops, S, C, B):
 
 
 def test_reverse_traversal_hints_do_not_change_results(ops):
-    """RAJNI_HINT_REVERSE_M / rajni_attention_fwd(reverse=1) only change the order in which tiles are visited."""
+    """RAJNI_HINT_REVERSE_M / rajni_attention_fwd_ex(reverse=1) only change the order in which tiles are visited."""
     g = torch.Generator().manual_seed(11)
     M, N, K = 3000, 768, 768
     a = dev(bf16_round(torch.randn(M, K, generator=g)), torch.bfloat16)
@@ -538,7 +538,8 @@ def test_reverse_traversal_hints_do_not_change_results(ops):
 @pytest.mark.parametrize("B,N,H,ratio", [(8, 197, 12, 0.88), (3, 577, 12, 0.88), (5, 197, 6, 0.7), (4, 197, 16, 0.9),
                                          (300, 197, 12, 0.8), (2, 33, 3, 0.5), (7, 32, 2, 0.9), (1, 2, 1, 1.0), (2, 257, 3, 0.6)])
 def test_score_select_split_path_is_bit_identical(ops, B, N, H, ratio):
-    """The two-launch path for small batches (rajni_score_select_split) must reproduce the fused kernel exactly."""
+    """The two-launch path for small batches (rajni_score_select_prefix with a workspace) must reproduce the fused kernel
+    exactly."""
     qkv = dev(make_qkv(B, N, H, 64, 900 + N + H), torch.bfloat16)
     keep = max(1, min(N - 1, orc.keep_count(N, ratio)))
     s0, i0, n0, r0 = ops.score_select(qkv, H, keep, want_scores=True, split=False)

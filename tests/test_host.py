@@ -102,6 +102,35 @@ def test_library_exports_every_declared_symbol():
     assert sorted(_lib.SIGNATURES) == names
 
 
+# ABI 11: one entry point per operation.  A name removed from this list must not come back with another signature: a
+# caller that binds by name would misbind silently.
+C_ABI = sorted("rajni_" + n for n in (
+    "abi_version", "last_error", "device_check", "launch_count",
+    "select_prefix", "score_select_prefix", "score_select_workspace_bytes", "score_select_needs_workspace",
+    "gather_rows",
+    "layernorm_strided", "layernorm_strided_f32", "layernorm_row_stats",
+    "mean_pool_layernorm", "mean_pool_layernorm_f32",
+    "gemm_bf16_ex", "gemm_workspace_bytes", "gemm_stream_k_plan", "gemm_row_stats_slots",
+    "attention_fwd_ex",
+    "patch_im2col_prefix",
+    "resize_workspace_bytes", "resize_center_crop_u8", "resize_status"))
+
+
+def test_c_abi_is_exactly_the_documented_surface():
+    """The header declares exactly these 23 functions (so no superseded sibling is left), the ctypes loader binds exactly
+    these, the library exports each, INTEGRATION.md documents each, and both sides report ABI 11."""
+    assert len(C_ABI) == 23
+    assert _declared_symbols() == C_ABI
+    assert sorted(_lib.SIGNATURES) == C_ABI
+    lib = ctypes.CDLL(_lib.LIB_PATH)
+    integ = open(os.path.join(ROOT, "INTEGRATION.md")).read()
+    for n in C_ABI:
+        assert hasattr(lib, n), f"{n} is not exported by {_lib.LIB_PATH}"
+        assert f"`{n}`" in integ, f"{n} is not documented in INTEGRATION.md"
+    assert _lib.ABI_VERSION == 11
+    assert _lib.load().rajni_abi_version() == 11
+
+
 def test_library_abi_version_and_error_string():
     lib = _lib.load()
     assert lib.rajni_abi_version() == _lib.ABI_VERSION

@@ -1,7 +1,7 @@
 """CPU-side tests of the two DeiT families (DeiT-III: LayerScale and a class token without a position; distilled DeiT: a
 distillation token kept through pruning and two heads): the DeiT reference (tests/deit_oracle.py) against the stand-ins'
 own forward and against the oracle at one prefix token, prefix-aware
-token counts, checkpoint loading and what is still refused, and the library's new entry points."""
+token counts, checkpoint loading and what is still refused."""
 import copy
 import os
 import re
@@ -12,7 +12,6 @@ import torch
 
 from oracle import rajni_oracle as orc
 from tests import deit_oracle as dorc
-from rajni_vit_b200 import _lib
 from rajni_vit_b200 import schedule as S
 from rajni_vit_b200.checkpoint import load_checkpoint, write_safetensors
 from rajni_vit_b200.packing import PackCache
@@ -21,7 +20,7 @@ from rajni_vit_b200.vit import (VIT_CONFIGS, VIT_VARIANT, LayerScale, VisionTran
 from rajni_vit_b200.wrapper.attention import keep_count
 from rajni_vit_b200.wrapper.model import RAJNIViTWrapper
 from tests.cases import E2E_CASES, MICRO_SCHEDULE, README_SCHEDULE, make_images, npz
-from tests.conftest import GOLDEN, ROOT
+from tests.conftest import GOLDEN
 
 DEIT3 = ["deit3_small_patch16_224", "deit3_medium_patch16_224", "deit3_base_patch16_224", "deit3_large_patch16_224",
          "deit3_base_patch16_384", "deit3_micro_patch16_64"]
@@ -267,14 +266,3 @@ def test_load_checkpoint_rejections():
     for extra in ("reg_token", "fc_norm.weight", "norm_pre.weight"):
         with pytest.raises(NotImplementedError, match=extra.split(".")[0]):
             load_checkpoint({**vit, extra: torch.zeros(1, 4, 128) if extra == "reg_token" else torch.ones(128)})
-
-
-# ------------------------------------------------------------------ the C ABI
-def test_new_entry_points_are_declared_and_exported():
-    import ctypes
-    text = re.sub(r"/\*.*?\*/", "", open(os.path.join(ROOT, "include", "rajni_b200.h")).read(), flags=re.S)
-    declared = set(re.findall(r"\b(rajni_[a-z0-9_]+)\s*\(", text))
-    lib = ctypes.CDLL(_lib.LIB_PATH)
-    for n in ("rajni_score_select_prefix", "rajni_select_prefix", "rajni_patch_im2col_prefix", "rajni_layernorm_strided"):
-        assert n in declared and n in _lib.SIGNATURES and hasattr(lib, n), n
-    assert _lib.load().rajni_abi_version() == 10

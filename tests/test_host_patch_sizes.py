@@ -1,9 +1,9 @@
 """CPU-side tests of the 8- and 32-pixel patch models: schedules and work per image, checkpoint loading into a model the
-wrapper accepts, the patch sizes it still refuses, and the library's ABI version and long-sequence score query."""
+wrapper accepts, the patch sizes it still refuses, and the library's long-sequence score query."""
 import pytest
 import torch
 
-from rajni_vit_b200 import _lib, ops
+from rajni_vit_b200 import ops
 from rajni_vit_b200 import schedule as S
 from rajni_vit_b200.checkpoint import load_checkpoint
 from rajni_vit_b200.vit import VIT_CONFIGS, VIT_PATCH, VisionTransformer, create_model
@@ -65,11 +65,6 @@ def test_wrapper_rejects_patch_sizes_that_are_not_multiples_of_8(p):
     base = VisionTransformer(img_size=p * 4, patch_size=p, embed_dim=128, depth=1, num_heads=2)
     with pytest.raises(NotImplementedError, match=f"kernel=\\({p}, {p}\\)"):
         RAJNIViTWrapper(base, {})
-
-
-def test_abi_version_is_10():
-    assert _lib.ABI_VERSION == 10
-    assert _lib.load().rajni_abi_version() == 10
 
 
 def test_score_workspace_query():

@@ -1,22 +1,17 @@
 """CPU-side tests of average-pooled heads (global_pool='avg' with fc_norm, MAE fine-tunes) and the pre-norm stem
 (norm_pre, a bias-free patch embedding, LayerNorm eps 1e-5: CLIP fine-tunes): the reference (tests/pool_prenorm_oracle.py)
 against the stand-ins' own forward and against the DeiT reference with neither feature, what the wrapper accepts and still
-refuses, checkpoint loading, and the library's new entry points."""
-import os
-import re
-
+refuses, and checkpoint loading."""
 import pytest
 import torch
 import torch.nn as nn
 
 from tests import deit_oracle as dorc
 from tests import pool_prenorm_oracle as porc
-from rajni_vit_b200 import _lib
 from rajni_vit_b200.checkpoint import load_checkpoint, write_safetensors
 from rajni_vit_b200.vit import VIT_CONFIGS, VIT_PATCH, VIT_POOL_PRENORM, create_model, randomize_trained_like
 from rajni_vit_b200.wrapper.model import RAJNIViTWrapper
 from tests.cases import MICRO_SCHEDULE, README_SCHEDULE, make_images
-from tests.conftest import ROOT
 
 POOLED = ["vit_base_patch16_224_mae", "vit_large_patch16_224_mae", "vit_micro_patch16_64_mae"]
 PRENORM = ["vit_base_patch16_clip_224", "vit_base_patch32_clip_224", "vit_base_patch16_clip_384", "vit_micro_patch16_64_clip"]
@@ -195,16 +190,3 @@ def test_load_checkpoint_rejections():
         load_checkpoint({**pooled_dist, "fc_norm.weight": torch.ones(128), "fc_norm.bias": torch.zeros(128)})
     with pytest.raises(KeyError, match="norm"):                               # no final norm at all
         load_checkpoint({k: v for k, v in vit.items() if not k.startswith("norm.")})
-
-
-# ------------------------------------------------------------------ the C ABI
-def test_new_entry_points_are_declared_and_exported():
-    import ctypes
-    text = re.sub(r"/\*.*?\*/", "", open(os.path.join(ROOT, "include", "rajni_b200.h")).read(), flags=re.S)
-    declared = set(re.findall(r"\b(rajni_[a-z0-9_]+)\s*\(", text))
-    lib = ctypes.CDLL(_lib.LIB_PATH)
-    for n in ("rajni_mean_pool_layernorm", "rajni_layernorm_row_stats"):
-        assert n in declared and n in _lib.SIGNATURES and hasattr(lib, n), n
-    integ = open(os.path.join(ROOT, "INTEGRATION.md")).read()
-    assert "rajni_mean_pool_layernorm" in integ and "rajni_layernorm_row_stats" in integ
-    assert _lib.load().rajni_abi_version() == 10

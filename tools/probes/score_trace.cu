@@ -22,7 +22,7 @@ int main(int argc, char** argv) {
     cudaEvent_t e0, e1; cudaEventCreate(&e0); cudaEventCreate(&e1);
     for (int i = 0; i < 6; ++i) {
         if (i == 5) cudaEventRecord(e0);
-        int rc = rajni_score_select_split(qkv[i % 3], B, N, C, H, keep, 1e-6f, nullptr, idx, nxt, rmap, ws, wb, 0);
+        int rc = rajni_score_select_prefix(qkv[i % 3], B, N, C, H, 1, keep, 1e-6f, nullptr, idx, nxt, rmap, ws, wb, 0);
         if (rc) { printf("rc=%d\n", rc); return 1; }
     }
     cudaEventRecord(e1);
