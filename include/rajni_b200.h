@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define RAJNI_ABI_VERSION 11     /* 11: one entry point per operation; the superseded calls are gone */
+#define RAJNI_ABI_VERSION 12     /* 12: the GEMM lost its split-K workspace (rajni_gemm_args is two fields shorter) */
 
 enum {
     RAJNI_OK = 0,
@@ -46,10 +46,8 @@ enum {
     RAJNI_EPI_OUT_F32 = 8,    /* store fp32 instead of bf16                      */
     RAJNI_EPI_LN_FOLD = 16,   /* A is the UN-normalised x; apply LayerNorm algebraically (see below)  */
     RAJNI_EPI_ROW_STATS = 32, /* also emit per-row partial (sum, sum of squares) of the stored values */
-    RAJNI_HINT_REVERSE_M = 64,/* walk the M tiles last-to-first: a consumer that starts where its producer
+    RAJNI_HINT_REVERSE_M = 64 /* walk the M tiles last-to-first: a consumer that starts where its producer
                                  finished finds those rows still in the 126 MB L2. Results are identical.   */
-    RAJNI_HINT_STREAM_K = 128 /* with a workspace: split the leftover tiles of the last wave along K wherever that is
-                                 possible, not only where the cost model expects a gain (tests, A/B timing).   */
 };
 
 int rajni_abi_version(void);
@@ -153,17 +151,8 @@ typedef struct rajni_gemm_args {
     long long ldd; const int32_t* out_row_map;
     const float* ln_stats; long long ln_stats_ld; int ln_slots; const float* ln_wsum; float ln_eps;
     float* row_stats; long long row_stats_ld;
-    /* optional stream-K scratch (may be NULL): >= rajni_gemm_workspace_bytes() bytes, 128-byte aligned, its first 4096 bytes
-     * ZERO before the first call (the kernels leave them zero).  With it, a CTA-pair GEMM with a long K whose tile count is
-     * not a multiple of the SM pairs splits the leftover tiles of the last wave along K over the pairs and reduces the fp32
-     * partials through this buffer (deterministic order).  Calls that share one workspace must be ordered on one stream. */
-    void* workspace; long long workspace_bytes;
 } rajni_gemm_args;
 int rajni_gemm_bf16_ex(const rajni_gemm_args* args, void* stream);
-size_t rajni_gemm_workspace_bytes(void);
-/* Host-side query, no launch: the number of tiles a GEMM of this shape and these flags would split along K when given a
- * workspace (0 = none) and, through sk_pairs (may be NULL), the number of CTA pairs that share the pieces. */
-int rajni_gemm_stream_k_plan(int M, int N, int K, int flags, int* sk_pairs);
 int rajni_gemm_row_stats_slots(int N);
 
 /* ---- a4: multi-head attention over kept tokens (attention.py:45-54)

@@ -14,8 +14,8 @@ LIB_PATH = os.path.join(_HERE, "csrc", "librajni_b200.so")
 
 RAJNI_OK, RAJNI_EINVAL, RAJNI_ECUDA, RAJNI_EARCH, RAJNI_ERANGE = 0, -1, -2, -3, -4
 ATTN_AUTO, ATTN_PIPE, ATTN_TC, ATTN_LONG = 0, 1, 2, 3
-EPI_BIAS, EPI_GELU, EPI_RESIDUAL, EPI_OUT_F32, EPI_LN_FOLD, EPI_ROW_STATS, HINT_REVERSE_M, HINT_STREAM_K = 1, 2, 4, 8, 16, 32, 64, 128
-ABI_VERSION = 11
+EPI_BIAS, EPI_GELU, EPI_RESIDUAL, EPI_OUT_F32, EPI_LN_FOLD, EPI_ROW_STATS, HINT_REVERSE_M = 1, 2, 4, 8, 16, 32, 64
+ABI_VERSION = 12
 
 
 class GemmArgs(Structure):
@@ -26,8 +26,7 @@ class GemmArgs(Structure):
                 ("ldd", c_longlong), ("out_row_map", c_void_p),
                 ("ln_stats", c_void_p), ("ln_stats_ld", c_longlong), ("ln_slots", c_int),
                 ("ln_wsum", c_void_p), ("ln_eps", c_float),
-                ("row_stats", c_void_p), ("row_stats_ld", c_longlong),
-                ("workspace", c_void_p), ("workspace_bytes", c_longlong)]
+                ("row_stats", c_void_p), ("row_stats_ld", c_longlong)]
 
 
 
@@ -55,8 +54,6 @@ SIGNATURES = {
                                               c_longlong, c_void_p]),
     "rajni_gemm_bf16_ex": (c_int, [POINTER(GemmArgs), c_void_p]),
     "rajni_gemm_row_stats_slots": (c_int, [c_int]),
-    "rajni_gemm_workspace_bytes": (c_size_t, []),
-    "rajni_gemm_stream_k_plan": (c_int, [c_int, c_int, c_int, c_int, c_void_p]),
     "rajni_attention_fwd_ex": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_float, c_int, c_int, c_void_p]),
     "rajni_resize_workspace_bytes": (c_size_t, [c_int, c_int]),
     "rajni_resize_center_crop_u8": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_size_t, c_void_p]),

@@ -74,61 +74,7 @@ struct GemmParams {
     float2* row_stats;          // [N >> stat_shift][row_stats_ld] partial (sum, sumsq) of the rows of D per 32- or 64-column slot, or null
     long long row_stats_ld;
     int stat_shift;             // 5 or 6: log2 of the slot width (rajni_gemm_row_stats_slots)
-    // stream-K tail (see "Stream-K" below): the first sk_tiles tiles are split along K over sk_pairs CTA pairs
-    int sk_tiles, sk_pairs, sk_units;   // sk_units = sk_tiles * k_blocks
-    float* sk_ws;               // fp32 partial accumulators: [pair][piece 0/1][cta rank][128][BN]
-    int* sk_flags;              // [2][2 * sk_tiles]: partials arrived / finishing warps done, per (tile, cta rank); zero between launches
 };
-
-// ---------------------------------------------------------------------------------------------------------------------
-// Stream-K tail.  tiles_m * tiles_n is rarely a multiple of the 74 CTA pairs: the last, partial wave costs a whole tile time
-// (173 x 3 tiles = 7.01 waves -> 8).  For long K the R = tiles % pairs leftover tiles are therefore taken FIRST and split along
-// K: their R * k_blocks k-blocks are dealt out evenly to sk_pairs CTA pairs (a contiguous range each, so a pair gets pieces of
-// at most two tiles), every pair then runs its whole tiles as before.  A piece's fp32 accumulator goes to a scratch slot
-// (thread = row, 128-byte runs) and a counter per (tile, CTA rank) is bumped; after its last whole tile each of the first
-// min(pieces, BN/64) contributors of a tile adds up ALL the pieces of its own 64-column slices (fixed order: deterministic)
-// and runs the usual fused epilogue on them - the fix-up is spread over the contributors, and by then the partials have
-// been in L2 for the length of the kernel, so nobody waits.  Every piece is written before any pair starts waiting: no
-// deadlock.  The last finisher zeroes the counters for the next launch (launches sharing a workspace are stream-ordered).
-struct SkPlan { int n, tile0, k00, k10, tile1, k11; };      // piece 0 = (tile0, [k00, k10)), piece 1 = (tile1, [0, k11))
-__device__ __forceinline__ int sk_bound(const GemmParams& p, int j) { return (int)(((long long)j * p.sk_units) / p.sk_pairs); }
-// the pair whose range holds k-block unit u: the largest j with sk_bound(j) <= u
-__device__ __forceinline__ int sk_pair_of(const GemmParams& p, int u) {
-    return (int)(((long long)(u + 1) * p.sk_pairs + p.sk_units - 1) / p.sk_units) - 1;
-}
-template <bool SK>
-__device__ __forceinline__ SkPlan sk_plan(const GemmParams& p, int pair) {
-    SkPlan s{0, 0, 0, 0, 0, 0};
-    if (SK && pair < p.sk_pairs) {
-        const int b0 = sk_bound(p, pair), b1 = sk_bound(p, pair + 1);
-        if (b1 > b0) {
-            const int t0 = b0 / p.k_blocks, t1 = (b1 - 1) / p.k_blocks;
-            s.tile0 = t0; s.k00 = b0 - t0 * p.k_blocks; s.k10 = min(b1 - t0 * p.k_blocks, p.k_blocks);
-            s.n = 1;
-            if (t1 > t0) { s.tile1 = t1; s.k11 = b1 - t1 * p.k_blocks; s.n = 2; }
-        }
-    }
-    return s;
-}
-// item `it` of a pair's sequence of accumulator-producing work: its stream-K pieces first, then whole tiles
-template <bool SK>
-__device__ __forceinline__ bool sk_item(const GemmParams& p, const SkPlan& plan, int pair, int stride, int num_tiles, int it,
-                                        int& tile, int& k0, int& k1) {
-    if (SK && it < plan.n) {
-        tile = it == 0 ? plan.tile0 : plan.tile1;
-        k0 = it == 0 ? plan.k00 : 0;
-        k1 = it == 0 ? plan.k10 : plan.k11;
-        return true;
-    }
-    tile = (SK ? p.sk_tiles : 0) + pair + (it - (SK ? plan.n : 0)) * stride;
-    k0 = 0; k1 = p.k_blocks;
-    return tile < num_tiles;
-}
-__device__ __forceinline__ int ld_acquire_gpu(const int* ptr) {
-    int v;
-    asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(ptr) : "memory");
-    return v;
-}
 
 // Exact-erf GELU (timm nn.GELU) evaluated as x*Phi(x) with
 //   Phi(-a) = 0.5 * 2^(-a*P(a)),  a = min(|x|, 6),  P = degree-4 fit of -log2(erfc(a/sqrt2))/a, weighted so that the error of
@@ -174,9 +120,9 @@ __device__ __forceinline__ float4 lds128(uint32_t addr) {
 // logic (they require N % BN == 0); MODE_GENERIC reads the runtime flags and handles every edge.
 enum { MODE_GENERIC = 0, MODE_BIAS = 1, MODE_BIAS_GELU = 2, MODE_BIAS_RES = 3 };
 
-// One 32-column chunk of one output row in the hot epilogues: cur = the fp32 accumulators (from TMEM, or summed stream-K
-// partials), r = the residual's 32 bf16.  Bias / LayerNorm fold / GELU / residual in packed fp32x2, bf16 row stores, and the
-// row statistics of the values as stored (MODE_BIAS_RES with row_stats).
+// One 32-column chunk of one output row in the hot epilogues: cur = the fp32 accumulators from TMEM, r = the residual's
+// 32 bf16.  Bias / LayerNorm fold / GELU / residual in packed fp32x2, bf16 row stores, and the row statistics of the values
+// as stored (MODE_BIAS_RES with row_stats).
 template <int MODE, bool LN>
 __device__ __forceinline__ void epi_chunk(const uint32_t (&cur)[32], const uint32_t (&r)[16], int ch, uint32_t sb, uint32_t sg,
                                           uint64_t rstd2, uint64_t mr2, uint64_t& sum2, uint64_t& sq2, bool wide_slots,
@@ -236,7 +182,7 @@ __device__ __forceinline__ void epi_chunk(const uint32_t (&cur)[32], const uint3
 }
 
 
-template <int BN, int CG, int MODE, bool LN, bool SK>
+template <int BN, int CG, int MODE, bool LN>
 __global__ void __launch_bounds__(kGemmThreads, 1)
 gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                  const GemmParams p) {
@@ -283,14 +229,13 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
         if (lane == 0) {
             int stage = 0;
             uint32_t phase = 0;
-            const SkPlan plan = sk_plan<SK>(p, first_tile);
-            int tile, k0, k1;
-            for (int it = 0; sk_item<SK>(p, plan, first_tile, tile_stride, num_tiles, it, tile, k0, k1); ++it) {
+            for (int it = 0; first_tile + it * tile_stride < num_tiles; ++it) {
+                const int tile = first_tile + it * tile_stride;
                 const int m_lin = tile / p.tiles_n, n_blk = tile % p.tiles_n;
                 const int m_blk = p.reverse_m ? p.tiles_m - 1 - m_lin : m_lin;
                 const int row_a = m_blk * (BM * CG) + (int)cta_rank * BM;
                 const int row_b = n_blk * BN + (int)cta_rank * Cfg::kBRows;
-                for (int kb = k0; kb < k1; ++kb) {
+                for (int kb = 0; kb < p.k_blocks; ++kb) {
                     mbar_wait(&empty_bar[stage], phase ^ 1);
                     if (CG == 2) {
                         const uint32_t lead_bar = mapa_u32(smem_u32(&full_bar[stage]), 0);
@@ -312,15 +257,13 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
             constexpr uint32_t idesc = umma_idesc_bf16(BM * CG, BN, 0, 0);
             int stage = 0;
             uint32_t phase = 0;
-            const SkPlan plan = sk_plan<SK>(p, first_tile);
-            int tile, k0, k1;
-            for (int local = 0; sk_item<SK>(p, plan, first_tile, tile_stride, num_tiles, local, tile, k0, k1); ++local) {
+            for (int local = 0; first_tile + local * tile_stride < num_tiles; ++local) {
                 const int acc = local & 1;
                 const uint32_t acc_phase = (local >> 1) & 1;
                 mbar_wait(&tmem_empty[acc], acc_phase ^ 1);          // epilogues have drained this accumulator
                 tc_fence_after();
                 const uint32_t d_tmem = tmem_base + acc * BN;
-                for (int kb = k0; kb < k1; ++kb) {
+                for (int kb = 0; kb < p.k_blocks; ++kb) {
                     mbar_wait(&full_bar[stage], phase);
                     tc_fence_after();
                     const uint32_t a_addr = smem_u32(s_a + stage * Cfg::kABytes);
@@ -330,8 +273,8 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
                         // advancing 16 bf16 along K = +32 bytes inside the 128-byte swizzle row
                         const uint64_t a_desc = umma_desc_sw128(a_addr + k * 32, 16, 1024);
                         const uint64_t b_desc = umma_desc_sw128(b_addr + k * 32, 16, 1024);
-                        if (CG == 2) umma_bf16_cg2(d_tmem, a_desc, b_desc, idesc, (uint32_t)(kb != k0 || k != 0));
-                        else umma_bf16(d_tmem, a_desc, b_desc, idesc, (uint32_t)(kb != k0 || k != 0));
+                        if (CG == 2) umma_bf16_cg2(d_tmem, a_desc, b_desc, idesc, (uint32_t)(kb != 0 || k != 0));
+                        else umma_bf16(d_tmem, a_desc, b_desc, idesc, (uint32_t)(kb != 0 || k != 0));
                     }
                     // frees the smem slot (in both CTAs of a pair) when these MMAs finish
                     if (CG == 2) umma_commit_cg2(&empty_bar[stage], 0x3); else umma_commit(&empty_bar[stage]);
@@ -356,7 +299,6 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
             const uint32_t sb = stg, sg = stg + HALF * 4;   // this warp's bias / weight-row-sum vectors
             __nv_bfloat16* const Dp = static_cast<__nv_bfloat16*>(p.D);
             const bool wide_slots = kRes && p.stat_shift == 6;   // 64-column statistics slots: two chunks each (NCH is even then)
-            const int pair = first_tile;
             // ---- state of the tile being finished (set by `setup`)
             int ncol0 = 0;
             bool valid = false;
@@ -364,8 +306,8 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
             __nv_bfloat16* dptr = nullptr;
             uint32_t rr[kRes ? NCH : 1][16];
             uint64_t rstd2 = 0, mr2 = 0;
-            // everything of a tile's epilogue that does not need the accumulator; `chunks`: bit c = this warp will process chunk c
-            auto setup = [&](int tile, uint32_t chunks) {
+            // everything of a tile's epilogue that does not need the accumulator
+            auto setup = [&](int tile) {
                 const int m_lin = tile / p.tiles_n, n_blk = tile % p.tiles_n;
                 const int m_blk = p.reverse_m ? p.tiles_m - 1 - m_lin : m_lin;
                 const int m = m_blk * (BM * CG) + (int)cta_rank * BM + sub * 32 + lane;
@@ -392,7 +334,6 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
                         const __nv_bfloat16* rptr = p.residual + (p.res_row_map ? (long long)__ldg(p.res_row_map + m) : (long long)m) * p.ldres + ncol0;
 #pragma unroll
                         for (int c = 0; c < NCH; ++c) {
-                            if (!((chunks >> c) & 1u)) continue;
                             ldg256(rptr + c * 32, *reinterpret_cast<uint32_t(*)[8]>(&rr[kRes ? c : 0][0]));      // (coherent: the residual may alias D)
                             ldg256(rptr + c * 32 + 16, *reinterpret_cast<uint32_t(*)[8]>(&rr[kRes ? c : 0][8]));
                         }
@@ -417,52 +358,11 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
             uint32_t va[32], vb[32];
             uint64_t sum2 = 0, sq2 = 0;                      // row statistics of the current slot (kRes)
             int local = 0;
-            if (SK) {
-                // ---- this pair's stream-K pieces come first: the fp32 partial goes to the pair's scratch slot, the tile is
-                //      finished after the whole tiles (below).  (A piece is never a whole tile: sk_decide.)
-                const int n_pieces = sk_plan<SK>(p, pair).n;
-                for (; local < n_pieces; ++local) {
-                    const SkPlan plan = sk_plan<SK>(p, pair);
-                    const int tile = local == 0 ? plan.tile0 : plan.tile1;
-                    const int acc = local & 1;
-                    const uint32_t taddr = tmem_base + ((uint32_t)(sub * 32) << 16) + (uint32_t)(acc * BN + half * HALF);
-                    // slot layout: [warp (sub, half)][chunk][4-column group][lane][4 fp32] - every warp store / load is 512 contiguous bytes
-                    float* slot = p.sk_ws + (size_t)((pair * 2 + local) * 2 + (int)cta_rank) * (BM * BN) + (size_t)(sub * 2 + half) * (32 * HALF) + lane * 4;
-                    mbar_wait(&tmem_full[acc], 0);
-                    tc_fence_after();
-                    tmem_ld32(taddr, va);
-#pragma unroll
-                    for (int ch = 0; ch < NCH; ++ch) {
-                        uint32_t (&cur)[32] = (ch & 1) ? vb : va;
-                        uint32_t (&nxt)[32] = (ch & 1) ? va : vb;
-                        tmem_ld_wait();
-                        if (ch + 1 < NCH) {
-                            tmem_ld32(taddr + (ch + 1) * 32, nxt);
-                        } else {
-                            tc_fence_before();
-                            __syncwarp();
-                            if (lane == 0) {
-                                if (CG == 2) mbar_arrive_cluster(mapa_u32(smem_u32(&tmem_empty[acc]), 0));
-                                else mbar_arrive(&tmem_empty[acc]);
-                            }
-                        }
-#pragma unroll
-                        for (int g = 0; g < 8; ++g)
-                            st_stream16(slot + (ch * 8 + g) * 128, make_uint4(cur[4 * g], cur[4 * g + 1], cur[4 * g + 2], cur[4 * g + 3]));
-                    }
-                    __syncwarp();
-                    if (lane == 0) {
-                        __threadfence();                     // the warp's stores (ordered before this by the __syncwarp) are visible first
-                        atomicAdd(p.sk_flags + tile * 2 + (int)cta_rank, 1);
-                    }
-                }
-            }
-            const int local0 = local;
-            for (int tile = (SK ? p.sk_tiles : 0) + pair; tile < num_tiles; tile += tile_stride, ++local) {
+            for (int tile = first_tile; tile < num_tiles; tile += tile_stride, ++local) {
                 const int acc = local & 1;
                 const uint32_t acc_phase = (local >> 1) & 1;
                 const uint32_t taddr = tmem_base + ((uint32_t)(sub * 32) << 16) + (uint32_t)(acc * BN + half * HALF);
-                setup(tile, 0xffffffffu);
+                setup(tile);
                 mbar_wait(&tmem_full[acc], acc_phase);
                 tc_fence_after();
                 tmem_ld32(taddr, va);
@@ -483,84 +383,6 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
                         }
                     }
                     epi_chunk<MODE, LN>(cur, rr[kRes ? ch : 0], ch, sb, sg, rstd2, mr2, sum2, sq2, wide_slots, valid, dptr, orow, ncol0, p);
-                }
-            }
-            // ---- stream-K: finish this pair's share of the split tiles it contributed to
-            for (int q = 0; SK && q < local0; ++q) {
-                int pair_o = pair;
-                asm volatile("" : "+r"(pair_o));                            // (recomputed here rather than kept live across the tile loop)
-                const SkPlan plan = sk_plan<SK>(p, pair_o);
-                const int t = q == 0 ? plan.tile0 : plan.tile1, u0 = t * p.k_blocks;
-                const int jf = sk_pair_of(p, u0), jl = sk_pair_of(p, u0 + p.k_blocks - 1);
-                const int pieces = jl - jf + 1, me = pair - jf;
-                constexpr int UNITS = BN / 64;                               // 64-column slices of a tile (= statistics slots)
-                const int nfin = pieces < UNITS ? pieces : UNITS;
-                if (me >= nfin) continue;
-                uint32_t mine = 0;
-#pragma unroll
-                for (int ch = 0; ch < NCH; ++ch) if ((((half * HALF + ch * 32) >> 6) % nfin) == me) mine |= 1u << ch;
-                int* const arrived = p.sk_flags + t * 2 + (int)cta_rank;
-                int* const done = arrived + 2 * p.sk_tiles;
-                setup(t, 0u);                                               // (the residual is fetched per chunk below)
-                if (mine != 0) {
-                    if (lane == 0) {
-                        // pieces * 8 epilogue warps of this CTA rank arrive; all of them were written before anybody waits here
-                        unsigned spins = 0;
-                        while (ld_acquire_gpu(arrived) < pieces * kEpiWarps) {
-                            __nanosleep(200);
-                            if (++spins > (1u << 24)) asm volatile("trap;");  // (seconds: a lost contributor must not hang the GPU)
-                        }
-                    }
-                    __syncwarp();
-                    // slot of contributor i: its first piece unless the pair's range began in the previous tile
-                    const int q0 = sk_bound(p, jf) == u0 ? 0 : 1;
-                    const size_t slot_floats = (size_t)2 * BM * BN;          // both CTA ranks of one piece
-                    const float* const base0 = p.sk_ws + ((size_t)(jf * 2 + q0) * 2 + (int)cta_rank) * (BM * BN) + (size_t)(sub * 2 + half) * (32 * HALF) + lane * 4;
-                    const float* const base1 = p.sk_ws + ((size_t)(jf * 2 + 2) * 2 + (int)cta_rank) * (BM * BN) + (size_t)(sub * 2 + half) * (32 * HALF) + lane * 4;
-                    const __nv_bfloat16* rptr = nullptr;
-                    if (kRes && valid) {
-                        const int m_lin = t / p.tiles_n;
-                        const int m = (p.reverse_m ? p.tiles_m - 1 - m_lin : m_lin) * (BM * CG) + (int)cta_rank * BM + sub * 32 + lane;
-                        rptr = p.residual + (p.res_row_map ? (long long)__ldg(p.res_row_map + m) : (long long)m) * p.ldres + ncol0;
-                    }
-#pragma unroll
-                    for (int ch = 0; ch < NCH; ++ch) {
-                        if (!((mine >> ch) & 1u)) continue;
-                        uint32_t r1[16];
-                        if (kRes && valid) {
-                            ldg256(rptr + ch * 32, *reinterpret_cast<uint32_t(*)[8]>(&r1[0]));
-                            ldg256(rptr + ch * 32 + 16, *reinterpret_cast<uint32_t(*)[8]>(&r1[8]));
-                        }
-                        // sum of the pieces in contributor order (deterministic); two pieces' loads in flight at a time
-                        float a32[32];
-#pragma unroll
-                        for (int j = 0; j < 32; ++j) a32[j] = 0.f;
-                        for (int i = 0; i < pieces; i += 2) {
-                            const float* s0 = (i == 0 ? base0 : base1 + (size_t)(i - 1) * 2 * slot_floats) + ch * 1024;
-                            const bool two = i + 1 < pieces;
-                            const float* s1 = base1 + (size_t)i * 2 * slot_floats + ch * 1024;
-                            float4 x[8], y[8];
-#pragma unroll
-                            for (int g = 0; g < 8; ++g) x[g] = __ldcg(reinterpret_cast<const float4*>(s0 + g * 128));
-#pragma unroll
-                            for (int g = 0; g < 8; ++g) y[g] = two ? __ldcg(reinterpret_cast<const float4*>(s1 + g * 128)) : make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll
-                            for (int g = 0; g < 8; ++g) { a32[4 * g] += x[g].x; a32[4 * g + 1] += x[g].y; a32[4 * g + 2] += x[g].z; a32[4 * g + 3] += x[g].w; }
-#pragma unroll
-                            for (int g = 0; g < 8; ++g) { a32[4 * g] += y[g].x; a32[4 * g + 1] += y[g].y; a32[4 * g + 2] += y[g].z; a32[4 * g + 3] += y[g].w; }
-                        }
-#pragma unroll
-                        for (int j = 0; j < 32; ++j) va[j] = __float_as_uint(a32[j]);
-                        epi_chunk<MODE, LN>(va, r1, ch, sb, sg, rstd2, mr2, sum2, sq2, wide_slots, valid, dptr, orow, ncol0, p);
-                    }
-                }
-                __syncwarp();
-                if (lane == 0) {
-                    // the last of the nfin * 8 finishing warps re-arms the counters for the next launch
-                    if (atomicAdd(done, 1) == nfin * kEpiWarps - 1) {
-                        *arrived = 0;
-                        *done = 0;
-                    }
                 }
             }
         } else {
@@ -744,39 +566,8 @@ int make_tmap_bf16_3d_ld(CUtensorMap* map, const void* base, long long batch, lo
     return 0;
 }
 
-// Stream-K scratch: a 4 KB header of counters, then one fp32 slot per (pair, piece, CTA rank) of 128 x 256 accumulators.
-constexpr size_t kSkHeaderBytes = 4096;
-constexpr int kSkMinKBlocks = 16;          // shorter K: a tile is too cheap for a fix-up to pay
-constexpr int kSkMinPiece = 8;             // k-blocks per pair at least (bounds the pieces per tile at k_blocks / 8 + 1)
-static size_t sk_workspace_bytes() { return kSkHeaderBytes + (size_t)(num_sms() / 2) * 2 * 2 * BM * 256 * sizeof(float); }
-
-// Decide whether the leftover tiles of the last wave are split along K (see "Stream-K" above).  Time is counted in k-blocks
-// of one pair: without the split the R leftover tiles cost a whole extra tile time (k_blocks); with it every sharing pair
-// gets ceil(R * k_blocks / pairs) k-blocks plus the fix-up - writing the fp32 partials (256 KB per pair and piece) and
-// reading them back costs ~`fix` k-block times, measured (profiles/r2_gemm_stream_k.md: 6-10 us with few pieces, 17-27 us
-// when every pair holds two).  The split must save at least 15 % of the whole call: that admits the short calls of small
-// shards (M = 6304, K = 3072: 41.0 -> 33.4 us) and rejects the long ones, where under the power cap an idle tail costs
-// little anyway (M = 44288: 153.9 vs 156.1 us).  Returns R (0: no split) and the number of pairs that share the pieces.
-static int sk_decide(int tiles, int pairs, int k_blocks, bool force, int* sk_pairs) {
-    static const char* env = getenv("RAJNI_GEMM_SK");                       // "0" disables, "1" forces wherever it is legal
-    static const int fix = getenv("RAJNI_GEMM_SK_FIX") ? atoi(getenv("RAJNI_GEMM_SK_FIX")) : 20;
-    if (env && env[0] == '0') return 0;
-    const int R = tiles % pairs, full = tiles / pairs;
-    if (R == 0 || k_blocks < kSkMinKBlocks) return 0;
-    long long units = (long long)R * k_blocks;
-    int sp = (int)(units / kSkMinPiece);
-    if (sp > pairs) sp = pairs;
-    if (sp < R) sp = R;                                                      // a pair's range never spans three tiles
-    const int per_pair = (int)((units + sp - 1) / sp);
-    if (per_pair >= k_blocks) return 0;                                      // nothing is split (and a piece is never a whole tile)
-    const bool forced = force || (env && env[0] == '1');
-    if (!forced && (long long)(k_blocks - per_pair - fix) * 100 < 15LL * (full + 1) * k_blocks) return 0;
-    *sk_pairs = sp;
-    return R;
-}
-
 template <int BN, int CG, int MODE, bool LN>
-static int launch_gemm_mode(const void* A, const void* W, GemmParams& p, void* ws, size_t ws_bytes, cudaStream_t stream) {
+static int launch_gemm_mode(const void* A, const void* W, GemmParams& p, cudaStream_t stream) {
     using Cfg = GemmCfg<BN, CG>;
     CUtensorMap ta, tb;
     if (int rc = make_tmap_bf16_2d(&ta, A, p.M, p.K, p.K, BM)) return rc;
@@ -789,23 +580,9 @@ static int launch_gemm_mode(const void* A, const void* W, GemmParams& p, void* w
     if (cta_cap > 0 && cta_cap < max_grid) max_grid = (cta_cap / CG) * CG;
     int grid = p.tiles_m * p.tiles_n * CG;
     if (grid > max_grid) grid = max_grid;
-    constexpr bool kSkCapable = BN == 256 && CG == 2 && MODE != MODE_GENERIC;
-    bool sk = false;
-    if (kSkCapable && ws != nullptr && ws_bytes >= sk_workspace_bytes() && (reinterpret_cast<uintptr_t>(ws) & 127u) == 0) {
-        int sp = 0;
-        const int R = sk_decide(p.tiles_m * p.tiles_n, max_grid / CG, p.k_blocks, (p.flags & RAJNI_HINT_STREAM_K) != 0, &sp);
-        if (R > 0) {
-            sk = true;
-            p.sk_tiles = R; p.sk_pairs = sp; p.sk_units = R * p.k_blocks;
-            p.sk_flags = static_cast<int*>(ws);
-            p.sk_ws = reinterpret_cast<float*>(static_cast<char*>(ws) + kSkHeaderBytes);
-            if (grid < sp * CG) grid = sp * CG;          // fewer tiles than pairs: the pieces still go to sk_pairs pairs
-        }
-    }
-    auto kern = gemm_bf16_kernel<BN, CG, MODE, LN, false>;
-    if constexpr (kSkCapable) { if (sk) kern = gemm_bf16_kernel<BN, CG, MODE, LN, true>; }
-    static int smem_granted[2][kMaxDevices] = {};
-    if (int rc = raise_smem_limit("gemm", kern, Cfg::kSmemBytes, smem_granted[sk ? 1 : 0])) return rc;
+    auto kern = gemm_bf16_kernel<BN, CG, MODE, LN>;
+    static int smem_granted[kMaxDevices] = {};
+    if (int rc = raise_smem_limit("gemm", kern, Cfg::kSmemBytes, smem_granted)) return rc;
     return launch_checked("gemm_bf16", kern, dim3(grid), dim3(kGemmThreads), Cfg::kSmemBytes, stream, CG, ta, tb, p);
 }
 
@@ -814,30 +591,30 @@ static bool aligned32(const void* ptr) { return (reinterpret_cast<uintptr_t>(ptr
 // Pick the compile-time epilogue.  The hot modes need: no column tail, 32-byte-aligned rows of D (and of
 // the residual), bf16 output, and one of the flag combinations below; everything else runs MODE_GENERIC.
 template <int BN, int CG>
-static int launch_gemm(const void* A, const void* W, GemmParams& p, void* ws, size_t ws_bytes, cudaStream_t stream) {
+static int launch_gemm(const void* A, const void* W, GemmParams& p, cudaStream_t stream) {
     const int ln = p.flags & RAJNI_EPI_LN_FOLD, stats = p.flags & RAJNI_EPI_ROW_STATS;
-    const int core = p.flags & ~(RAJNI_EPI_LN_FOLD | RAJNI_EPI_ROW_STATS | RAJNI_HINT_REVERSE_M | RAJNI_HINT_STREAM_K);
+    const int core = p.flags & ~(RAJNI_EPI_LN_FOLD | RAJNI_EPI_ROW_STATS | RAJNI_HINT_REVERSE_M);
     bool hot = p.N % BN == 0 && p.ldd % 16 == 0 && aligned32(p.D);
     if (core & RAJNI_EPI_RESIDUAL) hot = hot && p.ldres % 16 == 0 && aligned32(p.residual);
     if (hot) {
         if (core == RAJNI_EPI_BIAS && !stats)
-            return ln ? launch_gemm_mode<BN, CG, MODE_BIAS, true>(A, W, p, ws, ws_bytes, stream) : launch_gemm_mode<BN, CG, MODE_BIAS, false>(A, W, p, ws, ws_bytes, stream);
+            return ln ? launch_gemm_mode<BN, CG, MODE_BIAS, true>(A, W, p, stream) : launch_gemm_mode<BN, CG, MODE_BIAS, false>(A, W, p, stream);
         if (core == (RAJNI_EPI_BIAS | RAJNI_EPI_GELU) && !stats)
-            return ln ? launch_gemm_mode<BN, CG, MODE_BIAS_GELU, true>(A, W, p, ws, ws_bytes, stream) : launch_gemm_mode<BN, CG, MODE_BIAS_GELU, false>(A, W, p, ws, ws_bytes, stream);
+            return ln ? launch_gemm_mode<BN, CG, MODE_BIAS_GELU, true>(A, W, p, stream) : launch_gemm_mode<BN, CG, MODE_BIAS_GELU, false>(A, W, p, stream);
         if (core == (RAJNI_EPI_BIAS | RAJNI_EPI_RESIDUAL) && !ln)
-            return launch_gemm_mode<BN, CG, MODE_BIAS_RES, false>(A, W, p, ws, ws_bytes, stream);
+            return launch_gemm_mode<BN, CG, MODE_BIAS_RES, false>(A, W, p, stream);
     }
     RAJNI_REQUIRE(!ln && !stats, RAJNI_EINVAL,
                   "rajni_gemm_bf16_ex: LN_FOLD / ROW_STATS need N %% %d == 0, ldd/ldres multiples of 16 and 32-byte aligned rows "
                   "(N=%d ldd=%lld ldres=%lld flags=%d)", BN, p.N, p.ldd, p.ldres, p.flags);
-    return launch_gemm_mode<BN, CG, MODE_GENERIC, false>(A, W, p, ws, ws_bytes, stream);
+    return launch_gemm_mode<BN, CG, MODE_GENERIC, false>(A, W, p, stream);
 }
 
 // Tile width.  Generic epilogue: minimise padded columns (the 64-wide tile runs at ~2/3 rate, shared-memory bound).
 // `exact` (hot epilogues, no column-tail path): among the widths that divide N, the CTA-pair tiles (256 or 192 wide,
 // 256 rows) are preferred; between those two the one with fewer, fuller waves over the 74 CTA pairs wins
 // (e.g. N = 768, M = 44288: 173 x 3 tiles of 256 = 7.01 waves -> 8, but 173 x 4 tiles of 192 = 9.35 -> 10 x 3/4 = 7.5).
-static int pick_bn(int N, int M, int K, bool exact, bool no192, bool sk_ws, bool force_sk = false) {
+static int pick_bn(int N, int M, bool exact, bool no192) {
     if (exact) {
         static const char* force = getenv("RAJNI_GEMM_BN");                 // debugging aid: force a pair-tile width that divides N
         if (force && M > BM && N % atoi(force) == 0 && (atoi(force) == 256 || (atoi(force) == 192 && !no192) || atoi(force) == 128)) return -atoi(force);
@@ -848,14 +625,7 @@ static int pick_bn(int N, int M, int K, bool exact, bool no192, bool sk_ws, bool
             if (!pair || N % bn || (no192 && bn == 192)) continue;
             const long long tiles = (long long)((M + 2 * BM - 1) / (2 * BM)) * (N / bn);
             const int pairs = num_sms() / 2;
-            double waves = (double)((tiles + pairs - 1) / pairs);
-            if (bn == 256 && sk_ws) {
-                // the 256-wide tile can split its leftover tiles along K (stream-K): the last wave then costs a fraction
-                int sp = 0;
-                const int kb = (K + BK - 1) / BK;
-                if (sk_decide((int)tiles, pairs, kb, force_sk, &sp) > 0)
-                    waves = (double)(tiles / pairs) + (double)((tiles % pairs) * kb / sp + 20) / kb;
-            }
+            const double waves = (double)((tiles + pairs - 1) / pairs);
             // the 192-wide tile re-reads A once more per row block: it has to save 8 % of the wave time to be chosen
             // (the 128-wide pair tile re-reads A twice as often and halves the work per accumulator hand-over: 20 %)
             const double cost = waves * bn * (bn == 192 ? 1.08 : bn == 128 ? 1.2 : 1.0);
@@ -882,25 +652,6 @@ static int stat_shift_for(int N) { return N % 128 == 0 ? 6 : 5; }
 extern "C" int rajni_gemm_row_stats_slots(int N) {
     if (N <= 0 || N % 64 != 0) return 0;            // ROW_STATS needs whole tiles
     return N >> stat_shift_for(N);
-}
-
-extern "C" size_t rajni_gemm_workspace_bytes(void) { return sk_workspace_bytes(); }
-
-// Host-side query (no launch): how many tiles a hot-epilogue GEMM of this shape would split along K given a workspace,
-// and over how many CTA pairs.  0 = no stream-K (tile count already a multiple of the pairs, K too short, or no gain).
-extern "C" int rajni_gemm_stream_k_plan(int M, int N, int K, int flags, int* sk_pairs) {
-    if (sk_pairs) *sk_pairs = 0;
-    if (M <= BM || N <= 0 || N % 256 != 0 || K <= 0 || (flags & RAJNI_EPI_OUT_F32)) return 0;
-    // the entry point's own tile choice; only the 256-wide CTA-pair tile with a hot epilogue splits
-    const bool exact = (flags & (RAJNI_EPI_LN_FOLD | RAJNI_EPI_ROW_STATS)) != 0;
-    const bool force = (flags & RAJNI_HINT_STREAM_K) != 0;
-    const int bn = pick_bn(N, M, K, exact, (flags & RAJNI_EPI_ROW_STATS) && stat_shift_for(N) == 6, true, force);
-    if (bn != -256 && bn != 256) return 0;
-    int sp = 0;
-    const int tiles = ((M + 2 * BM - 1) / (2 * BM)) * (N / 256);
-    const int R = sk_decide(tiles, num_sms() / 2, (K + BK - 1) / BK, force, &sp);
-    if (sk_pairs && R > 0) *sk_pairs = sp;
-    return R;
 }
 
 extern "C" int rajni_gemm_bf16_ex(const rajni_gemm_args* a, void* stream) {
@@ -937,18 +688,17 @@ extern "C" int rajni_gemm_bf16_ex(const rajni_gemm_args* a, void* stream) {
     const bool exact = (flags & (RAJNI_EPI_LN_FOLD | RAJNI_EPI_ROW_STATS)) != 0;
     RAJNI_REQUIRE(!exact || N % 64 == 0, RAJNI_EINVAL, "rajni_gemm_bf16_ex: LN_FOLD / ROW_STATS need N %% 64 == 0 (N=%d)", N);
     // (a producer of 64-column statistics slots cannot use the 192-wide tile)
-    int bn = pick_bn(N, M, K, exact, (flags & RAJNI_EPI_ROW_STATS) && stat_shift_for(N) == 6,
-                     a->workspace != nullptr && (size_t)a->workspace_bytes >= sk_workspace_bytes(), (flags & RAJNI_HINT_STREAM_K) != 0);   // < 0: exact CTA-pair tile of width -bn
+    int bn = pick_bn(N, M, exact, (flags & RAJNI_EPI_ROW_STATS) && stat_shift_for(N) == 6);   // < 0: exact CTA-pair tile of width -bn
     auto s = static_cast<cudaStream_t>(stream);
     // wide problems run as CTA pairs (256 x 256 tiles); narrow ones keep single-CTA tiles
     static const bool force_cg1 = getenv("RAJNI_GEMM_CG1") != nullptr;     // debugging aid
     if (bn < 0 && force_cg1) bn = (-bn == 192) ? 64 : -bn;
     switch (bn) {
-        case -256: return launch_gemm<256, 2>(a->A, a->W, p, a->workspace, (size_t)a->workspace_bytes, s);
-        case -192: return launch_gemm<192, 2>(a->A, a->W, p, a->workspace, (size_t)a->workspace_bytes, s);
-        case -128: return launch_gemm<128, 2>(a->A, a->W, p, a->workspace, (size_t)a->workspace_bytes, s);
-        case 256: return (M > BM && !force_cg1) ? launch_gemm<256, 2>(a->A, a->W, p, a->workspace, (size_t)a->workspace_bytes, s) : launch_gemm<256, 1>(a->A, a->W, p, a->workspace, (size_t)a->workspace_bytes, s);
-        case 128: return launch_gemm<128, 1>(a->A, a->W, p, a->workspace, (size_t)a->workspace_bytes, s);
-        default: return launch_gemm<64, 1>(a->A, a->W, p, a->workspace, (size_t)a->workspace_bytes, s);
+        case -256: return launch_gemm<256, 2>(a->A, a->W, p, s);
+        case -192: return launch_gemm<192, 2>(a->A, a->W, p, s);
+        case -128: return launch_gemm<128, 2>(a->A, a->W, p, s);
+        case 256: return (M > BM && !force_cg1) ? launch_gemm<256, 2>(a->A, a->W, p, s) : launch_gemm<256, 1>(a->A, a->W, p, s);
+        case 128: return launch_gemm<128, 1>(a->A, a->W, p, s);
+        default: return launch_gemm<64, 1>(a->A, a->W, p, s);
     }
 }

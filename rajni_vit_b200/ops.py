@@ -10,7 +10,7 @@ import torch
 
 from . import _lib
 from ._lib import (EPI_BIAS, EPI_GELU, EPI_LN_FOLD, EPI_OUT_F32, EPI_RESIDUAL, EPI_ROW_STATS,  # noqa: F401  (re-exported)
-                   HINT_REVERSE_M, HINT_STREAM_K)
+                   HINT_REVERSE_M)
 
 _checked_devices = set()
 _prof = None        # list of (name, work, start_event, end_event) while profile_steps() runs
@@ -259,19 +259,16 @@ def gemm(a: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor], M: int,
          res_row_map: Optional[torch.Tensor] = None, out: Optional[torch.Tensor] = None,
          ldd: Optional[int] = None, out_row_map: Optional[torch.Tensor] = None, out_f32: bool = False,
          ln: Optional[tuple] = None, row_stats: Optional[torch.Tensor] = None, tag: str = "",
-         reverse: bool = False, workspace: Optional[torch.Tensor] = None, force_stream_k: bool = False) -> torch.Tensor:
+         reverse: bool = False) -> torch.Tensor:
     """out[orow(m), n] = epi(sum_k a[m,k] w[n,k]); a [M,K] bf16, w [N,K] bf16, bias fp32 [N].
 
     ``ln = (stats, slots, wsum, eps)``: LayerNorm folded in (a is the un-normalised x, w = W*gamma,
     bias = b + W beta, wsum[n] = sum_k w[n,k], stats fp32 [>=slots, rows, 2] partial sums of x's rows).
     ``row_stats`` fp32 [slots, rows, 2]: also emit the partial sums of the rows this GEMM stores.
-    ``reverse``: walk the M tiles last-to-first (L2 reuse hint; results identical).
-    ``workspace``: stream-K scratch from ``gemm_workspace(device)`` (optional): lets a long-K GEMM split the leftover tiles of
-    its last wave along K where the cost model expects a gain (``force_stream_k``: wherever it is possible).  Calls sharing
-    one workspace must be ordered on one stream."""
+    ``reverse``: walk the M tiles last-to-first (L2 reuse hint; results identical)."""
     flags = (EPI_BIAS if bias is not None else 0) | (EPI_GELU if gelu else 0) | \
             (EPI_RESIDUAL if residual is not None else 0) | (EPI_OUT_F32 if out_f32 else 0) | \
-            (HINT_REVERSE_M if reverse else 0) | (HINT_STREAM_K if force_stream_k else 0)
+            (HINT_REVERSE_M if reverse else 0)
     if out is None:
         out = torch.empty((M, N), device=a.device, dtype=torch.float32 if out_f32 else torch.bfloat16)
     args = _lib.GemmArgs(a.data_ptr(), w.data_ptr(), _ptr(bias), out.data_ptr(), M, N, K, flags,
@@ -285,29 +282,8 @@ def gemm(a: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor], M: int,
     if row_stats is not None:
         args.flags |= EPI_ROW_STATS
         args.row_stats, args.row_stats_ld = row_stats.data_ptr(), row_stats.shape[1]
-    if workspace is not None:
-        if workspace.device != a.device or workspace.dtype != torch.uint8:
-            raise ValueError("gemm: workspace must be a uint8 tensor on the operands' device (ops.gemm_workspace)")
-        args.workspace, args.workspace_bytes = workspace.data_ptr(), workspace.numel()
     _call("gemm:" + tag if tag else "gemm", 2.0 * M * N * K, _lib.load().rajni_gemm_bf16_ex, args, _stream(a))
     return out
-
-
-def gemm_workspace(device) -> torch.Tensor:
-    """Zero-initialised stream-K scratch for ``gemm(workspace=...)`` (rajni_gemm_workspace_bytes: ~38 MB on 148 SMs).
-    One per stream of GEMM calls; the kernels leave its counters zero, so it is reusable without clearing."""
-    with torch.cuda.device(device):
-        n = int(_lib.load().rajni_gemm_workspace_bytes())
-    return torch.zeros(n, device=device, dtype=torch.uint8)
-
-
-def stream_k_plan(M: int, N: int, K: int, flags: int):
-    """(tiles split along K, CTA pairs sharing them) for a GEMM of this shape given a workspace; (0, 0) = no stream-K.
-    Host-side query (rajni_gemm_stream_k_plan), no launch."""
-    import ctypes
-    sp = ctypes.c_int(0)
-    r = int(_lib.load().rajni_gemm_stream_k_plan(M, N, K, flags, ctypes.addressof(sp)))
-    return r, sp.value
 
 
 LONG_SEQ = 256          # above this many kept tokens the key-block kernel runs; it wants its rows compacted first

@@ -98,10 +98,6 @@ class RAJNIViTWrapper(nn.Module):
         self.avg_pool = False            # head on fc_norm(mean of the patch tokens) (global_pool='avg', MAE)
         self.headless = False            # head = Identity: forward returns the features the head would read (num_classes=0)
         self.input_norm: Optional[tuple] = None       # (mean[3], std[3]) for uint8 images, see set_input_normalization
-        # Stream-K tail of the fc2 GEMMs (gemm_tcgen05.cu): +1.4 % at 32 images per GPU, nothing at 64 and above.  OFF by default
-        # because the fp32 summation order of a split tile depends on the tile count, i.e. on the batch size: without it an
-        # image's logits are bit-identical whatever batch it is evaluated in (tests/test_gpu_e2e.py::test_full_batch_properties).
-        self.stream_k: bool = os.environ.get("RAJNI_STREAM_K", "0") == "1"
         self._validate()
 
     def set_input_normalization(self, mean, std) -> "RAJNIViTWrapper":
@@ -231,7 +227,7 @@ class RAJNIViTWrapper(nn.Module):
 
     # ------------------------------------------------------------------ workspace
     def _workspace(self, B: int, S: int, dev: torch.device):
-        key = (B, S, dev, self.stream_k)
+        key = (B, S, dev)
         ws = self._ws.get(key)
         if ws is not None:
             return ws
@@ -263,9 +259,6 @@ class RAJNIViTWrapper(nn.Module):
             stat_slots=ops.row_stats_slots(C),
             stats=torch.zeros((ops.row_stats_slots(C), B * N0, 2), device=dev, dtype=torch.float32),
             sel={},
-            # stream-K scratch of the long-K GEMMs (fc2), only when asked for: owned here like every other pointer a captured
-            # graph bakes in
-            gemm_ws=ops.gemm_workspace(dev) if self.stream_k else None,
             # scratch of the split score path (small batches, and sequences too long for the one-launch kernel at any batch):
             # owned here, so a captured graph's pointer lives with the graph.  Sized for N0, the longest sequence of the step.
             score_ws=(torch.empty(max(ops.score_workspace_bytes(B, N0, C, blk.attn.num_heads) for blk in self.blocks),
@@ -296,7 +289,7 @@ class RAJNIViTWrapper(nn.Module):
             return self._forward_eager(x)
         # what _forward_eager reads besides the input: the schedule of the pruned blocks (attention.py:25-32) ...
         sched = tuple((blk.attn.keep_ratio, blk.attn.update) if blk.has_pruner else None for blk in self.blocks)
-        key = (tuple(x.shape), x.dtype, x.device, self.training, sched, self.input_norm, self.stream_k)
+        key = (tuple(x.shape), x.dtype, x.device, self.training, sched, self.input_norm)
         # ... and the parameters.  Storage changes go through _apply / load_state_dict (which drop the graphs); in-place
         # updates bump the tensors' version counters, summed here over a parameter list that is built once.
         if self._param_list is None:
@@ -438,8 +431,7 @@ class RAJNIViTWrapper(nn.Module):
                 keep_log.append(None)
             ops.gemm(cur, f1w, f1b, M, hidden, C, gelu=True, out=ws["hid"], ldd=hidden,
                      ln=(stats, slots, f1sum, e2), tag="fc1", reverse=zig and not rev)                                    # model.py:59 (norm2 + fc1 + GELU)
-            ops.gemm(ws["hid"], f2w, f2b, M, C, hidden, residual=cur, ldres=C, out=cur, ldd=C, row_stats=stats, tag="fc2", reverse=rev,
-                     workspace=ws["gemm_ws"] if self.stream_k else None)
+            ops.gemm(ws["hid"], f2w, f2b, M, C, hidden, residual=cur, ldres=C, out=cur, ldd=C, row_stats=stats, tag="fc2", reverse=rev)
             rev = zig and not rev
 
         # ---- final norm on the CLS rows only (LayerNorm is row-wise) + head   model.py:65-66

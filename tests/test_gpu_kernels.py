@@ -256,66 +256,6 @@ def test_gemm_layernorm_folded(ops, M, C, N, gelu):
     assert not bad.any(), f"{int(bad.sum())} of {bad.numel()} elements out of tolerance; first at {bad.nonzero()[0].tolist()}"
 
 
-# Stream-K tail (gemm_tcgen05.cu): with a workspace, a long-K CTA-pair GEMM splits the leftover tiles of its last wave
-# along K over the pairs and reduces fp32 partials through scratch.  Shapes: tiles % 74 pairs = 1 (the 7.01-wave case of
-# 173-token blocks), 3, 26, 39 (of 74), fewer tiles than pairs (44: small shards), and vit_large's K = 4096.
-SK_CASES = [
-    # M, N, K, mode
-    (19200, 768, 3072, "res"),        # 75 x 3 = 225 tiles = 3 waves + 3
-    (22272, 768, 3072, "res"),        # 87 x 3 = 261 = 3 waves + 39
-    (2784, 1024, 4096, "res"),        # 11 x 4 = 44 tiles < 74 pairs
-    (6304, 768, 3072, "res"),         # 25 x 3 = 75 = 1 wave + 1
-    (6304, 1024, 4096, "res"),        # vit_large fc2: 25 x 4 = 100 = 1 wave + 26
-    (6304, 768, 3072, "bias"),
-    (2784, 1024, 4096, "gelu"),
-]
-
-
-@pytest.mark.parametrize("M,N,K,mode", SK_CASES)
-def test_gemm_stream_k_tail(ops, M, N, K, mode):
-    g = torch.Generator().manual_seed(M + N + K)
-    a = bf16_round(torch.randn(M, K, generator=g))
-    w = bf16_round(torch.randn(N, K, generator=g) / math.sqrt(K))
-    bias = torch.randn(N, generator=g)
-    A, W, Bv = dev(a, torch.bfloat16), dev(w, torch.bfloat16), dev(bias)
-    ref = A.float() @ W.float().t() + Bv
-    res = None
-    if mode == "gelu":
-        ref = torch.nn.functional.gelu(ref)
-    if mode == "res":
-        res = dev(bf16_round(torch.randn(M, N, generator=g)), torch.bfloat16)
-        ref = ref + res.float()
-    ws = ops.gemm_workspace("cuda")
-    slots = ops.row_stats_slots(N)
-    flags = ops.EPI_BIAS | (ops.EPI_GELU if mode == "gelu" else 0) | ((ops.EPI_RESIDUAL | ops.EPI_ROW_STATS) if mode == "res" else 0)
-    assert ops.stream_k_plan(M, N, K, flags | ops.HINT_STREAM_K)[0] > 0, "this shape is meant to take the stream-K path"
-
-    def run(workspace, in_place):
-        stats = torch.zeros((slots, M, 2), device="cuda") if mode == "res" else None
-        out = res.clone() if (in_place and res is not None) else torch.zeros((M, N), device="cuda", dtype=torch.bfloat16)
-        ops.gemm(A, W, Bv, M, N, K, gelu=mode == "gelu", residual=(out if in_place else res) if res is not None else None, ldres=N,
-                 out=out, ldd=N, row_stats=stats, workspace=workspace, force_stream_k=True)
-        torch.cuda.synchronize()
-        return out, stats
-
-    plain, plain_stats = run(None, False)
-    for rep in range(3):                                   # the counters re-arm themselves: the workspace is reusable as is
-        got, stats = run(ws, rep == 2)                     # (last repetition in place: residual aliases the output, like fc2)
-        report(f"stream-k gemm {M}x{N}x{K} {mode} rep {rep}", got.float(), ref)
-        bad = (got.float() - ref).abs() > BF16_RTOL * ref.abs() + 2e-3
-        assert not bad.any(), f"{int(bad.sum())} of {bad.numel()} elements out of tolerance; first at {bad.nonzero()[0].tolist()}"
-        assert int(ws[:4096].count_nonzero()) == 0, "stream-K counters were not re-armed"
-        # against the unsplit kernel: same products, fp32 sums in a different order -> at most one bf16 rounding step apart
-        assert ((got.float() - plain.float()).abs() <= 2.0 ** -7 * plain.float().abs() + 1e-3).all()
-        if stats is not None:
-            torch.testing.assert_close(stats.sum(dim=0)[:, 0].double(), got.double().sum(dim=1), rtol=1e-5, atol=1e-3)
-            torch.testing.assert_close(stats.sum(dim=0)[:, 1].double(), (got.double() ** 2).sum(dim=1), rtol=1e-5, atol=1e-3)
-    # deterministic: the pieces of a tile are summed in a fixed order
-    again, _ = run(ws, False)
-    got2, _ = run(ws, False)
-    assert torch.equal(again, got2)
-
-
 @pytest.mark.parametrize("ratio", [0.0, 10.0, 50.0, 100.0])
 def test_layernorm_fold_statistics_at_large_mean(ops, ratio):
     """The folded LayerNorm takes the variance as E[x^2] - mean^2 from fp32 partial sums (gemm_tcgen05.cu epilogue).

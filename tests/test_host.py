@@ -102,24 +102,24 @@ def test_library_exports_every_declared_symbol():
     assert sorted(_lib.SIGNATURES) == names
 
 
-# ABI 11: one entry point per operation.  A name removed from this list must not come back with another signature: a
-# caller that binds by name would misbind silently.
+# One entry point per operation (ABI 11); ABI 12 dropped the GEMM's split-K workspace calls.  A name removed from this list
+# must not come back with another signature: a caller that binds by name would misbind silently.
 C_ABI = sorted("rajni_" + n for n in (
     "abi_version", "last_error", "device_check", "launch_count",
     "select_prefix", "score_select_prefix", "score_select_workspace_bytes", "score_select_needs_workspace",
     "gather_rows",
     "layernorm_strided", "layernorm_strided_f32", "layernorm_row_stats",
     "mean_pool_layernorm", "mean_pool_layernorm_f32",
-    "gemm_bf16_ex", "gemm_workspace_bytes", "gemm_stream_k_plan", "gemm_row_stats_slots",
+    "gemm_bf16_ex", "gemm_row_stats_slots",
     "attention_fwd_ex",
     "patch_im2col_prefix",
     "resize_workspace_bytes", "resize_center_crop_u8", "resize_status"))
 
 
-def test_c_abi_is_exactly_the_documented_surface():
-    """The header declares exactly these 23 functions (so no superseded sibling is left), the ctypes loader binds exactly
-    these, the library exports each, INTEGRATION.md documents each, and both sides report ABI 11."""
-    assert len(C_ABI) == 23
+def test_c_abi_12_is_exactly_the_documented_surface():
+    """The header declares exactly these 21 functions (so no superseded sibling is left), the ctypes loader binds exactly
+    these, the library exports each, INTEGRATION.md documents each, and both sides report ABI 12."""
+    assert len(C_ABI) == 21
     assert _declared_symbols() == C_ABI
     assert sorted(_lib.SIGNATURES) == C_ABI
     lib = ctypes.CDLL(_lib.LIB_PATH)
@@ -127,8 +127,8 @@ def test_c_abi_is_exactly_the_documented_surface():
     for n in C_ABI:
         assert hasattr(lib, n), f"{n} is not exported by {_lib.LIB_PATH}"
         assert f"`{n}`" in integ, f"{n} is not documented in INTEGRATION.md"
-    assert _lib.ABI_VERSION == 11
-    assert _lib.load().rajni_abi_version() == 11
+    assert _lib.ABI_VERSION == 12
+    assert _lib.load().rajni_abi_version() == 12
 
 
 def test_library_abi_version_and_error_string():
@@ -361,42 +361,3 @@ def test_greedy_search_respects_the_floor_and_prefers_cheap_accuracy():
     sched0, hist0 = S.greedy_search(fake, depth, floor=90.0, blocks=[1, 4])
     assert sched0 == {} and len(hist0) == 1
 
-
-def test_gemm_stream_k_planner_host_logic():
-    """rajni_gemm_stream_k_plan is pure host code (no launch): which GEMM shapes split the leftover tiles of their last wave
-    along K, over how many CTA pairs (gemm_tcgen05.cu: sk_decide).  Also restates the kernel's unit -> pair arithmetic
-    (sk_bound / sk_pair_of / sk_plan) and checks that the pieces tile every k-block of every split tile exactly once."""
-    lib = _lib.load()
-    sp = ctypes.c_int(0)
-    res = _lib.EPI_BIAS | _lib.EPI_RESIDUAL | _lib.EPI_ROW_STATS
-
-    def plan(M, N, K, flags):
-        return int(lib.rajni_gemm_stream_k_plan(M, N, K, flags, ctypes.addressof(sp))), sp.value
-
-    pairs = 74 if not torch.cuda.is_available() else torch.cuda.get_device_properties(0).multi_processor_count // 2
-    if pairs == 74:
-        assert plan(6304, 768, 3072, res) == (1, 6)                # the 32-image shard: 75 tiles = one wave + 1
-        assert plan(44288, 768, 3072, res) == (0, 0)               # long call: an idle tail is cheap under the power cap
-        assert plan(44288, 768, 3072, res | _lib.HINT_STREAM_K) == (1, 6)
-        assert plan(50432, 768, 3072, res | _lib.HINT_STREAM_K) == (0, 0)     # 591 tiles = 7.99 waves, 73 left over: nothing to gain
-    assert plan(6304, 768, 768, res | _lib.HINT_STREAM_K) == (0, 0)            # K too short for a fix-up to pay
-    assert plan(100, 768, 3072, res | _lib.HINT_STREAM_K) == (0, 0)            # a single row block: no CTA-pair tiles
-    assert plan(6304, 1000, 3072, _lib.EPI_BIAS | _lib.HINT_STREAM_K) == (0, 0)   # column tail: generic epilogue, never split
-
-    # the kernel's partition of R * KB k-block units over `sp` pairs
-    for R, KB, n_sp in [(1, 48, 6), (39, 48, 74), (26, 64, 74), (3, 48, 18), (12, 48, 72), (44, 64, 74)]:
-        U = R * KB
-        bound = lambda j: (j * U) // n_sp                                             # noqa: E731  sk_bound
-        pair_of = lambda u: ((u + 1) * n_sp + U - 1) // U - 1                          # noqa: E731  sk_pair_of
-        cover = [0] * U
-        for j in range(n_sp):
-            b0, b1 = bound(j), bound(j + 1)
-            assert 0 < b1 - b0 < KB                                                    # a piece is never a whole tile
-            t0, t1 = b0 // KB, (b1 - 1) // KB
-            assert t1 - t0 <= 1                                                        # pieces of at most two tiles
-            pieces = [(t0, b0 - t0 * KB, min(b1 - t0 * KB, KB))] + ([(t1, 0, b1 - t1 * KB)] if t1 > t0 else [])
-            for t, k0, k1 in pieces:
-                for k in range(k0, k1):
-                    cover[t * KB + k] += 1
-            assert all(pair_of(u) == j for u in range(b0, b1))
-        assert cover == [1] * U
