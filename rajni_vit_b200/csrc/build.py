@@ -1,4 +1,5 @@
-"""Build librajni_b200.so in-tree with nvcc for sm_100a (cross-compiles without a GPU)."""
+"""Build librajni_b200.so (the model) and librajni_jpeg.so (the GPU JPEG decoder) in-tree with nvcc for sm_100a
+(cross-compiles without a GPU).  runtime.cu (error string, launch plumbing) is linked into both."""
 from __future__ import annotations
 
 import os
@@ -9,8 +10,14 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 LIB = os.path.join(HERE, "librajni_b200.so")
-SOURCES = ["capi.cu", "score_select.cu", "rowops.cu", "resize.cu", "gemm_tcgen05.cu", "attention.cu", "attention_pipe.cu", "attention_tc.cu", "attention_long.cu"]
-HEADERS = ["common.cuh", os.path.join(ROOT, "include", "rajni_b200.h")]
+JPEG_LIB = os.path.join(HERE, "librajni_jpeg.so")
+LIBS = {
+    LIB: ["runtime.cu", "capi.cu", "score_select.cu", "rowops.cu", "resize.cu", "gemm_tcgen05.cu", "attention.cu",
+          "attention_pipe.cu", "attention_tc.cu", "attention_long.cu"],
+    JPEG_LIB: ["runtime.cu", "jpeg.cu"],
+}
+SOURCES = list(dict.fromkeys(s for srcs in LIBS.values() for s in srcs))
+HEADERS = ["common.cuh", os.path.join(ROOT, "include", "rajni_b200.h"), os.path.join(ROOT, "include", "rajni_jpeg.h")]
 NVCC_FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]
 
@@ -18,10 +25,6 @@ NVCC_FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a",
 def _nvcc() -> str:
     cand = os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", "nvcc")
     return cand if os.path.exists(cand) else "nvcc"
-
-
-def _sources():
-    return [s for s in SOURCES if os.path.exists(os.path.join(HERE, s))]
 
 
 def _stale(target: str, deps) -> bool:
@@ -33,12 +36,10 @@ def _stale(target: str, deps) -> bool:
 
 def build(force: bool = False, verbose: bool = False) -> str:
     hdrs = [h if os.path.isabs(h) else os.path.join(HERE, h) for h in HEADERS]
-    objs = []
     jobs = []
-    for src in _sources():
+    for src in SOURCES:
         s = os.path.join(HERE, src)
         o = os.path.join(HERE, src[:-3] + ".o")
-        objs.append(o)
         if force or _stale(o, [s] + hdrs):
             cmd = [_nvcc(), *NVCC_FLAGS, "-c", s, "-o", o]
             if verbose:
@@ -55,8 +56,10 @@ def build(force: bool = False, verbose: bool = False) -> str:
         for out in ex.map(run, jobs):
             if verbose and out:
                 print(out, file=sys.stderr)
-    if force or jobs or _stale(LIB, objs):
-        run([_nvcc(), "-shared", "-o", LIB, *objs, "-gencode", "arch=compute_100a,code=sm_100a"])
+    for lib, srcs in LIBS.items():
+        objs = [os.path.join(HERE, src[:-3] + ".o") for src in srcs]
+        if force or jobs or _stale(lib, objs):
+            run([_nvcc(), "-shared", "-o", lib, *objs, "-gencode", "arch=compute_100a,code=sm_100a"])
     return LIB
 
 

@@ -1,52 +1,11 @@
-// Error string, launch counter and device check behind the C ABI.
-#include <atomic>
-#include <cstdarg>
-#include <cstdio>
-#include <cstdlib>
-
+// The C ABI's version, error string, launch counter and device check.
 #include "common.cuh"
-
-namespace rajni {
-
-static thread_local char g_error[512] = "";
-static std::atomic<uint64_t> g_launches{0};
-
-void set_error(const char* fmt, ...) {
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(g_error, sizeof(g_error), fmt, ap);
-    va_end(ap);
-}
-
-bool pdl_enabled() {
-    static const bool on = getenv("RAJNI_NO_PDL") == nullptr;
-    return on;
-}
-
-int current_device() {
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= kMaxDevices) dev = 0;
-    return dev;
-}
-
-void count_launch(int n) { g_launches.fetch_add((uint64_t)n, std::memory_order_relaxed); }
-
-int check_launch(const char* what) {
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) {
-        set_error("%s: launch failed: %s", what, cudaGetErrorString(e));
-        return RAJNI_ECUDA;
-    }
-    return RAJNI_OK;
-}
-
-}  // namespace rajni
 
 extern "C" int rajni_abi_version(void) { return RAJNI_ABI_VERSION; }
 
-extern "C" const char* rajni_last_error(void) { return rajni::g_error; }
+extern "C" const char* rajni_last_error(void) { return rajni::error_text(); }
 
-extern "C" uint64_t rajni_launch_count(void) { return rajni::g_launches.load(std::memory_order_relaxed); }
+extern "C" uint64_t rajni_launch_count(void) { return rajni::launches(); }
 
 extern "C" int rajni_device_check(void) {
     int dev = 0;

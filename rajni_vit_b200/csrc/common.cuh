@@ -14,8 +14,10 @@
 
 namespace rajni {
 
-// ------------------------------------------------------------------ host-side errors
+// ------------------------------------------------------------------ host-side errors (runtime.cu)
 void set_error(const char* fmt, ...);
+const char* error_text();             // the calling thread's last message
+uint64_t launches();
 void count_launch(int n = 1);
 int check_launch(const char* what);   // cudaGetLastError -> RAJNI_ECUDA
 
@@ -35,8 +37,8 @@ int check_launch(const char* what);   // cudaGetLastError -> RAJNI_ECUDA
 __device__ __forceinline__ void griddep_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void griddep_launch() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 
-bool pdl_enabled();      // capi.cu: false when RAJNI_NO_PDL is set
-int current_device();    // capi.cu: cudaGetDevice, 0 on error (indexes the per-device one-time flags below)
+bool pdl_enabled();      // runtime.cu: false when RAJNI_NO_PDL is set
+int current_device();    // runtime.cu: cudaGetDevice, 0 on error (indexes the per-device one-time flags below)
 constexpr int kMaxDevices = 64;
 
 template <typename... KArgs, typename... Args>

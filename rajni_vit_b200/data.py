@@ -107,3 +107,45 @@ class GpuPreprocessLoader:
     def __iter__(self):
         for frames, labels in self.loader:
             yield gpu_resize_center_crop(frames, self.device, self.size, self.crop), labels
+
+
+# ------------------------------------------------------------------ GPU JPEG decode (csrc/jpeg.cu) in front of the above
+def read_for_gpu_decode(path: str):
+    """``ImageFolder`` loader for ``GpuDecodeLoader``: a ``jpeg.JpegFile`` (bytes + parsed headers) when the GPU decoder
+    takes the file (host-only header parse), else the frame Pillow decodes (uint8 [H,W,3]) - progressive, CMYK, PNG named
+    .JPEG, images above Pillow's pixel limit and the like."""
+    from . import jpeg
+    with open(path, "rb") as f:
+        return jpeg.read_file(f.read())
+
+
+# The GPU decodes images one sequential decoder per image, so its throughput grows with the images in one launch: the
+# loader's batches are decoded in groups of at least this many images (2048 decoders fill a B200's 148 SMs ~14 deep).
+DECODE_GROUP_IMAGES = 2048
+
+
+class GpuDecodeLoader(GpuPreprocessLoader):
+    """``GpuPreprocessLoader`` for a loader whose items come from ``read_for_gpu_decode`` (+ ``collate_frames``): the JPEG
+    decode runs on ``device`` too (``jpeg.decode_batch``, several loader batches per launch, see DECODE_GROUP_IMAGES),
+    so the CPU workers only read files and parse headers.  Same ``(uint8 [B,3,crop,crop] CUDA tensor, labels)`` batches,
+    bit for bit."""
+
+    def __iter__(self):
+        from . import jpeg, ops
+        group, n = [], 0
+        it = iter(self.loader)
+        while True:
+            batch = next(it, None)
+            if batch is not None:
+                group.append(batch)
+                n += len(batch[0])
+            if group and (batch is None or n >= DECODE_GROUP_IMAGES):
+                frames, meta, max_h = jpeg.decode_batch([x for items, _ in group for x in items], self.device)
+                start = 0
+                for items, labels in group:
+                    yield ops.resize_center_crop(frames, meta[start:start + len(items)], max_h, size=self.size,
+                                                 crop=self.crop), labels
+                    start += len(items)
+                group, n = [], 0
+            if batch is None:
+                return

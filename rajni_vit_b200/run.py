@@ -14,6 +14,8 @@ Differences from the reference CLI, all deliberate (SURVEY.md section 5):
   * ``--uint8_input`` ships uint8 crops and normalises inside the patch kernel (extension; same logits, 4x fewer H2D bytes);
   * ``--gpu_preprocess`` leaves only the JPEG decode to the CPU workers: Resize(256, bicubic) + CenterCrop(224) run in
     ``csrc/resize.cu`` (bit-identical to torchvision on PIL images), ToTensor + Normalize in the patch kernel;
+  * ``--gpu_decode`` (implies ``--gpu_preprocess``) moves the JPEG decode to the GPU as well (``csrc/jpeg.cu``, frames
+    equal to Pillow's); the workers read files and decode on the CPU only what the GPU decoder does not take;
   * ``--ckpt file`` loads timm-named weights from a .safetensors / .pt file (no hub access needed);
   * under torchrun every rank decodes only its shard of each batch (``data.sharded_loader``);
   * without ``timm`` (not installable here) the stand-in ViT with random weights is used and the fact is printed;
@@ -52,9 +54,14 @@ def get_args(argv=None):
     ap.add_argument("--gpu_preprocess", action="store_true",
                     help="workers only decode; Resize(256, bicubic) + CenterCrop(224) + ToTensor + Normalize run on the GPU "
                          "(bit-identical to the torchvision pipeline; implies --uint8_input)")
+    ap.add_argument("--gpu_decode", action="store_true",
+                    help="decode baseline JPEGs on the GPU too (frames equal to Pillow's; other files are decoded by the "
+                         "workers); implies --gpu_preprocess")
     ap.add_argument("--uint8_input", action="store_true",
                     help="ship uint8 crops to the GPU and normalise inside the patch kernel (4x fewer H2D bytes; same logits)")
     args = ap.parse_args(argv)
+    if args.gpu_decode:
+        args.gpu_preprocess = True
     if args.gpu_preprocess:
         args.uint8_input = True
     if not args.data_path and args.synthetic <= 0:
@@ -90,12 +97,15 @@ def build_loader(args, image_size: int, rank: int = 0, world: int = 1):
     if args.gpu_preprocess:
         if image_size != 224:
             raise ValueError("--gpu_preprocess: the GPU resize kernel crops to 224 x 224")
-        from .data import GpuPreprocessLoader, collate_frames, decode_only, sharded_loader
-        ds = datasets.ImageFolder(args.data_path, decode_only)
+        from .data import (GpuDecodeLoader, GpuPreprocessLoader, collate_frames, decode_only, read_for_gpu_decode,
+                           sharded_loader)
+        ds = (datasets.ImageFolder(args.data_path, loader=read_for_gpu_decode) if args.gpu_decode else
+              datasets.ImageFolder(args.data_path, decode_only))
         kw = dict(num_workers=args.num_workers, pin_memory=False, collate_fn=collate_frames)
         inner = (sharded_loader(ds, args.batch_size, rank, world, **kw) if world > 1 else
                  torch.utils.data.DataLoader(ds, batch_size=args.batch_size, shuffle=False, drop_last=False, **kw))
-        return GpuPreprocessLoader(inner, torch.device(args.device if world == 1 else f"cuda:{torch.cuda.current_device()}"))
+        wrap = GpuDecodeLoader if args.gpu_decode else GpuPreprocessLoader
+        return wrap(inner, torch.device(args.device if world == 1 else f"cuda:{torch.cuda.current_device()}"))
     tail = [T.PILToTensor()] if args.uint8_input else [T.ToTensor(), T.Normalize(mean=IMAGENET_MEAN, std=IMAGENET_STD)]
     tf = T.Compose([T.Resize(int(image_size * 256 / 224), interpolation=T.InterpolationMode.BICUBIC), T.CenterCrop(image_size), *tail])
     ds = datasets.ImageFolder(args.data_path, tf)
