@@ -1,7 +1,7 @@
 """RAJNIAttention — drop-in for rajni/wrapper/attention.py:5-60 on sm_100a kernels."""
 from __future__ import annotations
 
-from typing import Optional
+from typing import Optional, Sequence
 
 import torch
 import torch.nn as nn
@@ -15,6 +15,30 @@ def keep_count(num_tokens: int, keep_ratio: float, prefix: int = 1) -> int:
     (rajni/wrapper/attention.py:31-32).  ``prefix``: the leading tokens that are always kept (1: CLS; 2: CLS and the
     distillation token of a distilled DeiT)."""
     return max(1, int(keep_ratio * (num_tokens - prefix)))
+
+
+def token_maps(keep_log: Sequence[Optional[torch.Tensor]], batch: int, num_tokens: int, device=None):
+    """Where each original token's latest row is after the blocks of ``keep_log``, and how many blocks it went through.
+
+    ``keep_log``: one entry per block run, None for a dense block and, for a pruned block, its ``keep_idx`` [B, N_{s+1}]
+    (the rows of the previous stage it keeps).  Stage s (the tokens between two pruned blocks, N_0 = ``num_tokens``) holds
+    its rows [B, N_s] at rows B·(N_0 + … + N_{s-1}) + b·N_s + j of one allocation.  A token dropped by pruned block k
+    keeps its row in the last stage that held it, at depth k; the tokens of the last stage are at depth len(keep_log).
+    -> (rows int32 [B, N0], depth int32 [B, N0]), indexed by original position (prefix tokens first, then the patches).
+    Torch index ops only (no host sync), so a CUDA graph can capture it."""
+    B, dev = batch, device
+    keeps = [(i, k) for i, k in enumerate(keep_log) if k is not None]
+    pos = torch.arange(num_tokens, device=dev).expand(B, num_tokens)        # original position of each stage row
+    rows = torch.empty((B, num_tokens), device=dev, dtype=torch.int32)
+    depth = torch.empty_like(rows)
+    base, n = 0, num_tokens
+    for end, keep in keeps + [(len(keep_log), None)]:
+        rows.scatter_(1, pos, torch.arange(base, base + B * n, device=dev, dtype=torch.int32).view(B, n))
+        depth.scatter_(1, pos, torch.full((B, n), end, device=dev, dtype=torch.int32))
+        if keep is not None:
+            pos = torch.gather(pos, 1, keep.long())
+            base, n = base + B * n, keep.shape[1]
+    return rows, depth
 
 
 class RAJNIAttention(nn.Module):

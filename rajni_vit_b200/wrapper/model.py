@@ -21,6 +21,11 @@ fc_norm, in one kernel) and a pre-norm stem (``norm_pre``, CLIP fine-tunes: one 
 that also writes block 0's LayerNorm statistics), with or without a patch-embedding bias.  A headless model (``head`` =
 Identity, timm's ``num_classes=0``: DINO and other backbones) returns its pooled, normalised features [B, C], stored in fp32
 by the final LayerNorm or pooling kernel itself.
+
+Token-level features as timm serves them to dense heads: ``forward_features`` ([B, N0, C], every token through the final
+norm) and ``forward_intermediates`` (the token map after chosen blocks).  A token pruned at block k keeps the row it had
+after block k-1, at its original position: each stage of the schedule gets its own rows, so no row is overwritten after
+the stage's last block, and one row gather puts them back in order (``token_maps``).
 """
 from __future__ import annotations
 
@@ -32,7 +37,35 @@ import torch.nn as nn
 
 from .. import ops
 from ..packing import PackCache
-from .attention import RAJNIAttention, keep_count
+from .attention import RAJNIAttention, keep_count, token_maps
+
+
+def feature_take_indices(num_blocks: int, indices=None) -> tuple:
+    """timm's ``feature_take_indices``: None -> every block, an int n -> the last n blocks, a sequence -> those blocks
+    (negative indices count from the end).  -> the block indices in ascending order, each once (the order in which
+    ``forward_intermediates`` returns the maps)."""
+    if indices is None:
+        indices = num_blocks
+    if isinstance(indices, int):
+        if not 0 < indices <= num_blocks:
+            raise ValueError(f"last-n ({indices}) is out of range (1 to {num_blocks})")
+        return tuple(range(num_blocks - indices, num_blocks))
+    take = set()
+    for i in indices:
+        idx = num_blocks + int(i) if int(i) < 0 else int(i)
+        if not 0 <= idx < num_blocks:
+            raise ValueError(f"feature index {idx} is out of range (0 to {num_blocks - 1})")
+        take.add(idx)
+    if not take:
+        raise ValueError("indices is empty")
+    return tuple(sorted(take))
+
+
+def _clone(y):
+    """A graph replay's outputs (a tensor, None, or tuples / lists of them) copied out of the graph's memory."""
+    if isinstance(y, (tuple, list)):
+        return type(y)(_clone(t) for t in y)
+    return None if y is None else y.clone()
 
 
 def _normalise_schedule(schedule: Dict) -> Dict[int, Dict]:
@@ -85,6 +118,7 @@ class RAJNIViTWrapper(nn.Module):
 
         self._last_stats = None
         self._last_keep_idx: List[Optional[torch.Tensor]] = []
+        self._last_token_depth: Optional[torch.Tensor] = None
         self._packs = PackCache()
         self._ws = {}
         self._graphs = {}
@@ -279,41 +313,103 @@ class RAJNIViTWrapper(nn.Module):
         ``AUTO_GRAPH_MAX_ROWS`` token rows, True / False force it (RAJNI_CUDA_GRAPH=1 / 0 in the environment do the same).
         A captured graph is dropped when any parameter changes (storage or version), on ``.to()`` / ``.bfloat16()`` /
         ``load_state_dict`` and when the input normalisation changes; results are bit-identical to the eager sequence."""
+        return self._run(x, ("forward",))
+
+    @torch.no_grad()
+    def forward_features(self, x: torch.Tensor) -> torch.Tensor:
+        """timm's ``forward_features``: every token after the last block through the final ``norm`` -> [B, N0, C], N0 the
+        un-pruned token count (prefix tokens first, then the patches in raster order).
+
+        A pruned token keeps the features it had when it was dropped: its row is its output of the last block that kept
+        it, normalised like the others, at its original position (``get_last_token_depth`` tells how many blocks each token
+        went through).  ``norm`` is a LayerNorm computed in fp32 (as a headless model's output), or Identity for an
+        average-pooled model, whose rows come out un-normalised and without ``fc_norm``, as in timm.  fp32 for fp32 or uint8
+        input, otherwise the input's dtype.  Every row is one the blocks of ``forward`` computed, bit for bit; the launches
+        are those of ``forward`` with the final LayerNorm and head replaced by one row gather and one LayerNorm over all
+        B·N0 rows.  CUDA graphs as in ``forward``, with a graph of its own."""
+        return self._run(x, ("forward_features", (), False, len(self.blocks), True))[0]
+
+    @torch.no_grad()
+    def forward_intermediates(self, x: torch.Tensor, indices=None, return_prefix_tokens: bool = False, norm: bool = False,
+                              stop_early: bool = False, output_fmt: str = "NCHW", intermediates_only: bool = False):
+        """timm's ``forward_intermediates``: the token map after each block of ``indices`` (an int n: the last n blocks; a
+        sequence of block indices, negative ones counted from the end; None: every block), in block order.
+
+        Each map follows the rule of ``forward_features`` at that depth: a token pruned earlier keeps the row it had when
+        it was dropped.  ``norm=True`` applies the final norm (fp32 LayerNorm, Identity for an average-pooled model).  As in
+        timm the prefix tokens are split off: 'NLC' gives [B, P, C] rows of the patches, 'NCHW' the patch grid [B, C, G, G]
+        -- a permuted view of [B, G, G, C] rows, not a contiguous tensor.  ``return_prefix_tokens`` pairs each map with its
+        prefix rows [B, prefix, C].  ``stop_early`` runs no block after the last one requested.  Returns the list of maps,
+        or (final features, maps) unless ``intermediates_only``; the final features are ``forward_features(x)`` (at the
+        depth reached, with ``stop_early``).  dtype as in ``forward_features``; each map costs one row gather, plus one
+        LayerNorm with ``norm=True``."""
+        if output_fmt not in ("NCHW", "NLC"):
+            raise ValueError(f"output_fmt={output_fmt!r}: 'NCHW' or 'NLC'")
+        take = feature_take_indices(len(self.blocks), indices)
+        depth = take[-1] + 1 if stop_early else len(self.blocks)
+        final, maps, _ = self._run(x, ("forward_intermediates", take, bool(norm), depth, not intermediates_only))
+        P0, B, G = self.prefix, x.shape[0], x.shape[2] // self.patch
+        prefix = [y[:, :P0] for y in maps]
+        maps = [y[:, P0:] for y in maps]
+        if output_fmt == "NCHW":
+            maps = [y.view(B, G, G, y.shape[-1]).permute(0, 3, 1, 2) for y in maps]
+        if return_prefix_tokens:
+            maps = list(zip(maps, prefix))
+        return maps if intermediates_only else (final, maps)
+
+    def get_last_token_depth(self) -> Optional[torch.Tensor]:
+        """int32 [B, N0]: how many blocks each token went through in the last ``forward_features`` /
+        ``forward_intermediates`` call (the model's depth, or the depth reached with ``stop_early``, for prefix tokens and
+        the tokens kept to the end).  None before the first such call."""
+        return self._last_token_depth
+
+    def _run(self, x: torch.Tensor, spec: tuple):
+        """``_forward_eager(x, spec)``, or the replay of a CUDA graph captured for this input shape and ``spec`` (see
+        ``forward``).  One graph per method stays resident, so that alternating methods do not recapture."""
         if x.device.type == "cuda" and x.device.index is not None and x.device.index != torch.cuda.current_device():
             with torch.cuda.device(x.device):          # the C ABI launches on the current device
-                return self.forward(x)
+                return self._run(x, spec)
         use = self.use_cuda_graph
         if use is None and x.dim() == 4:
             use = x.shape[0] * ((x.shape[2] // self.patch) * (x.shape[3] // self.patch) + self.prefix) <= AUTO_GRAPH_MAX_ROWS
         if not use or x.device.type != "cuda" or x.dim() != 4 or ops._prof is not None:      # (the per-kernel profiler times eager launches)
-            return self._forward_eager(x)
-        # what _forward_eager reads besides the input: the schedule of the pruned blocks (attention.py:25-32) ...
-        sched = tuple((blk.attn.keep_ratio, blk.attn.update) if blk.has_pruner else None for blk in self.blocks)
-        key = (tuple(x.shape), x.dtype, x.device, self.training, sched, self.input_norm)
-        # ... and the parameters.  Storage changes go through _apply / load_state_dict (which drop the graphs); in-place
-        # updates bump the tensors' version counters, summed here over a parameter list that is built once.
-        if self._param_list is None:
-            self._param_list = list(self.parameters())
-        wsig = sum(q._version for q in self._param_list)
-        entry = self._graphs.get(key)
-        if entry is None or entry[5] != wsig:
-            x_static = x.clone()
-            self._forward_eager(x_static)                       # builds packs and workspace, warms every kernel
-            torch.cuda.synchronize(x.device)
-            graph = torch.cuda.CUDAGraph()
-            # thread-local capture mode: a DataLoader's pin-memory thread may call into CUDA while this thread captures
-            with torch.cuda.graph(graph, capture_error_mode="thread_local"):
-                y_static = self._forward_eager(x_static)
-            entry = (graph, x_static, y_static, self._last_stats, self._last_keep_idx, wsig)
-            self._graphs = {key: entry}                         # one shape resident, like the workspace
-        graph, x_static, y_static, stats, keep, _ = entry
-        x_static.copy_(x)
-        graph.replay()
-        self._last_stats, self._last_keep_idx = stats, keep
-        return y_static.clone()
+            out = self._forward_eager(x, spec)
+        else:
+            # what _forward_eager reads besides the input: the schedule of the pruned blocks (attention.py:25-32) ...
+            sched = tuple((blk.attn.keep_ratio, blk.attn.update) if blk.has_pruner else None for blk in self.blocks)
+            key = (tuple(x.shape), x.dtype, x.device, self.training, sched, self.input_norm, spec)
+            # ... and the parameters.  Storage changes go through _apply / load_state_dict (which drop the graphs); in-place
+            # updates bump the tensors' version counters, summed here over a parameter list that is built once.
+            if self._param_list is None:
+                self._param_list = list(self.parameters())
+            wsig = sum(q._version for q in self._param_list)
+            entry = self._graphs.get(key)
+            if entry is None or entry[5] != wsig:
+                x_static = x.clone()
+                self._forward_eager(x_static, spec)             # builds packs and workspace, warms every kernel
+                torch.cuda.synchronize(x.device)
+                graph = torch.cuda.CUDAGraph()
+                # thread-local capture mode: a DataLoader's pin-memory thread may call into CUDA while this thread captures
+                with torch.cuda.graph(graph, capture_error_mode="thread_local"):
+                    y_static = self._forward_eager(x_static, spec)
+                entry = (graph, x_static, y_static, self._last_stats, self._last_keep_idx, wsig)
+                # one input shape resident, like the workspace, and one graph per method
+                self._graphs = {k: v for k, v in self._graphs.items() if k[:-1] == key[:-1] and k[-1][0] != spec[0]}
+                self._graphs[key] = entry
+            graph, x_static, y_static, stats, keep, _ = entry
+            x_static.copy_(x)
+            graph.replay()
+            self._last_stats, self._last_keep_idx = stats, keep
+            out = _clone(y_static)
+        if spec[0] != "forward":
+            self._last_token_depth = out[2]
+        return out
 
     @torch.no_grad()
-    def _forward_eager(self, x: torch.Tensor) -> torch.Tensor:
+    def _forward_eager(self, x: torch.Tensor, spec: tuple = ("forward",)):
+        """One pass of the launch sequence.  ``spec`` = ("forward",): -> logits (or pooled features).  Otherwise
+        (method, take, norm, depth, final): run ``depth`` blocks with every stage in a region of its own and return
+        (final token features or None unless ``final``, [token map after each block of ``take``], depth map)."""
         if x.dim() != 4 or x.shape[1] != 3 or x.shape[2] != x.shape[3] or x.shape[2] % self.patch:
             raise ValueError(f"expected images [B,3,S,S] with S a multiple of the patch size {self.patch}, got {tuple(x.shape)}")
         if x.device.type != "cuda":
@@ -337,7 +433,8 @@ class RAJNIViTWrapper(nn.Module):
         x = x.contiguous()
         B, _, S, _ = x.shape
         ws = self._workspace(B, S, x.device)
-        P, N, C = ws["P"], ws["N0"], ws["C"]
+        P, N0, C = ws["P"], ws["N0"], ws["C"]
+        N = N0                          # tokens entering the current block
         pk = self._packs
 
         # ---- patch + CLS + pos (model.py:31-37): im2col, then one GEMM whose epilogue adds
@@ -361,7 +458,16 @@ class RAJNIViTWrapper(nn.Module):
             return pos_, rows, sums if P0 > 1 else sums[0], sqs if P0 > 1 else sqs[0]
 
         pos, prefix_rows, pre_sum, pre_sumsq = pk.tensors(("pos", P), (m.pos_embed, m.cls_token, dist), _pos_pack)
-        cur, nxt = ws["xa"], ws["xb"]
+        features = spec[0] != "forward"
+        if features:
+            # every stage in a region of its own: a pruned block's proj writes the next stage, dense blocks stay in place,
+            # so the rows of a dropped token are still there at the end
+            _, take, take_norm, depth, final = spec
+            feat, regions = self._stage_regions(ws, B, x.device)
+            cur, nxt, maps = regions[0], None, []
+        else:
+            depth = len(self.blocks)
+            cur, nxt = ws["xa"], ws["xb"]
         stats, slots = ws["stats"], ws["stat_slots"]
         kpe = ws["cols"].shape[1]                                                   # 3 p^2
         ops.patch_im2col(x, self.patch, ws["cols"], prefix_rows, cur, C, row_stats=stats, stats_slots=slots,
@@ -381,6 +487,8 @@ class RAJNIViTWrapper(nn.Module):
         token_counts = []
         keep_log: List[Optional[torch.Tensor]] = []
         for i, blk in enumerate(self.blocks):
+            if i == depth:
+                break
             token_counts.append(N)                                                   # model.py:43
             H = blk.attn.num_heads
             # norm1 / norm2 are folded into the qkv / fc1 GEMMs: x itself is the A operand, the row statistics
@@ -416,6 +524,8 @@ class RAJNIViTWrapper(nn.Module):
                     ws["qkvc"] = torch.empty((B * ws["N0"], 3 * C), device=x.device, dtype=torch.bfloat16)
                 ops.attention(ws["qkv"], row_map, B, N, Np, C, H, float(attn.scale), out=ws["att"], reverse=zig and not rev,
                               compact=ws.get("qkvc"))
+                if features:
+                    nxt = regions[sum(k is not None for k in keep_log) + 1]
                 # proj + gathered residual: x_new[b,j] = x[b, keep_idx[b,j]] + proj(att)   model.py:55-58
                 ops.gemm(ws["att"], pw, pb, B * Np, C, C, residual=cur, ldres=C, res_row_map=row_map, out=nxt, ldd=C,
                          row_stats=stats, tag="proj", reverse=rev)
@@ -433,6 +543,15 @@ class RAJNIViTWrapper(nn.Module):
                      ln=(stats, slots, f1sum, e2), tag="fc1", reverse=zig and not rev)                                    # model.py:59 (norm2 + fc1 + GELU)
             ops.gemm(ws["hid"], f2w, f2b, M, C, hidden, residual=cur, ldres=C, out=cur, ldd=C, row_stats=stats, tag="fc2", reverse=rev)
             rev = zig and not rev
+            if features and i in take:          # before the next block overwrites this stage's rows in place
+                maps.append(self._token_features(feat, token_maps(keep_log, B, N0, x.device)[0], take_norm, out_dtype))
+
+        self._last_stats = {"token_counts": token_counts}                            # model.py:68
+        self._last_keep_idx = keep_log
+        if features:
+            # the final norm over all B*N0 rows in original order, instead of the final norm on the class rows + head
+            rows, depth_map = token_maps(keep_log, B, N0, x.device)
+            return (self._token_features(feat, rows, True, out_dtype) if final else None), maps, depth_map
 
         # ---- final norm on the CLS rows only (LayerNorm is row-wise) + head   model.py:65-66
         if self.headless:               # the head's input is the output, stored in fp32 by the kernel that computes it
@@ -460,10 +579,36 @@ class RAJNIViTWrapper(nn.Module):
                 ops.layernorm(cur, gn, bn, en, B, C, in_row_stride=N * C, in_offset=r * C, out=ws["cls"],
                               out_row_stride=2 * C, out_offset=r * C)
             logits = ops.gemm(ws["cls"], hw, hb, B, hw.shape[0], 2 * C, out_f32=True, tag="head")
-
-        self._last_stats = {"token_counts": token_counts}                            # model.py:68
-        self._last_keep_idx = keep_log
         return logits if out_dtype == torch.float32 else logits.to(out_dtype)
+
+    def _stage_regions(self, ws: dict, B: int, dev: torch.device):
+        """The allocation of every stage's rows (the layout of ``token_maps``) -> (all rows [B*sum(N_s), C], [stage s's
+        B*N_s rows]).  Kept in the workspace for the schedule's stage sizes; only the feature methods allocate it."""
+        counts = [ws["N0"]]
+        for blk in self.blocks:
+            if blk.has_pruner:
+                counts.append(keep_count(counts[-1], blk.attn.keep_ratio, self.prefix) + self.prefix)
+        st = ws.get("stages")
+        if st is None or st[0] != counts:
+            st = (counts, torch.empty((B * sum(counts), ws["C"]), device=dev, dtype=torch.bfloat16))
+            ws["stages"] = st
+            self._graphs = {}           # a captured graph points into the allocation it was captured with
+        feat, regions, off = st[1], [], 0
+        for n in counts:
+            regions.append(feat[off: off + B * n])
+            off += B * n
+        return feat, regions
+
+    def _token_features(self, feat: torch.Tensor, rows: torch.Tensor, norm: bool, out_dtype: torch.dtype) -> torch.Tensor:
+        """The rows ``rows`` [B, N0] (of ``token_maps``) of the stage allocation in one gather, through the final norm if
+        ``norm`` and the model has one (one fp32 LayerNorm) -> [B, N0, C] in ``out_dtype``."""
+        B, N0 = rows.shape
+        C = feat.shape[1]
+        y = ops.gather_rows(feat, rows.view(-1))
+        if norm and not self.avg_pool:
+            y = ops.layernorm(y, *self._packs.norm(self.m.norm), B * N0, C,
+                              out=torch.empty((B * N0, C), device=feat.device, dtype=torch.float32))
+        return y.view(B, N0, C).to(out_dtype)
 
     def _head_pack(self):
         m = self.m
