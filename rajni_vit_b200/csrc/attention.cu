@@ -13,10 +13,8 @@
 //                                    for bit.  (profiles/r2_attention_pipe.md, r2_attention_fullrow_ab.txt)
 //   else                           : attention_long.cu  (key blocks of 224, two passes; the 577-token configuration)
 //
-// RAJNI_ATTN_TC=1 sends every Np <= 256 call to attention_tc.cu, RAJNI_ATTN_PIPE=1 every Np_pad <= 224 call to
-// attention_pipe.cu (A/B timing; the tests run both).
-#include <cstdlib>
-
+// RAJNI_ATTN_AUTO picks by shape as above; any other `impl` runs that kernel, or fails where the shape is outside its range
+// (the tests run each kernel this way).
 #include "common.cuh"
 
 namespace rajni {
@@ -39,13 +37,12 @@ extern "C" int rajni_attention_fwd_ex(const void* qkv, const int32_t* row_map, v
     RAJNI_REQUIRE(row_map || N_src == Np, RAJNI_EINVAL, "rajni_attention_fwd_ex: N_src != Np needs a row_map");
     RAJNI_REQUIRE(impl >= RAJNI_ATTN_AUTO && impl <= RAJNI_ATTN_LONG, RAJNI_EINVAL, "rajni_attention_fwd_ex: impl %d", impl);
     if (impl == RAJNI_ATTN_AUTO) {
-        static const bool force_tc = getenv("RAJNI_ATTN_TC") != nullptr, force_pipe = getenv("RAJNI_ATTN_PIPE") != nullptr;
         const int np_pad = (Np + 15) & ~15;
         const int sms = num_sms();
         const long long items = (long long)B * H;
         const bool big = Np > 128;
         const bool one_tile = Np > 64 && Np <= 128 && (row_map == nullptr ? items >= sms : items <= 4LL * sms);
-        if (np_pad <= 224 && (force_pipe || (!force_tc && (big || one_tile)))) impl = RAJNI_ATTN_PIPE;
+        if (np_pad <= 224 && (big || one_tile)) impl = RAJNI_ATTN_PIPE;
         else impl = Np <= 256 ? RAJNI_ATTN_TC : RAJNI_ATTN_LONG;
     }
     int rc = 0;

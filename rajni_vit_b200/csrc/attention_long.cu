@@ -36,14 +36,6 @@ constexpr int kAlQBytes = 128 * 128;            // one Q tile; two of them (the 
 constexpr int kAlOCol = 2 * kAlKB;                 // 448
 constexpr int kAlSmem = 2 * kAlQBytes + kAlStages * kAlStageBytes + 256 + 1024;
 
-// Optional event trace (tools/probes/attn_long_trace.cu builds this file with -DRAJNI_ATTN_TRACE): clock64 stamps of CTA 0.
-#ifdef RAJNI_ATTN_TRACE
-__device__ long long g_al_trace[32 * 32];
-#define AL_TRACE(n, slot) do { if (blockIdx.x == 0 && (n) < 32) g_al_trace[(n) * 32 + (slot)] = clock64(); } while (0)
-#else
-#define AL_TRACE(n, slot) do { } while (0)
-#endif
-
 struct AttnLongParams {
     const __nv_bfloat16* qkv;
     const int32_t* row_map;
@@ -113,7 +105,6 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_c
                 const int b = bh / p.H, h = bh - b * p.H;
                 const int qb = n & 1;
                 mbar_wait(&q_empty[qb], ((n >> 1) & 1) ^ 1);
-                AL_TRACE(n, 0);
                 mbar_expect_tx(&q_full[qb], kAlQBytes);
                 tma_load_3d(smem_gen + qb * kAlQBytes, &tmap_q, &q_full[qb], h * 64, qt * 128, b);      // rows past the image: zero-filled
                 for (int pass = 0; pass < 2; ++pass) {
@@ -124,7 +115,6 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_c
                         mbar_expect_tx(&full_bar[stage], pass ? 2 * kAlPlane : kAlPlane);
                         tma_load_3d(sk, &tmap_kv, &full_bar[stage], p.C + h * 64, j * kAlKB, b);
                         if (pass) tma_load_3d(sk + kAlPlane, &tmap_kv, &full_bar[stage], 2 * p.C + h * 64, j * kAlKB, b);
-                        AL_TRACE(n, 1 + pass * 3 + (j < 3 ? j : 2));
                     }
                 }
             }
@@ -152,7 +142,6 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_c
             if (lw == 0) {
                 const int qb = n & 1;
                 mbar_wait(&q_empty[qb], ((n >> 1) & 1) ^ 1);
-                if (lane == 0) AL_TRACE(n, 0);
                 long long grow[32];
 #pragma unroll
                 for (int i = 0; i < 32; ++i) {
@@ -195,7 +184,6 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_c
                         }
                     }
                     cp_async_arrive_noinc(&full_bar[stage]);
-                    if (lane == 0) AL_TRACE(n, 1 + pass * 3 + (j < 3 ? j : 2));
                 }
             }
         }
@@ -237,13 +225,10 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_c
             for (int n = 0; n < n_mine; ++n) {
                 qd = qd0 + (uint64_t)(((n & 1) * kAlQBytes) >> 4);
                 mbar_wait(&q_full[n & 1], (n >> 1) & 1);
-                AL_TRACE(n, 8);
                 // ---- pass 1: scores only
                 for (int j = 0; j < nb; ++j) issue_s(j, j & 1, true);
                 // ---- pass 2: S_{j+1} is queued before P_j V_j so that it overlaps the softmax of block j
-                AL_TRACE(n, 9);
                 int st_cur = issue_s(0, 0, false);
-                AL_TRACE(n, 10);
                 mbar_wait(o_free, (n & 1) ^ 1);                                  // previous item's O has been read out
                 for (int j = 0; j < nb; ++j) {
                     int st_next = -1;
@@ -259,7 +244,6 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_c
                         umma_bf16_ts(tmem_base + kAlOCol, tmem_base + buf * kAlKB + k * 8, vd + (uint64_t)(k * (2048 >> 4)), idesc_o,
                                      (j | k) != 0);
                     umma_commit(&empty_bar[st_cur]);                             // K_j / V_j may be overwritten
-                    AL_TRACE(n, 11 + (j < 3 ? j : 2));
                     st_cur = st_next;
                 }
                 umma_commit(o_full);
@@ -281,7 +265,6 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_c
             const int b = bh / p.H, h = bh - b * p.H;
             const bool warp_live = qt * 128 + rbase < Np;                         // any valid query row in this warp
             // ---------------- pass 1: row maxima ----------------
-            if (tid == 0) AL_TRACE(n, 16);
             float mx0 = -INFINITY, mx1 = -INFINITY;
             for (int j = 0; j < nb; ++j) {
                 const int buf = j & 1;
@@ -323,7 +306,6 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_c
                 }
                 tc_fence_before();
                 mbar_arrive(&s_free[buf]);
-                if (tid == 0) AL_TRACE(n, 17 + (j < 3 ? j : 2));
             }
             mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 1));
             mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 1));
@@ -402,7 +384,6 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_c
                 }
                 tc_fence_before();
                 mbar_arrive(&p_full[buf]);
-                if (tid == 0) AL_TRACE(n, 20 + (j < 3 ? j : 2));
             }
             sum0 += __shfl_xor_sync(0xffffffffu, sum0, 1);
             sum1 += __shfl_xor_sync(0xffffffffu, sum1, 1);
@@ -411,7 +392,6 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_c
             // ---------------- O / rowsum -> bf16 -> global ----------------
             mbar_wait(o_full, n & 1);
             tc_fence_after();
-            if (tid == 0) AL_TRACE(n, 23);
             if (warp_live) {
                 uint32_t o[32];
                 tmem_ld16x256_x8(twin + kAlOCol, o);
@@ -435,7 +415,6 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_c
                         *reinterpret_cast<uint32_t*>(dst + 8 * g) =
                             float2_to_bf16x2(__uint_as_float(o[4 * g + 2]) * inv, __uint_as_float(o[4 * g + 3]) * inv);
                 }
-                if (tid == 0) AL_TRACE(n, 24);
             } else {
                 tc_fence_before();
                 mbar_arrive(o_free);

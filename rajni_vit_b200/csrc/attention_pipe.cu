@@ -34,14 +34,11 @@
 namespace rajni {
 
 constexpr int kApHelpWarp0 = 8;
-#ifndef AP_MMA_WARP
-#define AP_MMA_WARP 15
-#endif
 // The MMA issuer sits on scheduler 3 (warp id % 4): its neighbours there are the exp warps of TMEM lanes 96..127, which have
 // no rows at all in the second tile of a 129..224-token item - an issuer next to busy exp warps gets so few issue slots that
 // queueing one P V takes 2200 cycles instead of 1300 (profiles/r2_attention_pipe.md).
-constexpr int kApMmaWarp = AP_MMA_WARP;
-constexpr int kApLoaderWarp0 = 12;                                             // three loader warps: 12..14 (or 13..15)
+constexpr int kApMmaWarp = 15;
+constexpr int kApLoaderWarp0 = 12;                                             // three loader warps: 12..14
 constexpr int kApWg3Warp0 = 12;
 constexpr int kApLoaderThreads = 96;
 constexpr int kApLoaderGroups = kApLoaderThreads / 8;                          // 8 lanes move one token's 128-byte head slice
@@ -50,22 +47,10 @@ constexpr int kApThreads = 512;
 constexpr int kApMaxStages = 4;
 constexpr int kApMaxBufs = 4;
 constexpr int kApSumSlots = 8;
-#ifndef AP_POLY_EVERY
-#define AP_POLY_EVERY 0
-#endif
-constexpr int kApPolyEvery = AP_POLY_EVERY;               // one exponential in this many is a polynomial on the FMA pipe (0: all on MUFU)
 constexpr int kApOutStage = 4 * 4096;                                          // 32 rows x 128 B per helper warp
 constexpr int kApAuxBytes = 2 * 2 * 128 * 4 + kApSumSlots * 2 * 128 * 4;       // half-row maxima (2 parities), partial row sums
 constexpr int kApBarBytes = 320;
 constexpr int kApSmemBudget = 227 * 1024 - 1024 - kApOutStage - kApAuxBytes - kApBarBytes;
-
-#ifdef RAJNI_ATTN_TRACE
-__device__ int g_ap_dbg;
-__device__ long long g_ap_trace[64 * 16];
-#define AP_TRACE(g, slot) do { if (blockIdx.x == 0 && (g) < 64) g_ap_trace[(g) * 16 + (slot)] = clock64(); } while (0)
-#else
-#define AP_TRACE(g, slot) do { } while (0)
-#endif
 
 struct AttnPipeParams {
     const __nv_bfloat16* qkv;
@@ -75,7 +60,6 @@ struct AttnPipeParams {
     int split;                                  // key columns [0, split) -> exp warps 0-3, [split, Np_pad) -> warps 4-7
     int fullrow;                                // one-tile items of <= 112 keys: a thread takes its WHOLE row, warps 0-3 the even tiles, 4-7 the odd ones
     int plane_bytes, stages, reverse;
-    int dbg;                                    // experiments (tools/probes, RAJNI_ATTN_TRACE builds only): skip parts of the work
     float scale_log2;
 };
 
@@ -113,19 +97,6 @@ struct ApCursor {
     }
 };
 
-// 2^x on the FMA/ALU pipes (x >= -125 after the clamp): round x to the nearest integer with the 1.5*2^23 trick, a cubic
-// for 2^f on f in [-0.5, 0.5] (relative error 2.2e-4, a twentieth of a bf16 ulp), the integer added into the exponent field.
-// One exponential in kApPolyEvery goes this way: MUFU.EX2 (16 results/clk/SM) is what bounds the exp warps, the FMA pipe idles.
-__device__ __forceinline__ float ap_ex2_poly(float x) {
-    x = fmaxf(x, -125.f);
-    const float t = x + 12582912.f;
-    const float f = x - (t - 12582912.f);
-    float q = fmaf(0.05286743f, f, 0.24215189f);
-    q = fmaf(q, f, 0.69358677f);
-    q = fmaf(q, f, 0.99996275f);
-    return __uint_as_float(__float_as_uint(q) + (__float_as_uint(t) << 23));
-}
-
 // One exp-warp thread's share of a tile: the half row [cb, cb + 32*N32 + 16*HAS16) of S (TMEM row `sb`) -> P at `pcol`.
 // Straight-line for a given (N32, HAS16): no branch between the 16-column groups, so MUFU.EX2 never drains.
 //   s[0..95] = the 32-column pieces, s[96..111] = the 16-column piece.  The thread holds its WHOLE half row before the row
@@ -138,7 +109,7 @@ __device__ __forceinline__ float ap_ex2_poly(float x) {
 // Returns the half row's sum of p.
 template <int N32, int HAS16>
 __device__ __forceinline__ float ap_exp_half(uint32_t sb, int cb, uint32_t pcol, int Np, float sl2, float* pm_mine, const float* pm_other,
-                                             int bar_id, int bar_n, uint64_t* taken_bar, bool drop16, int lane, bool trace_lane, int g) {
+                                             int bar_id, int bar_n, uint64_t* taken_bar, bool drop16, int lane) {
     constexpr int NCOL = 32 * N32 + 16 * HAS16;
     constexpr int LAST = HAS16 ? 96 : 32 * N32 - 16;                          // registers of the half's last 16 columns
     constexpr int W16 = 16 * N32;                                             // P pairs of the 16-column piece go to s[W16..]
@@ -150,7 +121,6 @@ __device__ __forceinline__ float ap_exp_half(uint32_t sb, int cb, uint32_t pcol,
     tc_fence_before();
     __syncwarp();
     if (lane == 0) mbar_arrive(taken_bar);
-    if (trace_lane) AP_TRACE(g, 4);
     if (cb + NCOL > Np) {
 #pragma unroll
         for (int i = 0; i < 16; ++i) if (cb + NCOL - 16 + i >= Np) s[LAST + i] = 0xff800000u;      // -inf
@@ -167,20 +137,14 @@ __device__ __forceinline__ float ap_exp_half(uint32_t sb, int cb, uint32_t pcol,
     *pm_mine = mx;
     ap_bar_sync(bar_id, bar_n);                                               // the two warps that share these 32 rows
     const float mb = fmaxf(mx, *pm_other) * sl2;
-    if (trace_lane) AP_TRACE(g, 5);
-#ifdef RAJNI_ATTN_TRACE
-    if (g_ap_dbg & 2) return mb;
-#endif
     float sum0 = 0.f, sum1 = 0.f;
-    // p = exp2(s * scale * log2e - max) for registers R0..R0+N -> bf16 pairs at W0..; column c of the row takes the
-    // polynomial when c % kApPolyEvery == kApPolyEvery - 1 (cb and R0 are multiples of 16, so the register index decides)
+    // p = exp2(s * scale * log2e - max) for registers R0..R0+N -> bf16 pairs at W0..
     auto exp_run = [&](auto r0_c, auto w0_c, auto n_c) {
         constexpr int R0 = decltype(r0_c)::value, W0 = decltype(w0_c)::value, N = decltype(n_c)::value;
 #pragma unroll
         for (int j = 0; j < N; j += 2) {
             const float x0 = fmaf(__uint_as_float(s[R0 + j]), sl2, -mb), x1 = fmaf(__uint_as_float(s[R0 + j + 1]), sl2, -mb);
-            const float e0 = ex2_approx(x0);
-            const float e1 = (kApPolyEvery > 0 && (j + 1) % (kApPolyEvery > 0 ? kApPolyEvery : 1) == kApPolyEvery - 1) ? ap_ex2_poly(x1) : ex2_approx(x1);
+            const float e0 = ex2_approx(x0), e1 = ex2_approx(x1);
             sum0 += e0;
             sum1 += e1;
             s[W0 + (j >> 1)] = float2_to_bf16x2(e0, e1);
@@ -196,7 +160,6 @@ __device__ __forceinline__ float ap_exp_half(uint32_t sb, int cb, uint32_t pcol,
         exp_run(integral_constant<int, 96>{}, integral_constant<int, W16>{}, integral_constant<int, 16>{});
         if (N32 == 0 && drop16) { sum0 = 0.f; sum1 = 0.f; }
     }
-    if (trace_lane) AP_TRACE(g, 10);
     // P pairs are contiguous in s[0 .. NCOL/2): 32 + 16 + 8 columns at most
     if (NCOL >= 64) tmem_st32(pcol, *reinterpret_cast<uint32_t(*)[32]>(&s[0]));
     if ((NCOL / 2) & 16) tmem_st16(pcol + ((NCOL / 2) & 32), *reinterpret_cast<uint32_t(*)[16]>(&s[(NCOL / 2) & 32]));
@@ -393,7 +356,6 @@ attention_pipe_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid
             auto issue_s = [&]() {
                 mbar_wait(&qk_full[s.stage], s.stage_ph);
                 tc_fence_after();
-                AP_TRACE(s.g, 0);
                 const uint64_t qd = qd0 + (uint64_t)((s.stage * stage_bytes + s.j * (128 * 128)) >> 4);
                 const uint64_t kd = kd0 + (uint64_t)((s.stage * stage_bytes) >> 4);
                 const uint32_t d = tmem_base + s.buf * p.s_stride;
@@ -402,7 +364,6 @@ attention_pipe_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid
                     umma_bf16(d, qd + (uint64_t)(k * 2), kd + (uint64_t)(k * 2), idesc_s, k != 0);
                 umma_commit(&s_full[s.buf]);
                 if (s.j == p.tpi - 1) umma_commit(&qk_empty[s.stage]);         // the item's last S: its Q and K planes may be refilled
-                AP_TRACE(s.g, 1);
                 s.advance(p);
             };
             // Fixed issue order with BLOCKING waits (a polling issuer takes issue slots from the exp warps of its scheduler):
@@ -422,17 +383,14 @@ attention_pipe_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid
                 mbar_wait(&v_full[v.stage], v.stage_ph);
                 mbar_wait(&o_empty[ob], ob ? o_ph1 : o_ph0);
                 tc_fence_after();
-                AP_TRACE(v.g, 2);
                 const uint64_t vd = vd0 + (uint64_t)((v.stage * stage_bytes) >> 4);
                 const uint32_t pb = tmem_base + v.buf * p.s_stride;
                 const uint32_t d = tmem_base + p.o_col + ob * 64;
                 uint64_t vdk = vd;
                 for (int k = 0; k < nk0; ++k, vdk += (2048 >> 4)) umma_bf16_ts(d, pb + k * 8, vdk, idesc_o, k != 0);
                 for (int k = 0; k < nk - nk0; ++k, vdk += (2048 >> 4)) umma_bf16_ts(d, pb + p2 + k * 8, vdk, idesc_o, 1);
-                AP_TRACE(v.g, 12);
                 umma_commit(&o_full[ob]);
                 if (v.j == p.tpi - 1) umma_commit(&stage_empty[v.stage]);     // the item's last product: the stage may be refilled
-                AP_TRACE(v.g, 3);
                 if (ob) o_ph1 ^= 1; else o_ph0 ^= 1;
                 if (++ob == p.n_obuf) ob = 0;
                 if (s.g < G) issue_s();                                       // into the buffer this PV has just released
@@ -452,12 +410,7 @@ attention_pipe_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid
         for (; e.g < G; e.advance(p)) {
             mbar_wait(&o_full[ob], ob ? o_ph1 : o_ph0);
             tc_fence_after();
-            if (hq == 0 && lane == 0) AP_TRACE(e.g, 6);
-#ifdef RAJNI_ATTN_TRACE
-            const bool live = e.j * 128 + hq * 32 < Np && !(p.dbg & 4);
-#else
             const bool live = e.j * 128 + hq * 32 < Np;
-#endif
             uint32_t o0[32], o1[32];
             if (live) {
                 const uint32_t ocol = lane_base + p.o_col + ob * 64;
@@ -492,7 +445,6 @@ attention_pipe_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid
                     bulk_commit_group();
                 }
             }
-            if (hq == 0 && lane == 0) AP_TRACE(e.g, 7);
             if (ob) o_ph1 ^= 1; else o_ph0 ^= 1;
             if (++ob == p.n_obuf) ob = 0;
             if (++slot == kApSumSlots) slot = 0;
@@ -549,10 +501,6 @@ attention_pipe_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid
         } else
         for (; c.g < G; c.advance(p)) {
             mbar_wait(&s_full[c.buf], c.buf_ph);
-            if (warp == 0 && lane == 0) AP_TRACE(c.g, 8);
-#ifdef RAJNI_ATTN_TRACE
-            if (p.dbg & 1) { __syncwarp(); if (lane == 0) { mbar_arrive(&s_taken[c.buf]); mbar_arrive(&p_full[c.buf]); } if (++slot == kApSumSlots) slot = 0; continue; }
-#endif
             if (c.j * 128 + q * 32 < Np && has_cols) {
                 tc_fence_after();
                 const uint32_t sb = lane_base + c.buf * p.s_stride;
@@ -560,10 +508,9 @@ attention_pipe_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid
                 float* pm_mine = pm + half * 128 + row;
                 const float* pm_other = p.split < Np_pad ? pm + (half ^ 1) * 128 + row : pm_mine;
                 const int bar_n = p.split < Np_pad ? 64 : 32;
-                const bool tl = warp == 0 && lane == 0;
                 float sum;
 #define AP_HALF(N32_, H16_) ap_exp_half<N32_, H16_>(sb, cb, sb + (half ? p.split : 0), Np, sl2, pm_mine, pm_other, 1 + q + (bar_n == 32 ? 4 * half : 0), \
-                                                    bar_n, &s_taken[c.buf], drop16, lane, tl, c.g)
+                                                    bar_n, &s_taken[c.buf], drop16, lane)
                 switch (nch) {                                                // warp-uniform: one straight-line body per width
                     case 7: sum = AP_HALF(3, 1); break;
                     case 6: sum = AP_HALF(3, 0); break;
@@ -584,7 +531,6 @@ attention_pipe_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid
             }
             __syncwarp();
             if (lane == 0) mbar_arrive(&p_full[c.buf]);
-            if (warp == 0 && lane == 0) AP_TRACE(c.g, 9);
             if (++slot == kApSumSlots) slot = 0;
         }
     }
@@ -606,10 +552,6 @@ int launch_attention_pipe(const void* qkv, const int32_t* row_map, void* out, in
     p.row_map = row_map;
     p.N_src = N_src; p.Np = Np; p.Np_pad = Np_pad; p.C = C; p.H = H;
     p.reverse = reverse;
-#ifdef RAJNI_ATTN_TRACE
-    p.dbg = getenv("AP_DEBUG") ? atoi(getenv("AP_DEBUG")) : 0;
-    cudaMemcpyToSymbol(g_ap_dbg, &p.dbg, sizeof(int));
-#endif
     p.BH = B * H;
     p.tpi = Np > 128 ? 2 : 1;
     p.scale_log2 = scale * 1.4426950408889634f;
@@ -642,9 +584,7 @@ int launch_attention_pipe(const void* qkv, const int32_t* row_map, void* out, in
     if (int rc = make_tmap_bf16_3d_box(&tmap_out, out, B, Np, C, 32)) return rc;
     static int smem_granted[kMaxDevices] = {};
     if (int rc = raise_smem_limit("attention_pipe", attention_pipe_kernel, smem, smem_granted)) return rc;
-    int grid = p.BH < num_sms() ? p.BH : num_sms();
-    static const int cta_cap = getenv("RAJNI_ATTN_MAX_CTAS") ? atoi(getenv("RAJNI_ATTN_MAX_CTAS")) : 0;      // experiments: share the GPU
-    if (cta_cap > 0 && grid > cta_cap) grid = cta_cap;
+    const int grid = p.BH < num_sms() ? p.BH : num_sms();
     const int rc = launch_checked("attention_pipe", attention_pipe_kernel, dim3(grid), dim3(kApThreads), (size_t)smem, stream, 1,
                                   tmap, tmap_out, p);
     return rc ? rc : 1;

@@ -43,15 +43,6 @@ constexpr int kAtTileCols = 256;
 constexpr int kAtOutStage = kAtSoftmaxWarps * 32 * 128;                        // output staging: 32 rows x 128 B per softmax warp
 constexpr int kAtSmemBudget = 224 * 1024 - kAtOutStage;                        // stages; barriers and alignment on top
 
-// Optional event trace (tools/probes/attn_trace.cu builds this file with -DRAJNI_ATTN_TRACE): clock64 stamps of
-// CTA 0's pipeline events, one row of 32 slots per unit.  Compiles to nothing in the library.
-#ifdef RAJNI_ATTN_TRACE
-__device__ long long g_attn_trace[64 * 32];
-#define AT_TRACE(n, slot) do { if (blockIdx.x == 0 && (n) < 64) g_attn_trace[(n) * 32 + (slot)] = clock64(); } while (0)
-#else
-#define AT_TRACE(n, slot) do { } while (0)
-#endif
-
 struct AttnTcParams {
     const __nv_bfloat16* qkv;
     const int32_t* row_map;
@@ -133,7 +124,6 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_c
                 const int u = blockIdx.x + n * gridDim.x;
                 const int nsub = p.two_tiles ? 1 : (unit_item(p, u, 1) >= 0 ? 2 : 1);
                 mbar_wait(&empty_bar[stage], phase ^ 1);
-                AT_TRACE(n, 0);
                 mbar_expect_tx(&qk_full[stage], 2u * plane_tx * nsub);
                 mbar_expect_tx(&v_full[stage], plane_tx * nsub);
                 uint8_t* sq = smem_gen + stage * stage_bytes;
@@ -145,7 +135,6 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_c
                         tma_load_3d(sq + pl * p.plane_bytes + t * (128 * 128), &tmap_qkv, pl < 2 ? &qk_full[stage] : &v_full[stage],
                                     pl * p.C + h * 64, 0, b);
                     }
-                AT_TRACE(n, 1);
                 if (++stage == p.stages) { stage = 0; phase ^= 1; }
             }
         }
@@ -182,7 +171,6 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_c
             }
             if (p.two_tiles) hcol[1] = hcol[0];
             mbar_wait(&empty_bar[stage], phase ^ 1);
-            if (lt == 0) AT_TRACE(n, 0);
             const uint32_t sq = smem_base + stage * stage_bytes, sk = sq + p.plane_bytes, sv = sk + p.plane_bytes;
 #pragma unroll
             for (int pass = 0; pass < 2; ++pass) {                    // pass 0: Q and K (what S needs), pass 1: V
@@ -206,7 +194,6 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_c
                 }
                 cp_async_arrive_noinc(pass == 0 ? &qk_full[stage] : &v_full[stage]);
             }
-            if (lt == 0) AT_TRACE(n, 1);
             if (++stage == p.stages) { stage = 0; phase ^= 1; }
         }
     } else if (warp == kAtMmaWarp) {
@@ -248,7 +235,6 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_c
                         }
                         if (ok) {
                             tc_fence_after();
-                            AT_TRACE(n, 4 + 4 * t);
                             const uint64_t vd = vd0 + (uint64_t)((st * stage_bytes + t * kv_stride) >> 4);
                             for (int k = 0; k < p.split_col / 16; ++k)
                                 umma_bf16_ts(tt + p.o_col, tt + k * 8, vd + (uint64_t)(k * (2048 >> 4)), idesc_o, k != 0);
@@ -267,13 +253,11 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_c
                         }
                         if (ok) {
                             tc_fence_after();
-                            if (!half_done[t]) AT_TRACE(n, 4 + 4 * t);
                             const uint64_t vd = vd0 + (uint64_t)((st * stage_bytes + t * kv_stride) >> 4);
                             for (int k = half_done[t] ? p.split_col / 16 : 0; k < nk; ++k)
                                 umma_bf16_ts(tt + p.o_col, tt + k * 8, vd + (uint64_t)(k * (2048 >> 4)), idesc_o, k != 0);
                             half_done[t] = false;
                             umma_commit(&o_full[t]);
-                            AT_TRACE(n, 5 + 4 * t);
                             pv_next[t] = n + 1;
                             if (++pv_stage[t] == p.stages) { pv_stage[t] = 0; pv_phase[t] ^= 1; }
                             const int tiles_n = (n == n_mine - 1 && cnt[1] < n_mine) ? 1 : 2;
@@ -291,7 +275,7 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_c
                         const int st = s_stage[t];
                         bool ok = true;
                         if (qk_seen <= n) {
-                            if (mbar_test(&qk_full[st], s_phase[t])) { qk_seen = n + 1; AT_TRACE(n, 2); }
+                            if (mbar_test(&qk_full[st], s_phase[t])) qk_seen = n + 1;
                             else ok = false;
                         }
                         if (ok && !p.o_outside && n > 0) ok = mbar_test(&o_empty[t], (n - 1) & 1);   // O sits inside S's columns
@@ -300,14 +284,12 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_c
                         if (ok && t == 1 && n == 0 && cnt[0] > 0) ok = mbar_test(&p_full[0], 0);
                         if (ok) {
                             tc_fence_after();
-                            AT_TRACE(n, 6 + 4 * t);
                             const uint64_t qd = qd0 + (uint64_t)((st * stage_bytes + t * (128 * 128)) >> 4);
                             const uint64_t kd = kd0 + (uint64_t)((st * stage_bytes + t * kv_stride) >> 4);
 #pragma unroll
                             for (int k = 0; k < 4; ++k)
                                 umma_bf16(tt, qd + (uint64_t)(k * 2), kd + (uint64_t)(k * 2), idesc_s, k != 0);
                             umma_commit(&s_full[t]);
-                            AT_TRACE(n, 7 + 4 * t);
                             s_next[t] = n + 1;
                             if (++s_stage[t] == p.stages) { s_stage[t] = 0; s_phase[t] ^= 1; }
                             did = true;
@@ -333,7 +315,6 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_c
             const int item_b = item / p.H, item_h = item - item_b * p.H;       // (before the wait for S: off the critical path)
             mbar_wait(&s_full[t], ph);
             tc_fence_after();
-            if ((tid & 127) == 0) AT_TRACE(n, 12 + 8 * t);
             float sum = 1.f;
             if (warp_live) {
                 uint32_t va[32], vb[32];
@@ -365,7 +346,6 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_c
                     max32(va, c0);
                     if (c0 + 32 < whi) max32(vb, c0 + 32);
                 }
-                if ((tid & 127) == 0) AT_TRACE(n, 13 + 8 * t);
                 // ---- pass 2: p = exp2((s - max) * scale * log2 e), row sum, bf16 P back into TMEM.
                 // P chunk c lands on columns [16c, 16c+16): always behind the S columns still to be read.
                 // The row sum is taken in the order attention_pipe.cu takes it - even and odd columns of the key halves
@@ -434,7 +414,6 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_c
                 mbar_arrive(&p_half[t]);
             }
             tc_fence_before();
-            if ((tid & 127) == 0) AT_TRACE(n, 14 + 8 * t);
             mbar_arrive(&p_full[t]);
             // ---- O = P V done -> normalise, store
             if (warp_live) {                  // while P V runs: the previous store must have read the staging buffer
@@ -443,7 +422,6 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_c
             }
             mbar_wait(&o_full[t], ph);
             tc_fence_after();
-            if ((tid & 127) == 0) AT_TRACE(n, 15 + 8 * t);
             if (warp_live) {
                 uint32_t o0[32], o1[32];
                 tmem_ld32(trow + p.o_col, o0);
@@ -451,7 +429,6 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_c
                 tmem_ld_wait();
                 tc_fence_before();
                 mbar_arrive(&o_empty[t]);
-                if ((tid & 127) == 0) AT_TRACE(n, 16 + 8 * t);
                 // The warp's 32 rows x 128 B go out as ONE TMA store (3-d map: rows past the image's Np are clipped), staged
                 // in shared memory with the 128-byte swizzle.  (Against 32-byte st.global per row: -3 % kernel time.)
                 const uint32_t s_out = smem_base + p.stages * stage_bytes + warp * 4096;
@@ -473,7 +450,6 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_c
                     tma_store_3d(&tmap_out, s_out, item_h * 64, q - lane, item_b);
                     bulk_commit_group();
                 }
-                if ((tid & 127) == 0) AT_TRACE(n, 17 + 8 * t);
             } else {
                 tc_fence_before();
                 mbar_arrive(&o_empty[t]);
@@ -521,8 +497,7 @@ int launch_attention_tc(const void* qkv, const int32_t* row_map, void* out, int 
     p.ksplit = ((p.Np_pad / 2) + 15) & ~15;
     p.o_outside = p.Np_pad <= 192;
     p.o_col = p.o_outside ? 192 : 128;
-    static const bool nosplit = getenv("RAJNI_ATTN_NOSPLIT") != nullptr;      // A/B switch
-    p.split_col = (p.o_outside && !nosplit && p.Np_pad >= 64) ? ((p.Np_pad / 2 + 31) & ~31) : 0;
+    p.split_col = (p.o_outside && p.Np_pad >= 64) ? ((p.Np_pad / 2 + 31) & ~31) : 0;
     if (p.split_col >= p.Np_pad) p.split_col = 0;
     // a plane holds the Q (or K, or V) rows of a stage; tile 1's Q rows / the second head start at row 128
     const int plane_rows = p.two_tiles ? p.Np_pad : 128 + p.Np_pad;
@@ -540,9 +515,7 @@ int launch_attention_tc(const void* qkv, const int32_t* row_map, void* out, int 
     auto kern = packed ? attention_tc_kernel<true> : attention_tc_kernel<false>;
     static int smem_granted[2][kMaxDevices] = {};
     if (int rc = raise_smem_limit("attention_tc", kern, smem, smem_granted[packed])) return rc;
-    int grid = p.n_units < num_sms() ? p.n_units : num_sms();
-    static const int cta_cap = getenv("RAJNI_ATTN_MAX_CTAS") ? atoi(getenv("RAJNI_ATTN_MAX_CTAS")) : 0;      // experiments: share the GPU
-    if (cta_cap > 0 && grid > cta_cap) grid = cta_cap;
+    const int grid = p.n_units < num_sms() ? p.n_units : num_sms();
     const int rc = launch_checked("attention_tc", kern, dim3(grid), dim3(kAtThreads), (size_t)smem, stream, 1, tmap, tmap_out, p);
     return rc ? rc : 1;
 }

@@ -37,7 +37,6 @@ int check_launch(const char* what);   // cudaGetLastError -> RAJNI_ECUDA
 __device__ __forceinline__ void griddep_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void griddep_launch() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 
-bool pdl_enabled();      // runtime.cu: false when RAJNI_NO_PDL is set
 int current_device();    // runtime.cu: cudaGetDevice, 0 on error (indexes the per-device one-time flags below)
 constexpr int kMaxDevices = 64;
 
@@ -58,11 +57,9 @@ inline cudaError_t launch_kernel(void (*kern)(KArgs...), dim3 grid, dim3 block, 
         attr[n].val.clusterDim.z = 1;
         ++n;
     }
-    if (pdl_enabled()) {
-        attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[n].val.programmaticStreamSerializationAllowed = 1;
-        ++n;
-    }
+    attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[n].val.programmaticStreamSerializationAllowed = 1;
+    ++n;
     cfg.attrs = attr;
     cfg.numAttrs = n;
     return cudaLaunchKernelEx(&cfg, kern, std::forward<Args>(args)...);

@@ -28,7 +28,6 @@
 // per 32-column chunk; the GEMM that CONSUMES LN(x) (qkv / fc1) runs on x itself with
 // gamma-scaled weights and applies  acc*rstd + (-mean*rstd)*wsum[n] + bias'[n]  in its epilogue.
 #include <cuda.h>
-#include <cstdlib>
 
 #include "common.cuh"
 
@@ -575,9 +574,7 @@ static int launch_gemm_mode(const void* A, const void* W, GemmParams& p, cudaStr
     p.tiles_m = (p.M + BM * CG - 1) / (BM * CG);
     p.tiles_n = (p.N + BN - 1) / BN;
     p.k_blocks = (p.K + BK - 1) / BK;
-    int max_grid = (num_sms() / CG) * CG;
-    static const int cta_cap = getenv("RAJNI_GEMM_MAX_CTAS") ? atoi(getenv("RAJNI_GEMM_MAX_CTAS")) : 0;     // experiments: leave SMs free
-    if (cta_cap > 0 && cta_cap < max_grid) max_grid = (cta_cap / CG) * CG;
+    const int max_grid = (num_sms() / CG) * CG;
     int grid = p.tiles_m * p.tiles_n * CG;
     if (grid > max_grid) grid = max_grid;
     auto kern = gemm_bf16_kernel<BN, CG, MODE, LN>;
@@ -616,8 +613,6 @@ static int launch_gemm(const void* A, const void* W, GemmParams& p, cudaStream_t
 // (e.g. N = 768, M = 44288: 173 x 3 tiles of 256 = 7.01 waves -> 8, but 173 x 4 tiles of 192 = 9.35 -> 10 x 3/4 = 7.5).
 static int pick_bn(int N, int M, bool exact, bool no192) {
     if (exact) {
-        static const char* force = getenv("RAJNI_GEMM_BN");                 // debugging aid: force a pair-tile width that divides N
-        if (force && M > BM && N % atoi(force) == 0 && (atoi(force) == 256 || (atoi(force) == 192 && !no192) || atoi(force) == 128)) return -atoi(force);
         const bool pair = M > BM;
         int best = 0;
         double best_cost = 0;
@@ -688,16 +683,14 @@ extern "C" int rajni_gemm_bf16_ex(const rajni_gemm_args* a, void* stream) {
     const bool exact = (flags & (RAJNI_EPI_LN_FOLD | RAJNI_EPI_ROW_STATS)) != 0;
     RAJNI_REQUIRE(!exact || N % 64 == 0, RAJNI_EINVAL, "rajni_gemm_bf16_ex: LN_FOLD / ROW_STATS need N %% 64 == 0 (N=%d)", N);
     // (a producer of 64-column statistics slots cannot use the 192-wide tile)
-    int bn = pick_bn(N, M, exact, (flags & RAJNI_EPI_ROW_STATS) && stat_shift_for(N) == 6);   // < 0: exact CTA-pair tile of width -bn
+    const int bn = pick_bn(N, M, exact, (flags & RAJNI_EPI_ROW_STATS) && stat_shift_for(N) == 6);   // < 0: exact CTA-pair tile of width -bn
     auto s = static_cast<cudaStream_t>(stream);
     // wide problems run as CTA pairs (256 x 256 tiles); narrow ones keep single-CTA tiles
-    static const bool force_cg1 = getenv("RAJNI_GEMM_CG1") != nullptr;     // debugging aid
-    if (bn < 0 && force_cg1) bn = (-bn == 192) ? 64 : -bn;
     switch (bn) {
         case -256: return launch_gemm<256, 2>(a->A, a->W, p, s);
         case -192: return launch_gemm<192, 2>(a->A, a->W, p, s);
         case -128: return launch_gemm<128, 2>(a->A, a->W, p, s);
-        case 256: return (M > BM && !force_cg1) ? launch_gemm<256, 2>(a->A, a->W, p, s) : launch_gemm<256, 1>(a->A, a->W, p, s);
+        case 256: return M > BM ? launch_gemm<256, 2>(a->A, a->W, p, s) : launch_gemm<256, 1>(a->A, a->W, p, s);
         case 128: return launch_gemm<128, 1>(a->A, a->W, p, s);
         default: return launch_gemm<64, 1>(a->A, a->W, p, s);
     }

@@ -2,7 +2,6 @@
 #include <atomic>
 #include <cstdarg>
 #include <cstdio>
-#include <cstdlib>
 
 #include "common.cuh"
 
@@ -16,11 +15,6 @@ void set_error(const char* fmt, ...) {
     va_start(ap, fmt);
     vsnprintf(g_error, sizeof(g_error), fmt, ap);
     va_end(ap);
-}
-
-bool pdl_enabled() {
-    static const bool on = getenv("RAJNI_NO_PDL") == nullptr;
-    return on;
 }
 
 int current_device() {

@@ -28,17 +28,6 @@ constexpr int kSelWarps = kSelThreads / 32;
 constexpr int kHeadDim = 64;
 constexpr int kVmSmemStride = kHeadDim + 1;     // value rows in shared memory: thread-per-row reads without bank conflicts
 
-// Optional event trace (tools/probes/score_trace.cu builds this file with -DRAJNI_SCORE_TRACE): globaltimer stamps (ns) of
-// one CTA's thread 0.
-#ifdef RAJNI_SCORE_TRACE
-__device__ long long g_sc_trace[64 * 16];
-__device__ int g_sc_trace_cta;
-__device__ __forceinline__ long long sc_now() { long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); return t; }
-#define SC_TRACE(row, slot) do { if (threadIdx.x == 0 && (int)blockIdx.x == g_sc_trace_cta && (row) < 64) g_sc_trace[(row) * 16 + (slot)] = sc_now(); } while (0)
-#else
-#define SC_TRACE(row, slot) do { } while (0)
-#endif
-
 struct ScoreSelectParams {
     const __nv_bfloat16* qkv;   // [B,N,3C] or null (select-only)
     const float* scores_in;     // [B,N] when qkv == null
@@ -375,12 +364,11 @@ __device__ __forceinline__ float row_dist2(const float* row, const float* mu) {
 // VS: float stride of the value rows (kVmSmemStride in shared memory, kHeadDim in the workspace).  sm.logit may point into the
 // workspace too (score_tail_ws_kernel): same reads, same arithmetic, same bits.
 template <int NT, int VS = kVmSmemStride>
-__device__ void score_tail(const SelSmem& sm, const float* vm, const ScoreSelectParams& p, int b, int trace_row = 0) {
+__device__ void score_tail(const SelSmem& sm, const float* vm, const ScoreSelectParams& p, int b) {
     const int N = p.N, H = p.H;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int vs = VS;
     const float inv_h = 1.0f / (float)H;
-    SC_TRACE(32 + trace_row, 4);
     // ---- mean over tokens of the head-averaged value (importance.py:25): 8 interleaved partial sums per dim, then their sum
     {
         const int d = tid & 63;
@@ -399,10 +387,8 @@ __device__ void score_tail(const SelSmem& sm, const float* vm, const ScoreSelect
         }
         tail_sync<NT>();
     }
-    SC_TRACE(32 + trace_row, 5);
     // ---- r[n] = || vm[n] - mu ||  (importance.py:27): thread per token
     for (int n = tid; n < N; n += NT) sm.r[n] = sqrtf(row_dist2(vm + (size_t)n * vs, sm.mu));
-    SC_TRACE(32 + trace_row, 6);
     // ---- per-head softmax statistics over all N tokens (importance.py:20): warp per head
     for (int h = warp; h < H; h += NT / 32) {
         float* l = sm.logit + (size_t)h * N;
@@ -418,7 +404,6 @@ __device__ void score_tail(const SelSmem& sm, const float* vm, const ScoreSelect
         s = warp_sum(s);
         if (lane == 0) sm.hstat[h] = s;
     }
-    SC_TRACE(32 + trace_row, 7);
     // ---- z-score of r with the unbiased std (importance.py:28-32)
     const float* r = sm.r;
     const float mu = block_sum<NT>([&](int v) { float t = 0.f; for (int n = v; n < N; n += kSelThreads) t += r[n]; return t; },
@@ -426,7 +411,6 @@ __device__ void score_tail(const SelSmem& sm, const float* vm, const ScoreSelect
     const float var = block_sum<NT>([&](int v) { float t = 0.f; for (int n = v; n < N; n += kSelThreads) { float d = r[n] - mu; t += d * d; } return t; },
                                     sm.scratch) / (float)(N - 1);
     const float sd = sqrtf(var) + p.eps;
-    SC_TRACE(32 + trace_row, 8);
     for (int n = tid; n < N; n += NT) {
         float a = 0.f;
         for (int h = 0; h < H; ++h) a += sm.logit[(size_t)h * N + n] / sm.hstat[h];
@@ -437,9 +421,7 @@ __device__ void score_tail(const SelSmem& sm, const float* vm, const ScoreSelect
         if (p.scores_out) p.scores_out[(size_t)b * N + n] = sc;
     }
     tail_sync<NT>();
-    SC_TRACE(32 + trace_row, 9);
     if (p.keep_idx != nullptr) select_any<NT>(sm, p, b);
-    SC_TRACE(32 + trace_row, 10);
 }
 
 // CPL = 16-byte chunks per lane per plane = ceil(C / 256).

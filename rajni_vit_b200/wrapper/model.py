@@ -29,7 +29,6 @@ the stage's last block, and one row gather puts them back in order (``token_maps
 """
 from __future__ import annotations
 
-import os
 from typing import Dict, List, Optional
 
 import torch
@@ -124,8 +123,7 @@ class RAJNIViTWrapper(nn.Module):
         self._graphs = {}
         self._param_list = None
         # None = automatic: replay a captured CUDA graph when the batch is small enough to be launch-bound
-        env = os.environ.get("RAJNI_CUDA_GRAPH", "")
-        self.use_cuda_graph: Optional[bool] = None if env == "" else env != "0"
+        self.use_cuda_graph: Optional[bool] = None
         self.prefix = 1                  # leading tokens that are always kept (set by _validate: 2 for a distilled DeiT)
         self.no_embed_class = False      # pos_embed covers the patches only (DeiT-III)
         self.pre_norm = False            # norm_pre LayerNorm after the embedding (CLIP)
@@ -310,7 +308,7 @@ class RAJNIViTWrapper(nn.Module):
         """model.py:30-69.  The launch sequence of a given input shape can be captured once into a CUDA graph and replayed:
         the 68 launches of a step cost ~13 us of host time each, which dominates small batches (vit_tiny at batch 8:
         0.88 -> 0.53 ms per step).  ``use_cuda_graph`` = None (default) replays when the batch has at most
-        ``AUTO_GRAPH_MAX_ROWS`` token rows, True / False force it (RAJNI_CUDA_GRAPH=1 / 0 in the environment do the same).
+        ``AUTO_GRAPH_MAX_ROWS`` token rows, True / False force it.
         A captured graph is dropped when any parameter changes (storage or version), on ``.to()`` / ``.bfloat16()`` /
         ``load_state_dict`` and when the input normalisation changes; results are bit-identical to the eager sequence."""
         return self._run(x, ("forward",))
@@ -481,8 +479,7 @@ class RAJNIViTWrapper(nn.Module):
 
         # Zig-zag traversal: every persistent kernel walks its row tiles in the direction opposite to the kernel that
         # produced its main operand, so it starts on the rows that kernel wrote last and that still sit in L2.
-        zig = os.environ.get("RAJNI_NO_ZIGZAG") is None       # A/B switch for profiling
-        rev = zig                      # the embed GEMM walked forward
+        rev = True                     # the embed GEMM walked forward
         scores = None
         token_counts = []
         keep_log: List[Optional[torch.Tensor]] = []
@@ -522,7 +519,7 @@ class RAJNIViTWrapper(nn.Module):
                     ops.select(scores, keep, keep_idx=keep_idx, next_scores=next_scores, row_map=row_map, prefix=P0)
                 if Np > ops.LONG_SEQ and "qkvc" not in ws:                             # compaction buffer, long sequences only
                     ws["qkvc"] = torch.empty((B * ws["N0"], 3 * C), device=x.device, dtype=torch.bfloat16)
-                ops.attention(ws["qkv"], row_map, B, N, Np, C, H, float(attn.scale), out=ws["att"], reverse=zig and not rev,
+                ops.attention(ws["qkv"], row_map, B, N, Np, C, H, float(attn.scale), out=ws["att"], reverse=not rev,
                               compact=ws.get("qkvc"))
                 if features:
                     nxt = regions[sum(k is not None for k in keep_log) + 1]
@@ -535,14 +532,14 @@ class RAJNIViTWrapper(nn.Module):
                 N = Np
                 M = B * N
             else:
-                ops.attention(ws["qkv"], None, B, N, N, C, H, float(blk.attn.scale), out=ws["att"], reverse=zig and not rev)
+                ops.attention(ws["qkv"], None, B, N, N, C, H, float(blk.attn.scale), out=ws["att"], reverse=not rev)
                 ops.gemm(ws["att"], pw, pb, M, C, C, residual=cur, ldres=C, out=cur, ldd=C, row_stats=stats, tag="proj", reverse=rev)   # in place
                 scores = None                                                         # model.py:63
                 keep_log.append(None)
             ops.gemm(cur, f1w, f1b, M, hidden, C, gelu=True, out=ws["hid"], ldd=hidden,
-                     ln=(stats, slots, f1sum, e2), tag="fc1", reverse=zig and not rev)                                    # model.py:59 (norm2 + fc1 + GELU)
+                     ln=(stats, slots, f1sum, e2), tag="fc1", reverse=not rev)                                    # model.py:59 (norm2 + fc1 + GELU)
             ops.gemm(ws["hid"], f2w, f2b, M, C, hidden, residual=cur, ldres=C, out=cur, ldd=C, row_stats=stats, tag="fc2", reverse=rev)
-            rev = zig and not rev
+            rev = not rev
             if features and i in take:          # before the next block overwrites this stage's rows in place
                 maps.append(self._token_features(feat, token_maps(keep_log, B, N0, x.device)[0], take_norm, out_dtype))
 

@@ -1,4 +1,5 @@
-"""Images/s of the five BASELINE configs on ONE GPU at their per-GPU batch (device-resident inputs, CUDA events)."""
+"""Images/s of the five BASELINE configs on ONE GPU at their per-GPU batch (device-resident inputs, CUDA events).
+usage: python tools/config_bench.py [--eager] [name filter ...]   (--eager: no CUDA-graph replay; default: automatic)"""
 import os
 import sys
 
@@ -22,12 +23,13 @@ CASES = [("C1 vit_tiny  bs8", "vit_tiny_patch16_224", C1, 8, 224),
          ("B/8  vit_base_patch8  bs64  README", "vit_base_patch8_224", README, 64, 224),
          ("B/8  vit_base_patch8  bs256 dense", "vit_base_patch8_224", {}, 256, 224),
          ("B/8  vit_base_patch8  bs256 README", "vit_base_patch8_224", README, 256, 224)]
-only = sys.argv[1:]
+eager = "--eager" in sys.argv
+only = [a for a in sys.argv[1:] if a != "--eager"]
 for name, model_name, sched, B, S in CASES:
     if only and not any(o in name for o in only):
         continue
     m = RAJNIViTWrapper(create_model(model_name, seed=0), sched).cuda().eval()
-    m.use_cuda_graph = {"": None, "0": False}.get(os.environ.get("RAJNI_CUDA_GRAPH", ""), True)     # default: automatic
+    m.use_cuda_graph = False if eager else None
     x = torch.randn(B, 3, S, S, device="cuda")
     for _ in range(5):
         m(x)

@@ -1,7 +1,7 @@
-// Stand-alone check + timing + event trace of attention_pipe.cu against attention_tc.cu (the round-1 kernel) and a CPU
+// Stand-alone check + timing of attention_pipe.cu against attention_tc.cu (the round-1 kernel) and a CPU
 // double-precision reference on sampled (image, head) pairs.
 // build (from tools/probes):
-//   nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -lineinfo -DRAJNI_ATTN_TRACE --expt-relaxed-constexpr \
+//   nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -lineinfo --expt-relaxed-constexpr \
 //        attn_pipe_check.cu -o attn_pipe_check -L../../rajni_vit_b200/csrc -lrajni_b200 -lcuda -Xlinker -rpath='$ORIGIN/../../rajni_vit_b200/csrc'
 #include <cmath>
 #include <cstdio>
@@ -108,22 +108,6 @@ int main(int argc, char** argv) {
         if (B >= 32) printf("   tc %.1f us  pipe %.1f us  (%.2fx, %.0f TF/s)", ms0 * 1e3, ms1 * 1e3, ms0 / ms1, 4.0 * B * Np * Np * C / (ms1 * 1e-3) / 1e12);
         printf("\n");
         fflush(stdout);
-#ifdef RAJNI_ATTN_TRACE
-        if (B == 256 && getenv("AP_TRACE")) {
-            static long long tr[64 * 16];
-            cudaMemcpyFromSymbol(tr, rajni::g_ap_trace, sizeof(tr));
-            const char* names[15] = {"S:beg", "S:end", "PV:beg", "PV:end", "ld:done", "max:done", "epi:beg", "epi:end", "exp:beg", "exp:end", "math:end", "prefetch", "PV:k1", "w:beg", "w:end"};
-            const long long t0 = tr[0];
-            printf("tile");
-            for (int s = 0; s < 15; ++s) printf(" %8s", names[s]);
-            printf("\n");
-            for (int g = 0; g < 24; ++g) {
-                printf("%4d", g);
-                for (int s = 0; s < 15; ++s) printf(" %8lld", tr[g * 16 + s] ? tr[g * 16 + s] - t0 : -1);
-                printf("\n");
-            }
-        }
-#endif
         cudaFree(qkv); cudaFree(out0); cudaFree(out1); cudaFree(rmap);
     }
     // NaN isolation (dense call): image 1 all-NaN must not touch image 0's output

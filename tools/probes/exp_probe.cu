@@ -7,7 +7,7 @@
 // build: nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -I../../rajni_vit_b200/csrc exp_probe.cu -o exp_probe
 #include <cstdio>
 #include "common.cuh"
-namespace rajni { void set_error(const char*, ...) {} void count_launch(int) {} int check_launch(const char*) { return 0; } bool pdl_enabled() { return false; } int current_device() { return 0; } }
+namespace rajni { void set_error(const char*, ...) {} void count_launch(int) {} int check_launch(const char*) { return 0; } int current_device() { return 0; } }
 using namespace rajni;
 __device__ __forceinline__ float ex2f(float x) { float y; asm volatile("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 __device__ __forceinline__ uint32_t prmt(uint32_t a, uint32_t b, uint32_t sel) { uint32_t d; asm volatile("prmt.b32 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(b), "r"(sel)); return d; }

@@ -2,7 +2,7 @@
 // the ceiling of the GEMM main loop.   build: nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -I../../rajni_vit_b200/csrc mma2_probe.cu -o mma2_probe
 #include <cstdio>
 #include "common.cuh"
-namespace rajni { void set_error(const char*, ...) {} void count_launch(int) {} int check_launch(const char*) { return 0; } bool pdl_enabled() { return false; } }
+namespace rajni { void set_error(const char*, ...) {} void count_launch(int) {} int check_launch(const char*) { return 0; } }
 using namespace rajni;
 
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(128) mma2_kernel(int N, int reps, int nacc, long long* out) {

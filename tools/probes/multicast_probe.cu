@@ -8,7 +8,7 @@
 #include <cstdio>
 #include <cuda.h>
 #include "common.cuh"
-namespace rajni { void set_error(const char*, ...) {} void count_launch(int) {} int check_launch(const char*) { return 0; } bool pdl_enabled() { return false; } int current_device() { return 0; } }
+namespace rajni { void set_error(const char*, ...) {} void count_launch(int) {} int check_launch(const char*) { return 0; } int current_device() { return 0; } }
 using namespace rajni;
 
 struct Result { int done[4]; float first[4]; };
